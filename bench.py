@@ -5,6 +5,7 @@
   python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...   # one rank per GPU (NCCL)
   python bench.py --gpus N --engine single ...                                   # ONE process, C++ multi-GPU engine
   python bench.py --impl reference [--steps K] [--warmup W]                      # the reference's CPU engine
+  python bench.py ... --dump-outputs DIR                                         # + the last timed step's match lists as DIR/*.npy
 
 Metric (BASELINE.json): image-pairs/sec on SIFT-128 descriptor sets; a *step* is one pass of the hot path — 2-NN + ratio
 (0.85 "all" / 0.6 "good", fine_matching_graph.cc:42-43) + mutual cross-check — over the whole candidate pair list.
@@ -79,7 +80,51 @@ def parse_args():
     ap.add_argument("--parity-pairs", type=int, default=-1, help="pairs checked against the CPU oracle after the timed regions")
     ap.add_argument("--mutual", type=int, default=1, help="1 = ratio + mutual cross-check (headline), 0 = ratio only")
     ap.add_argument("--no-int8-peak", action="store_true", help="skip the cuBLAS int8 GEMM peak measurement (rank 0, N = 1)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write the match lists of the last timed step as DIR/<name>.npy (rank 0's pairs; "
+                         "see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the lists of the native path; the reference arm keeps none")
+    return args
+
+
+DUMP_BYTES = 64 << 20   # all files written by --dump-outputs together
+
+
+def dump_outputs(out_dir: str, pairs: np.ndarray, res) -> None:
+    """--dump-outputs: the match lists a caller of the timed call receives, as DIR/<name>.npy, so that two builds can be
+    compared output for output.  Indices and flags are float32 (exact: all below 2^24), offsets float64:
+      pairs [k, 2]     (ref, query) image ids of the written pairs, ascending (independent of the staging order and engine)
+      ok [k]           1 = matched, 0 = gated (fewer than 20 keypoints)
+      offsets [k + 1]  pair p's matches are matches[offsets[p]:offsets[p + 1]]
+      matches [n, 2]   (ref row, query row) of every match
+      good [n]         1 = the match also passes the 'good' ratio
+    Every pair when the files fit in DUMP_BYTES; otherwise a fixed sample of whole pairs: the longest prefix that fits of a
+    permutation of the ascending list drawn with seed 0, written in ascending order."""
+    pairs = np.asarray(pairs)
+    n = len(pairs)
+    offs = np.asarray(res.offsets[:n + 1], np.int64)
+    counts = np.diff(offs)
+    per_pair = 8 + 4 + 8 + counts * (8 + (4 if res.good is not None else 0))
+    budget = DUMP_BYTES - 5 * 128                       # one .npy header per file
+    keep = np.lexsort((pairs[:, 1], pairs[:, 0]))
+    if per_pair.sum() > budget:
+        perm = np.random.default_rng(0).permutation(n)
+        keep = keep[np.sort(perm[:int(np.searchsorted(np.cumsum(per_pair[keep[perm]]), budget, side="right"))])]
+    new_offs = np.concatenate([[0], np.cumsum(counts[keep])]).astype(np.int64)
+    rows = np.repeat(offs[keep] - new_offs[:-1], counts[keep]) + np.arange(new_offs[-1])
+    arrays = {"pairs": pairs[keep].astype(np.float32), "ok": np.asarray(res.ok[:n])[keep].astype(np.float32),
+              "offsets": new_offs.astype(np.float64), "matches": np.asarray(res.matches)[rows].astype(np.float32)}
+    if res.good is not None:
+        arrays["good"] = np.asarray(res.good)[rows].astype(np.float32)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    print(f"[bench] --dump-outputs: match lists of {len(keep)} of {n} pairs ({int(new_offs[-1])} matches) written to {out_dir}",
+          file=sys.stderr, flush=True)
 
 
 def measured_peaks():
@@ -571,6 +616,13 @@ def run_native_ranks(args):
         total_ms = float(tt.item())
     pairs_done = float(len(pairs) * args.steps)   # all ranks together match the whole list once per step
     value = pairs_done / (total_ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        # the resident call leaves its lists in HBM and returns only their count: the same call on the same table through
+        # msfm_match_pairs copies them to the host, and must find exactly as many
+        res = m.match_pairs(my_pairs, RATIO_ALL, capacity=n_matches, **kw)
+        if len(res.matches) != n_matches:
+            raise RuntimeError(f"msfm_match_pairs found {len(res.matches)} matches, the timed resident call {n_matches}")
+        dump_outputs(args.dump_outputs, my_pairs, res)
 
     # ---- end to end through the public API from host buffers, staging pipelined against matching
     e2e, sampled_local = None, []
@@ -888,6 +940,8 @@ def run_native_single(args):
     total_ms = float(sum(dev_ms))
     value = len(pairs) * args.steps / (total_ms * 1e-3)
     n_matches = len(res.matches)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, pairs_sorted, res)   # before the e2e steps reuse the result buffers
 
     list_off = np.zeros((len(pairs) + 1,), np.int64)
 

@@ -100,6 +100,43 @@ def test_bench_reference_arm_contract():
     assert line["gpu_launches"] == 0
 
 
+@pytest.mark.parametrize("budget", [64 << 20, 1 << 20])
+def test_bench_dump_outputs(tmp_path, monkeypatch, budget):
+    """`bench.py --dump-outputs`: whole match lists of every pair, or of a seeded sample of pairs when they exceed the
+    budget; float files only, within the budget, every written list equal to its source, the same bytes whatever the
+    order the pairs were matched in."""
+    import bench
+    from metricsfm_b200.matcher import MatchResult
+    monkeypatch.setattr(bench, "DUMP_BYTES", budget)
+    rng = np.random.default_rng(5)
+    n = 200
+    pairs = np.stack([np.arange(n), np.arange(n) + 1], 1).astype(np.int32)
+    counts = rng.integers(0, 4000, size=n)
+    counts[::7] = 0
+    offs = np.concatenate([[0], np.cumsum(counts)]).astype(np.int64)
+    res = MatchResult(offs, (counts > 0).astype(np.int32), rng.integers(0, 8192, size=(offs[-1], 2)).astype(np.int32),
+                      rng.integers(0, 2, size=offs[-1]).astype(np.uint8))
+    bench.dump_outputs(str(tmp_path / "a"), pairs, res)
+    order = rng.permutation(n)                                        # the same lists, matched in another order
+    rows = np.concatenate([np.arange(offs[p], offs[p + 1]) for p in order])
+    shuffled = MatchResult(np.concatenate([[0], np.cumsum(counts[order])]), res.ok[order], res.matches[rows], res.good[rows])
+    bench.dump_outputs(str(tmp_path / "b"), pairs[order], shuffled)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["good.npy", "matches.npy", "offsets.npy", "ok.npy", "pairs.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= budget
+    for f in files:
+        assert (tmp_path / "a" / f).read_bytes() == (tmp_path / "b" / f).read_bytes(), f
+    got = {f[:-4]: np.load(tmp_path / "a" / f) for f in files}
+    assert all(a.dtype in (np.float32, np.float64) for a in got.values())
+    p = got["pairs"][:, 0].astype(np.int64)                          # pair p of the list is (p, p + 1)
+    assert (np.diff(p) > 0).all() and (len(p) == n) == (budget == 64 << 20) and len(p) > 0
+    o = got["offsets"].astype(np.int64)
+    for k, src in enumerate(p):
+        np.testing.assert_array_equal(got["matches"][o[k]:o[k + 1]], res.pair(src))
+        np.testing.assert_array_equal(got["good"][o[k]:o[k + 1]], res.pair_good(src))
+        assert got["ok"][k] == res.ok[src]
+
+
 def test_numa_pinning_helper_never_raises():
     """pin_to_gpu_numa_node() reports what it did and leaves the process alone when NVML / the device is missing."""
     import os
