@@ -11,7 +11,8 @@
  *              -> msfm_upload_f32 / msfm_upload_u8 (build, once per image), msfm_knn2 (query), msfm_release (free)
  *   seam S2  FeatureMatching::KNNMatchingWithGeoVerify(kp1, kp2, int* id, float* dis, matches)
  *            src/feature/feature_matching.h:57-58, feature_matching.cpp:477-501 (caller-supplied kNN arrays)
- *              -> msfm_knn2 fills exactly those id/dis arrays ([2*Nquery], (nn0,nn1) interleaved, squared L2)
+ *              -> msfm_knn2 fills exactly those id/dis arrays ([2*Nquery], (nn0,nn1) interleaved, squared L2);
+ *                 msfm_knn2_pairs fills them for a whole pair list, optionally exact in fp32 on float rows
  *   seam S3  bool Matcher(vector<KeyPoint>&, Mat&, vector<KeyPoint>&, Mat&, vector<pair<int,int>>&)
  *            src/feature/feature_matching.h:33-35 (KNNMatching), feature_matching_cuda_sift.h:34-36 (Run)
  *              -> msfm_match_pairs with n_pairs = 1 (host shim: metricsfm_b200/host/feature_matching_b200.h)
@@ -32,6 +33,7 @@
  * Float regime: float rows are quantised to u8 by the packer, so d0/d1 carries a relative error of a few 1e-3; with
  *   msfm_config.keep_float + msfm_params.rescore_band the rows near a ratio threshold are decided on exact fp32
  *   distances instead (the match lists then agree with an fp32 brute-force matcher to <= 1e-4 of the matches).
+ *   msfm_knn2_pairs with MSFM_KNN_EXACT_F32 returns the kNN arrays of an fp32 matcher itself, bit for bit.
  */
 #ifndef MSFM_MATCH_H_
 #define MSFM_MATCH_H_
@@ -191,8 +193,27 @@ msfm_status msfm_table_ptrs(const msfm_ctx *ctx, void **desc_arena, void **norm_
 msfm_status msfm_download_packed(msfm_ctx *ctx, int32_t image_id, uint8_t *desc_out, uint32_t *norms_out);
 
 /* ---- kNN query in FLANN layout (seams S1/S2) ------------------------------------------------------------------- */
-/* ids[2*Nq], dists[2*Nq] host buffers, Nq = rows of image `query_id`.  No min_keypoints gate (FLANN has none). */
+/* ids[2*Nq], dists[2*Nq] host buffers, Nq = rows of image `query_id`.  No min_keypoints gate (FLANN has none).
+ * Distances are those of the packed u8 rows (float uploads: quantised units); msfm_knn2_pairs with MSFM_KNN_EXACT_F32
+ * gives the fp32 ones. */
 msfm_status msfm_knn2(msfm_ctx *ctx, int32_t ref_id, int32_t query_id, int32_t *ids, float *dists);
+
+#define MSFM_KNN_EXACT_F32 1u   /* msfm_knn2_pairs flag */
+
+/* FLANN-layout 2-NN of every query row of every pair in one call.  Pair p's rows are rows
+ * [offsets[p], offsets[p+1]) of ids/dists: ids[2r..2r+1] = (nn0, nn1), dists[2r..2r+1] = (d0, d1), missing
+ * neighbour = (-1, +inf).  offsets[n_pairs+1] in query rows; ids/dists hold 2*row_capacity entries.  No min_keypoints gate.
+ * flags 0: exactly msfm_knn2 per pair (squared L2 of the packed u8 rows).
+ * MSFM_KNN_EXACT_F32: every pair's images must have been uploaded with msfm_upload_f32* on a keep_float context with
+ *   the same scale; ids/dists are then those of an exhaustive fp32 matcher on the caller's float rows: squared L2
+ *   accumulated in index order with separate multiply and add (nanoflann.hpp:376-383), in the caller's units, lowest
+ *   index on ties for nn0 and nn1, bit for bit.  (A pair with an empty image needs no float rows.)  Finite rows only.
+ * Errors (before any launch): INVALID_ARG for a null buffer, negative n_pairs / row_capacity, unknown flag bits, or
+ * EXACT_F32 on a pair without retained float rows or with two scales (the message names the pair); the image-id
+ * statuses; CAPACITY when the pairs' query rows exceed row_capacity.  msfm_last_timing: as msfm_match_pairs with
+ * rescore_band (match_kernel_ms = forward launches; the collect pass counts under finalize_ms). */
+msfm_status msfm_knn2_pairs(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pairs, uint32_t flags,
+                            int64_t *offsets, int32_t *ids, float *dists, int64_t row_capacity);
 /* Per reference row j of ref_id: best query row (lowest index on ties) and its squared distance. */
 msfm_status msfm_colbest(msfm_ctx *ctx, int32_t ref_id, int32_t query_id, int32_t *best_query, float *best_dist);
 
@@ -254,8 +275,12 @@ msfm_status msfm_geo_ransac(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pai
 
 /* ---- GPU-side cross-check kernel (CUDA cores, dp4a); used by the tests to localise faults, never by the fast path */
 msfm_status msfm_knn2_crosscheck(msfm_ctx *ctx, int32_t ref_id, int32_t query_id, int32_t *ids, float *dists);
-/* Test hook: capacity of the float regime's event list (-1 = default sizing; 0 forces the brute-force fallback). */
+/* Test hook: capacity of the float regime's event list (-1 = default sizing; 0 forces the brute-force fallback).
+ * Applies to msfm_match_pairs' rescore_band and to msfm_knn2_pairs' MSFM_KNN_EXACT_F32 alike. */
 msfm_status msfm_test_set_band_event_cap(msfm_ctx *ctx, int64_t cap);
+/* Test hook: for the last MSFM_KNN_EXACT_F32 call of msfm_knn2_pairs, the events the collect path scored and the
+ * batches whose event list overflowed, i.e. that the brute force decided.  Either pointer may be NULL. */
+msfm_status msfm_test_last_knn_stats(msfm_ctx *ctx, int64_t *events, int32_t *brute_force_batches);
 /* Test hook: 1 routes every pair's mutual check through the tensor twin pass (the fallback of the bound-based check). */
 msfm_status msfm_test_force_twin_pass(msfm_ctx *ctx, int32_t on);
 /* Test hook: 1 switches off the forward pass's dead-row rule (rows whose two nearest neighbours already violate every

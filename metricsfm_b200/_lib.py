@@ -26,6 +26,7 @@ EXPORTED_SYMBOLS = [
     "msfm_download_packed", "msfm_knn2", "msfm_colbest", "msfm_match_pairs", "msfm_match_pairs_resident",
     "msfm_last_timing", "msfm_get_stream", "msfm_knn2_crosscheck", "msfm_geo_verify", "msfm_geo_ransac",
     "msfm_upload_f32_batch_async", "msfm_get_upload_stream", "msfm_wait_event", "msfm_test_set_band_event_cap", "msfm_test_force_twin_pass", "msfm_test_disable_pruning", "msfm_reserve_batch_async", "msfm_host_alloc", "msfm_host_free", "msfm_device_memory",
+    "msfm_knn2_pairs", "msfm_test_last_knn_stats",
 ]
 
 
@@ -60,6 +61,7 @@ class Params(C.Structure):
 
 
 RATIO_REJECT_GT = 1  # msfm_params.flags: SLAMGPS::FeatureMatching's rule (slam_gps.cc:470-477)
+KNN_EXACT_F32 = 1    # msfm_knn2_pairs flag: fp32 neighbours and distances of the retained float rows
 
 
 class GeoParams(C.Structure):
@@ -116,6 +118,8 @@ def load() -> C.CDLL:
     L.msfm_table_ptrs.argtypes = [vp, C.POINTER(vp), C.POINTER(vp), _i64p, _i64p]
     L.msfm_download_packed.argtypes = [vp, C.c_int32, vp, vp]
     L.msfm_knn2.argtypes = [vp, C.c_int32, C.c_int32, vp, vp]
+    L.msfm_knn2_pairs.argtypes = [vp, vp, C.c_int64, C.c_uint32, vp, vp, vp, C.c_int64]
+    L.msfm_test_last_knn_stats.argtypes = [vp, _i64p, _i32p]
     L.msfm_colbest.argtypes = [vp, C.c_int32, C.c_int32, vp, vp]
     L.msfm_match_pairs.argtypes = [vp, vp, C.c_int64, C.POINTER(Params), C.POINTER(Result)]
     L.msfm_match_pairs_resident.argtypes = [vp, vp, C.c_int64, C.POINTER(Params), _i64p]

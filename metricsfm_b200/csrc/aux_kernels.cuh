@@ -16,8 +16,11 @@ namespace msfm {
 // One warp per row; lane l owns bytes 4l..4l+3.  rows_padded - rows pad rows get zero bytes and kNormPad norms.
 // The side table stores column keys, ckey = -8*||row||^2 + (7 - row%8) (see match_kernel.cuh), not raw norms.
 // Quantisation rule (mirrored by oracle_quantize_f32): q = min(255, max(0, rint(x * scale))), NaN -> 0.
+// resid (keep_float contexts, else null): per row the quantisation residual r = ||scale*x - q||_2, rounded up, and
+// *rmax the largest residual of the image (the exact kNN mode's candidate bound, see exact_threshold).
 __global__ void pack_f32_kernel(const float *__restrict__ src, int64_t src_stride_floats, int rows, int rows_padded,
-                                float scale, uint8_t *__restrict__ dst, int32_t *__restrict__ ckeys) {
+                                float scale, uint8_t *__restrict__ dst, int32_t *__restrict__ ckeys,
+                                float *__restrict__ resid = nullptr, float *__restrict__ rmax = nullptr) {
     const int warps_per_block = blockDim.x >> 5;
     const int lane = threadIdx.x & 31;
     for (int r = blockIdx.x * warps_per_block + (threadIdx.x >> 5); r < rows_padded; r += gridDim.x * warps_per_block) {
@@ -26,6 +29,7 @@ __global__ void pack_f32_kernel(const float *__restrict__ src, int64_t src_strid
             const float *s = src + (int64_t)r * src_stride_floats + lane * 4;
             const float f[4] = {s[0], s[1], s[2], s[3]};
             uint32_t acc = 0;
+            double e2 = 0.0;  // x*scale is exact in double (24 x 24 bit significands), so is its distance to q
 #pragma unroll
             for (int k = 0; k < 4; ++k) {
                 float x = rintf(f[k] * scale);
@@ -34,10 +38,23 @@ __global__ void pack_f32_kernel(const float *__restrict__ src, int64_t src_strid
                 const uint32_t qv = (uint32_t)x;
                 packed |= qv << (8 * k);
                 acc += qv * qv;
+                if (resid) {
+                    const double e = (double)f[k] * (double)scale - (double)qv;
+                    e2 += e * e;
+                }
             }
 #pragma unroll
             for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xFFFFFFFFu, acc, o);
             nrm = acc;
+            if (resid) {
+#pragma unroll
+                for (int o = 16; o > 0; o >>= 1) e2 += __shfl_xor_sync(0xFFFFFFFFu, e2, o);
+                if (lane == 0) {
+                    const float rv = __double2float_ru(__dsqrt_ru(e2));
+                    resid[r] = rv;
+                    atomicMax(reinterpret_cast<int *>(rmax), __float_as_int(rv));  // >= +0: the bits order like the values
+                }
+            }
         }
         reinterpret_cast<uint32_t *>(dst + (int64_t)r * kDim)[lane] = packed;
         if (lane == 0) ckeys[r] = make_ckey(nrm, r);
@@ -201,11 +218,56 @@ struct BandParams {
     unsigned long long *event_keys;  // [event_cap]
     const unsigned int *event_count;
     uint32_t event_cap;
+    // exact kNN mode (msfm_knn2_pairs with MSFM_KNN_EXACT_F32): every query row is a band row, and its fp32 (nn0, nn1,
+    // d0, d1) go to these FLANN-layout arrays at row knn_off + q instead of a ratio decision into the kNN scratch
+    int32_t *out_ids = nullptr;
+    float *out_dists = nullptr;
 };
 
 // Quantised-distance threshold under which a reference row may still be an fp32 top-2 neighbour of a band row whose
 // quantised second-best distance is d1.
 __device__ __forceinline__ int band_threshold(int d1) { return d1 + (d1 >> 5) + 256; }
+
+// Exact kNN mode: a quantised-distance threshold T(q) that provably holds every fp32 top-2 neighbour of query row x.
+// With s the scale, q_y the packed row of y and r_y = ||s*y - q_y|| its quantisation residual (clamping included), the
+// triangle inequality gives  | s*||x-y|| - ||q_x-q_y|| | <= r_x + r_y <= r_x + R  (R: largest residual of the reference
+// image).  The two quantised nearest neighbours are therefore both within s*||x-y|| <= sqrt(d1_q) + r_x + R, so the fp32
+// second-nearest distance is at most that, and every fp32 top-2 row y has ||q_x-q_y|| <= sqrt(d1_q) + 2(r_x + R).
+// Slack: the fp32 distance sum (128 products accumulated in order, with the rounding of the differences) is within a
+// relative 130 * 2^-24 of the real value; that widens the squared bound by (1 + 130 * 2^-24)^2 < 1 + 2^-15.  The
+// residuals are rounded up where they are stored and every step here rounds up, so T(q) is an upper bound.
+// d1 < 0 (the reference image has fewer than two rows): every reference row is a candidate.
+constexpr int kExactThrAll = 1 << 24;  // > 128 * 255^2, every quantised distance
+__device__ __forceinline__ int exact_threshold(int d1, float rx, float rmax) {
+    if (d1 < 0) return kExactThrAll;
+    const float root = __fadd_ru(__fsqrt_ru((float)d1), __fmul_ru(2.0f, __fadd_ru(rx, rmax)));
+    const float t = __fmul_ru(__fmul_ru(root, root), 1.0f + 1.0f / 32768.0f);
+    return t >= (float)kExactThrAll ? kExactThrAll : (int)ceilf(t);
+}
+
+// Exact kNN mode, per batch: every query row of pair p becomes a "band row" (rows knn_off .. knn_off + qry_rows of the
+// candidate scratch) with its own threshold exact_threshold(d1_q, r_x, R_ref).  Grid (pairs, row chunks).
+__global__ void __launch_bounds__(256) mark_exact_kernel(const BandParams bp, const float *__restrict__ resid,
+                                                         const float *__restrict__ img_rmax) {
+    const PairDesc pd = bp.pairs[blockIdx.x];
+    if (blockIdx.y == 0 && threadIdx.x == 0) bp.band_counts[blockIdx.x] = pd.qry_rows;
+    const float rmax = pd.ref_rows > 0 ? img_rmax[pd.ref_img] : 0.0f;
+    for (int q = blockIdx.y * blockDim.x + threadIdx.x; q < pd.qry_rows; q += gridDim.y * blockDim.x) {
+        const int4 k = merge_knn_shares(bp.knn, pd.knn_off + q, bp.nshare);
+        const int64_t row = pd.knn_off + q;
+        bp.band_q[row] = q;
+        bp.band_thr[row] = exact_threshold(k.y >= 0 ? k.w : -1, resid[pd.qry_off + q], rmax);
+        bp.band_state[2 * row] = ~0ull;
+        bp.band_state[2 * row + 1] = ~0ull;
+    }
+    // the rows' packed descriptors + column keys into the scratch image the collect pass queries
+    const int lane = threadIdx.x & 31, nwarps = blockDim.x >> 5;
+    for (int q = blockIdx.y * nwarps + (threadIdx.x >> 5); q < pd.qry_rows; q += gridDim.y * nwarps) {
+        const int64_t src = pd.qry_off + q, dst = pd.knn_off + q;
+        reinterpret_cast<uint32_t *>(bp.cand_desc + dst * kDim)[lane] = reinterpret_cast<const uint32_t *>(bp.desc_arena + src * kDim)[lane];
+        if (lane == 0) bp.cand_ckeys[dst] = bp.ckeys[src];
+    }
+}
 
 __global__ void __launch_bounds__(1024) mark_band_kernel(const BandParams bp) {
     __shared__ int warp_excl[32];
@@ -254,6 +316,14 @@ __device__ __forceinline__ bool fknn_less(float da, int ia, float db, int ib) { 
 
 // Decision of one band row from its fp32 nearest (b0, c0i) and second nearest (b1, c1i) reference rows (-1: none).
 __device__ __forceinline__ void write_rescored(const BandParams &bp, const PairDesc &pd, int q, float b0, int c0i, float b1, int c1i) {
+    if (bp.out_ids) {  // exact kNN mode: FLANN layout, missing neighbour = (-1, +inf)
+        const int64_t row = pd.knn_off + q;
+        bp.out_ids[2 * row] = c0i;
+        bp.out_ids[2 * row + 1] = c1i;
+        bp.out_dists[2 * row] = c0i >= 0 ? b0 : INFINITY;
+        bp.out_dists[2 * row + 1] = c1i >= 0 ? b1 : INFINITY;
+        return;
+    }
     int flags = 0;
     if (c0i >= 0 && c1i >= 0) {
         const float r = __fdiv_rn(b0, b1);
@@ -359,9 +429,9 @@ __global__ void __launch_bounds__(256) rescore_band_kernel(const BandParams bp, 
                 if (qi < nq) {
                     const int q = bp.band_q[pd.knn_off + c0 + qi];
                     na = ckey_to_norm(bp.ckeys[pd.qry_off + q]);
-                    // Prefilter on the quantised distance: a row whose integer distance exceeds the integer second
-                    // best by more than ~3 % (ten times the quantisation error) cannot be an fp32 top-2 neighbour.
-                    thr = band_threshold(merge_knn_shares(bp.knn, pd.knn_off + q, bp.nshare).w);
+                    // Prefilter on the quantised distance, the threshold the collect pass used: band_threshold of the
+                    // row's integer second best (~3 %, ten times the quantisation error), or exact_threshold.
+                    thr = bp.band_thr[pd.knn_off + c0 + qi];
                 }
                 s_na[qi] = na;
                 s_thr[qi] = thr;

@@ -44,6 +44,11 @@ constexpr int64_t kBatchMaxQueryRows = 16ll << 20;
 constexpr int64_t kBatchMaxQueryRowsMutual = 16ll << 20;  // mutual: + 128 B of gathered candidate row per query row
 constexpr int64_t kBatchMaxPairs = 16384;
 constexpr int64_t kBatchMaxRefRows = 16ll << 20;  // mutual: 8 B of column table per reference row of the batch
+// msfm_knn2_pairs exact mode: every query row goes through the collect pass (~10 events per row on unit-norm SIFT at
+// 8192 rows, p99 28), so its batches are smaller and its event list holds 16 events per row: 1 Mi rows -> 16 Mi events
+// x 24 B = 400 MB.  An overflow stays correct (brute force) but must not be the common case.
+constexpr int64_t kBatchMaxQueryRowsExact = 1ll << 20;
+constexpr int64_t kExactEventsPerRow = 16;
 
 struct DeviceBuf {
     void *ptr = nullptr;
@@ -98,6 +103,8 @@ struct msfm_ctx {
     uint8_t *desc = nullptr;
     int32_t *norms = nullptr;  // column-key arena: ckey = -8*||row||^2 + (7 - row%8), see match_kernel.cuh
     float *fdesc = nullptr;    // keep_float: the callers' float rows, same row offsets as `desc` (512 B per row)
+    float *resid = nullptr;    // keep_float: quantisation residual ||scale*x - q|| per row (pack_f32_kernel), same offsets
+    float *img_rmax = nullptr; // keep_float: [max_images] largest residual per image (0 after release)
     bool own_arena = false;
     CUtensorMap *d_maps = nullptr;
     CUtensorMap *h_maps = nullptr;  // pinned mirror of d_maps: tensor maps are uploaded without a host sync
@@ -112,6 +119,9 @@ struct msfm_ctx {
     DeviceBuf band_q, band_counts;  // float regime: query rows near a ratio threshold, per pair
     DeviceBuf band_thr, band_state, band_events, band_event_keys, band_event_count;  // ... and the collect pass over them
     int64_t band_event_cap_override = -1;  // msfm_test_set_band_event_cap (tests: 0 forces the brute-force fallback)
+    DeviceBuf knn_ids, knn_dists, knn_ids_b, knn_dists_b;  // msfm_knn2_pairs: FLANN-layout rows of a batch (two sets, see match_pairs_impl)
+    int64_t knn_events = 0;         // last exact-mode msfm_knn2_pairs: events scored by the collect path ...
+    int32_t knn_brute_batches = 0;  // ... and batches whose event list overflowed (brute force)
     bool force_twin = false;               // msfm_test_force_twin_pass
 #ifdef MSFM_DYNAMIC_ITEMS       // A/B builds only: work items drawn from a device counter instead of the static walk
     bool dynamic_items = true;
@@ -543,6 +553,18 @@ msfm_status wait_list_copy(msfm_ctx *ctx) {
     return MSFM_OK;
 }
 
+// A list copy still in flight when a call fails half-way must not outlive the call: the caller may free the
+// destination buffers as soon as it sees the error.  (On success wait_list_copy has already cleared the flag.)
+struct DrainListCopy {
+    msfm_ctx *c;
+    ~DrainListCopy() {
+        if (c->d2h_in_flight) {
+            cudaStreamSynchronize(c->d2h_stream);
+            c->d2h_in_flight = false;
+        }
+    }
+};
+
 msfm_status accumulate_kernel_time(msfm_ctx *ctx, cudaEvent_t e0, cudaEvent_t e1) {
     float ms = 0.f;
     MSFM_CUDA(ctx, cudaEventElapsedTime(&ms, e0, e1));
@@ -599,17 +621,7 @@ msfm_status match_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pa
         if ((st = check_image_id(ctx, pairs[i].query, true)) != MSFM_OK) return st;
     }
     ctx->timing = msfm_timing{};
-    // A list copy still in flight when the call fails half-way must not outlive the call: the caller may free the
-    // destination buffers as soon as it sees the error.  (On success wait_list_copy has already cleared the flag.)
-    struct DrainListCopy {
-        msfm_ctx *c;
-        ~DrainListCopy() {
-            if (c->d2h_in_flight) {
-                cudaStreamSynchronize(c->d2h_stream);
-                c->d2h_in_flight = false;
-            }
-        }
-    } drain_list_copy{ctx};
+    DrainListCopy drain_list_copy{ctx};
     MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_begin, ctx->stream));
     const bool mutual = params->mutual != 0;
     const bool want_good = params->ratio_good > 0.0f && (resident || out->has_good);
@@ -874,6 +886,180 @@ msfm_status match_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pa
     return MSFM_OK;
 }
 
+// msfm_knn2_pairs (and msfm_knn2, its one-pair flags-0 form).  Per batch of consecutive pairs: the forward 2-NN without
+// pruning, then either the FLANN conversion of the kNN scratch (integer distances) or, in exact mode, the collect pass
+// over every query row under its bound T(q) (mark_exact_kernel), fp32 scoring of the events and the FLANN rows written
+// by finish_band_kernel (rescore_band_kernel when the event list overflowed).  A batch's rows go back to the host on
+// the list-copy stream under the next batch's kernels, as in match_pairs_impl.
+msfm_status knn2_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pairs, uint32_t flags, int64_t *offsets, int32_t *ids,
+                            float *dists, int64_t row_capacity) {
+    if (!ctx) return MSFM_ERR_INVALID_ARG;
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    if (n_pairs < 0 || (n_pairs > 0 && !pairs) || !offsets || !ids || !dists || row_capacity < 0)
+        return fail(ctx, MSFM_ERR_INVALID_ARG, "null pair list / output buffer, negative n_pairs or negative row_capacity");
+    if (flags & ~MSFM_KNN_EXACT_F32) return fail(ctx, MSFM_ERR_INVALID_ARG, "unknown flag bits 0x%x", flags & ~MSFM_KNN_EXACT_F32);
+    const bool exact = (flags & MSFM_KNN_EXACT_F32) != 0;
+    msfm_status st;
+    int64_t rows_total = 0;
+    for (int64_t i = 0; i < n_pairs; ++i) {
+        if ((st = check_image_id(ctx, pairs[i].ref, true)) != MSFM_OK) return st;
+        if ((st = check_image_id(ctx, pairs[i].query, true)) != MSFM_OK) return st;
+        rows_total += ctx->images[pairs[i].query].rows;
+    }
+    if (rows_total > row_capacity)
+        return fail(ctx, MSFM_ERR_CAPACITY, "output too small: the pairs have %lld query rows, row_capacity is %lld", (long long)rows_total,
+                    (long long)row_capacity);
+    if (exact) {
+        if (!ctx->fdesc) return fail(ctx, MSFM_ERR_INVALID_ARG, "MSFM_KNN_EXACT_F32 needs a keep_float context");
+        for (int64_t i = 0; i < n_pairs; ++i) {
+            const ImageSlot &r = ctx->images[pairs[i].ref], &q = ctx->images[pairs[i].query];
+            if (r.rows == 0 || q.rows == 0) continue;  // nothing to score: the rows read "absent" either way
+            if (!r.has_float || !q.has_float)
+                return fail(ctx, MSFM_ERR_INVALID_ARG, "MSFM_KNN_EXACT_F32: pair %lld: image %d has no retained float rows (upload it with msfm_upload_f32*)",
+                            (long long)i, !r.has_float ? pairs[i].ref : pairs[i].query);
+            if (r.scale != q.scale)
+                return fail(ctx, MSFM_ERR_INVALID_ARG, "MSFM_KNN_EXACT_F32: pair %lld: images %d and %d were quantised with different scales (%g, %g)",
+                            (long long)i, pairs[i].ref, pairs[i].query, (double)r.scale, (double)q.scale);
+            if (!(r.scale * r.scale > 0.0f))  // the plan marks float pairs by scale^2 > 0
+                return fail(ctx, MSFM_ERR_INVALID_ARG, "MSFM_KNN_EXACT_F32: pair %lld: scale %g is too small", (long long)i, (double)r.scale);
+        }
+    }
+    MSFM_CUDA(ctx, cudaSetDevice(ctx->device));
+    offsets[0] = 0;
+    for (int64_t i = 0; i < n_pairs; ++i) offsets[i + 1] = offsets[i] + ctx->images[pairs[i].query].rows;
+    ctx->timing = msfm_timing{};
+    if (exact) { ctx->knn_events = 0; ctx->knn_brute_batches = 0; }
+    DrainListCopy drain_list_copy{ctx};
+    MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_begin, ctx->stream));
+    const int64_t max_rows = exact ? kBatchMaxQueryRowsExact : kBatchMaxQueryRows;
+    int64_t next = 0;
+    auto carve = [&](BatchPlan &plan) {
+        plan = BatchPlan();  // no pruning: exact 2-NN rows
+        plan.rescoring = exact;
+        while (next < n_pairs && (int64_t)plan.pairs.size() < kBatchMaxPairs) {
+            const int64_t qr = ctx->images[pairs[next].query].rows;
+            if (!plan.pairs.empty() && plan.query_rows + qr > max_rows) break;
+            plan_add_pair(ctx, plan, next, pairs[next].ref, pairs[next].query);
+            ++next;
+        }
+        finish_plan(ctx, plan);
+    };
+    BatchPlan cur, ahead;
+    bool have = next < n_pairs;
+    if (have) carve(cur);
+    for (int64_t batch_no = 0; have; ++batch_no) {
+        BatchPlan &plan = cur;
+        const int nb = (int)plan.pairs.size();
+        const int64_t row_base = offsets[plan.src_index.front()];
+        bool carved_next = false;
+        if (plan.query_rows > 0) {
+            const size_t rows = (size_t)plan.query_rows;
+            DeviceBuf &oi = batch_no & 1 ? ctx->knn_ids_b : ctx->knn_ids, &od = batch_no & 1 ? ctx->knn_dists_b : ctx->knn_dists;
+            if ((st = ensure(ctx, oi, rows * 8)) != MSFM_OK) return st;
+            if ((st = ensure(ctx, od, rows * 8)) != MSFM_OK) return st;
+            size_t event_cap = 0;
+            if (exact) {
+                event_cap = std::min<size_t>(ctx->band_event_cap_override >= 0 ? (size_t)ctx->band_event_cap_override : rows * kExactEventsPerRow + 65536,
+                                             UINT32_MAX);
+                if ((st = ensure_cand_scratch(ctx, plan.query_rows)) != MSFM_OK) return st;
+                if ((st = ensure(ctx, ctx->band_q, rows * 4)) != MSFM_OK) return st;
+                if ((st = ensure(ctx, ctx->band_counts, (size_t)nb * 4)) != MSFM_OK) return st;
+                if ((st = ensure(ctx, ctx->band_thr, rows * 4)) != MSFM_OK) return st;
+                if ((st = ensure(ctx, ctx->band_state, rows * 16)) != MSFM_OK) return st;
+                if ((st = ensure(ctx, ctx->band_events, std::max<size_t>(event_cap, 1) * 16)) != MSFM_OK) return st;
+                if ((st = ensure(ctx, ctx->band_event_keys, std::max<size_t>(event_cap, 1) * 8)) != MSFM_OK) return st;
+                if ((st = ensure(ctx, ctx->band_event_count, 4)) != MSFM_OK) return st;
+            }
+            // ---- forward 2-NN (exact rows: the plan carries no pruning)
+            if ((st = run_match_stage(ctx, plan)) != MSFM_OK) return st;
+            unsigned int h_events = 0;
+            if (exact) {
+                MSFM_CUDA(ctx, cudaMemsetAsync(ctx->band_event_count.ptr, 0, 4, ctx->stream));
+                msfm::BandParams bp;
+                bp.pairs = static_cast<const PairDesc *>(ctx->pairdesc.ptr);
+                bp.knn = static_cast<int4 *>(ctx->knn.ptr);
+                bp.nshare = kCsplit;
+                bp.ratio = bp.ratio_good = bp.max_dist_sq = bp.band = 0.0f;
+                bp.reject_gt = 0;
+                bp.band_q = static_cast<int32_t *>(ctx->band_q.ptr);
+                bp.band_counts = static_cast<int32_t *>(ctx->band_counts.ptr);
+                bp.fdesc = ctx->fdesc;
+                bp.desc_arena = ctx->desc;
+                bp.ckeys = ctx->norms;
+                bp.band_thr = static_cast<int32_t *>(ctx->band_thr.ptr);
+                bp.band_state = static_cast<unsigned long long *>(ctx->band_state.ptr);
+                bp.cand_desc = static_cast<uint8_t *>(ctx->cand_desc.ptr);
+                bp.cand_ckeys = static_cast<int32_t *>(ctx->cand_ckeys.ptr);
+                bp.events = static_cast<const int4 *>(ctx->band_events.ptr);
+                bp.event_keys = static_cast<unsigned long long *>(ctx->band_event_keys.ptr);
+                bp.event_count = static_cast<const unsigned int *>(ctx->band_event_count.ptr);
+                bp.event_cap = (uint32_t)event_cap;
+                bp.out_ids = static_cast<int32_t *>(oi.ptr);
+                bp.out_dists = static_cast<float *>(od.ptr);
+                int32_t max_q = 0;
+                for (const PairDesc &pd : plan.pairs) max_q = std::max(max_q, pd.qry_rows);
+                const int gy = std::max(1, std::min(64, (max_q + 255) / 256));
+                msfm::mark_exact_kernel<<<dim3(nb, gy), 256, 0, ctx->stream>>>(bp, ctx->resid, ctx->img_rmax);
+                MSFM_CUDA(ctx, cudaGetLastError());
+                // tensor pass in collect mode over every query row, fp32 scoring of what it listed, FLANN rows
+                if (!plan.band_items.empty() &&
+                    (st = launch_match_kernel(ctx, plan.items.size() + plan.twin_items.size(), plan.band_items.size(), true, bp.event_cap)) != MSFM_OK)
+                    return st;
+                msfm::score_events_kernel<<<4 * ctx->num_sms, 256, 0, ctx->stream>>>(bp);
+                msfm::second_events_kernel<<<4 * ctx->num_sms, 256, 0, ctx->stream>>>(bp);
+                msfm::finish_band_kernel<<<nb, 256, 0, ctx->stream>>>(bp);
+                // brute-force search on CUDA cores under the same thresholds: returns at once unless the event list overflowed
+                const int gx = std::min(nb, 4 * ctx->num_sms);
+                const int gyb = std::max(1, std::min(32, (4 * ctx->num_sms + gx - 1) / gx));
+                msfm::rescore_band_kernel<<<dim3(gx, gyb), 256, 0, ctx->stream>>>(bp, nb);
+                MSFM_CUDA(ctx, cudaGetLastError());
+                ctx->timing.total_launches += 6;
+                MSFM_CUDA(ctx, cudaMemcpyAsync(&h_events, ctx->band_event_count.ptr, 4, cudaMemcpyDeviceToHost, ctx->stream));
+            } else {
+                msfm::knn_to_flann_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, ctx->stream>>>(static_cast<const int4 *>(ctx->knn.ptr), (int)rows, kCsplit,
+                                                                                             static_cast<int32_t *>(oi.ptr), static_cast<float *>(od.ptr));
+                MSFM_CUDA(ctx, cudaGetLastError());
+                ctx->timing.total_launches += 1;
+            }
+            MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_f1, ctx->stream));
+            // ---- plan the next batch while this one runs
+            have = next < n_pairs;
+            if (have) carve(ahead);
+            carved_next = true;
+            MSFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+            if (exact) {
+                if (h_events > event_cap) ctx->knn_brute_batches += 1;
+                else ctx->knn_events += h_events;
+            }
+            if ((st = accumulate_kernel_time(ctx, ctx->ev_k0, ctx->ev_k1)) != MSFM_OK) return st;
+            {
+                float ms_all = 0.f, ms_a = 0.f;
+                MSFM_CUDA(ctx, cudaEventElapsedTime(&ms_all, ctx->ev_k0, ctx->ev_f1));
+                MSFM_CUDA(ctx, cudaEventElapsedTime(&ms_a, ctx->ev_k0, ctx->ev_k1));
+                ctx->timing.finalize_ms += ms_all - ms_a;
+            }
+            if ((st = wait_list_copy(ctx)) != MSFM_OK) return st;  // the previous batch's rows (copied under this batch's kernels)
+            MSFM_CUDA(ctx, cudaStreamWaitEvent(ctx->d2h_stream, ctx->ev_f1, 0));
+            MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_d2h0, ctx->d2h_stream));
+            MSFM_CUDA(ctx, cudaMemcpyAsync(ids + 2 * row_base, oi.ptr, rows * 8, cudaMemcpyDeviceToHost, ctx->d2h_stream));
+            MSFM_CUDA(ctx, cudaMemcpyAsync(dists + 2 * row_base, od.ptr, rows * 8, cudaMemcpyDeviceToHost, ctx->d2h_stream));
+            MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_d2h1, ctx->d2h_stream));
+            ctx->d2h_in_flight = true;
+            ctx->timing.d2h_bytes += (int64_t)rows * 16;
+        }
+        if (!carved_next) {
+            have = next < n_pairs;
+            if (have) carve(ahead);
+        }
+        std::swap(cur, ahead);
+    }
+    if ((st = wait_list_copy(ctx)) != MSFM_OK) return st;
+    MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_end, ctx->stream));
+    MSFM_CUDA(ctx, cudaEventSynchronize(ctx->ev_end));
+    MSFM_CUDA(ctx, cudaEventElapsedTime(&ctx->timing.total_ms, ctx->ev_begin, ctx->ev_end));
+    return MSFM_OK;
+}
+
 }  // namespace
 
 // =====================================================================================================================
@@ -979,6 +1165,9 @@ msfm_status msfm_create(const msfm_config *cfg, msfm_ctx **out) {
     }
     if (cfg->keep_float) {
         if (cudaMalloc(&ctx->fdesc, (size_t)ctx->arena_rows * kDim * sizeof(float)) != cudaSuccess) return bail(MSFM_ERR_OUT_OF_MEMORY);
+        if (cudaMalloc(&ctx->resid, (size_t)ctx->arena_rows * sizeof(float)) != cudaSuccess) return bail(MSFM_ERR_OUT_OF_MEMORY);
+        if (cudaMalloc(&ctx->img_rmax, (size_t)ctx->max_images * sizeof(float)) != cudaSuccess) return bail(MSFM_ERR_OUT_OF_MEMORY);
+        if (cudaMemset(ctx->img_rmax, 0, (size_t)ctx->max_images * sizeof(float)) != cudaSuccess) return bail(MSFM_ERR_CUDA);
     }
     // one tensor map per image + one for the candidate scratch
     if (cudaMalloc(&ctx->d_maps, (size_t)(ctx->max_images + 1) * sizeof(CUtensorMap)) != cudaSuccess) return bail(MSFM_ERR_OUT_OF_MEMORY);
@@ -1032,7 +1221,9 @@ msfm_status msfm_destroy(msfm_ctx *ctx) {
         cudaFree(ctx->dbg_stats.ptr);
     }
     if (ctx->fdesc) cudaFree(ctx->fdesc);
-    DeviceBuf *bufs[] = {&ctx->band_q, &ctx->band_counts, &ctx->band_thr, &ctx->band_state, &ctx->band_events, &ctx->band_event_keys, &ctx->band_event_count, &ctx->cand_q, &ctx->cand_j, &ctx->cand_d0, &ctx->cand_good, &ctx->cand_counts, &ctx->cand_desc, &ctx->cand_ckeys, &ctx->colbest, &ctx->twin_counts, &ctx->item_counter, &ctx->tilemin,
+    if (ctx->resid) cudaFree(ctx->resid);
+    if (ctx->img_rmax) cudaFree(ctx->img_rmax);
+    DeviceBuf *bufs[] = {&ctx->knn_ids, &ctx->knn_dists, &ctx->knn_ids_b, &ctx->knn_dists_b, &ctx->band_q, &ctx->band_counts, &ctx->band_thr, &ctx->band_state, &ctx->band_events, &ctx->band_event_keys, &ctx->band_event_count, &ctx->cand_q, &ctx->cand_j, &ctx->cand_d0, &ctx->cand_good, &ctx->cand_counts, &ctx->cand_desc, &ctx->cand_ckeys, &ctx->colbest, &ctx->twin_counts, &ctx->item_counter, &ctx->tilemin,
                          &ctx->staging, &ctx->knn, &ctx->matches, &ctx->good, &ctx->counts, &ctx->offsets,
                          &ctx->pairdesc, &ctx->items, &ctx->tight_matches, &ctx->tight_good, &ctx->tight_matches_b, &ctx->tight_good_b};
     for (DeviceBuf *b : bufs)
@@ -1287,7 +1478,8 @@ static msfm_status upload_f32_enqueue(msfm_ctx *ctx, int32_t image_id, const flo
         MSFM_CUDA_UPLOAD(ctx, mine, cudaMemcpyAsync(stage, desc, bytes, cudaMemcpyHostToDevice, ctx->upload_stream));
     }
     const int blocks = std::max(1, std::min(4 * ctx->num_sms, (s.rows_padded + 7) / 8));
-    msfm::pack_f32_kernel<<<blocks, 256, 0, ctx->upload_stream>>>(src, src_stride, rows, s.rows_padded, scale, ctx->desc + off * kDim, ctx->norms + off);
+    msfm::pack_f32_kernel<<<blocks, 256, 0, ctx->upload_stream>>>(src, src_stride, rows, s.rows_padded, scale, ctx->desc + off * kDim, ctx->norms + off,
+                                                                  ctx->resid ? ctx->resid + off : nullptr, ctx->img_rmax ? ctx->img_rmax + image_id : nullptr);
     MSFM_CUDA_UPLOAD(ctx, mine, cudaGetLastError());
     return MSFM_OK;
 }
@@ -1367,7 +1559,8 @@ msfm_status msfm_upload_f32_batch_async(msfm_ctx *ctx, int32_t n, const int32_t 
     for (const Job &j : jobs) {  // quantise + key
         const ImageSlot &sl = ctx->images[j.id];
         const int blocks = std::max(1, std::min(4 * ctx->num_sms, (sl.rows_padded + 7) / 8));
-        msfm::pack_f32_kernel<<<blocks, 256, 0, ctx->upload_stream>>>(j.src, kDim, j.rows, sl.rows_padded, scale, ctx->desc + sl.off * kDim, ctx->norms + sl.off);
+        msfm::pack_f32_kernel<<<blocks, 256, 0, ctx->upload_stream>>>(j.src, kDim, j.rows, sl.rows_padded, scale, ctx->desc + sl.off * kDim, ctx->norms + sl.off,
+                                                                      ctx->resid ? ctx->resid + sl.off : nullptr, ctx->img_rmax ? ctx->img_rmax + j.id : nullptr);
         MSFM_CUDA_UPLOAD(ctx, uploaded, cudaGetLastError());
     }
     if (stage) MSFM_CUDA_UPLOAD(ctx, uploaded, cudaEventRecord(stage->done, ctx->upload_stream));
@@ -1386,6 +1579,8 @@ msfm_status msfm_release(msfm_ctx *ctx, int32_t image_id) {
     ImageSlot &s = ctx->images[image_id];
     arena_free(ctx, s.off, s.rows_padded);
     s = ImageSlot{};
+    // the next image under this id starts from a zero largest residual (the packer only raises it)
+    if (ctx->img_rmax) MSFM_CUDA(ctx, cudaMemsetAsync(ctx->img_rmax + image_id, 0, sizeof(float), ctx->upload_stream));
     return MSFM_OK;
 }
 
@@ -1396,6 +1591,7 @@ msfm_status msfm_release_all(msfm_ctx *ctx) {
     MSFM_CUDA(ctx, cudaStreamSynchronize(ctx->upload_stream));
     MSFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     for (ImageSlot &s : ctx->images) s = ImageSlot{};
+    if (ctx->img_rmax) MSFM_CUDA(ctx, cudaMemsetAsync(ctx->img_rmax, 0, (size_t)ctx->max_images * sizeof(float), ctx->upload_stream));
     ctx->free_list.clear();
     ctx->rows_high_water = 0;
     recycle_marks(ctx);
@@ -1439,30 +1635,15 @@ msfm_status msfm_download_packed(msfm_ctx *ctx, int32_t image_id, uint8_t *desc_
 }
 
 msfm_status msfm_knn2(msfm_ctx *ctx, int32_t ref_id, int32_t query_id, int32_t *ids, float *dists) {
-    if (!ctx) return MSFM_ERR_INVALID_ARG;
-    std::lock_guard<std::mutex> lock(ctx->mu);
-    if (!ids || !dists) return fail(ctx, MSFM_ERR_INVALID_ARG, "null output buffer");
-    MSFM_CUDA(ctx, cudaSetDevice(ctx->device));
-    BatchPlan plan;
-    msfm_status st = knn_single(ctx, ref_id, query_id, plan);
-    if (st != MSFM_OK) return st;
-    const int n = (int)plan.query_rows;
-    if (n == 0) return MSFM_OK;
-    if ((st = ensure(ctx, ctx->tight_matches, (size_t)n * 8)) != MSFM_OK) return st;
-    if ((st = ensure(ctx, ctx->matches, (size_t)n * 8)) != MSFM_OK) return st;
-    int32_t *d_ids = static_cast<int32_t *>(ctx->tight_matches.ptr);
-    float *d_dists = static_cast<float *>(ctx->matches.ptr);
-    msfm::knn_to_flann_kernel<<<(n + 255) / 256, 256, 0, ctx->stream>>>(static_cast<const int4 *>(ctx->knn.ptr), n, kCsplit, d_ids, d_dists);
-    MSFM_CUDA(ctx, cudaGetLastError());
-    ctx->timing.total_launches += 1;
-    MSFM_CUDA(ctx, cudaMemcpyAsync(ids, d_ids, (size_t)n * 8, cudaMemcpyDeviceToHost, ctx->stream));
-    MSFM_CUDA(ctx, cudaMemcpyAsync(dists, d_dists, (size_t)n * 8, cudaMemcpyDeviceToHost, ctx->stream));
-    MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_end, ctx->stream));
-    MSFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    ctx->timing.d2h_bytes = (int64_t)n * 16;
-    if ((st = accumulate_kernel_time(ctx, ctx->ev_k0, ctx->ev_k1)) != MSFM_OK) return st;
-    MSFM_CUDA(ctx, cudaEventElapsedTime(&ctx->timing.total_ms, ctx->ev_begin, ctx->ev_end));
-    return MSFM_OK;
+    // the one-pair, integer-distance form of msfm_knn2_pairs (the caller's arrays hold the query image's rows)
+    const msfm_pair pair{ref_id, query_id};
+    int64_t offsets[2];
+    return knn2_pairs_impl(ctx, &pair, 1, 0u, offsets, ids, dists, INT64_MAX);
+}
+
+msfm_status msfm_knn2_pairs(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pairs, uint32_t flags, int64_t *offsets, int32_t *ids,
+                            float *dists, int64_t row_capacity) {
+    return knn2_pairs_impl(ctx, pairs, n_pairs, flags, offsets, ids, dists, row_capacity);
 }
 
 msfm_status msfm_colbest(msfm_ctx *ctx, int32_t ref_id, int32_t query_id, int32_t *best_query, float *best_dist) {
@@ -1597,6 +1778,14 @@ msfm_status msfm_test_set_band_event_cap(msfm_ctx *ctx, int64_t cap) {
     if (!ctx) return MSFM_ERR_INVALID_ARG;
     std::lock_guard<std::mutex> lock(ctx->mu);
     ctx->band_event_cap_override = cap;
+    return MSFM_OK;
+}
+
+msfm_status msfm_test_last_knn_stats(msfm_ctx *ctx, int64_t *events, int32_t *brute_force_batches) {
+    if (!ctx) return MSFM_ERR_INVALID_ARG;
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    if (events) *events = ctx->knn_events;
+    if (brute_force_batches) *brute_force_batches = ctx->knn_brute_batches;
     return MSFM_OK;
 }
 

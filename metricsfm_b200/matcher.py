@@ -223,6 +223,34 @@ class Matcher:
         self._check(self._L.msfm_knn2(self._h, ref_id, query_id, ids.ctypes.data, dists.ctypes.data))
         return ids, dists
 
+    def knn2_pairs(self, pairs, exact_f32: bool = False):
+        """msfm_knn2_pairs: FLANN-layout 2-NN of every query row of every pair in one call.  Returns (offsets [n+1] int64,
+        ids [rows, 2] int32, dists [rows, 2] float32); pair p owns rows offsets[p]:offsets[p+1].  exact_f32: neighbours and
+        distances of an exhaustive fp32 matcher on the retained float rows (float uploads on a keep_float context, one
+        scale per pair); otherwise the integer distances of msfm_knn2."""
+        pa = self._pairs(pairs)
+        n = pa.shape[0]
+        rows_cache = {}
+        total = 0
+        for q in pa[:, 1]:
+            q = int(q)
+            if q not in rows_cache:
+                rows_cache[q] = self.image_info(q)[0]
+            total += rows_cache[q]
+        offsets = np.zeros((n + 1,), np.int64)
+        ids = np.empty((max(total, 1), 2), np.int32)
+        dists = np.empty((max(total, 1), 2), np.float32)
+        flags = _lib.KNN_EXACT_F32 if exact_f32 else 0
+        self._check(self._L.msfm_knn2_pairs(self._h, pa.ctypes.data, n, flags, offsets.ctypes.data, ids.ctypes.data,
+                                            dists.ctypes.data, total))
+        return offsets, ids[:total], dists[:total]
+
+    def _test_last_knn_stats(self):
+        """(events scored by the collect path, batches decided by the brute force) of the last exact knn2_pairs call."""
+        ev, bf = C.c_int64(), C.c_int32()
+        self._check(self._L.msfm_test_last_knn_stats(self._h, C.byref(ev), C.byref(bf)))
+        return ev.value, bf.value
+
     def knn2_crosscheck(self, ref_id: int, query_id: int):
         n, _ = self.image_info(query_id)
         ids = np.empty((n, 2), dtype=np.int32)
