@@ -31,8 +31,8 @@
  *   argmin_q' d(q',nn0) == q (lowest q' on ties); a pair with M < min_keypoints or N < min_keypoints is rejected
  *   as a whole (ok = 0, no matches), like feature_matching.cpp:30-33.  Missing neighbours: id = -1, dist = +inf.
  * Float regime: float rows are quantised to u8 by the packer, so d0/d1 carries a relative error of a few 1e-3; with
- *   msfm_config.keep_float + msfm_params.rescore_band the rows near a ratio threshold are decided on exact fp32
- *   distances instead (the match lists then agree with an fp32 brute-force matcher to <= 1e-4 of the matches).
+ *   msfm_config.keep_float + msfm_params.rescore_band the rows near a ratio threshold are decided on the exact fp32
+ *   top-2 instead (rows outside the band keep the integer decision, see msfm_params.rescore_band).
  *   msfm_knn2_pairs with MSFM_KNN_EXACT_F32 returns the kNN arrays of an fp32 matcher itself, bit for bit.
  */
 #ifndef MSFM_MATCH_H_
@@ -86,11 +86,16 @@ typedef struct msfm_params {
     int32_t min_keypoints; /* pairs with fewer rows on either side are rejected; reference value 20 */
     int32_t orientation;   /* 0: emit (ref_index, query_index)  fine_matching_graph.cc:121,127
                               1: emit (query_index, ref_index)  feature_matching.cpp:60-61 */
-    float rescore_band;    /* float regime (both images uploaded with msfm_upload_f32 on a keep_float context):
-                              > 0: query rows whose quantised d0/d1 lies within ratio*(1 +- band) or
-                              ratio_good*(1 +- band) are re-scored by exact fp32 brute force on the retained float
-                              rows (squared L2 accumulated in index order like nanoflann.hpp:376-383) and the ratio
-                              tests are repeated on the fp32 distances; 0 = decide on the quantised distances */
+    float rescore_band;    /* float regime (both images uploaded with msfm_upload_f32 on a keep_float context with the
+                              same scale s; any other pair, and band 0, follows the integer rule):
+                              > 0: a query row whose quantised 2-NN both exist and whose fl(d0/d1) lies within
+                              ratio*(1 +- band) or ratio_good*(1 +- band) (a NaN ratio never does) is decided on
+                              its exact fp32 top-2 (b0, b1) over the retained float rows (squared L2 accumulated in
+                              index order like nanoflann.hpp:376-383, lowest index on ties; the candidates are found
+                              under a proven bound): the ratio tests on fl(b0/b1), max_dist_sq on fl(b0*fl(s*s)), the
+                              match on the fp32 nearest row.  Every other row keeps the integer decision.  The mutual
+                              check of these pairs is a heuristic filter of the one-way list (not exact in fp32).
+                              0 = integer rule */
     uint32_t flags;        /* MSFM_RATIO_* bits; 0 = the strict rule of MATCH-SPEC */
 } msfm_params;
 
@@ -278,8 +283,9 @@ msfm_status msfm_knn2_crosscheck(msfm_ctx *ctx, int32_t ref_id, int32_t query_id
 /* Test hook: capacity of the float regime's event list (-1 = default sizing; 0 forces the brute-force fallback).
  * Applies to msfm_match_pairs' rescore_band and to msfm_knn2_pairs' MSFM_KNN_EXACT_F32 alike. */
 msfm_status msfm_test_set_band_event_cap(msfm_ctx *ctx, int64_t cap);
-/* Test hook: for the last MSFM_KNN_EXACT_F32 call of msfm_knn2_pairs, the events the collect path scored and the
- * batches whose event list overflowed, i.e. that the brute force decided.  Either pointer may be NULL. */
+/* Test hook: for the last MSFM_KNN_EXACT_F32 call of msfm_knn2_pairs or the last msfm_match_pairs call with
+ * rescore_band > 0 on a keep_float context, whichever came later, the events the collect path scored and the batches
+ * whose event list overflowed, i.e. that the brute force decided.  Either pointer may be NULL. */
 msfm_status msfm_test_last_knn_stats(msfm_ctx *ctx, int64_t *events, int32_t *brute_force_batches);
 /* Test hook: 1 routes every pair's mutual check through the tensor twin pass (the fallback of the bound-based check). */
 msfm_status msfm_test_force_twin_pass(msfm_ctx *ctx, int32_t on);

@@ -186,15 +186,16 @@ __device__ __forceinline__ int block_rank(bool keep, int &running, int *warp_exc
 //                        nanoflann.hpp:376-383 compiled without contraction), repeats the ratio tests on those
 //                        distances and overwrites the row's kNN entry with the decision
 // Rows outside the band keep the integer decision: their ratio is off the threshold by many times the quantisation error.
-// The fp32 work is confined to the reference rows whose QUANTISED distance is within ~3 % of the row's quantised second
-// best (ten times the quantisation error) -- only those can be fp32 top-2 neighbours.  They are found by the matching
-// kernel itself in "collect" mode (mark_band_kernel gathers the band rows into the candidate scratch image; the tensor
-// pass lists every reference row under the per-row threshold as an event), then
+// The fp32 work is confined to the reference rows whose QUANTISED distance is within the bound T(q) of exact_threshold
+// -- only those can be fp32 top-2 neighbours, so a band row is decided on its exact fp32 top-2.  They are found by
+// the matching kernel itself in "collect" mode (mark_band_kernel gathers the band rows into the candidate scratch
+// image; the tensor pass lists every reference row under the per-row threshold as an event), then
 //   score_events_kernel / second_events_kernel   fp32 distance per event, best and second best per band row (atomicMin
 //                                                on (distance bits, reference row): lowest index wins ties)
 //   finish_band_kernel                           the ratio tests on those distances, kNN entry overwritten
 // rescore_band_kernel does the same search with a dp4a brute force on CUDA cores; it runs only when the event list
-// overflowed (pathological inputs with many near-duplicates) and is the cross-check of the tests.
+// overflowed (bands much wider than the recommended 0.02, inputs full of near-duplicates) and is the cross-check of the
+// tests.
 constexpr int kRescoredFlag = 0x40000000;  // in knn[row].x: {id0 | flag, bit0 keep | bit1 good, int d0, fp32 d0 bits}
 constexpr int kRescoreRows = 16;           // band rows a CTA scores together against the reference image
 
@@ -224,11 +225,8 @@ struct BandParams {
     float *out_dists = nullptr;
 };
 
-// Quantised-distance threshold under which a reference row may still be an fp32 top-2 neighbour of a band row whose
-// quantised second-best distance is d1.
-__device__ __forceinline__ int band_threshold(int d1) { return d1 + (d1 >> 5) + 256; }
-
-// Exact kNN mode: a quantised-distance threshold T(q) that provably holds every fp32 top-2 neighbour of query row x.
+// A quantised-distance threshold T(q) that provably holds every fp32 top-2 neighbour of query row x (the band rows of
+// msfm_match_pairs and every row of the exact kNN mode).
 // With s the scale, q_y the packed row of y and r_y = ||s*y - q_y|| its quantisation residual (clamping included), the
 // triangle inequality gives  | s*||x-y|| - ||q_x-q_y|| | <= r_x + r_y <= r_x + R  (R: largest residual of the reference
 // image).  The two quantised nearest neighbours are therefore both within s*||x-y|| <= sqrt(d1_q) + r_x + R, so the fp32
@@ -269,12 +267,16 @@ __global__ void __launch_bounds__(256) mark_exact_kernel(const BandParams bp, co
     }
 }
 
-__global__ void __launch_bounds__(1024) mark_band_kernel(const BandParams bp) {
+// Float regime, per batch: lists pair p's band rows (rows knn_off .. knn_off + band_count_p of the candidate scratch),
+// each with the threshold exact_threshold(d1_q, r_x, R_ref).
+__global__ void __launch_bounds__(1024) mark_band_kernel(const BandParams bp, const float *__restrict__ resid,
+                                                         const float *__restrict__ img_rmax) {
     __shared__ int warp_excl[32];
     __shared__ int chunk_total;
     const PairDesc pd = bp.pairs[blockIdx.x];
     int running = 0;
     if (pd.fscale2 > 0.0f) {
+        const float rmax = img_rmax[pd.ref_img];
         for (int base = 0; base < pd.qry_rows; base += blockDim.x) {
             const int q = base + threadIdx.x;
             bool in_band = false;
@@ -289,13 +291,11 @@ __global__ void __launch_bounds__(1024) mark_band_kernel(const BandParams bp) {
                 }
             }
             const int slot = block_rank(in_band, running, warp_excl, &chunk_total);
-            if (in_band) {
+            if (in_band) {  // both neighbours exist: d1q >= 0
                 bp.band_q[pd.knn_off + slot] = q;
-                if (bp.band_thr) {
-                    bp.band_thr[pd.knn_off + slot] = band_threshold(d1q);
-                    bp.band_state[2 * (pd.knn_off + slot)] = ~0ull;
-                    bp.band_state[2 * (pd.knn_off + slot) + 1] = ~0ull;
-                }
+                bp.band_thr[pd.knn_off + slot] = exact_threshold(d1q, resid[pd.qry_off + q], rmax);
+                bp.band_state[2 * (pd.knn_off + slot)] = ~0ull;
+                bp.band_state[2 * (pd.knn_off + slot) + 1] = ~0ull;
             }
         }
     }
@@ -429,8 +429,7 @@ __global__ void __launch_bounds__(256) rescore_band_kernel(const BandParams bp, 
                 if (qi < nq) {
                     const int q = bp.band_q[pd.knn_off + c0 + qi];
                     na = ckey_to_norm(bp.ckeys[pd.qry_off + q]);
-                    // Prefilter on the quantised distance, the threshold the collect pass used: band_threshold of the
-                    // row's integer second best (~3 %, ten times the quantisation error), or exact_threshold.
+                    // Prefilter on the quantised distance: the threshold the collect pass used (exact_threshold)
                     thr = bp.band_thr[pd.knn_off + c0 + qi];
                 }
                 s_na[qi] = na;

@@ -120,8 +120,8 @@ struct msfm_ctx {
     DeviceBuf band_thr, band_state, band_events, band_event_keys, band_event_count;  // ... and the collect pass over them
     int64_t band_event_cap_override = -1;  // msfm_test_set_band_event_cap (tests: 0 forces the brute-force fallback)
     DeviceBuf knn_ids, knn_dists, knn_ids_b, knn_dists_b;  // msfm_knn2_pairs: FLANN-layout rows of a batch (two sets, see match_pairs_impl)
-    int64_t knn_events = 0;         // last exact-mode msfm_knn2_pairs: events scored by the collect path ...
-    int32_t knn_brute_batches = 0;  // ... and batches whose event list overflowed (brute force)
+    int64_t knn_events = 0;         // last exact-mode msfm_knn2_pairs or re-scoring msfm_match_pairs: events scored by
+    int32_t knn_brute_batches = 0;  // the collect path, and batches whose event list overflowed (brute force)
     bool force_twin = false;               // msfm_test_force_twin_pass
 #ifdef MSFM_DYNAMIC_ITEMS       // A/B builds only: work items drawn from a device counter instead of the static walk
     bool dynamic_items = true;
@@ -626,6 +626,7 @@ msfm_status match_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pa
     const bool mutual = params->mutual != 0;
     const bool want_good = params->ratio_good > 0.0f && (resident || out->has_good);
     const int64_t max_rows = mutual ? kBatchMaxQueryRowsMutual : kBatchMaxQueryRows;
+    if (params->rescore_band > 0.0f && ctx->fdesc) { ctx->knn_events = 0; ctx->knn_brute_batches = 0; }
     int64_t written = 0;  // matches written to the caller so far
     int64_t total = 0;
     if (!resident) out->offsets[0] = 0;
@@ -682,6 +683,8 @@ msfm_status match_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pa
             if ((st = ensure(ctx, ctx->cand_d0, rows * 4)) != MSFM_OK) return st;
             if ((st = ensure(ctx, ctx->cand_good, rows)) != MSFM_OK) return st;
             const bool float_rescoring = plan.rescoring && plan.any_float;
+            size_t event_cap = 0;
+            unsigned int h_events = 0;  // events of the collect pass, read back with the batch's offsets
             if ((mutual || float_rescoring) && (st = ensure_cand_scratch(ctx, plan.query_rows)) != MSFM_OK) return st;
             if ((st = ensure(ctx, ctx->matches, rows * sizeof(int2))) != MSFM_OK) return st;
             if (want_good && (st = ensure(ctx, ctx->good, rows)) != MSFM_OK) return st;
@@ -695,7 +698,12 @@ msfm_status match_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pa
             if ((st = run_match_stage(ctx, plan)) != MSFM_OK) return st;
             // ---- float regime: rows near a ratio threshold are decided on exact fp32 distances
             if (float_rescoring) {
-                const size_t event_cap = ctx->band_event_cap_override >= 0 ? (size_t)ctx->band_event_cap_override : rows / 2 + 65536;
+                // Event list: half an event per query row of the batch.  Measured on tools/float_regime_bench.py (780
+                // pairs of 8192-row unit-norm images in one batch, ratio 0.85, band 0.02): 1.14 % of the query rows are
+                // band rows, with 10.05 events each under T(q), 0.73 M events against a cap of 3.26 M, no overflow
+                // (profiles/float_regime_bound_1gpu.json).  Wide bands overflow it and the brute force decides the
+                // batch, with the same result.
+                event_cap = ctx->band_event_cap_override >= 0 ? (size_t)ctx->band_event_cap_override : rows / 2 + 65536;
                 if ((st = ensure(ctx, ctx->band_q, rows * 4)) != MSFM_OK) return st;
                 if ((st = ensure(ctx, ctx->band_counts, (size_t)nb * 4)) != MSFM_OK) return st;
                 if ((st = ensure(ctx, ctx->band_thr, rows * 4)) != MSFM_OK) return st;
@@ -726,7 +734,7 @@ msfm_status match_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pa
                 bp.event_keys = static_cast<unsigned long long *>(ctx->band_event_keys.ptr);
                 bp.event_count = static_cast<const unsigned int *>(ctx->band_event_count.ptr);
                 bp.event_cap = (uint32_t)event_cap;
-                msfm::mark_band_kernel<<<nb, 1024, 0, ctx->stream>>>(bp);
+                msfm::mark_band_kernel<<<nb, 1024, 0, ctx->stream>>>(bp, ctx->resid, ctx->img_rmax);
                 MSFM_CUDA(ctx, cudaGetLastError());
                 // tensor pass in collect mode over the gathered band rows, then fp32 scoring of what it listed
                 if (!plan.band_items.empty() &&
@@ -819,8 +827,13 @@ msfm_status match_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pa
             unsigned int twin_pairs = 0;
             MSFM_CUDA(ctx, cudaMemcpyAsync(batch_offsets.data(), ctx->offsets.ptr, (size_t)(nb + 1) * 8, cudaMemcpyDeviceToHost, ctx->stream));
             if (mutual) MSFM_CUDA(ctx, cudaMemcpyAsync(&twin_pairs, static_cast<int32_t *>(ctx->twin_counts.ptr) + nb, 4, cudaMemcpyDeviceToHost, ctx->stream));
+            if (float_rescoring) MSFM_CUDA(ctx, cudaMemcpyAsync(&h_events, ctx->band_event_count.ptr, 4, cudaMemcpyDeviceToHost, ctx->stream));
             MSFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
             ctx->timing.twin_pairs += (int32_t)twin_pairs;
+            if (float_rescoring) {
+                if (h_events > event_cap) ctx->knn_brute_batches += 1;
+                else ctx->knn_events += h_events;
+            }
             ctx->timing.d2h_bytes += (nb + 1) * 8;
             if ((st = accumulate_kernel_time(ctx, ctx->ev_k0, ctx->ev_k1)) != MSFM_OK) return st;
             if ((st = accumulate_kernel_time(ctx, ctx->ev_k2, ctx->ev_k3)) != MSFM_OK) return st;

@@ -246,7 +246,8 @@ class Matcher:
         return offsets, ids[:total], dists[:total]
 
     def _test_last_knn_stats(self):
-        """(events scored by the collect path, batches decided by the brute force) of the last exact knn2_pairs call."""
+        """(events scored by the collect path, batches decided by the brute force) of the last exact knn2_pairs call or
+        re-scoring match_pairs call (rescore_band > 0 on a keep_float context)."""
         ev, bf = C.c_int64(), C.c_int32()
         self._check(self._L.msfm_test_last_knn_stats(self._h, C.byref(ev), C.byref(bf)))
         return ev.value, bf.value

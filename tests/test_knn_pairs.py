@@ -2,8 +2,8 @@
 or exact in fp32 on the retained float rows (MSFM_KNN_EXACT_F32).
 
 The CPU test restates the exact mode's candidate bound T(q) (aux_kernels.cuh, exact_threshold) in numpy and checks that
-it holds every fp32 top-2 neighbour, including on rows built so that the float regime's heuristic band misses one.  The
-GPU tests compare the call with msfm_knn2, the CPU oracle and the golden vectors, bit for bit."""
+it holds every fp32 top-2 neighbour, including on rows built so that the float regime's former heuristic threshold misses
+one.  The GPU tests compare the call with msfm_knn2, the CPU oracle and the golden vectors, bit for bit."""
 import ctypes as C
 
 import numpy as np
@@ -38,7 +38,7 @@ def _exact_threshold(d1q, rx, rmax):
 
 
 def _heuristic_threshold(d1q):
-    """msfm_match_pairs' re-scoring band (band_threshold): d1 + d1/32 + 256."""
+    """The re-scoring threshold msfm_match_pairs used before it took T(q): d1 + d1/32 + 256."""
     return d1q + np.floor(d1q / 32.0) + 256.0
 
 
