@@ -23,12 +23,7 @@
 //   over the B ring (immediate addresses) and they sleep between polls (see the comment at the role dispatch).
 // MODE 1 ("collect", float regime) replaces the top-2 merge by "append every element under the row's fixed threshold
 // to an event list"; everything else is shared.
-// Work distribution (template parameter DYN):
-//   DYN = false  static: CTA b takes items b, b + grid, ...; every role walks that list on its own.
-//   DYN = true   the loader draws items from a device counter (atomicAdd) and publishes each index in a small shared-memory
-//                ring (s_item / i_full barriers) as soon as it knows it, i.e. one to two items ahead of the MMAs; issuers and
-//                epilogue warps read it there (-1 ends the CTA).  Items go to whichever CTA is free: a CTA that cannot be
-//                placed at launch (a collective or a packer kernel occupies its SM) simply finds nothing left.
+// Work distribution: CTA b takes items b, b + grid, ...; every role walks that list on its own.
 // Pipelines (all mbarrier based):
 //   A ring (2 deep)     : query strips of a work item, STRIPS x [128 rows x 128 B]
 //   B ring (STAGES)     : reference tiles [TILE_N rows x 128 B]
@@ -103,8 +98,6 @@ struct MatchKernelParams {
     uint32_t event_cap;
     const unsigned int *gate;     // optional: the whole launch returns at once when *gate == 0 (mutual twin pass with no
                                   // pair left for the tensor path, see select_candidates_kernel)
-    unsigned int *next_item;      // work-item counter of this launch (zero at launch): CTAs draw items from it, so a CTA that
-                                  // starts late (another kernel sits on its SM) or meets cheap items does not hold the launch up
     uint32_t prune_q8;            // "dead row" rule of the forward pass (see the epilogue): a row whose two nearest neighbours
                                   // so far satisfy d0 > (prune_q8 / 256) * d1 only follows its NEAREST neighbour exactly.
                                   // kNoPrune = off (exact 2-NN of every row: msfm_knn2, twin and collect passes)
@@ -139,11 +132,9 @@ struct MatchKernelCfg {
     static constexpr int kSmemTmin = kSmemKey + kKeySlots * TILE_N * 4;        // [kKeySlots] int4: the tile's smallest reference norm
     static constexpr int kSmemShare = kSmemTmin + kKeySlots * 16;              // [STRIPS*128 rows][CSPLIT] int4
     static constexpr int kSmemBar = kSmemShare + STRIPS * kStripRows * CSPLIT * 16;
-    static constexpr int kItemSlots = 8;  // published work-item indices (the loader runs at most two items ahead of the MMAs)
-    static constexpr int kNumBars = 2 + 2 + STAGES + STAGES + 2 * TBUFS * STRIPS + kItemSlots;
+    static constexpr int kNumBars = 2 + 2 + STAGES + STAGES + 2 * TBUFS * STRIPS;
     static constexpr int kSmemTmemPtr = kSmemBar + kNumBars * 8;
-    static constexpr int kSmemItems = kSmemTmemPtr + 16;
-    static constexpr int kSmemBytes = kSmemItems + kItemSlots * 4;
+    static constexpr int kSmemBytes = kSmemTmemPtr + 16;
     static constexpr int kSmemAlloc = kSmemBytes + 1024;  // slack for manual 1024-byte alignment
     static_assert(kTmemCols == 32 || kTmemCols == 64 || kTmemCols == 128 || kTmemCols == 256 || kTmemCols == 512,
                   "TMEM allocation must be a power of two in [32, 512] columns");
@@ -189,7 +180,7 @@ __device__ __forceinline__ int prune_score(int S0, int S1, int na, int rho8, int
     return dead ? S0 : S1;
 }
 
-template <int STRIPS, int TILE_N, int STAGES, int CSPLIT, int TBUFS, bool DEBUG, int MODE = 0, bool DYN = false>
+template <int STRIPS, int TILE_N, int STAGES, int CSPLIT, int TBUFS, bool DEBUG, int MODE = 0>
 __global__ void __launch_bounds__(MatchKernelCfg<STRIPS, TILE_N, STAGES, CSPLIT, TBUFS>::kThreads, 1)
 match_pairs_kernel(const MatchKernelParams p) {
     using Cfg = MatchKernelCfg<STRIPS, TILE_N, STAGES, CSPLIT, TBUFS>;
@@ -209,9 +200,7 @@ match_pairs_kernel(const MatchKernelParams p) {
     uint64_t *b_empty = b_full + STAGES;             // [STAGES]
     uint64_t *t_full = b_empty + STAGES;             // [TBUFS][STRIPS]
     uint64_t *t_empty = t_full + TBUFS * STRIPS;     // [TBUFS][STRIPS]
-    uint64_t *i_full = t_empty + TBUFS * STRIPS;     // [kItemSlots] (DYN) item index published
     uint32_t *tmem_ptr = reinterpret_cast<uint32_t *>(smem + Cfg::kSmemTmemPtr);
-    volatile int32_t *s_item = reinterpret_cast<volatile int32_t *>(smem + Cfg::kSmemItems);
 
     const int warp = __shfl_sync(0xFFFFFFFFu, (int)(threadIdx.x >> 5), 0);  // warp-uniform by construction: lets the compiler keep
                                                                             // everything derived from it in uniform registers
@@ -224,7 +213,6 @@ match_pairs_kernel(const MatchKernelParams p) {
         for (int i = 0; i < 2; ++i) { ptx::mbar_init(&a_full[i], 1); ptx::mbar_init(&a_empty[i], STRIPS); }
         for (int i = 0; i < STAGES; ++i) { ptx::mbar_init(&b_full[i], 1); ptx::mbar_init(&b_empty[i], STRIPS); }
         for (int i = 0; i < TBUFS * STRIPS; ++i) { ptx::mbar_init(&t_full[i], 1); ptx::mbar_init(&t_empty[i], 4 * CSPLIT); }
-        for (int i = 0; i < Cfg::kItemSlots; ++i) ptx::mbar_init(&i_full[i], 1);
         ptx::fence_mbar_init();
     }
     if (warp == Cfg::kEpiWarps + 1) ptx::tmem_alloc<Cfg::kTmemCols>(tmem_ptr);
@@ -268,21 +256,11 @@ match_pairs_kernel(const MatchKernelParams p) {
             const int4 *tminp = nullptr;
             auto next_item = [&]() -> bool {  // next item with work; fetches its query strips
                 for (;;) {
-                    const int idx = DYN ? (int)atomicAdd(p.next_item, 1u) : (cur += (int)gridDim.x);
-                    if (idx >= p.n_items) {
-                        if (DYN) {  // end marker
-                            s_item[a % Cfg::kItemSlots] = -1;
-                            ptx::mbar_arrive(&i_full[a % Cfg::kItemSlots]);
-                        }
-                        return false;
-                    }
+                    const int idx = (cur += (int)gridDim.x);
+                    if (idx >= p.n_items) return false;
                     const WorkItem wi = p.items[idx];
                     const PairDesc pd = p.pairs[wi.pair];
                     if (pd.cand_idx >= 0 && wi.row0 >= p.counts[pd.cand_idx]) continue;  // item past the candidate list
-                    if (DYN) {  // published before the strips are even requested: the other roles prefetch the descriptors
-                        s_item[a % Cfg::kItemSlots] = idx;
-                        ptx::mbar_arrive(&i_full[a % Cfg::kItemSlots]);
-                    }
                     const CUtensorMap *qmap = p.maps + pd.qry_img;
                     const uint32_t abuf = a & 1;
                     LOADER_WAIT(&a_empty[abuf], ((a >> 1) & 1) ^ 1);
@@ -339,18 +317,11 @@ match_pairs_kernel(const MatchKernelParams p) {
             uint32_t a = 0, abuf = 0, a_lo = 0, round = 0;
             auto next_item = [&]() -> bool {  // next item with work; waits for its query strips
                 for (;;) {
-                    int idx;
-                    if (DYN) {
-                        ISSUER_WAIT(&i_full[a % Cfg::kItemSlots], (a / Cfg::kItemSlots) & 1);
-                        idx = s_item[a % Cfg::kItemSlots];
-                        if (idx < 0) return false;
-                    } else {
-                        idx = (cur += (int)gridDim.x);
-                        if (idx >= p.n_items) return false;
-                    }
+                    const int idx = (cur += (int)gridDim.x);
+                    if (idx >= p.n_items) return false;
                     const WorkItem wi = p.items[idx];
                     const PairDesc pd = p.pairs[wi.pair];
-                    if (!DYN && pd.cand_idx >= 0 && wi.row0 >= p.counts[pd.cand_idx]) continue;
+                    if (pd.cand_idx >= 0 && wi.row0 >= p.counts[pd.cand_idx]) continue;
                     abuf = a & 1;
                     ISSUER_WAIT(&a_full[abuf], (a >> 1) & 1);
                     a_lo = a_lo0 + abuf * (Cfg::kABytes >> 4);
@@ -429,20 +400,11 @@ match_pairs_kernel(const MatchKernelParams p) {
         // ring positions all derive from ONE running tile counter g (TBUFS and kKeySlots are powers of two)
         static_assert((TBUFS & (TBUFS - 1)) == 0 && (Cfg::kKeySlots & (Cfg::kKeySlots - 1)) == 0, "ring sizes must be powers of two");
         uint32_t g = 0, a = 0;
-        const uint32_t i_full_base = ptx::smem_u32(i_full);
-        for (int cur = blockIdx.x;; cur += gridDim.x) {
-            int item = cur;
-            if (DYN) {  // published by the loader one to two items ahead of the MMAs
-                ptx::mbar_wait_a(i_full_base + (a % Cfg::kItemSlots) * 8, (a / Cfg::kItemSlots) & 1);
-                item = s_item[a % Cfg::kItemSlots];
-                if (item < 0) break;
-            } else if (item >= p.n_items) {
-                break;
-            }
+        for (int item = blockIdx.x; item < p.n_items; item += gridDim.x) {
             const WorkItem wi = p.items[item];
             const PairDesc pd = p.pairs[wi.pair];
             const int qry_rows = pd.cand_idx >= 0 ? p.counts[pd.cand_idx] : pd.qry_rows;
-            if (!DYN && wi.row0 >= qry_rows) continue;  // item past the candidate list (never published when DYN)
+            if (wi.row0 >= qry_rows) continue;  // item past the candidate list
             const int q = wi.row0 + row_local;
             const bool valid = q < qry_rows;
             const int na = valid ? ckey_to_norm((pd.cand_idx >= 0 ? p.cand_ckeys : p.ckeys)[pd.qry_off + q]) : 0;

@@ -114,7 +114,6 @@ struct msfm_ctx {
     DeviceBuf dbg_stats;  // debug flag 8: per-phase cycle counters of the matching kernel, dumped at destroy
     DeviceBuf cand_q, cand_j, cand_d0, cand_good, cand_counts, cand_desc, cand_ckeys;  // one-way candidates + gathered rows
     DeviceBuf tilemin;       // per reference tile: smallest squared norm (tile_min_kernel, refreshed per batch)
-    DeviceBuf item_counter;  // work-item counter of the matching launch in flight (zeroed before every launch)
     DeviceBuf colbest, twin_counts;  // mutual check: per-pair column table (nearest claimant per reference row); [n_pairs] + gate word
     DeviceBuf band_q, band_counts;  // float regime: query rows near a ratio threshold, per pair
     DeviceBuf band_thr, band_state, band_events, band_event_keys, band_event_count;  // ... and the collect pass over them
@@ -123,17 +122,7 @@ struct msfm_ctx {
     int64_t knn_events = 0;         // last exact-mode msfm_knn2_pairs or re-scoring msfm_match_pairs: events scored by
     int32_t knn_brute_batches = 0;  // the collect path, and batches whose event list overflowed (brute force)
     bool force_twin = false;               // msfm_test_force_twin_pass
-#ifdef MSFM_DYNAMIC_ITEMS       // A/B builds only: work items drawn from a device counter instead of the static walk
-    bool dynamic_items = true;
-#else
-    bool dynamic_items = false;
-#endif
-#ifdef MSFM_NO_PRUNE_DEFAULT   // A/B builds only
-    bool no_prune = true;
-#else
-    bool no_prune = false;
-#endif
-    // ^ msfm_test_disable_pruning: the forward pass keeps exact 2-NN rows for every query row
+    bool no_prune = false;                 // msfm_test_disable_pruning: the forward pass keeps exact 2-NN rows for every query row
     DeviceBuf staging, knn, matches, good, counts, offsets, pairdesc, items, tight_matches, tight_good;
     DeviceBuf tight_matches_b, tight_good_b;  // second set: a batch's lists are copied out while the next batch is gathered
     void *h_pinned = nullptr;
@@ -232,18 +221,22 @@ void arena_free(msfm_ctx *ctx, int64_t off, int64_t rows_padded) {
     ctx->free_list.swap(merged);
 }
 
-// One 2-D tensor map per image: inner dim 128 bytes, outer dim = exact row count, so that TMA zero-fills rows past
-// the image end (ragged sizes need no masking of the operands).
-msfm_status write_tensor_map(msfm_ctx *ctx, int32_t image_id, int64_t off, int32_t rows) {
-    CUtensorMap m;
-    memset(&m, 0, sizeof m);
-    cuuint64_t dims[2] = {(cuuint64_t)kDim, (cuuint64_t)std::max(rows, 1)};
+// 2-D tensor map over `rows` packed rows at `base`: inner dim 128 bytes, outer dim = exact row count, so that TMA
+// zero-fills rows past the end (ragged sizes need no masking of the operands); 64-row boxes, 128-byte swizzle.
+CUresult encode_row_map(const msfm_ctx *ctx, void *base, int64_t rows, CUtensorMap *m) {
+    memset(m, 0, sizeof *m);
+    cuuint64_t dims[2] = {(cuuint64_t)kDim, (cuuint64_t)rows};
     cuuint64_t strides[1] = {(cuuint64_t)kDim};
     cuuint32_t box[2] = {(cuuint32_t)kDim, (cuuint32_t)msfm::kBoxRows};
     cuuint32_t estr[2] = {1u, 1u};
-    CUresult r = ctx->encode(&m, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, ctx->desc + off * kDim, dims, strides, box, estr,
-                             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    return ctx->encode(m, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, base, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                       CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+}
+
+// One tensor map per image, in the image's slot.
+msfm_status write_tensor_map(msfm_ctx *ctx, int32_t image_id, int64_t off, int32_t rows) {
+    CUtensorMap m;
+    const CUresult r = encode_row_map(ctx, ctx->desc + off * kDim, std::max(rows, 1), &m);
     if (r != CUDA_SUCCESS) return fail(ctx, MSFM_ERR_CUDA, "cuTensorMapEncodeTiled failed with CUresult %d", (int)r);
     // The pinned slot of this image may still be in flight from an earlier upload of the same id (release + re-upload):
     // copies on one stream execute in order, and the slot is only rewritten after msfm_release* synchronised the streams.
@@ -255,6 +248,16 @@ msfm_status write_tensor_map(msfm_ctx *ctx, int32_t image_id, int64_t off, int32
 msfm_status check_image_id(msfm_ctx *ctx, int32_t id, bool must_exist) {
     if (id < 0 || id >= ctx->max_images) return fail(ctx, MSFM_ERR_INVALID_ARG, "image id %d outside [0, %d)", id, ctx->max_images);
     if (must_exist && !ctx->images[id].present) return fail(ctx, MSFM_ERR_NOT_FOUND, "image id %d has not been uploaded", id);
+    return MSFM_OK;
+}
+
+// Every pair of a caller's list names two uploaded images.
+msfm_status check_pairs(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pairs) {
+    msfm_status st;
+    for (int64_t i = 0; i < n_pairs; ++i) {
+        if ((st = check_image_id(ctx, pairs[i].ref, true)) != MSFM_OK) return st;
+        if ((st = check_image_id(ctx, pairs[i].query, true)) != MSFM_OK) return st;
+    }
     return MSFM_OK;
 }
 
@@ -335,10 +338,15 @@ struct BatchPlan {
     int64_t knn_rows() const { return mutual ? 2 * query_rows : query_rows; }
 };
 
-// collect = false: 2-NN of the items' query rows (forward pairs and mutual twins).  collect = true: the items are band
-// twins; every reference row within band_thr of a band row is appended to the event list instead.
-msfm_status launch_match_kernel(msfm_ctx *ctx, size_t first_item, size_t n_items, bool collect = false, uint32_t event_cap = 0, bool twin = false,
-                                uint32_t prune_q8 = msfm::kNoPrune) {
+// The passes of the matching kernel over a batch's work items [first_item, first_item + n_items):
+//   forward  2-NN of the forward pairs' query rows, with the dead-row rule `value` (prune_q8)
+//   twin     2-NN of the mutual twins' candidate rows, skipped on the device unless select_candidates_kernel routed a pair
+//   collect  the items are band twins: every reference row within band_thr of a band row is appended to the event list,
+//            which holds `value` events
+enum class Pass { forward, twin, collect };
+
+msfm_status launch_match_kernel(msfm_ctx *ctx, Pass pass, size_t first_item, size_t n_items, uint32_t value = 0) {
+    const bool collect = pass == Pass::collect, twin = pass == Pass::twin;
     msfm::MatchKernelParams kp;
     kp.maps = ctx->d_maps;
     kp.ckeys = ctx->norms;
@@ -350,29 +358,19 @@ msfm_status launch_match_kernel(msfm_ctx *ctx, size_t first_item, size_t n_items
     kp.gate = twin ? reinterpret_cast<const unsigned int *>(static_cast<const int32_t *>(ctx->twin_counts.ptr) + ctx->twin_gate_index) : nullptr;
     kp.events = static_cast<int4 *>(ctx->band_events.ptr);
     kp.event_count = static_cast<unsigned int *>(ctx->band_event_count.ptr);
-    kp.event_cap = event_cap;
+    kp.event_cap = collect ? value : 0;
     kp.pairs = static_cast<const PairDesc *>(ctx->pairdesc.ptr);
     kp.items = static_cast<const WorkItem *>(ctx->items.ptr) + first_item;
     kp.n_items = (int32_t)n_items;
     kp.stats = static_cast<unsigned long long *>(ctx->dbg_stats.ptr);  // null unless MSFM_DEBUG_FLAGS & 8
     kp.debug_flags = ctx->debug_flags;
     kp.knn = static_cast<int4 *>(ctx->knn.ptr);
-    kp.prune_q8 = (collect || twin || ctx->no_prune) ? msfm::kNoPrune : prune_q8;
+    kp.prune_q8 = (pass == Pass::forward && !ctx->no_prune) ? value : msfm::kNoPrune;
     const int grid = std::max(1, std::min<int>(ctx->num_sms, kp.n_items));
-    const bool dyn = ctx->dynamic_items && !collect && !ctx->debug_flags;
-    kp.next_item = nullptr;
-    if (dyn) {  // the launch's work-item counter
-        msfm_status st = ensure(ctx, ctx->item_counter, 256);
-        if (st != MSFM_OK) return st;
-        MSFM_CUDA(ctx, cudaMemsetAsync(ctx->item_counter.ptr, 0, 4, ctx->stream));
-        kp.next_item = static_cast<unsigned int *>(ctx->item_counter.ptr);
-    }
     if (collect)
         msfm::match_pairs_kernel<kStrips, kTileN, kStages, kCsplit, kTbufs, false, 1><<<grid, KCfg::kThreads, KCfg::kSmemAlloc, ctx->stream>>>(kp);
     else if (ctx->debug_flags)
         msfm::match_pairs_kernel<kStrips, kTileN, kStages, kCsplit, kTbufs, true><<<grid, KCfg::kThreads, KCfg::kSmemAlloc, ctx->stream>>>(kp);
-    else if (dyn)
-        msfm::match_pairs_kernel<kStrips, kTileN, kStages, kCsplit, kTbufs, false, 0, true><<<grid, KCfg::kThreads, KCfg::kSmemAlloc, ctx->stream>>>(kp);
     else
         msfm::match_pairs_kernel<kStrips, kTileN, kStages, kCsplit, kTbufs, false><<<grid, KCfg::kThreads, KCfg::kSmemAlloc, ctx->stream>>>(kp);
     MSFM_CUDA(ctx, cudaGetLastError());
@@ -389,14 +387,7 @@ msfm_status ensure_cand_scratch(msfm_ctx *ctx, int64_t rows) {
     if (ctx->cand_desc.ptr && ctx->cand_desc.bytes >= (size_t)rows * kDim) return MSFM_OK;
     if ((st = ensure(ctx, ctx->cand_desc, (size_t)rows * kDim)) != MSFM_OK) return st;
     CUtensorMap m;
-    memset(&m, 0, sizeof m);
-    cuuint64_t dims[2] = {(cuuint64_t)kDim, (cuuint64_t)(ctx->cand_desc.bytes / kDim)};
-    cuuint64_t strides[1] = {(cuuint64_t)kDim};
-    cuuint32_t box[2] = {(cuuint32_t)kDim, (cuuint32_t)msfm::kBoxRows};
-    cuuint32_t estr[2] = {1u, 1u};
-    CUresult r = ctx->encode(&m, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, ctx->cand_desc.ptr, dims, strides, box, estr,
-                             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    const CUresult r = encode_row_map(ctx, ctx->cand_desc.ptr, (int64_t)(ctx->cand_desc.bytes / kDim), &m);
     if (r != CUDA_SUCCESS) return fail(ctx, MSFM_ERR_CUDA, "cuTensorMapEncodeTiled (candidate scratch) failed with CUresult %d", (int)r);
     MSFM_CUDA(ctx, cudaMemcpyAsync(ctx->d_maps + ctx->max_images, &m, sizeof m, cudaMemcpyHostToDevice, ctx->stream));
     MSFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
@@ -504,7 +495,7 @@ msfm_status run_match_stage(msfm_ctx *ctx, const BatchPlan &plan) {
         ctx->timing.total_launches += 1;
     }
     MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_k0, ctx->stream));
-    if (!plan.items.empty() && (st = launch_match_kernel(ctx, 0, plan.items.size(), false, 0, false, plan.prune_q8)) != MSFM_OK) return st;
+    if (!plan.items.empty() && (st = launch_match_kernel(ctx, Pass::forward, 0, plan.items.size(), plan.prune_q8)) != MSFM_OK) return st;
     MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_k1, ctx->stream));
     ctx->timing.int8_ops += plan.ops;
     return MSFM_OK;
@@ -565,11 +556,108 @@ struct DrainListCopy {
     }
 };
 
+// Start copying a batch's result arrays to the host on the list-copy stream, behind the batch's last kernel (ev_f1).  The
+// second range is skipped when it is empty.  wait_list_copy waits for the copy.
+msfm_status start_list_copy(msfm_ctx *ctx, void *dst0, const void *src0, size_t bytes0, void *dst1, const void *src1, size_t bytes1) {
+    MSFM_CUDA(ctx, cudaStreamWaitEvent(ctx->d2h_stream, ctx->ev_f1, 0));
+    MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_d2h0, ctx->d2h_stream));
+    MSFM_CUDA(ctx, cudaMemcpyAsync(dst0, src0, bytes0, cudaMemcpyDeviceToHost, ctx->d2h_stream));
+    if (bytes1) MSFM_CUDA(ctx, cudaMemcpyAsync(dst1, src1, bytes1, cudaMemcpyDeviceToHost, ctx->d2h_stream));
+    MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_d2h1, ctx->d2h_stream));
+    ctx->d2h_in_flight = true;
+    ctx->timing.d2h_bytes += (int64_t)(bytes0 + bytes1);
+    return MSFM_OK;
+}
+
 msfm_status accumulate_kernel_time(msfm_ctx *ctx, cudaEvent_t e0, cudaEvent_t e1) {
     float ms = 0.f;
     MSFM_CUDA(ctx, cudaEventElapsedTime(&ms, e0, e1));
     ctx->timing.match_kernel_ms += ms;
     return MSFM_OK;
+}
+
+// Device time of a batch that has completed: the forward pass [ev_k0, ev_k1] and, when the batch recorded them, the twin
+// pass [ev_k2, ev_k3] are matching-kernel time; the rest of [ev_k0, ev_f1] is finalize time.
+msfm_status add_batch_times(msfm_ctx *ctx, bool twin_events) {
+    float ms_all = 0.f, ms_fw = 0.f, ms_twin = 0.f;
+    MSFM_CUDA(ctx, cudaEventElapsedTime(&ms_all, ctx->ev_k0, ctx->ev_f1));
+    MSFM_CUDA(ctx, cudaEventElapsedTime(&ms_fw, ctx->ev_k0, ctx->ev_k1));
+    if (twin_events) MSFM_CUDA(ctx, cudaEventElapsedTime(&ms_twin, ctx->ev_k2, ctx->ev_k3));
+    ctx->timing.match_kernel_ms += ms_fw + ms_twin;
+    ctx->timing.finalize_ms += ms_all - ms_fw - ms_twin;
+    return MSFM_OK;
+}
+
+// ---- Collect stage of the float regime: the band rows of a re-scoring msfm_match_pairs, every query row of an exact
+// msfm_knn2_pairs.  The caller's mark kernel gathers the rows and their thresholds into the candidate scratch; the
+// matching kernel's collect pass lists every reference row under a row's threshold, the events are scored in fp32 and
+// finish_band_kernel decides each row.  When the event list overflows, the dp4a brute force decides the batch instead.
+
+// Capacity of the event list: `allowance` + 65 536, or the test override; the kernels count events in 32 bits.
+size_t collect_event_cap(const msfm_ctx *ctx, size_t allowance) {
+    return std::min<size_t>(ctx->band_event_cap_override >= 0 ? (size_t)ctx->band_event_cap_override : allowance + 65536, UINT32_MAX);
+}
+
+msfm_status ensure_collect_scratch(msfm_ctx *ctx, size_t rows, size_t n_pairs, size_t event_cap) {
+    msfm_status st;
+    if ((st = ensure(ctx, ctx->band_q, rows * 4)) != MSFM_OK) return st;
+    if ((st = ensure(ctx, ctx->band_counts, n_pairs * 4)) != MSFM_OK) return st;
+    if ((st = ensure(ctx, ctx->band_thr, rows * 4)) != MSFM_OK) return st;
+    if ((st = ensure(ctx, ctx->band_state, rows * 16)) != MSFM_OK) return st;
+    if ((st = ensure(ctx, ctx->band_events, std::max<size_t>(event_cap, 1) * 16)) != MSFM_OK) return st;
+    if ((st = ensure(ctx, ctx->band_event_keys, std::max<size_t>(event_cap, 1) * 8)) != MSFM_OK) return st;
+    return ensure(ctx, ctx->band_event_count, 4);
+}
+
+// The collect stage's parameters over the current batch's scratch.  The ratio rule fields are left at zero and the
+// FLANN outputs null: msfm_match_pairs sets the former, msfm_knn2_pairs the latter.
+msfm::BandParams collect_params(const msfm_ctx *ctx, size_t event_cap) {
+    msfm::BandParams bp;
+    bp.pairs = static_cast<const PairDesc *>(ctx->pairdesc.ptr);
+    bp.knn = static_cast<int4 *>(ctx->knn.ptr);
+    bp.nshare = kCsplit;
+    bp.ratio = bp.ratio_good = bp.max_dist_sq = bp.band = 0.0f;
+    bp.reject_gt = 0;
+    bp.band_q = static_cast<int32_t *>(ctx->band_q.ptr);
+    bp.band_counts = static_cast<int32_t *>(ctx->band_counts.ptr);
+    bp.fdesc = ctx->fdesc;
+    bp.desc_arena = ctx->desc;
+    bp.ckeys = ctx->norms;
+    bp.band_thr = static_cast<int32_t *>(ctx->band_thr.ptr);
+    bp.band_state = static_cast<unsigned long long *>(ctx->band_state.ptr);
+    bp.cand_desc = static_cast<uint8_t *>(ctx->cand_desc.ptr);
+    bp.cand_ckeys = static_cast<int32_t *>(ctx->cand_ckeys.ptr);
+    bp.events = static_cast<const int4 *>(ctx->band_events.ptr);
+    bp.event_keys = static_cast<unsigned long long *>(ctx->band_event_keys.ptr);
+    bp.event_count = static_cast<const unsigned int *>(ctx->band_event_count.ptr);
+    bp.event_cap = (uint32_t)event_cap;
+    return bp;
+}
+
+// Everything after the mark kernel: the collect pass over the plan's band items, fp32 scoring of the events, the rows'
+// decisions, and the brute force, which returns at once unless the event list overflowed.
+msfm_status run_collect_pass(msfm_ctx *ctx, const BatchPlan &plan, const msfm::BandParams &bp) {
+    msfm_status st;
+    if (!plan.band_items.empty() &&
+        (st = launch_match_kernel(ctx, Pass::collect, plan.items.size() + plan.twin_items.size(), plan.band_items.size(), bp.event_cap)) != MSFM_OK)
+        return st;
+    const int nb = (int)plan.pairs.size();
+    msfm::score_events_kernel<<<4 * ctx->num_sms, 256, 0, ctx->stream>>>(bp);
+    msfm::second_events_kernel<<<4 * ctx->num_sms, 256, 0, ctx->stream>>>(bp);
+    msfm::finish_band_kernel<<<nb, 256, 0, ctx->stream>>>(bp);
+    const int gx = std::min(nb, 4 * ctx->num_sms);
+    const int gy = std::max(1, std::min(32, (4 * ctx->num_sms + gx - 1) / gx));
+    msfm::rescore_band_kernel<<<dim3(gx, gy), 256, 0, ctx->stream>>>(bp, nb);
+    MSFM_CUDA(ctx, cudaGetLastError());
+    ctx->timing.total_launches += 4;
+    return MSFM_OK;
+}
+
+// `events` is the collect pass's event count, read back after the batch: more than the list holds means the brute force
+// decided the batch.
+void note_collect_events(msfm_ctx *ctx, unsigned int events, size_t event_cap) {
+    if (events > event_cap) ctx->knn_brute_batches += 1;
+    else ctx->knn_events += events;
 }
 
 // kNN of a single pair into scratch (no gate).  Caller holds the lock.
@@ -616,10 +704,7 @@ msfm_status match_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pa
         return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_result needs offsets, ok and matches buffers");
     if (!(params->ratio > 0.0f)) return fail(ctx, MSFM_ERR_INVALID_ARG, "ratio must be > 0");
     msfm_status st;
-    for (int64_t i = 0; i < n_pairs; ++i) {
-        if ((st = check_image_id(ctx, pairs[i].ref, true)) != MSFM_OK) return st;
-        if ((st = check_image_id(ctx, pairs[i].query, true)) != MSFM_OK) return st;
-    }
+    if ((st = check_pairs(ctx, pairs, n_pairs)) != MSFM_OK) return st;
     ctx->timing = msfm_timing{};
     DrainListCopy drain_list_copy{ctx};
     MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_begin, ctx->stream));
@@ -643,7 +728,8 @@ msfm_status match_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pa
     // Batches are carved (host-only work: pair descriptors + work items) one ahead, while the previous batch runs on the GPU.
     struct Carved { BatchPlan plan; int64_t first = 0, last = 0; };
     int64_t next = 0;
-    auto carve = [&](Carved &c) {
+    auto carve = [&](Carved &c) -> bool {  // false: no pair left
+        if (next >= n_pairs) return false;
         c.plan = BatchPlan();
         c.plan.mutual = mutual;
         c.plan.rescoring = params->rescore_band > 0.0f && ctx->fdesc != nullptr;
@@ -665,90 +751,54 @@ msfm_status match_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pa
         }
         c.last = next;
         finish_plan(ctx, c.plan);
+        return true;
     };
     Carved cur, ahead;
-    bool have = next < n_pairs;
-    if (have) carve(cur);
-    int64_t batch_no = 0;  // picks the set of tight list buffers (the other set may still be on its way to the host)
-    while (have) {
+    bool have = carve(cur);
+    for (int64_t batch_no = 0; have; ++batch_no) {  // batch_no picks the set of tight list buffers (the other set may still be on its way to the host)
         BatchPlan &plan = cur.plan;
         const int64_t first = cur.first, last = cur.last;
-        bool have_next = false, carved_next = false;
         const int nb = (int)plan.pairs.size();
-        std::vector<int64_t> batch_offsets;
-        if (nb > 0 && plan.query_rows > 0) {
-            const size_t rows = (size_t)plan.query_rows;
+        const bool work = nb > 0 && plan.query_rows > 0;
+        const size_t rows = (size_t)plan.query_rows;
+        const bool float_rescoring = plan.rescoring && plan.any_float;
+        // Event list: half an event per query row of the batch.  Measured on tools/float_regime_bench.py (780 pairs of
+        // 8192-row unit-norm images in one batch, ratio 0.85, band 0.02): 1.14 % of the query rows are band rows, with
+        // 10.05 events each under T(q), 0.73 M events against a cap of 3.26 M, no overflow
+        // (profiles/float_regime_bound_1gpu.json).  Wide bands overflow it and the brute force decides the batch, with
+        // the same result.
+        const size_t event_cap = float_rescoring ? collect_event_cap(ctx, rows / 2) : 0;
+        // (a buffer that has to grow is not the one a list copy is still reading: see wait_list_copy below)
+        DeviceBuf &tm = batch_no & 1 ? ctx->tight_matches_b : ctx->tight_matches, &tg = batch_no & 1 ? ctx->tight_good_b : ctx->tight_good;
+        if (work) {
             if ((st = ensure(ctx, ctx->cand_q, rows * 4)) != MSFM_OK) return st;
             if ((st = ensure(ctx, ctx->cand_j, rows * 4)) != MSFM_OK) return st;
             if ((st = ensure(ctx, ctx->cand_d0, rows * 4)) != MSFM_OK) return st;
             if ((st = ensure(ctx, ctx->cand_good, rows)) != MSFM_OK) return st;
-            const bool float_rescoring = plan.rescoring && plan.any_float;
-            size_t event_cap = 0;
-            unsigned int h_events = 0;  // events of the collect pass, read back with the batch's offsets
             if ((mutual || float_rescoring) && (st = ensure_cand_scratch(ctx, plan.query_rows)) != MSFM_OK) return st;
+            if (float_rescoring && (st = ensure_collect_scratch(ctx, rows, nb, event_cap)) != MSFM_OK) return st;
             if ((st = ensure(ctx, ctx->matches, rows * sizeof(int2))) != MSFM_OK) return st;
             if (want_good && (st = ensure(ctx, ctx->good, rows)) != MSFM_OK) return st;
             if ((st = ensure(ctx, ctx->counts, (size_t)nb * 4)) != MSFM_OK) return st;
             if ((st = ensure(ctx, ctx->offsets, (size_t)(nb + 1) * 8)) != MSFM_OK) return st;
-            // (a buffer that has to grow is not the one a list copy is still reading: see wait_list_copy below)
-            DeviceBuf &tm = batch_no & 1 ? ctx->tight_matches_b : ctx->tight_matches, &tg = batch_no & 1 ? ctx->tight_good_b : ctx->tight_good;
             if ((st = ensure(ctx, tm, rows * sizeof(int2))) != MSFM_OK) return st;
             if (want_good && (st = ensure(ctx, tg, rows)) != MSFM_OK) return st;
             // ---- forward 2-NN
             if ((st = run_match_stage(ctx, plan)) != MSFM_OK) return st;
             // ---- float regime: rows near a ratio threshold are decided on exact fp32 distances
             if (float_rescoring) {
-                // Event list: half an event per query row of the batch.  Measured on tools/float_regime_bench.py (780
-                // pairs of 8192-row unit-norm images in one batch, ratio 0.85, band 0.02): 1.14 % of the query rows are
-                // band rows, with 10.05 events each under T(q), 0.73 M events against a cap of 3.26 M, no overflow
-                // (profiles/float_regime_bound_1gpu.json).  Wide bands overflow it and the brute force decides the
-                // batch, with the same result.
-                event_cap = ctx->band_event_cap_override >= 0 ? (size_t)ctx->band_event_cap_override : rows / 2 + 65536;
-                if ((st = ensure(ctx, ctx->band_q, rows * 4)) != MSFM_OK) return st;
-                if ((st = ensure(ctx, ctx->band_counts, (size_t)nb * 4)) != MSFM_OK) return st;
-                if ((st = ensure(ctx, ctx->band_thr, rows * 4)) != MSFM_OK) return st;
-                if ((st = ensure(ctx, ctx->band_state, rows * 16)) != MSFM_OK) return st;
-                if ((st = ensure(ctx, ctx->band_events, std::max<size_t>(event_cap, 1) * 16)) != MSFM_OK) return st;
-                if ((st = ensure(ctx, ctx->band_event_keys, std::max<size_t>(event_cap, 1) * 8)) != MSFM_OK) return st;
-                if ((st = ensure(ctx, ctx->band_event_count, 4)) != MSFM_OK) return st;
                 MSFM_CUDA(ctx, cudaMemsetAsync(ctx->band_event_count.ptr, 0, 4, ctx->stream));
-                msfm::BandParams bp;
-                bp.pairs = static_cast<const PairDesc *>(ctx->pairdesc.ptr);
-                bp.knn = static_cast<int4 *>(ctx->knn.ptr);
-                bp.nshare = kCsplit;
+                msfm::BandParams bp = collect_params(ctx, event_cap);
                 bp.ratio = params->ratio;
                 bp.ratio_good = params->ratio_good;
                 bp.max_dist_sq = params->max_dist_sq;
                 bp.band = params->rescore_band;
                 bp.reject_gt = (params->flags & MSFM_RATIO_REJECT_GT) ? 1 : 0;
-                bp.band_q = static_cast<int32_t *>(ctx->band_q.ptr);
-                bp.band_counts = static_cast<int32_t *>(ctx->band_counts.ptr);
-                bp.fdesc = ctx->fdesc;
-                bp.desc_arena = ctx->desc;
-                bp.ckeys = ctx->norms;
-                bp.band_thr = static_cast<int32_t *>(ctx->band_thr.ptr);
-                bp.band_state = static_cast<unsigned long long *>(ctx->band_state.ptr);
-                bp.cand_desc = static_cast<uint8_t *>(ctx->cand_desc.ptr);
-                bp.cand_ckeys = static_cast<int32_t *>(ctx->cand_ckeys.ptr);
-                bp.events = static_cast<const int4 *>(ctx->band_events.ptr);
-                bp.event_keys = static_cast<unsigned long long *>(ctx->band_event_keys.ptr);
-                bp.event_count = static_cast<const unsigned int *>(ctx->band_event_count.ptr);
-                bp.event_cap = (uint32_t)event_cap;
                 msfm::mark_band_kernel<<<nb, 1024, 0, ctx->stream>>>(bp, ctx->resid, ctx->img_rmax);
                 MSFM_CUDA(ctx, cudaGetLastError());
+                ctx->timing.total_launches += 1;
                 // tensor pass in collect mode over the gathered band rows, then fp32 scoring of what it listed
-                if (!plan.band_items.empty() &&
-                    (st = launch_match_kernel(ctx, plan.items.size() + plan.twin_items.size(), plan.band_items.size(), true, bp.event_cap)) != MSFM_OK)
-                    return st;
-                msfm::score_events_kernel<<<4 * ctx->num_sms, 256, 0, ctx->stream>>>(bp);
-                msfm::second_events_kernel<<<4 * ctx->num_sms, 256, 0, ctx->stream>>>(bp);
-                msfm::finish_band_kernel<<<nb, 256, 0, ctx->stream>>>(bp);
-                // brute-force search on CUDA cores: returns at once unless the event list overflowed
-                const int gx = std::min(nb, 4 * ctx->num_sms);
-                const int gy = std::max(1, std::min(32, (4 * ctx->num_sms + gx - 1) / gx));
-                msfm::rescore_band_kernel<<<dim3(gx, gy), 256, 0, ctx->stream>>>(bp, nb);
-                MSFM_CUDA(ctx, cudaGetLastError());
-                ctx->timing.total_launches += 5;
+                if ((st = run_collect_pass(ctx, plan, bp)) != MSFM_OK) return st;
             }
             // ---- ratio test -> one-way candidates; mutual check from the forward results (column table + dangerous rows),
             //      pairs too ambiguous for that are routed to the tensor twin pass
@@ -790,7 +840,7 @@ msfm_status match_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pa
             // ---- tensor twin pass (nearest query row of every candidate's reference row) for the routed pairs only
             MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_k2, ctx->stream));
             if (mutual && !plan.twin_items.empty() &&
-                (st = launch_match_kernel(ctx, plan.items.size(), plan.twin_items.size(), false, 0, true)) != MSFM_OK)
+                (st = launch_match_kernel(ctx, Pass::twin, plan.items.size(), plan.twin_items.size())) != MSFM_OK)
                 return st;
             MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_k3, ctx->stream));
             // ---- emission, offsets, tight gather
@@ -818,32 +868,22 @@ msfm_status match_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pa
             MSFM_CUDA(ctx, cudaGetLastError());
             MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_f1, ctx->stream));
             ctx->timing.total_launches += 3;
-            // ---- plan the next batch while this one runs
-            have_next = next < n_pairs;
-            if (have_next) carve(ahead);
-            carved_next = true;
+        }
+        // ---- plan the next batch while this one runs
+        have = carve(ahead);
+        std::vector<int64_t> batch_offsets;
+        if (work) {
             // ---- results
             batch_offsets.resize(nb + 1);
-            unsigned int twin_pairs = 0;
+            unsigned int twin_pairs = 0, h_events = 0;
             MSFM_CUDA(ctx, cudaMemcpyAsync(batch_offsets.data(), ctx->offsets.ptr, (size_t)(nb + 1) * 8, cudaMemcpyDeviceToHost, ctx->stream));
             if (mutual) MSFM_CUDA(ctx, cudaMemcpyAsync(&twin_pairs, static_cast<int32_t *>(ctx->twin_counts.ptr) + nb, 4, cudaMemcpyDeviceToHost, ctx->stream));
             if (float_rescoring) MSFM_CUDA(ctx, cudaMemcpyAsync(&h_events, ctx->band_event_count.ptr, 4, cudaMemcpyDeviceToHost, ctx->stream));
             MSFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
             ctx->timing.twin_pairs += (int32_t)twin_pairs;
-            if (float_rescoring) {
-                if (h_events > event_cap) ctx->knn_brute_batches += 1;
-                else ctx->knn_events += h_events;
-            }
+            if (float_rescoring) note_collect_events(ctx, h_events, event_cap);
             ctx->timing.d2h_bytes += (nb + 1) * 8;
-            if ((st = accumulate_kernel_time(ctx, ctx->ev_k0, ctx->ev_k1)) != MSFM_OK) return st;
-            if ((st = accumulate_kernel_time(ctx, ctx->ev_k2, ctx->ev_k3)) != MSFM_OK) return st;
-            {
-                float ms_all = 0.f, ms_a = 0.f, ms_b = 0.f;
-                MSFM_CUDA(ctx, cudaEventElapsedTime(&ms_all, ctx->ev_k0, ctx->ev_f1));
-                MSFM_CUDA(ctx, cudaEventElapsedTime(&ms_a, ctx->ev_k0, ctx->ev_k1));
-                MSFM_CUDA(ctx, cudaEventElapsedTime(&ms_b, ctx->ev_k2, ctx->ev_k3));
-                ctx->timing.finalize_ms += ms_all - ms_a - ms_b;
-            }
+            if ((st = add_batch_times(ctx, true)) != MSFM_OK) return st;
             const int64_t bt = batch_offsets[nb];
             total += bt;
             if ((st = wait_list_copy(ctx)) != MSFM_OK) return st;  // the previous batch's lists (copied under this batch's kernels)
@@ -852,19 +892,12 @@ msfm_status match_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pa
                 uint8_t *dst_g = nullptr;
                 if (out->sink(out->user, written, bt, &dst_m, &dst_g) != 0 || !dst_m)
                     return fail(ctx, MSFM_ERR_CAPACITY, "match buffer too small: need at least %lld entries", (long long)(written + bt));
+                if (dst_g && !want_good) memset(dst_g, 0, (size_t)bt);
                 // The lists leave on their own stream, ordered behind this batch's gather (ev_f1); the next batch's kernels
                 // start right away on the main stream and write the OTHER set of tight buffers.  At most one list copy is
                 // in flight: the previous one was waited for above, before the sink could move the host buffers.
-                MSFM_CUDA(ctx, cudaStreamWaitEvent(ctx->d2h_stream, ctx->ev_f1, 0));
-                MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_d2h0, ctx->d2h_stream));
-                MSFM_CUDA(ctx, cudaMemcpyAsync(dst_m, tm.ptr, (size_t)bt * sizeof(int2), cudaMemcpyDeviceToHost, ctx->d2h_stream));
-                if (dst_g) {
-                    if (want_good) MSFM_CUDA(ctx, cudaMemcpyAsync(dst_g, tg.ptr, (size_t)bt, cudaMemcpyDeviceToHost, ctx->d2h_stream));
-                    else memset(dst_g, 0, (size_t)bt);
-                }
-                MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_d2h1, ctx->d2h_stream));
-                ctx->d2h_in_flight = true;
-                ctx->timing.d2h_bytes += bt * (int64_t)(sizeof(int2) + (dst_g && want_good ? 1 : 0));
+                if ((st = start_list_copy(ctx, dst_m, tm.ptr, (size_t)bt * sizeof(int2), dst_g, tg.ptr, dst_g && want_good ? (size_t)bt : 0)) != MSFM_OK)
+                    return st;
             }
         }
         // ---- host bookkeeping for pairs [first, last)
@@ -883,13 +916,7 @@ msfm_status match_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pa
             }
             written = out->offsets[last];
         }
-        if (!carved_next) {
-            have_next = next < n_pairs;
-            if (have_next) carve(ahead);
-        }
         std::swap(cur, ahead);
-        have = have_next;
-        ++batch_no;
     }
     if ((st = wait_list_copy(ctx)) != MSFM_OK) return st;
     MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_end, ctx->stream));
@@ -913,12 +940,9 @@ msfm_status knn2_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pai
     if (flags & ~MSFM_KNN_EXACT_F32) return fail(ctx, MSFM_ERR_INVALID_ARG, "unknown flag bits 0x%x", flags & ~MSFM_KNN_EXACT_F32);
     const bool exact = (flags & MSFM_KNN_EXACT_F32) != 0;
     msfm_status st;
+    if ((st = check_pairs(ctx, pairs, n_pairs)) != MSFM_OK) return st;
     int64_t rows_total = 0;
-    for (int64_t i = 0; i < n_pairs; ++i) {
-        if ((st = check_image_id(ctx, pairs[i].ref, true)) != MSFM_OK) return st;
-        if ((st = check_image_id(ctx, pairs[i].query, true)) != MSFM_OK) return st;
-        rows_total += ctx->images[pairs[i].query].rows;
-    }
+    for (int64_t i = 0; i < n_pairs; ++i) rows_total += ctx->images[pairs[i].query].rows;
     if (rows_total > row_capacity)
         return fail(ctx, MSFM_ERR_CAPACITY, "output too small: the pairs have %lld query rows, row_capacity is %lld", (long long)rows_total,
                     (long long)row_capacity);
@@ -946,7 +970,8 @@ msfm_status knn2_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pai
     MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_begin, ctx->stream));
     const int64_t max_rows = exact ? kBatchMaxQueryRowsExact : kBatchMaxQueryRows;
     int64_t next = 0;
-    auto carve = [&](BatchPlan &plan) {
+    auto carve = [&](BatchPlan &plan) -> bool {  // false: no pair left
+        if (next >= n_pairs) return false;
         plan = BatchPlan();  // no pruning: exact 2-NN rows
         plan.rescoring = exact;
         while (next < n_pairs && (int64_t)plan.pairs.size() < kBatchMaxPairs) {
@@ -956,57 +981,30 @@ msfm_status knn2_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pai
             ++next;
         }
         finish_plan(ctx, plan);
+        return true;
     };
     BatchPlan cur, ahead;
-    bool have = next < n_pairs;
-    if (have) carve(cur);
+    bool have = carve(cur);
     for (int64_t batch_no = 0; have; ++batch_no) {
         BatchPlan &plan = cur;
         const int nb = (int)plan.pairs.size();
         const int64_t row_base = offsets[plan.src_index.front()];
-        bool carved_next = false;
-        if (plan.query_rows > 0) {
-            const size_t rows = (size_t)plan.query_rows;
-            DeviceBuf &oi = batch_no & 1 ? ctx->knn_ids_b : ctx->knn_ids, &od = batch_no & 1 ? ctx->knn_dists_b : ctx->knn_dists;
+        const bool work = plan.query_rows > 0;
+        const size_t rows = (size_t)plan.query_rows;
+        const size_t event_cap = exact ? collect_event_cap(ctx, rows * kExactEventsPerRow) : 0;
+        DeviceBuf &oi = batch_no & 1 ? ctx->knn_ids_b : ctx->knn_ids, &od = batch_no & 1 ? ctx->knn_dists_b : ctx->knn_dists;
+        if (work) {
             if ((st = ensure(ctx, oi, rows * 8)) != MSFM_OK) return st;
             if ((st = ensure(ctx, od, rows * 8)) != MSFM_OK) return st;
-            size_t event_cap = 0;
             if (exact) {
-                event_cap = std::min<size_t>(ctx->band_event_cap_override >= 0 ? (size_t)ctx->band_event_cap_override : rows * kExactEventsPerRow + 65536,
-                                             UINT32_MAX);
                 if ((st = ensure_cand_scratch(ctx, plan.query_rows)) != MSFM_OK) return st;
-                if ((st = ensure(ctx, ctx->band_q, rows * 4)) != MSFM_OK) return st;
-                if ((st = ensure(ctx, ctx->band_counts, (size_t)nb * 4)) != MSFM_OK) return st;
-                if ((st = ensure(ctx, ctx->band_thr, rows * 4)) != MSFM_OK) return st;
-                if ((st = ensure(ctx, ctx->band_state, rows * 16)) != MSFM_OK) return st;
-                if ((st = ensure(ctx, ctx->band_events, std::max<size_t>(event_cap, 1) * 16)) != MSFM_OK) return st;
-                if ((st = ensure(ctx, ctx->band_event_keys, std::max<size_t>(event_cap, 1) * 8)) != MSFM_OK) return st;
-                if ((st = ensure(ctx, ctx->band_event_count, 4)) != MSFM_OK) return st;
+                if ((st = ensure_collect_scratch(ctx, rows, nb, event_cap)) != MSFM_OK) return st;
             }
             // ---- forward 2-NN (exact rows: the plan carries no pruning)
             if ((st = run_match_stage(ctx, plan)) != MSFM_OK) return st;
-            unsigned int h_events = 0;
             if (exact) {
                 MSFM_CUDA(ctx, cudaMemsetAsync(ctx->band_event_count.ptr, 0, 4, ctx->stream));
-                msfm::BandParams bp;
-                bp.pairs = static_cast<const PairDesc *>(ctx->pairdesc.ptr);
-                bp.knn = static_cast<int4 *>(ctx->knn.ptr);
-                bp.nshare = kCsplit;
-                bp.ratio = bp.ratio_good = bp.max_dist_sq = bp.band = 0.0f;
-                bp.reject_gt = 0;
-                bp.band_q = static_cast<int32_t *>(ctx->band_q.ptr);
-                bp.band_counts = static_cast<int32_t *>(ctx->band_counts.ptr);
-                bp.fdesc = ctx->fdesc;
-                bp.desc_arena = ctx->desc;
-                bp.ckeys = ctx->norms;
-                bp.band_thr = static_cast<int32_t *>(ctx->band_thr.ptr);
-                bp.band_state = static_cast<unsigned long long *>(ctx->band_state.ptr);
-                bp.cand_desc = static_cast<uint8_t *>(ctx->cand_desc.ptr);
-                bp.cand_ckeys = static_cast<int32_t *>(ctx->cand_ckeys.ptr);
-                bp.events = static_cast<const int4 *>(ctx->band_events.ptr);
-                bp.event_keys = static_cast<unsigned long long *>(ctx->band_event_keys.ptr);
-                bp.event_count = static_cast<const unsigned int *>(ctx->band_event_count.ptr);
-                bp.event_cap = (uint32_t)event_cap;
+                msfm::BandParams bp = collect_params(ctx, event_cap);
                 bp.out_ids = static_cast<int32_t *>(oi.ptr);
                 bp.out_dists = static_cast<float *>(od.ptr);
                 int32_t max_q = 0;
@@ -1014,20 +1012,9 @@ msfm_status knn2_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pai
                 const int gy = std::max(1, std::min(64, (max_q + 255) / 256));
                 msfm::mark_exact_kernel<<<dim3(nb, gy), 256, 0, ctx->stream>>>(bp, ctx->resid, ctx->img_rmax);
                 MSFM_CUDA(ctx, cudaGetLastError());
+                ctx->timing.total_launches += 1;
                 // tensor pass in collect mode over every query row, fp32 scoring of what it listed, FLANN rows
-                if (!plan.band_items.empty() &&
-                    (st = launch_match_kernel(ctx, plan.items.size() + plan.twin_items.size(), plan.band_items.size(), true, bp.event_cap)) != MSFM_OK)
-                    return st;
-                msfm::score_events_kernel<<<4 * ctx->num_sms, 256, 0, ctx->stream>>>(bp);
-                msfm::second_events_kernel<<<4 * ctx->num_sms, 256, 0, ctx->stream>>>(bp);
-                msfm::finish_band_kernel<<<nb, 256, 0, ctx->stream>>>(bp);
-                // brute-force search on CUDA cores under the same thresholds: returns at once unless the event list overflowed
-                const int gx = std::min(nb, 4 * ctx->num_sms);
-                const int gyb = std::max(1, std::min(32, (4 * ctx->num_sms + gx - 1) / gx));
-                msfm::rescore_band_kernel<<<dim3(gx, gyb), 256, 0, ctx->stream>>>(bp, nb);
-                MSFM_CUDA(ctx, cudaGetLastError());
-                ctx->timing.total_launches += 6;
-                MSFM_CUDA(ctx, cudaMemcpyAsync(&h_events, ctx->band_event_count.ptr, 4, cudaMemcpyDeviceToHost, ctx->stream));
+                if ((st = run_collect_pass(ctx, plan, bp)) != MSFM_OK) return st;
             } else {
                 msfm::knn_to_flann_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, ctx->stream>>>(static_cast<const int4 *>(ctx->knn.ptr), (int)rows, kCsplit,
                                                                                              static_cast<int32_t *>(oi.ptr), static_cast<float *>(od.ptr));
@@ -1035,34 +1022,17 @@ msfm_status knn2_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pai
                 ctx->timing.total_launches += 1;
             }
             MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_f1, ctx->stream));
-            // ---- plan the next batch while this one runs
-            have = next < n_pairs;
-            if (have) carve(ahead);
-            carved_next = true;
-            MSFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-            if (exact) {
-                if (h_events > event_cap) ctx->knn_brute_batches += 1;
-                else ctx->knn_events += h_events;
-            }
-            if ((st = accumulate_kernel_time(ctx, ctx->ev_k0, ctx->ev_k1)) != MSFM_OK) return st;
-            {
-                float ms_all = 0.f, ms_a = 0.f;
-                MSFM_CUDA(ctx, cudaEventElapsedTime(&ms_all, ctx->ev_k0, ctx->ev_f1));
-                MSFM_CUDA(ctx, cudaEventElapsedTime(&ms_a, ctx->ev_k0, ctx->ev_k1));
-                ctx->timing.finalize_ms += ms_all - ms_a;
-            }
-            if ((st = wait_list_copy(ctx)) != MSFM_OK) return st;  // the previous batch's rows (copied under this batch's kernels)
-            MSFM_CUDA(ctx, cudaStreamWaitEvent(ctx->d2h_stream, ctx->ev_f1, 0));
-            MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_d2h0, ctx->d2h_stream));
-            MSFM_CUDA(ctx, cudaMemcpyAsync(ids + 2 * row_base, oi.ptr, rows * 8, cudaMemcpyDeviceToHost, ctx->d2h_stream));
-            MSFM_CUDA(ctx, cudaMemcpyAsync(dists + 2 * row_base, od.ptr, rows * 8, cudaMemcpyDeviceToHost, ctx->d2h_stream));
-            MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_d2h1, ctx->d2h_stream));
-            ctx->d2h_in_flight = true;
-            ctx->timing.d2h_bytes += (int64_t)rows * 16;
         }
-        if (!carved_next) {
-            have = next < n_pairs;
-            if (have) carve(ahead);
+        // ---- plan the next batch while this one runs
+        have = carve(ahead);
+        if (work) {
+            unsigned int h_events = 0;
+            if (exact) MSFM_CUDA(ctx, cudaMemcpyAsync(&h_events, ctx->band_event_count.ptr, 4, cudaMemcpyDeviceToHost, ctx->stream));
+            MSFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+            if (exact) note_collect_events(ctx, h_events, event_cap);
+            if ((st = add_batch_times(ctx, false)) != MSFM_OK) return st;
+            if ((st = wait_list_copy(ctx)) != MSFM_OK) return st;  // the previous batch's rows (copied under this batch's kernels)
+            if ((st = start_list_copy(ctx, ids + 2 * row_base, oi.ptr, rows * 8, dists + 2 * row_base, od.ptr, rows * 8)) != MSFM_OK) return st;
         }
         std::swap(cur, ahead);
     }
@@ -1191,8 +1161,6 @@ msfm_status msfm_create(const msfm_config *cfg, msfm_ctx **out) {
                              cudaFuncAttributeMaxDynamicSharedMemorySize, KCfg::kSmemAlloc) != cudaSuccess ||
         cudaFuncSetAttribute(msfm::match_pairs_kernel<kStrips, kTileN, kStages, kCsplit, kTbufs, false, 1>,
                              cudaFuncAttributeMaxDynamicSharedMemorySize, KCfg::kSmemAlloc) != cudaSuccess ||
-        cudaFuncSetAttribute(msfm::match_pairs_kernel<kStrips, kTileN, kStages, kCsplit, kTbufs, false, 0, true>,
-                             cudaFuncAttributeMaxDynamicSharedMemorySize, KCfg::kSmemAlloc) != cudaSuccess ||
         cudaFuncSetAttribute(msfm::select_candidates_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msfm::kSelectSmemBytes) != cudaSuccess)
         return bail(MSFM_ERR_CUDA);
     if (ctx->debug_flags & 8u) {
@@ -1236,7 +1204,7 @@ msfm_status msfm_destroy(msfm_ctx *ctx) {
     if (ctx->fdesc) cudaFree(ctx->fdesc);
     if (ctx->resid) cudaFree(ctx->resid);
     if (ctx->img_rmax) cudaFree(ctx->img_rmax);
-    DeviceBuf *bufs[] = {&ctx->knn_ids, &ctx->knn_dists, &ctx->knn_ids_b, &ctx->knn_dists_b, &ctx->band_q, &ctx->band_counts, &ctx->band_thr, &ctx->band_state, &ctx->band_events, &ctx->band_event_keys, &ctx->band_event_count, &ctx->cand_q, &ctx->cand_j, &ctx->cand_d0, &ctx->cand_good, &ctx->cand_counts, &ctx->cand_desc, &ctx->cand_ckeys, &ctx->colbest, &ctx->twin_counts, &ctx->item_counter, &ctx->tilemin,
+    DeviceBuf *bufs[] = {&ctx->knn_ids, &ctx->knn_dists, &ctx->knn_ids_b, &ctx->knn_dists_b, &ctx->band_q, &ctx->band_counts, &ctx->band_thr, &ctx->band_state, &ctx->band_events, &ctx->band_event_keys, &ctx->band_event_count, &ctx->cand_q, &ctx->cand_j, &ctx->cand_d0, &ctx->cand_good, &ctx->cand_counts, &ctx->cand_desc, &ctx->cand_ckeys, &ctx->colbest, &ctx->twin_counts, &ctx->tilemin,
                          &ctx->staging, &ctx->knn, &ctx->matches, &ctx->good, &ctx->counts, &ctx->offsets,
                          &ctx->pairdesc, &ctx->items, &ctx->tight_matches, &ctx->tight_good, &ctx->tight_matches_b, &ctx->tight_good_b};
     for (DeviceBuf *b : bufs)

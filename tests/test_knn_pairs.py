@@ -185,6 +185,9 @@ def test_exact_mode_equals_fp32_matcher_unit_norm(oracle_mod, native_lib):
         offsets, ids, dists = m.knn2_pairs([(4, 5)], exact_f32=True)
         events, brute = m._test_last_knn_stats()
         assert brute == 0 and events >= 8192
+        # pull_plan, tile_min, forward, mark_exact, collect, score_events, second_events, finish_band, rescore_band
+        t = m.timing()
+        assert t["total_launches"] == 9 and t["match_launches"] == 2
         _assert_exact(oracle_mod, imgs, [(4, 5)], offsets, ids, dists)
         int_offsets, int_ids, _ = m.knn2_pairs([(4, 5)])
         assert (int_ids != ids).any()  # quantised units do pick other neighbours: the reason the exact mode exists
