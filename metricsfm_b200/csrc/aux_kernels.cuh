@@ -118,35 +118,17 @@ __global__ void pull_plan_kernel(const uint4 *__restrict__ host_src, uint4 *__re
     }
 }
 
-// ------------------------------------------------------------------------------------------------ kNN shares
-// The matching kernel leaves `nshare` partial results per query row (one per column share).  Each is sorted
-// (d0,id0) <= (d1,id1); absent entries are (INT_MAX, -1).  The row's result is the two smallest (d, id) pairs.
-__device__ __forceinline__ bool knn_less(int da, int ia, int db, int ib) { return da < db || (da == db && ia < ib); }
-__device__ __forceinline__ int4 load_knn_share(const int4 *__restrict__ knn, int64_t idx) {
-    int4 v = knn[idx];
-    if (v.x < 0) v.z = INT_MAX;  // rows of work-less pairs are memset to -1
+// ------------------------------------------------------------------------------------------------ kNN records
+// The matching kernel leaves one record {id0, id1, d0, d1} per query row, sorted (d0,id0) <= (d1,id1); an absent
+// neighbour is (id -1, d INT_MAX).  load_knn() returns a record in which an id of -1 and a distance of INT_MAX always
+// come together, whichever of the two was written.
+__device__ __forceinline__ int4 load_knn(const int4 *__restrict__ knn, int64_t row) {
+    int4 v = knn[row];
+    if (v.x < 0) v.z = INT_MAX;  // rows of work-less pairs are memset to -1; seeded placeholders carry id -1
     if (v.y < 0) v.w = INT_MAX;
+    if (v.z == INT_MAX) v.x = -1;
+    if (v.w == INT_MAX) v.y = -1;
     return v;
-}
-__device__ __forceinline__ int4 merge_knn_shares(const int4 *__restrict__ knn, int64_t row, int nshare) {
-    int4 r = load_knn_share(knn, row * nshare);
-    for (int s = 1; s < nshare; ++s) {
-        const int4 o = load_knn_share(knn, row * nshare + s);
-        int4 m;
-        if (knn_less(o.z, o.x, r.z, r.x)) {  // o first
-            m.x = o.x; m.z = o.z;
-            const bool o2 = knn_less(o.w, o.y, r.z, r.x);
-            m.y = o2 ? o.y : r.x; m.w = o2 ? o.w : r.z;
-        } else {
-            m.x = r.x; m.z = r.z;
-            const bool r2 = knn_less(r.w, r.y, o.z, o.x);
-            m.y = r2 ? r.y : o.x; m.w = r2 ? r.w : o.z;
-        }
-        r = m;
-    }
-    if (r.z == INT_MAX) r.x = -1;
-    if (r.w == INT_MAX) r.y = -1;
-    return r;
 }
 
 // ------------------------------------------------------------------------------------------------ finalize
@@ -202,7 +184,6 @@ constexpr int kRescoreRows = 16;           // band rows a CTA scores together ag
 struct BandParams {
     const PairDesc *pairs;
     int4 *knn;
-    int32_t nshare;
     float ratio, ratio_good, max_dist_sq, band;
     int32_t reject_gt;     // ratio rule, see SelectParams
     int32_t *band_q;       // [forward kNN rows], pair p writes from row knn_off
@@ -251,7 +232,7 @@ __global__ void __launch_bounds__(256) mark_exact_kernel(const BandParams bp, co
     if (blockIdx.y == 0 && threadIdx.x == 0) bp.band_counts[blockIdx.x] = pd.qry_rows;
     const float rmax = pd.ref_rows > 0 ? img_rmax[pd.ref_img] : 0.0f;
     for (int q = blockIdx.y * blockDim.x + threadIdx.x; q < pd.qry_rows; q += gridDim.y * blockDim.x) {
-        const int4 k = merge_knn_shares(bp.knn, pd.knn_off + q, bp.nshare);
+        const int4 k = load_knn(bp.knn, pd.knn_off + q);
         const int64_t row = pd.knn_off + q;
         bp.band_q[row] = q;
         bp.band_thr[row] = exact_threshold(k.y >= 0 ? k.w : -1, resid[pd.qry_off + q], rmax);
@@ -282,7 +263,7 @@ __global__ void __launch_bounds__(1024) mark_band_kernel(const BandParams bp, co
             bool in_band = false;
             int d1q = 0;
             if (q < pd.qry_rows) {
-                const int4 k = merge_knn_shares(bp.knn, pd.knn_off + q, bp.nshare);
+                const int4 k = load_knn(bp.knn, pd.knn_off + q);
                 d1q = k.w;
                 if (k.x >= 0 && k.y >= 0) {
                     const float r = __fdiv_rn((float)k.z, (float)k.w);
@@ -346,8 +327,7 @@ __device__ __forceinline__ void write_rescored(const BandParams &bp, const PairD
     out.y = flags;
     out.z = di;
     out.w = __float_as_int(b0);
-    bp.knn[(pd.knn_off + q) * bp.nshare] = out;
-    for (int s = 1; s < bp.nshare; ++s) bp.knn[(pd.knn_off + q) * bp.nshare + s] = make_int4(-1, -1, INT_MAX, INT_MAX);
+    bp.knn[pd.knn_off + q] = out;
 }
 
 // fp32 squared distance of every collected event; best (distance, reference row) per band row.
@@ -538,7 +518,6 @@ constexpr int kCandGood = 1, kCandKilled = 2;  // bits of cand_good[]
 struct SelectParams {
     const PairDesc *pairs;
     const int4 *knn;
-    int32_t nshare;
     float ratio, ratio_good, max_dist_sq;
     int32_t reject_gt;         // ratio rule: 0 accept iff r < ratio; 1 accept iff !(r > ratio) (slam_gps.cc:470-477)
     int32_t *cand_q, *cand_j;  // [forward kNN rows], pair p writes from row knn_off
@@ -644,7 +623,7 @@ __global__ void __launch_bounds__(1024) select_candidates_kernel(const SelectPar
         const int q0 = base + threadIdx.x * kSelRows;  // this thread's rows are consecutive: thread order = row order
 #pragma unroll
         for (int r = 0; r < kSelRows; ++r)
-            k[r] = (q0 + r < pd.qry_rows) ? merge_knn_shares(sp.knn, pd.knn_off + q0 + r, sp.nshare) : make_int4(-1, -1, INT_MAX, INT_MAX);
+            k[r] = (q0 + r < pd.qry_rows) ? load_knn(sp.knn, pd.knn_off + q0 + r) : make_int4(-1, -1, INT_MAX, INT_MAX);
         unsigned keep = 0, good = 0;
         int d0max = -1;
 #pragma unroll
@@ -695,7 +674,7 @@ __global__ void __launch_bounds__(1024) select_candidates_kernel(const SelectPar
             if (!single) {
 #pragma unroll
                 for (int r = 0; r < kSelRows; ++r)
-                    k[r] = (q0 + r < pd.qry_rows) ? merge_knn_shares(sp.knn, pd.knn_off + q0 + r, sp.nshare) : make_int4(-1, -1, INT_MAX, INT_MAX);
+                    k[r] = (q0 + r < pd.qry_rows) ? load_knn(sp.knn, pd.knn_off + q0 + r) : make_int4(-1, -1, INT_MAX, INT_MAX);
             }
 #pragma unroll
             for (int r = 0; r < kSelRows; ++r)
@@ -867,8 +846,7 @@ __global__ void __launch_bounds__(1024) select_candidates_kernel(const SelectPar
 struct EmitParams {
     const PairDesc *pairs;
     const int4 *knn;
-    int32_t nshare;
-    int64_t twin_base;         // twin kNN row of candidate i of pair p = twin_base + knn_off + i
+    int64_t twin_base;        // twin kNN row of candidate i of pair p = twin_base + knn_off + i
     const int32_t *cand_q, *cand_j;
     const uint8_t *cand_good;
     const int32_t *cand_counts;
@@ -908,7 +886,7 @@ __global__ void __launch_bounds__(1024) emit_matches_kernel(const EmitParams ep)
             flags = ep.cand_good[pd.knn_off + i];
             if (ep.mutual && !twin) keep = (flags & kCandKilled) == 0;
             if (twin) {
-                const int4 tw = merge_knn_shares(ep.knn, ep.twin_base + pd.knn_off + i, ep.nshare);
+                const int4 tw = load_knn(ep.knn, ep.twin_base + pd.knn_off + i);
                 keep = tw.x == q;
                 if (ep.fdesc && pd.fscale2 > 0.0f && tw.x >= 0 && tw.y >= 0 && (tw.x == q || tw.y == q)) {
                     // two query rows within the quantisation slack of reference row j: decide on fp32 distances
@@ -982,11 +960,11 @@ __global__ void gather_matches_kernel(const PairDesc *__restrict__ pairs, const 
 }
 
 // kNN scratch {id0,id1,d0,d1} -> FLANN layout ids[2q..], dists[2q..] (float), one pair.
-__global__ void knn_to_flann_kernel(const int4 *__restrict__ knn, int rows, int nshare, int32_t *__restrict__ ids,
+__global__ void knn_to_flann_kernel(const int4 *__restrict__ knn, int rows, int32_t *__restrict__ ids,
                                     float *__restrict__ dists) {
     const int q = blockIdx.x * blockDim.x + threadIdx.x;
     if (q >= rows) return;
-    const int4 k = merge_knn_shares(knn, q, nshare);
+    const int4 k = load_knn(knn, q);
     ids[2 * q] = k.x;
     ids[2 * q + 1] = k.y;
     dists[2 * q] = k.x >= 0 ? (float)k.z : __int_as_float(0x7f800000);
@@ -994,11 +972,11 @@ __global__ void knn_to_flann_kernel(const int4 *__restrict__ knn, int rows, int 
 }
 
 // Nearest neighbour only (used for the "best query of each reference row" query).
-__global__ void knn_best_kernel(const int4 *__restrict__ knn, int rows, int nshare, int32_t *__restrict__ best,
+__global__ void knn_best_kernel(const int4 *__restrict__ knn, int rows, int32_t *__restrict__ best,
                                 float *__restrict__ dist) {
     const int j = blockIdx.x * blockDim.x + threadIdx.x;
     if (j >= rows) return;
-    const int4 k = merge_knn_shares(knn, j, nshare);
+    const int4 k = load_knn(knn, j);
     best[j] = k.x;
     dist[j] = k.x >= 0 ? (float)k.z : __int_as_float(0x7f800000);
 }

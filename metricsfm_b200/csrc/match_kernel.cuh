@@ -10,10 +10,10 @@
 // /root/reference/SfM/src/graph/fine_matching_graph.cc:99 (and slam_gps.cc:463, feature_matching.cpp:44,336,409)
 // with the brute-force/mutual-best semantics of the declared GPU matchers (SiftGPU.h:303-308, cudaSift sift.h:97).
 //
-// Roles per CTA (4*STRIPS*CSPLIT epilogue warps + 1 + STRIPS auxiliary warps padded to whole warpgroups; one CTA per SM,
+// Roles per CTA (4*STRIPS epilogue warps + 1 + STRIPS auxiliary warps padded to whole warpgroups; one CTA per SM,
 // persistent over work items):
-//   epilogue warps  warp w owns TMEM lanes 32*(w%4).. of query strip (w/4)%STRIPS and the column share w/(4*STRIPS)
-//                   of every tile (thread = query row x column share)
+//   epilogue warps  warp w owns TMEM lanes 32*(w%4).. of query strip w/4 and all TILE_N columns of every tile
+//                   (thread = query row)
 //   next warp       TMA producer (one elected lane)
 //   next STRIPS     MMA issuers, one per query strip (one elected lane each; the first also owns the TMEM allocation):
 //                   spreads the issue instructions over the four SM sub-partitions and lets every strip advance as soon
@@ -89,8 +89,8 @@ struct MatchKernelParams {
     uint32_t debug_flags;         // timing experiments only (results are wrong): 1 = skip the exact phase,
                                   // 2 = no epilogue work at all, 4 = TMEM loads + hand-back only
     unsigned long long *stats;    // optional debug counter (slow-path group visits); null in production
-    int4 *knn;                    // [sum qry_rows][CSPLIT] partial {id0, id1, d0, d1} per column share; id = -1 /
-                                  // d = INT_MAX when absent; consumers merge the shares with merge_knn_shares()
+    int4 *knn;                    // [sum qry_rows] {id0, id1, d0, d1} per query row; id = -1 / d = INT_MAX when absent;
+                                  // consumers read it with load_knn()
     // MODE 1 ("collect", float regime): instead of a top-2 the kernel lists every (query row, reference row) whose
     // squared distance is <= cand_d0[row], as {scratch row, reference row, cand_idx, 0}
     int4 *events;
@@ -104,11 +104,11 @@ struct MatchKernelParams {
 };
 constexpr uint32_t kNoPrune = 4096;  // ((d1 >> 8) + 1) * 4096 >= 16 * d1 > d0 for every row, and fits in 32 bits (d < 2^25)
 
-template <int STRIPS, int TILE_N, int STAGES, int CSPLIT, int TBUFS>
+template <int STRIPS, int TILE_N, int STAGES, int TBUFS>
 struct MatchKernelCfg {
-    // CSPLIT warps share one (strip, 32-row quarter) and split the tile's columns between them; TBUFS accumulator
-    // buffers per strip let the MMA of tile t+1 run under the epilogue of tile t.
-    static constexpr int kEpiWarps = 4 * STRIPS * CSPLIT;
+    // One epilogue warp per (strip, 32-row quarter); TBUFS accumulator buffers per strip let the MMA of tile t+1 run
+    // under the epilogue of tile t.
+    static constexpr int kEpiWarps = 4 * STRIPS;
     static constexpr int kAuxWarps = (1 + STRIPS + 3) / 4 * 4;       // TMA producer + one MMA issuer per strip, padded to warpgroups
     static constexpr int kThreads = (kEpiWarps + kAuxWarps) * 32;
     // Registers: the launch gives every thread 65536 / kThreads (a multiple of 8); the auxiliary warpgroups hand most of
@@ -116,7 +116,6 @@ struct MatchKernelCfg {
     static constexpr int kAuxRegs = 32;
     static constexpr int kLaunchRegs = 65536 / kThreads / 8 * 8;
     static constexpr int kEpiRegs = (kLaunchRegs * kThreads - kAuxWarps * 32 * kAuxRegs) / (kEpiWarps * 32) / 8 * 8;
-    static constexpr int kColsPerWarp = TILE_N / CSPLIT;
     // The producer may refill a key slot once the MMAs that share its B stage have completed; those were issued after
     // every epilogue warp released the accumulator buffer TBUFS tiles earlier; a warp releases a buffer before it has
     // finished reading that tile's keys, but it must finish before it can release the next one:
@@ -130,8 +129,7 @@ struct MatchKernelCfg {
     static constexpr int kSmemB = kSmemA + 2 * kABytes;
     static constexpr int kSmemKey = kSmemB + STAGES * kBBytes;
     static constexpr int kSmemTmin = kSmemKey + kKeySlots * TILE_N * 4;        // [kKeySlots] int4: the tile's smallest reference norm
-    static constexpr int kSmemShare = kSmemTmin + kKeySlots * 16;              // [STRIPS*128 rows][CSPLIT] int4
-    static constexpr int kSmemBar = kSmemShare + STRIPS * kStripRows * CSPLIT * 16;
+    static constexpr int kSmemBar = kSmemTmin + kKeySlots * 16;
     static constexpr int kNumBars = 2 + 2 + STAGES + STAGES + 2 * TBUFS * STRIPS;
     static constexpr int kSmemTmemPtr = kSmemBar + kNumBars * 8;
     static constexpr int kSmemBytes = kSmemTmemPtr + 16;
@@ -141,8 +139,7 @@ struct MatchKernelCfg {
     static_assert(TILE_N % kBoxRows == 0 && TILE_N <= 256, "reference tile is loaded as 64-row TMA boxes; UMMA N <= 256");
     static_assert(kAlignRows % TILE_N == 0, "image padding must cover whole reference tiles");
     static_assert(TILE_N == kKeyTileRows, "the minimum-norm table is kept per reference tile");
-    static_assert(CSPLIT == 1 || CSPLIT == 2, "one or two warps per (strip, quarter)");
-    static_assert(kColsPerWarp % 16 == 0 && kColsPerWarp / 8 <= 32, "one flag bit per group of 8 columns");
+    static_assert(TILE_N % 16 == 0 && TILE_N / 8 <= 32, "one flag bit per group of 8 columns");
     static_assert(kThreads <= 1024, "too many warps");
     static_assert(kSmemAlloc <= 227 * 1024, "shared memory budget");
 };
@@ -180,10 +177,10 @@ __device__ __forceinline__ int prune_score(int S0, int S1, int na, int rho8, int
     return dead ? S0 : S1;
 }
 
-template <int STRIPS, int TILE_N, int STAGES, int CSPLIT, int TBUFS, bool DEBUG, int MODE = 0>
-__global__ void __launch_bounds__(MatchKernelCfg<STRIPS, TILE_N, STAGES, CSPLIT, TBUFS>::kThreads, 1)
+template <int STRIPS, int TILE_N, int STAGES, int TBUFS, bool DEBUG, int MODE = 0>
+__global__ void __launch_bounds__(MatchKernelCfg<STRIPS, TILE_N, STAGES, TBUFS>::kThreads, 1)
 match_pairs_kernel(const MatchKernelParams p) {
-    using Cfg = MatchKernelCfg<STRIPS, TILE_N, STAGES, CSPLIT, TBUFS>;
+    using Cfg = MatchKernelCfg<STRIPS, TILE_N, STAGES, TBUFS>;
     // No static shared memory is declared, so the dynamic window starts at shared offset 0 (1024-byte aligned, as
     // the 128B-swizzled operand tiles require); checked once below.
     extern __shared__ __align__(1024) uint8_t smem[];
@@ -192,7 +189,6 @@ match_pairs_kernel(const MatchKernelParams p) {
     uint8_t *sB = smem + Cfg::kSmemB;
     int32_t *sKey = reinterpret_cast<int32_t *>(smem + Cfg::kSmemKey);
     int4 *sTmin = reinterpret_cast<int4 *>(smem + Cfg::kSmemTmin);
-    int4 *sShare = reinterpret_cast<int4 *>(smem + Cfg::kSmemShare);
     uint64_t *bars = reinterpret_cast<uint64_t *>(smem + Cfg::kSmemBar);
     uint64_t *a_full = bars;                         // [2]
     uint64_t *a_empty = a_full + 2;                  // [2]
@@ -212,12 +208,10 @@ match_pairs_kernel(const MatchKernelParams p) {
         // A buffers and B stages are released by the commits of all STRIPS MMA issuers
         for (int i = 0; i < 2; ++i) { ptx::mbar_init(&a_full[i], 1); ptx::mbar_init(&a_empty[i], STRIPS); }
         for (int i = 0; i < STAGES; ++i) { ptx::mbar_init(&b_full[i], 1); ptx::mbar_init(&b_empty[i], STRIPS); }
-        for (int i = 0; i < TBUFS * STRIPS; ++i) { ptx::mbar_init(&t_full[i], 1); ptx::mbar_init(&t_empty[i], 4 * CSPLIT); }
+        for (int i = 0; i < TBUFS * STRIPS; ++i) { ptx::mbar_init(&t_full[i], 1); ptx::mbar_init(&t_empty[i], 4); }
         ptx::fence_mbar_init();
     }
     if (warp == Cfg::kEpiWarps + 1) ptx::tmem_alloc<Cfg::kTmemCols>(tmem_ptr);
-    if (warp < Cfg::kEpiWarps)  // threshold-sharing slots {score, item tag} start out "no information"
-        for (int i = threadIdx.x; i < STRIPS * kStripRows * CSPLIT; i += Cfg::kEpiWarps * 32) sShare[i] = make_int4(0, 0, -1, 0);
     ptx::tc_fence_before();
     __syncthreads();
     ptx::tc_fence_after();
@@ -366,40 +360,32 @@ match_pairs_kernel(const MatchKernelParams p) {
         }
       }
     } else {
-        // =========================================================== epilogue (thread = query row x column share)
+        // =========================================================== epilogue (thread = query row)
         ptx::setmaxnreg_inc<(Cfg::kEpiRegs > 232 ? 232 : Cfg::kEpiRegs)>();
         // Scores s = 2*acc - ||r||^2 (maximise; d = ||q||^2 - s).
-        // Phase 1 (filter): stream this warp's share of the strip's accumulator tile through registers once and keep
+        // Phase 1 (filter): stream the warp's rows of the strip's accumulator tile through registers once and keep
         //   only the maximum RAW accumulator of every group of 8 columns; a group is flagged when that maximum exceeds
-        //   T = floor((theta + min||r||^2 over the share) / 2) in any lane.  theta is a lower bound of the row's final
+        //   T = floor((theta + min||r||^2 over the tile) / 2) in any lane.  theta is a lower bound of the row's final
         //   second-best score, so an unflagged group cannot enter the row's top-2
         //   (2*acc - nb_j <= 2*acc - nbmin <= theta) and costs ~0.45 instructions per element.
         // Phase 2 (exact): flagged groups (a few per tile) are re-read from TMEM and scored exactly with packed keys
         //   (branch-free top-2-of-8 network + merge), in ascending column order; ties never displace (strict >), hence
-        //   lowest-index tie-breaking inside a share.  Then the accumulator is handed back to the MMA warp.
-        // Column shares (CSPLIT = 2): the two threads of a row keep independent top-2 states over their own columns
-        //   (merged by the consumer kernels) but publish their two best scores;
-        //   theta = max(own S1, partner S1 - 1, min(own S0, partner S0 - 1)).
-        //   The "- 1" keeps every element that merely TIES the partner's second best in play, because the partner's
-        //   columns may lie to the right of it; elements strictly below two known scores can never reach the top-2.
-        const int share = warp / (4 * STRIPS);
-        const int strip = (warp >> 2) % STRIPS;
+        //   lowest-index tie-breaking.  Then the accumulator is handed back to the MMA warp.
+        // Each thread holds the row's whole top-2 state and writes the row's one kNN record at the end of the item.
+        const int strip = warp >> 2;
         const int quarter = warp & 3;
         const int row_local = strip * kStripRows + quarter * 32 + lane;
-        const uint32_t warp_taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + strip * TILE_N + share * Cfg::kColsPerWarp;
-        constexpr int kCols = Cfg::kColsPerWarp;
+        const uint32_t warp_taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + strip * TILE_N;
         constexpr int kAbsent = -0x08000000;  // scores below this are pad columns / "no neighbour"
         // everything the tile loop touches in shared memory, as 32-bit shared addresses
-        const uint32_t my_slot = ptx::smem_u32(sShare + row_local * CSPLIT + share);
-        const uint32_t peer_slot = ptx::smem_u32(sShare + row_local * CSPLIT + (share ^ (CSPLIT - 1)));
-        const uint32_t key_base = ptx::smem_u32(sKey) + share * kCols * 4;
+        const uint32_t key_base = ptx::smem_u32(sKey);
         const uint32_t tmin_base = ptx::smem_u32(sTmin);
         const uint32_t t_full_base = ptx::smem_u32(t_full + strip);
         const uint32_t t_empty_base = ptx::smem_u32(t_empty + strip);
         // ring positions are carried incrementally (no divisions in the tile loop)
         // ring positions all derive from ONE running tile counter g (TBUFS and kKeySlots are powers of two)
         static_assert((TBUFS & (TBUFS - 1)) == 0 && (Cfg::kKeySlots & (Cfg::kKeySlots - 1)) == 0, "ring sizes must be powers of two");
-        uint32_t g = 0, a = 0;
+        uint32_t g = 0;
         for (int item = blockIdx.x; item < p.n_items; item += gridDim.x) {
             const WorkItem wi = p.items[item];
             const PairDesc pd = p.pairs[wi.pair];
@@ -424,13 +410,13 @@ match_pairs_kernel(const MatchKernelParams p) {
             // the running-top-2 records of such rows (most rows of an image pair) never reach the exact phase.  A row that
             // ends dead reports d1 := d0: "rejected", and still a valid lower bound of its distance to every row but nn0,
             // which is what the mutual check's dangerous-row bound needs (select_candidates_kernel).
-            const int rho8 = (MODE == 0 && CSPLIT == 1 && pd.cand_idx < 0) ? (int)p.prune_q8 : (int)kNoPrune;  // shares keep partial states
+            const int rho8 = (MODE == 0 && pd.cand_idx < 0) ? (int)p.prune_q8 : (int)kNoPrune;
             const int ntiles = (pd.ref_rows + TILE_N - 1) / TILE_N;
             long long acc_wait = 0, acc_load = 0, acc_p1 = 0, acc_p2 = 0, acc_hot = 0, acc_first = 0;
             int theta = prune_score(S0, S1, na, rho8, kAbsent);  // pruning score of the row, refreshed after every hot tile
-            int jtile = share * kCols;  // first column of this warp's share in the current tile
+            int jtile = 0;  // first column of the current tile
             for (int t = 0; t < ntiles; ++t, jtile += TILE_N) {
-                // ---- pull this warp's whole share of the accumulator tile into registers and release TMEM at once
+                // ---- pull the warp's rows of the whole accumulator tile into registers and release TMEM at once
                 long long c0 = 0, c1 = 0, c2 = 0, c3 = 0;
                 const bool prof = DEBUG && (p.debug_flags & 8u) && p.stats != nullptr;
                 if (prof) c0 = clock64();
@@ -440,21 +426,14 @@ match_pairs_kernel(const MatchKernelParams p) {
                 ptx::tc_fence_after();
                 if (prof) c1 = clock64();
                 const uint32_t tile_taddr = warp_taddr + buf * (STRIPS * TILE_N);
-                uint32_t acc[kCols / 16][16];
+                uint32_t acc[TILE_N / 16][16];
 #pragma unroll
-                for (int c = 0; c < kCols / 16; ++c) ptx::tmem_ld_32x32b_x16(tile_taddr + c * 16, acc[c]);
+                for (int c = 0; c < TILE_N / 16; ++c) ptx::tmem_ld_32x32b_x16(tile_taddr + c * 16, acc[c]);
                 // ---- while the loads fly: column keys of the tile, smallest reference norm, pruning threshold
                 // (the tile's keys and minimum norm landed before its MMAs were issued: they share the B stage's barrier)
                 const uint32_t ck = key_base + ks * (TILE_N * 4);
                 const int nbmin = ptx::lds_s32(tmin_base + ks * 16);  // smallest reference norm of the tile (tile_min_kernel)
-                int th = theta;  // dead rows are pruned against their best score, the others against their second best
-                if (CSPLIT > 1) {
-                    // peer's {S0 - 1, S1 - 1, item tag}: the row's final second best is >= its own S1, >= the peer's S1
-                    // and >= min(S0_own, S0_peer); peer scores count minus one (see above)
-                    const int4 peer = ptx::lds_v4_volatile(peer_slot);
-                    if ((uint32_t)peer.z == a) th = __vimax3_s32(th, peer.y, min(S0, peer.x));
-                }
-                const int T = (th + nbmin) >> 1;
+                const int T = (theta + nbmin) >> 1;  // dead rows are pruned against their best score, the others against their second best
                 ptx::tmem_ld_wait();
                 ptx::tc_fence_before();
                 __syncwarp();
@@ -465,9 +444,9 @@ match_pairs_kernel(const MatchKernelParams p) {
                 } else {
                     // ---- phase 1: can any column of this tile still matter to some lane?  (maximum of the raw accumulators
                     //      per group of 8 columns, then of the tile: one vote; most tiles late in an item end here)
-                    int gm[kCols / 8];
+                    int gm[TILE_N / 8];
 #pragma unroll
-                    for (int gq = 0; gq < kCols / 8; ++gq) {
+                    for (int gq = 0; gq < TILE_N / 8; ++gq) {
                         const uint32_t *v = &acc[gq / 2][8 * (gq & 1)];
                         const int m1 = __vimax3_s32((int)v[0], (int)v[1], (int)v[2]);
                         const int m2 = __vimax3_s32((int)v[3], (int)v[4], (int)v[5]);
@@ -476,19 +455,18 @@ match_pairs_kernel(const MatchKernelParams p) {
                     }
                     int tm = gm[0];
 #pragma unroll
-                    for (int gq = 1; gq + 1 < kCols / 8; gq += 2) tm = __vimax3_s32(tm, gm[gq], gm[gq + 1]);
-                    tm = max(tm, gm[kCols / 8 - 1]);
+                    for (int gq = 1; gq + 1 < TILE_N / 8; gq += 2) tm = __vimax3_s32(tm, gm[gq], gm[gq + 1]);
+                    tm = max(tm, gm[TILE_N / 8 - 1]);
                     const bool tile_hot = __any_sync(0xFFFFFFFFu, tm > T);
                     if (prof) c3 = clock64();
-                    bool touched = false;
                     if (tile_hot) {
                         // ---- which groups?  (one vote and one branch per group: only paid by tiles that have one)
-                        bool hot[kCols / 8];
+                        bool hot[TILE_N / 8];
 #pragma unroll
-                        for (int gq = 0; gq < kCols / 8; ++gq) hot[gq] = __any_sync(0xFFFFFFFFu, gm[gq] > T);
+                        for (int gq = 0; gq < TILE_N / 8; ++gq) hot[gq] = __any_sync(0xFFFFFFFFu, gm[gq] > T);
                         // ---- phase 2: exact scoring of the hot groups straight from the registers
 #pragma unroll
-                        for (int gq = 0; gq < kCols / 8; ++gq) {
+                        for (int gq = 0; gq < TILE_N / 8; ++gq) {
                             if (hot[gq] && !(DEBUG && (p.debug_flags & 1u))) {
                                 const uint32_t *v = &acc[gq / 2][8 * (gq & 1)];
                                 const int4 c0 = ptx::lds_v4(ck + gq * 32);
@@ -509,15 +487,12 @@ match_pairs_kernel(const MatchKernelParams p) {
                                     top2_of8(key, g0, g1);
                                     merge_top2(g0 >> 3, jb8 | (g0 & 7), g1 >> 3, jb8 | (g1 & 7), S0, J0, S1, J1);  // columns stay packed: see the item's end
                                 }
-                                touched = true;
                                 if (prof) ++acc_hot;
                             }
                         }
                         // the row's pruning score for the next tiles (only a hot tile can change it)
                         theta = prune_score(S0, S1, na, rho8, kAbsent);
                     }
-                    if (CSPLIT > 1 && touched)
-                        ptx::sts_v4_volatile(my_slot, max(S0, INT_MIN + 1) - 1, max(S1, INT_MIN + 1) - 1, (int)a, 0);
                 }
                 if (prof) {  // per-warp cycle accounting of the tile loop (debug flag 8)
                     const long long c4 = clock64();
@@ -525,7 +500,7 @@ match_pairs_kernel(const MatchKernelParams p) {
                     if (t == 0) acc_first = c1 - c0;  // ... of the item's first tile (the item-switch bubble)
                     acc_load += c2 - c1;  // TMEM loads + keys + threshold + hand-back
                     acc_p1 += c3 - c2;    // phase 1
-                    acc_p2 += c4 - c3;    // phase 2 + publish
+                    acc_p2 += c4 - c3;    // phase 2
                 }
                 ++g;
             }
@@ -549,9 +524,8 @@ match_pairs_kernel(const MatchKernelParams p) {
                 out.y = (S1 > kAbsent && J1 >= 0) ? (J1 ^ 7) : -1;
                 out.z = (S0 > kAbsent) ? na - S0 : INT_MAX;
                 out.w = (S1 > kAbsent) ? na - S1 : INT_MAX;
-                p.knn[(pd.knn_off + q) * CSPLIT + share] = out;
+                p.knn[pd.knn_off + q] = out;
             }
-            ++a;
         }
     }
 

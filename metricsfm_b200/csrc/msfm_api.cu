@@ -34,9 +34,8 @@ using msfm::WorkItem;
 constexpr int kStrips = 4;   // query strips (128 rows each) per work item
 constexpr int kTileN = 64;   // reference rows per tile (UMMA N)
 constexpr int kStages = 8;   // B-tile ring depth
-constexpr int kCsplit = 1;   // epilogue warps per (strip, quarter): column shares
 constexpr int kTbufs = 2;    // TMEM accumulator buffers per strip
-using KCfg = msfm::MatchKernelCfg<kStrips, kTileN, kStages, kCsplit, kTbufs>;
+using KCfg = msfm::MatchKernelCfg<kStrips, kTileN, kStages, kTbufs>;
 constexpr int kItemRows = kStrips * msfm::kStripRows;
 
 // Per-batch scratch bounds (rows).  16 Mi query rows -> 256 MiB kNN scratch + 128 MiB match scratch.
@@ -368,11 +367,11 @@ msfm_status launch_match_kernel(msfm_ctx *ctx, Pass pass, size_t first_item, siz
     kp.prune_q8 = (pass == Pass::forward && !ctx->no_prune) ? value : msfm::kNoPrune;
     const int grid = std::max(1, std::min<int>(ctx->num_sms, kp.n_items));
     if (collect)
-        msfm::match_pairs_kernel<kStrips, kTileN, kStages, kCsplit, kTbufs, false, 1><<<grid, KCfg::kThreads, KCfg::kSmemAlloc, ctx->stream>>>(kp);
+        msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, false, 1><<<grid, KCfg::kThreads, KCfg::kSmemAlloc, ctx->stream>>>(kp);
     else if (ctx->debug_flags)
-        msfm::match_pairs_kernel<kStrips, kTileN, kStages, kCsplit, kTbufs, true><<<grid, KCfg::kThreads, KCfg::kSmemAlloc, ctx->stream>>>(kp);
+        msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, true><<<grid, KCfg::kThreads, KCfg::kSmemAlloc, ctx->stream>>>(kp);
     else
-        msfm::match_pairs_kernel<kStrips, kTileN, kStages, kCsplit, kTbufs, false><<<grid, KCfg::kThreads, KCfg::kSmemAlloc, ctx->stream>>>(kp);
+        msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, false><<<grid, KCfg::kThreads, KCfg::kSmemAlloc, ctx->stream>>>(kp);
     MSFM_CUDA(ctx, cudaGetLastError());
     ctx->timing.match_launches += 1;
     ctx->timing.total_launches += 1;
@@ -465,7 +464,7 @@ msfm_status run_match_stage(msfm_ctx *ctx, const BatchPlan &plan) {
     const size_t pd_pad = (pd_bytes + 15) / 16 * 16, it_pad = (it_fw + it_tw + 15) / 16 * 16;
     if ((st = ensure(ctx, ctx->pairdesc, pd_pad)) != MSFM_OK) return st;
     if ((st = ensure(ctx, ctx->items, it_pad)) != MSFM_OK) return st;
-    if ((st = ensure(ctx, ctx->knn, (size_t)plan.knn_rows() * kCsplit * sizeof(int4))) != MSFM_OK) return st;
+    if ((st = ensure(ctx, ctx->knn, (size_t)plan.knn_rows() * sizeof(int4))) != MSFM_OK) return st;
     if ((st = ensure(ctx, ctx->cand_counts, plan.pairs.size() * 4)) != MSFM_OK) return st;
     if ((st = ensure_pinned(ctx, pd_pad + it_pad + 64)) != MSFM_OK) return st;
     if ((st = wait_for_uploads(ctx, plan.need_seq)) != MSFM_OK) return st;  // asynchronous uploads of the batch's images
@@ -486,7 +485,7 @@ msfm_status run_match_stage(msfm_ctx *ctx, const BatchPlan &plan) {
         MSFM_CUDA(ctx, cudaGetLastError());
         ctx->timing.total_launches += 1;
     }
-    if (plan.has_empty) MSFM_CUDA(ctx, cudaMemsetAsync(ctx->knn.ptr, 0xFF, (size_t)plan.query_rows * kCsplit * sizeof(int4), ctx->stream));
+    if (plan.has_empty) MSFM_CUDA(ctx, cudaMemsetAsync(ctx->knn.ptr, 0xFF, (size_t)plan.query_rows * sizeof(int4), ctx->stream));
     if (plan.row_hi > plan.row_lo) {  // smallest norm per reference tile, over the arena rows this batch can touch
         if ((st = ensure(ctx, ctx->tilemin, (size_t)(ctx->arena_rows / msfm::kKeyTileRows + 1) * sizeof(int4))) != MSFM_OK) return st;
         const int64_t tile0 = plan.row_lo / msfm::kKeyTileRows, tile1 = (plan.row_hi + msfm::kKeyTileRows - 1) / msfm::kKeyTileRows;
@@ -615,7 +614,6 @@ msfm::BandParams collect_params(const msfm_ctx *ctx, size_t event_cap) {
     msfm::BandParams bp;
     bp.pairs = static_cast<const PairDesc *>(ctx->pairdesc.ptr);
     bp.knn = static_cast<int4 *>(ctx->knn.ptr);
-    bp.nshare = kCsplit;
     bp.ratio = bp.ratio_good = bp.max_dist_sq = bp.band = 0.0f;
     bp.reject_gt = 0;
     bp.band_q = static_cast<int32_t *>(ctx->band_q.ptr);
@@ -812,7 +810,6 @@ msfm_status match_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pa
             msfm::SelectParams sp;
             sp.pairs = static_cast<const PairDesc *>(ctx->pairdesc.ptr);
             sp.knn = static_cast<const int4 *>(ctx->knn.ptr);
-            sp.nshare = kCsplit;
             sp.ratio = params->ratio;
             sp.ratio_good = params->ratio_good;
             sp.max_dist_sq = params->max_dist_sq;
@@ -847,7 +844,6 @@ msfm_status match_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pa
             msfm::EmitParams ep;
             ep.pairs = sp.pairs;
             ep.knn = sp.knn;
-            ep.nshare = kCsplit;
             ep.twin_base = plan.query_rows;
             ep.cand_q = sp.cand_q;
             ep.cand_j = sp.cand_j;
@@ -1016,7 +1012,7 @@ msfm_status knn2_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pai
                 // tensor pass in collect mode over every query row, fp32 scoring of what it listed, FLANN rows
                 if ((st = run_collect_pass(ctx, plan, bp)) != MSFM_OK) return st;
             } else {
-                msfm::knn_to_flann_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, ctx->stream>>>(static_cast<const int4 *>(ctx->knn.ptr), (int)rows, kCsplit,
+                msfm::knn_to_flann_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, ctx->stream>>>(static_cast<const int4 *>(ctx->knn.ptr), (int)rows,
                                                                                              static_cast<int32_t *>(oi.ptr), static_cast<float *>(od.ptr));
                 MSFM_CUDA(ctx, cudaGetLastError());
                 ctx->timing.total_launches += 1;
@@ -1155,11 +1151,11 @@ msfm_status msfm_create(const msfm_config *cfg, msfm_ctx **out) {
     // one tensor map per image + one for the candidate scratch
     if (cudaMalloc(&ctx->d_maps, (size_t)(ctx->max_images + 1) * sizeof(CUtensorMap)) != cudaSuccess) return bail(MSFM_ERR_OUT_OF_MEMORY);
     if (cudaMallocHost(&ctx->h_maps, (size_t)(ctx->max_images + 1) * sizeof(CUtensorMap)) != cudaSuccess) return bail(MSFM_ERR_OUT_OF_MEMORY);
-    if (cudaFuncSetAttribute(msfm::match_pairs_kernel<kStrips, kTileN, kStages, kCsplit, kTbufs, false>,
+    if (cudaFuncSetAttribute(msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, false>,
                              cudaFuncAttributeMaxDynamicSharedMemorySize, KCfg::kSmemAlloc) != cudaSuccess ||
-        cudaFuncSetAttribute(msfm::match_pairs_kernel<kStrips, kTileN, kStages, kCsplit, kTbufs, true>,
+        cudaFuncSetAttribute(msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, true>,
                              cudaFuncAttributeMaxDynamicSharedMemorySize, KCfg::kSmemAlloc) != cudaSuccess ||
-        cudaFuncSetAttribute(msfm::match_pairs_kernel<kStrips, kTileN, kStages, kCsplit, kTbufs, false, 1>,
+        cudaFuncSetAttribute(msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, false, 1>,
                              cudaFuncAttributeMaxDynamicSharedMemorySize, KCfg::kSmemAlloc) != cudaSuccess ||
         cudaFuncSetAttribute(msfm::select_candidates_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msfm::kSelectSmemBytes) != cudaSuccess)
         return bail(MSFM_ERR_CUDA);
@@ -1642,7 +1638,7 @@ msfm_status msfm_colbest(msfm_ctx *ctx, int32_t ref_id, int32_t query_id, int32_
     if ((st = ensure(ctx, ctx->matches, (size_t)m * 4)) != MSFM_OK) return st;
     int32_t *d_best = static_cast<int32_t *>(ctx->tight_matches.ptr);
     float *d_dist = static_cast<float *>(ctx->matches.ptr);
-    msfm::knn_best_kernel<<<(m + 255) / 256, 256, 0, ctx->stream>>>(static_cast<const int4 *>(ctx->knn.ptr), m, kCsplit, d_best, d_dist);
+    msfm::knn_best_kernel<<<(m + 255) / 256, 256, 0, ctx->stream>>>(static_cast<const int4 *>(ctx->knn.ptr), m, d_best, d_dist);
     MSFM_CUDA(ctx, cudaGetLastError());
     MSFM_CUDA(ctx, cudaMemcpyAsync(best_query, d_best, (size_t)m * 4, cudaMemcpyDeviceToHost, ctx->stream));
     MSFM_CUDA(ctx, cudaMemcpyAsync(best_dist, d_dist, (size_t)m * 4, cudaMemcpyDeviceToHost, ctx->stream));
@@ -1901,7 +1897,7 @@ msfm_status msfm_knn2_crosscheck(msfm_ctx *ctx, int32_t ref_id, int32_t query_id
                                                                          static_cast<int4 *>(ctx->knn.ptr));
     int32_t *d_ids = static_cast<int32_t *>(ctx->tight_matches.ptr);
     float *d_dists = static_cast<float *>(ctx->matches.ptr);
-    msfm::knn_to_flann_kernel<<<(n + 255) / 256, 256, 0, ctx->stream>>>(static_cast<const int4 *>(ctx->knn.ptr), n, 1, d_ids, d_dists);
+    msfm::knn_to_flann_kernel<<<(n + 255) / 256, 256, 0, ctx->stream>>>(static_cast<const int4 *>(ctx->knn.ptr), n, d_ids, d_dists);
     MSFM_CUDA(ctx, cudaGetLastError());
     MSFM_CUDA(ctx, cudaMemcpyAsync(ids, d_ids, (size_t)n * 8, cudaMemcpyDeviceToHost, ctx->stream));
     MSFM_CUDA(ctx, cudaMemcpyAsync(dists, d_dists, (size_t)n * 8, cudaMemcpyDeviceToHost, ctx->stream));

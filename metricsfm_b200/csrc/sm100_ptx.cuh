@@ -42,14 +42,6 @@ __device__ __forceinline__ uint2 lds_v2_volatile(uint32_t addr) {
     asm volatile("ld.volatile.shared.v2.u32 {%0, %1}, [%2];" : "=r"(v.x), "=r"(v.y) : "r"(addr) : "memory");
     return v;
 }
-__device__ __forceinline__ int4 lds_v4_volatile(uint32_t addr) {
-    int4 v;
-    asm volatile("ld.volatile.shared.v4.s32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(addr) : "memory");
-    return v;
-}
-__device__ __forceinline__ void sts_v4_volatile(uint32_t addr, int x, int y, int z, int w) {
-    asm volatile("st.volatile.shared.v4.s32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(x), "r"(y), "r"(z), "r"(w) : "memory");
-}
 __device__ __forceinline__ void sts_v2_volatile(uint32_t addr, uint32_t x, uint32_t y) {
     asm volatile("st.volatile.shared.v2.u32 [%0], {%1, %2};" ::"r"(addr), "r"(x), "r"(y) : "memory");
 }

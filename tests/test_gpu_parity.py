@@ -304,19 +304,19 @@ def test_cpp_host_shim_matches_oracle(oracle_mod, native_lib, tmp_path):
 
 def test_adversarial_norm_spread_and_near_ties(oracle_mod, matcher):
     """Inputs that defeat the pruning filter (huge spread of reference norms, scores within 1 of each other across
-    column shares and tiles): results must stay bit-exact, only slower."""
+    columns and tiles): results must stay bit-exact, only slower."""
     rng = np.random.default_rng(91)
     ref = rng.integers(0, 256, size=(1300, 128), dtype=np.uint8)
     ref[::3] //= 8                      # a third of the rows with tiny norms, interleaved inside every tile
     ref[1::7] = 255 - ref[1::7] // 16   # and some with huge norms
     qry = rng.integers(0, 256, size=(700, 128), dtype=np.uint8)
-    # near-ties: copies of a query row differing by +-1 in one coordinate, scattered over tiles and both column shares
+    # near-ties: copies of a query row differing by +-1 in one coordinate, scattered over columns of several tiles
     base = qry[5].copy()
     for n, j in enumerate((3, 70, 130, 200, 640, 705, 1290)):
         r = base.copy()
         r[n] = np.clip(int(r[n]) + (1 if n % 2 else -1), 0, 255)
         ref[j] = r
-    ref[64] = base                      # exact hit in the second column share of tile 0
+    ref[64] = base                      # exact hit in the first column of tile 1
     ref[900] = base                     # and an equal-distance duplicate far to the right (must lose the tie)
     _upload_pair(matcher, ref, qry)
     ids, dists = _check_knn(oracle_mod, matcher, ref, qry)
