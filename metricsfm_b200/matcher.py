@@ -322,11 +322,14 @@ class Matcher:
         return total.value
 
     def geo_verify(self, pairs, result: "MatchResult", image_xy: dict, *, th_epipolar: float = 3.0, min_points: int = 30,
-                   min_inliers: int = 30, iters: int = 1024, seed: int = 0, ransac_only: bool = False):
+                   min_inliers: int = 30, iters: int = 1024, seed: int = 0, ransac_only: bool = False,
+                   pair_index_base: int = 0):
         """Batched GeoVerificationFundamental (utils/geo_verification.cc:30-79) of the pairs of a match_pairs result
         (orientation 0, ratio_good set).  image_xy: {image id: [n, 2] float32 centred keypoints}.  Returns
         (pair_ok [n] int32, pair_inliers [n] int32, keep [total] uint8, F [n, 3, 3] float64).  ransac_only: msfm_geo_ransac —
-        `result.good` selects the participating matches and `keep` is the RANSAC consensus mask instead of the F-filter."""
+        `result.good` selects the participating matches and `keep` is the RANSAC consensus mask instead of the F-filter.
+        pair_index_base: global index of the first pair in the RANSAC counter, so that a pair list verified in slices
+        draws the same hypotheses as in one call."""
         pa = self._pairs(pairs)
         n = pa.shape[0]
         n_images = int(pa.max()) + 1 if n else 0
@@ -337,7 +340,7 @@ class Matcher:
                 xy_keep.append(a)
                 ptrs[i] = a.ctypes.data
                 npts[i] = a.shape[0]
-        gp = _lib.GeoParams(th_epipolar, min_points, min_inliers, iters, seed, 0)
+        gp = _lib.GeoParams(th_epipolar, min_points, min_inliers, iters, seed, pair_index_base)
         total = int(result.offsets[n])
         ok = np.zeros((max(n, 1),), np.int32)
         inl = np.zeros((max(n, 1),), np.int32)

@@ -8,6 +8,7 @@ import pytest
 
 from conftest import GOLDEN_CASES
 from metricsfm_b200 import synth
+from oracle.geo_oracle import two_view_scene as _two_view_scene
 
 pytestmark = pytest.mark.gpu
 
@@ -517,21 +518,6 @@ def test_build_match_graph_driver_writes_reference_files(oracle_mod, native_lib,
 
 
 # ---------------------------------------------------------------------------------------------------- geo-verification
-def _two_view_scene(rng, n_true, n_out, noise=0.5, f=3000.0):
-    """Centred pixel coordinates of n_true correspondences of a rigid scene in two views + n_out random outliers."""
-    X = np.concatenate([rng.uniform(-40, 40, (n_true, 2)), rng.uniform(60, 140, (n_true, 1))], 1)
-    ang = np.deg2rad(rng.uniform(4, 10))
-    R = np.array([[np.cos(ang), 0, np.sin(ang)], [0, 1, 0], [-np.sin(ang), 0, np.cos(ang)]])
-    t = np.array([rng.uniform(8, 15), rng.uniform(-2, 2), rng.uniform(-1, 1)])
-    p1 = f * X[:, :2] / X[:, 2:3]
-    Xc = X @ R.T + t
-    p2 = f * Xc[:, :2] / Xc[:, 2:3]
-    p1 = p1 + rng.normal(0, noise, p1.shape)
-    p2 = p2 + rng.normal(0, noise, p2.shape)
-    o1, o2 = rng.uniform(-1800, 1800, (n_out, 2)), rng.uniform(-1800, 1800, (n_out, 2))
-    return np.concatenate([p1, o1]).astype(np.float32), np.concatenate([p2, o2]).astype(np.float32)
-
-
 def test_geo_verification_against_opencv_and_restatement(matcher):
     """Batched GPU GeoVerificationFundamental (utils/geo_verification.cc:30-79): stage B is exact given F (numpy
     restatement); stage A agrees with cv2.findFundamentalMat(FM_RANSAC, 3 px) on decisions and inlier sets."""
