@@ -34,6 +34,22 @@
  *   msfm_config.keep_float + msfm_params.rescore_band the rows near a ratio threshold are decided on the exact fp32
  *   top-2 instead (rows outside the band keep the integer decision, see msfm_params.rescore_band).
  *   msfm_knn2_pairs with MSFM_KNN_EXACT_F32 returns the kNN arrays of an fp32 matcher itself, bit for bit.
+ *
+ * GUIDED-SPEC (msfm_match_pairs_guided): MATCH-SPEC with the candidate set of every query row restricted to the
+ *   reference rows consistent with the pair's fundamental matrix.  F is given as msfm_geo_verify writes it
+ *   (double[9], row-major, p_q^T F p_r = 0 with p_r a keypoint of the reference image and p_q one of the query image,
+ *   centred feature-file coordinates) and rounded once to float f[9]; t2 = th*th in fp32 (th = th_epipolar).  Every
+ *   operation below is one IEEE fp32 rounding, with no fused multiply-add:
+ *     query row q at (xq, yq):     a_k = ((f[k]*xq) + (f[3+k]*yq)) + f[6+k]         k = 0, 1, 2
+ *     reference row j at (xj, yj): b_k = ((f[3k]*xj) + (f[3k+1]*yj)) + f[3k+2]     k = 0, 1
+ *     s = ((a0*xj) + (a1*yj)) + a2,  na = (a0*a0) + (a1*a1),  nb = (b0*b0) + (b1*b1)
+ *     element (q, j) is allowed iff s*s <= t2 * min(na, nb)
+ *   i.e. the larger of the two squared one-sided epipolar distances is at most th^2 (msfm_geo_verify's stage-A inlier
+ *   test without the division; msfm_geo_verify contracts to FMAs, so an element within rounding reach of th^2 may be
+ *   decided differently there).  nn0 / nn1 are the two closest allowed reference rows (lowest index on ties); a row with
+ *   fewer than two allowed rows gets id -1 / +inf and is rejected.  Ratio, ratio_good, max_dist_sq, MSFM_RATIO_REJECT_GT,
+ *   orientation and the min_keypoints gate (on the images' rows) are those of MATCH-SPEC; the mutual check keeps
+ *   (q, nn0) iff q is the closest allowed query row of nn0 (lowest index on ties).
  */
 #ifndef MSFM_MATCH_H_
 #define MSFM_MATCH_H_
@@ -277,6 +293,20 @@ msfm_status msfm_geo_ransac(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pai
                             const int32_t (*matches)[2], const uint8_t *use, const float *const *image_xy,
                             const int32_t *image_npts, int32_t n_images, const msfm_geo_params *gp, int32_t *pair_ok,
                             int32_t *pair_inliers, uint8_t *inlier_mask, double *F);
+
+/* ---- guided re-matching of verified pairs (GUIDED-SPEC above) ------------------------------------------------- */
+/* msfm_match_pairs with each query row's 2-NN searched only among the reference rows consistent with F[p] (typically
+ * msfm_geo_verify's F of the pairs with pair_ok).  image_xy / image_npts / n_images as in msfm_geo_verify; image_npts[i]
+ * must equal the uploaded rows of every image a pair touches.  Results, batches and msfm_last_timing as in
+ * msfm_match_pairs; with mutual = 1 every pair takes the tensor twin pass (timing.twin_pairs counts them).
+ * Errors (before any launch): the statuses of msfm_match_pairs, and INVALID_ARG (the message names the pair or image)
+ * for a null F, image_xy or image_npts; a pair naming an image >= n_images; a touched image without keypoints, with
+ * image_npts different from its uploaded rows, or with a non-finite coordinate; an F with a non-finite entry or that
+ * is zero after rounding to fp32; th_epipolar not finite or not > 0; rescore_band != 0 (no float regime under a gate). */
+msfm_status msfm_match_pairs_guided(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pairs, const msfm_params *params,
+                                    const double (*F)[9], float th_epipolar,
+                                    const float *const *image_xy, const int32_t *image_npts, int32_t n_images,
+                                    msfm_result *out);
 
 /* ---- GPU-side cross-check kernel (CUDA cores, dp4a); used by the tests to localise faults, never by the fast path */
 msfm_status msfm_knn2_crosscheck(msfm_ctx *ctx, int32_t ref_id, int32_t query_id, int32_t *ids, float *dists);

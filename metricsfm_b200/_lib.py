@@ -26,7 +26,7 @@ EXPORTED_SYMBOLS = [
     "msfm_download_packed", "msfm_knn2", "msfm_colbest", "msfm_match_pairs", "msfm_match_pairs_resident",
     "msfm_last_timing", "msfm_get_stream", "msfm_knn2_crosscheck", "msfm_geo_verify", "msfm_geo_ransac",
     "msfm_upload_f32_batch_async", "msfm_get_upload_stream", "msfm_wait_event", "msfm_test_set_band_event_cap", "msfm_test_force_twin_pass", "msfm_test_disable_pruning", "msfm_reserve_batch_async", "msfm_host_alloc", "msfm_host_free", "msfm_device_memory",
-    "msfm_knn2_pairs", "msfm_test_last_knn_stats",
+    "msfm_knn2_pairs", "msfm_test_last_knn_stats", "msfm_match_pairs_guided",
 ]
 
 
@@ -122,6 +122,8 @@ def load() -> C.CDLL:
     L.msfm_test_last_knn_stats.argtypes = [vp, _i64p, _i32p]
     L.msfm_colbest.argtypes = [vp, C.c_int32, C.c_int32, vp, vp]
     L.msfm_match_pairs.argtypes = [vp, vp, C.c_int64, C.POINTER(Params), C.POINTER(Result)]
+    L.msfm_match_pairs_guided.argtypes = [vp, vp, C.c_int64, C.POINTER(Params), vp, C.c_float, vp, vp, C.c_int32,
+                                          C.POINTER(Result)]
     L.msfm_match_pairs_resident.argtypes = [vp, vp, C.c_int64, C.POINTER(Params), _i64p]
     L.msfm_last_timing.argtypes = [vp, C.POINTER(Timing)]
     L.msfm_get_stream.argtypes = [vp, C.POINTER(vp)]

@@ -22,7 +22,8 @@
 //   The service warps share issue slots with the epilogue warps of their sub-partition: their tile loops are unrolled
 //   over the B ring (immediate addresses) and they sleep between polls (see the comment at the role dispatch).
 // MODE 1 ("collect", float regime) replaces the top-2 merge by "append every element under the row's fixed threshold
-// to an event list"; everything else is shared.
+// to an event list"; MODE 2 ("guided") bars the elements that fail an epipolar gate from the top-2 in the exact phase;
+// everything else is shared.
 // Work distribution: CTA b takes items b, b + grid, ...; every role walks that list on its own.
 // Pipelines (all mbarrier based):
 //   A ring (2 deep)     : query strips of a work item, STRIPS x [128 rows x 128 B]
@@ -92,15 +93,29 @@ struct MatchKernelParams {
     int4 *knn;                    // [sum qry_rows] {id0, id1, d0, d1} per query row; id = -1 / d = INT_MAX when absent;
                                   // consumers read it with load_knn()
     // MODE 1 ("collect", float regime): instead of a top-2 the kernel lists every (query row, reference row) whose
-    // squared distance is <= cand_d0[row], as {scratch row, reference row, cand_idx, 0}
-    int4 *events;
-    unsigned int *event_count;    // total events seen (may exceed event_cap: the consumer then falls back)
-    uint32_t event_cap;
+    // squared distance is <= cand_d0[row], as {scratch row, reference row, cand_idx, 0}.
+    // MODE 2 ("guided", msfm_match_pairs_guided): only elements that pass the epipolar gate (epi_allowed) can enter a
+    // row's top-2.  Forward item of pair p: row = query row, columns = reference rows, F = fmat[p]; twin item of pair p
+    // (cand_idx = p): row = candidate i, whose reference row is cand_j[qry_off + i], columns = query rows, same F.
+    // The two modes share these fields, which keeps the parameter block (and the code of modes 0 and 1) as it was.
+    union {
+        int4 *events;
+        const float2 *xy;         // MODE 2: keypoints (x, y), indexed like the column-key arena
+    };
+    union {
+        unsigned int *event_count;  // total events seen (may exceed event_cap: the consumer then falls back)
+        const float *fmat;          // MODE 2: [forward pairs of the batch][9] F rounded to fp32, row-major
+    };
+    union {
+        uint32_t event_cap;
+        const int32_t *cand_j;      // MODE 2: reference row of every gathered candidate (twin items)
+    };
     const unsigned int *gate;     // optional: the whole launch returns at once when *gate == 0 (mutual twin pass with no
                                   // pair left for the tensor path, see select_candidates_kernel)
     uint32_t prune_q8;            // "dead row" rule of the forward pass (see the epilogue): a row whose two nearest neighbours
                                   // so far satisfy d0 > (prune_q8 / 256) * d1 only follows its NEAREST neighbour exactly.
                                   // kNoPrune = off (exact 2-NN of every row: msfm_knn2, twin and collect passes)
+    float t2;                     // MODE 2: th_epipolar^2, rounded to fp32
 };
 constexpr uint32_t kNoPrune = 4096;  // ((d1 >> 8) + 1) * 4096 >= 16 * d1 > d0 for every row, and fits in 32 bits (d < 2^25)
 
@@ -175,6 +190,18 @@ __device__ __forceinline__ int prune_score(int S0, int S1, int na, int rho8, int
     const int d0 = (int)((uint32_t)na - (uint32_t)S0), d1 = (int)((uint32_t)na - (uint32_t)S1);
     const bool dead = (S1 > absent) && (d0 > (d1 >> 8) * rho8 + rho8);
     return dead ? S0 : S1;
+}
+
+// Epipolar gate of GUIDED-SPEC (include/msfm_match.h).  Query line a = F^T (xq, yq, 1), reference line b = F (xj, yj, 1),
+// s = a . (xj, yj, 1): element (q, j) is allowed iff s^2 <= t2 * min(|a|^2, |b|^2) over the first two components.  Every
+// operation is one fp32 rounding (no contraction), so the forward item (row q) and the twin item (row j) decide an element
+// identically, and a numpy float32 restatement reproduces it bit for bit.
+__device__ __forceinline__ float epi_lin(float u, float x, float v, float y, float w) {  // ((u*x) + (v*y)) + w
+    return __fadd_rn(__fadd_rn(__fmul_rn(u, x), __fmul_rn(v, y)), w);
+}
+__device__ __forceinline__ float epi_sq(float u, float v) { return __fadd_rn(__fmul_rn(u, u), __fmul_rn(v, v)); }
+__device__ __forceinline__ bool epi_allowed(float s, float na, float nb, float t2) {
+    return __fmul_rn(s, s) <= __fmul_rn(t2, nb < na ? nb : na);
 }
 
 template <int STRIPS, int TILE_N, int STAGES, int TBUFS, bool DEBUG, int MODE = 0>
@@ -410,7 +437,30 @@ match_pairs_kernel(const MatchKernelParams p) {
             // the running-top-2 records of such rows (most rows of an image pair) never reach the exact phase.  A row that
             // ends dead reports d1 := d0: "rejected", and still a valid lower bound of its distance to every row but nn0,
             // which is what the mutual check's dangerous-row bound needs (select_candidates_kernel).
-            const int rho8 = (MODE == 0 && pd.cand_idx < 0) ? (int)p.prune_q8 : (int)kNoPrune;
+            // Under the epipolar gate (MODE 2) the rule stays on: it only reasons about elements that can enter the row's
+            // top-2, and the gate only removes elements (barred ones never reach the running state).
+            const int rho8 = (MODE != 1 && pd.cand_idx < 0) ? (int)p.prune_q8 : (int)kNoPrune;
+            // Guided items: the row's half of the gate, once per item.  Forward row (query q): g = (a0, a1, a2, |a|^2);
+            // twin row (candidate of reference row j): g = (xj, yj, b0, b1), gn = |b|^2.
+            float g0 = 0.f, g1 = 0.f, g2 = 0.f, g3 = 0.f, gn = 0.f;
+            const float *fm = nullptr;
+            if (MODE == 2) {
+                fm = p.fmat + 9 * (pd.cand_idx >= 0 ? pd.cand_idx : wi.pair);
+                if (valid && pd.cand_idx < 0) {
+                    const float2 k = p.xy[pd.qry_off + q];
+                    g0 = epi_lin(fm[0], k.x, fm[3], k.y, fm[6]);
+                    g1 = epi_lin(fm[1], k.x, fm[4], k.y, fm[7]);
+                    g2 = epi_lin(fm[2], k.x, fm[5], k.y, fm[8]);
+                    g3 = epi_sq(g0, g1);
+                } else if (valid) {
+                    const float2 k = p.xy[p.pairs[pd.cand_idx].ref_off + p.cand_j[pd.qry_off + q]];
+                    g0 = k.x;
+                    g1 = k.y;
+                    g2 = epi_lin(fm[0], k.x, fm[1], k.y, fm[2]);
+                    g3 = epi_lin(fm[3], k.x, fm[4], k.y, fm[5]);
+                    gn = epi_sq(g2, g3);
+                }
+            }
             const int ntiles = (pd.ref_rows + TILE_N - 1) / TILE_N;
             long long acc_wait = 0, acc_load = 0, acc_p1 = 0, acc_p2 = 0, acc_hot = 0, acc_first = 0;
             int theta = prune_score(S0, S1, na, rho8, kAbsent);  // pruning score of the row, refreshed after every hot tile
@@ -471,10 +521,36 @@ match_pairs_kernel(const MatchKernelParams p) {
                                 const uint32_t *v = &acc[gq / 2][8 * (gq & 1)];
                                 const int4 c0 = ptx::lds_v4(ck + gq * 32);
                                 const int4 c1 = ptx::lds_v4(ck + gq * 32 + 16);
-                                const int key[8] = {16 * (int)v[0] + c0.x, 16 * (int)v[1] + c0.y, 16 * (int)v[2] + c0.z,
-                                                    16 * (int)v[3] + c0.w, 16 * (int)v[4] + c1.x, 16 * (int)v[5] + c1.y,
-                                                    16 * (int)v[6] + c1.z, 16 * (int)v[7] + c1.w};
+                                int key[8] = {16 * (int)v[0] + c0.x, 16 * (int)v[1] + c0.y, 16 * (int)v[2] + c0.z,
+                                              16 * (int)v[3] + c0.w, 16 * (int)v[4] + c1.x, 16 * (int)v[5] + c1.y,
+                                              16 * (int)v[6] + c1.z, 16 * (int)v[7] + c1.w};
                                 const int jb8 = jtile + gq * 8;
+                                if (MODE == 2) {
+                                    // the group's 8 column keypoints (64 bytes, L2-resident); a barred element gets the
+                                    // smallest key, whose score lies below kAbsent: it can only fill an empty slot as
+                                    // "no neighbour" and loses against every allowed element
+                                    const float4 *kp = reinterpret_cast<const float4 *>(p.xy + pd.ref_off + jb8);
+#pragma unroll
+                                    for (int h = 0; h < 4; ++h) {
+                                        const float4 c = __ldg(kp + h);
+                                        const float cx[2] = {c.x, c.z}, cy[2] = {c.y, c.w};
+#pragma unroll
+                                        for (int e = 0; e < 2; ++e) {
+                                            bool ok;
+                                            if (pd.cand_idx < 0) {  // column = reference row j
+                                                const float b0 = epi_lin(__ldg(fm + 0), cx[e], __ldg(fm + 1), cy[e], __ldg(fm + 2));
+                                                const float b1 = epi_lin(__ldg(fm + 3), cx[e], __ldg(fm + 4), cy[e], __ldg(fm + 5));
+                                                ok = epi_allowed(epi_lin(g0, cx[e], g1, cy[e], g2), g3, epi_sq(b0, b1), p.t2);
+                                            } else {                // column = query row q
+                                                const float a0 = epi_lin(__ldg(fm + 0), cx[e], __ldg(fm + 3), cy[e], __ldg(fm + 6));
+                                                const float a1 = epi_lin(__ldg(fm + 1), cx[e], __ldg(fm + 4), cy[e], __ldg(fm + 7));
+                                                const float a2 = epi_lin(__ldg(fm + 2), cx[e], __ldg(fm + 5), cy[e], __ldg(fm + 8));
+                                                ok = epi_allowed(epi_lin(a0, g0, a1, g1, a2), epi_sq(a0, a1), gn, p.t2);
+                                            }
+                                            if (!ok) key[2 * h + e] = INT_MIN;
+                                        }
+                                    }
+                                }
                                 if (MODE == 1) {
 #pragma unroll
                                     for (int i = 0; i < 8; ++i)
@@ -516,7 +592,7 @@ match_pairs_kernel(const MatchKernelParams p) {
                 atomicAdd(p.stats + 8 + 2 * quarter, (unsigned long long)acc_wait);  // per SM sub-partition
                 atomicAdd(p.stats + 9 + 2 * quarter, (unsigned long long)(acc_load + acc_p1 + acc_p2));
             }
-            if (valid && MODE == 0) {
+            if (valid && MODE != 1) {
                 if (prune_score(S0, S1, na, rho8, kAbsent) != S1) S1 = S0;  // ended dead: d1 := d0 (lower bound)
                 int4 out;
                 out.x = (S0 > kAbsent && J0 >= 0) ? (J0 ^ 7) : -1;  // low three bits hold 7 - (column mod 8), as in the packed keys;

@@ -5,6 +5,7 @@
 //   match_pairs_kernel (tcgen05)  ->  finalize_kernel  ->  scan_counts_kernel  ->  gather_matches_kernel  ->  D2H.
 // There is deliberately no CPU or non-sm_100 fallback: msfm_create fails with MSFM_ERR_UNSUPPORTED elsewhere.
 #include <algorithm>
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
@@ -122,6 +123,10 @@ struct msfm_ctx {
     int32_t knn_brute_batches = 0;  // the collect path, and batches whose event list overflowed (brute force)
     bool force_twin = false;               // msfm_test_force_twin_pass
     bool no_prune = false;                 // msfm_test_disable_pruning: the forward pass keeps exact 2-NN rows for every query row
+    DeviceBuf kp_xy;                       // msfm_match_pairs_guided: keypoints (x, y) per arena row (allocated on the first call)
+    const float *guided_f = nullptr;       // F matrices (fp32) of the current batch of a guided call, null otherwise: set per batch
+                                           // by run_match_stage (they travel in the pair-descriptor upload)
+    float guided_t2 = 0.0f;                // ... and th_epipolar^2
     DeviceBuf staging, knn, matches, good, counts, offsets, pairdesc, items, tight_matches, tight_good;
     DeviceBuf tight_matches_b, tight_good_b;  // second set: a batch's lists are copied out while the next batch is gathered
     void *h_pinned = nullptr;
@@ -334,6 +339,7 @@ struct BatchPlan {
     uint32_t prune_q8 = msfm::kNoPrune;  // forward pass: dead-row rule of the matching kernel (match_kernel.cuh); off = exact 2-NN rows
     bool has_empty = false;          // some pair has no work items: its kNN rows must read "absent"
     bool any_float = false;          // some pair has retained float rows on both sides (rescoring possible)
+    std::vector<float> fmat;         // guided call: F of every forward pair, 9 floats each (uploaded after the descriptors)
     int64_t knn_rows() const { return mutual ? 2 * query_rows : query_rows; }
 };
 
@@ -355,9 +361,18 @@ msfm_status launch_match_kernel(msfm_ctx *ctx, Pass pass, size_t first_item, siz
     kp.counts = static_cast<const int32_t *>(collect ? ctx->band_counts.ptr : ctx->twin_counts.ptr);
     // mutual twin pass: the launch returns at once unless select_candidates_kernel routed some pair to it
     kp.gate = twin ? reinterpret_cast<const unsigned int *>(static_cast<const int32_t *>(ctx->twin_counts.ptr) + ctx->twin_gate_index) : nullptr;
-    kp.events = static_cast<int4 *>(ctx->band_events.ptr);
-    kp.event_count = static_cast<unsigned int *>(ctx->band_event_count.ptr);
-    kp.event_cap = collect ? value : 0;
+    const bool guided = ctx->guided_f != nullptr && !collect;
+    if (guided) {
+        kp.xy = static_cast<const float2 *>(ctx->kp_xy.ptr);
+        kp.fmat = ctx->guided_f;
+        kp.cand_j = static_cast<const int32_t *>(ctx->cand_j.ptr);
+        kp.t2 = ctx->guided_t2;
+    } else {
+        kp.events = static_cast<int4 *>(ctx->band_events.ptr);
+        kp.event_count = static_cast<unsigned int *>(ctx->band_event_count.ptr);
+        kp.event_cap = collect ? value : 0;
+        kp.t2 = 0.0f;
+    }
     kp.pairs = static_cast<const PairDesc *>(ctx->pairdesc.ptr);
     kp.items = static_cast<const WorkItem *>(ctx->items.ptr) + first_item;
     kp.n_items = (int32_t)n_items;
@@ -368,6 +383,10 @@ msfm_status launch_match_kernel(msfm_ctx *ctx, Pass pass, size_t first_item, siz
     const int grid = std::max(1, std::min<int>(ctx->num_sms, kp.n_items));
     if (collect)
         msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, false, 1><<<grid, KCfg::kThreads, KCfg::kSmemAlloc, ctx->stream>>>(kp);
+    else if (guided && ctx->debug_flags)
+        msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, true, 2><<<grid, KCfg::kThreads, KCfg::kSmemAlloc, ctx->stream>>>(kp);
+    else if (guided)
+        msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, false, 2><<<grid, KCfg::kThreads, KCfg::kSmemAlloc, ctx->stream>>>(kp);
     else if (ctx->debug_flags)
         msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, true><<<grid, KCfg::kThreads, KCfg::kSmemAlloc, ctx->stream>>>(kp);
     else
@@ -457,7 +476,8 @@ msfm_status run_match_stage(msfm_ctx *ctx, const BatchPlan &plan) {
     msfm_status st;
     const size_t fw_bytes = plan.pairs.size() * sizeof(PairDesc);
     const size_t tw_bytes = plan.twins.size() * sizeof(PairDesc), bt_bytes = plan.band_twins.size() * sizeof(PairDesc);
-    const size_t pd_bytes = fw_bytes + tw_bytes + bt_bytes;
+    const size_t f_bytes = plan.fmat.size() * sizeof(float);
+    const size_t pd_bytes = fw_bytes + tw_bytes + bt_bytes + f_bytes;
     const size_t it_fw = plan.items.size() * sizeof(WorkItem);
     const size_t it_tw = (plan.twin_items.size() + plan.band_items.size()) * sizeof(WorkItem);
     // both parts padded to whole 16-byte words for the pull kernel
@@ -473,6 +493,8 @@ msfm_status run_match_stage(msfm_ctx *ctx, const BatchPlan &plan) {
     memcpy(hp, plan.pairs.data(), fw_bytes);
     if (tw_bytes) memcpy(hp + fw_bytes, plan.twins.data(), tw_bytes);
     if (bt_bytes) memcpy(hp + fw_bytes + tw_bytes, plan.band_twins.data(), bt_bytes);
+    if (f_bytes) memcpy(hp + fw_bytes + tw_bytes + bt_bytes, plan.fmat.data(), f_bytes);
+    ctx->guided_f = f_bytes ? reinterpret_cast<const float *>(static_cast<const char *>(ctx->pairdesc.ptr) + fw_bytes + tw_bytes + bt_bytes) : nullptr;
     memcpy(hp + pd_pad, plan.items.data(), it_fw);
     if (!plan.twin_items.empty()) memcpy(hp + pd_pad + it_fw, plan.twin_items.data(), plan.twin_items.size() * sizeof(WorkItem));
     if (!plan.band_items.empty())
@@ -693,8 +715,77 @@ int caller_sink(void *user, int64_t first, int64_t n, int32_t (**m)[2], uint8_t 
     return 0;
 }
 
+// The epipolar gate of msfm_match_pairs_guided, as the caller passed it.
+struct GuidedArgs {
+    const double (*F)[9];
+    float th;
+    const float *const *image_xy;
+    const int32_t *image_npts;
+    int32_t n_images;
+};
+
+// Everything msfm_match_pairs_guided rejects is rejected here, before any launch.  On success `fq` holds every pair's F
+// rounded to fp32.  The image ids have been checked.
+msfm_status check_guided(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pairs, const msfm_params *params, const GuidedArgs &g,
+                         std::vector<float> &fq) {
+    if (params->rescore_band != 0.0f) return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_match_pairs_guided: rescore_band must be 0");
+    if (!std::isfinite(g.th) || !(g.th > 0.0f))
+        return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_match_pairs_guided: th_epipolar %g must be finite and > 0", (double)g.th);
+    if (n_pairs == 0) return MSFM_OK;
+    if (!g.F) return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_match_pairs_guided: null F");
+    if (!g.image_xy || !g.image_npts) return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_match_pairs_guided: null image_xy / image_npts");
+    std::vector<char> checked((size_t)std::max(g.n_images, 0), 0);
+    fq.resize((size_t)n_pairs * 9);
+    for (int64_t p = 0; p < n_pairs; ++p) {
+        for (const int32_t i : {pairs[p].ref, pairs[p].query}) {
+            if (i >= g.n_images)
+                return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_match_pairs_guided: pair %lld names image %d, outside [0, n_images = %d)",
+                            (long long)p, i, g.n_images);
+            if (checked[i]) continue;
+            checked[i] = 1;
+            const int32_t rows = ctx->images[i].rows;
+            if (g.image_npts[i] != rows)
+                return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_match_pairs_guided: image %d has %d keypoints and %d uploaded rows", i,
+                            g.image_npts[i], rows);
+            if (rows > 0 && !g.image_xy[i]) return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_match_pairs_guided: image %d has no keypoints", i);
+            for (int64_t k = 0; k < 2ll * rows; ++k)
+                if (!std::isfinite(g.image_xy[i][k]))
+                    return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_match_pairs_guided: keypoint %lld of image %d is not finite", (long long)(k / 2), i);
+        }
+        bool nonzero = false;
+        for (int k = 0; k < 9; ++k) {
+            const float f = (float)g.F[p][k];  // one rounding to nearest
+            if (!std::isfinite(f))
+                return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_match_pairs_guided: F of pair %lld has a non-finite entry (in fp32)", (long long)p);
+            nonzero = nonzero || f != 0.0f;
+            fq[(size_t)p * 9 + k] = f;
+        }
+        if (!nonzero) return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_match_pairs_guided: F of pair %lld is zero", (long long)p);
+    }
+    return MSFM_OK;
+}
+
+// Keypoints of the images a guided call touches, to their arena rows of ctx->kp_xy (on the matching stream).
+msfm_status upload_keypoints(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pairs, const GuidedArgs &g) {
+    msfm_status st;
+    const bool fresh = ctx->kp_xy.ptr == nullptr;
+    if ((st = ensure(ctx, ctx->kp_xy, (size_t)ctx->arena_rows * sizeof(float2))) != MSFM_OK) return st;
+    if (fresh) MSFM_CUDA(ctx, cudaMemsetAsync(ctx->kp_xy.ptr, 0, ctx->kp_xy.bytes, ctx->stream));
+    std::vector<char> sent((size_t)g.n_images, 0);
+    for (int64_t p = 0; p < n_pairs; ++p)
+        for (const int32_t i : {pairs[p].ref, pairs[p].query}) {
+            if (sent[i] || ctx->images[i].rows == 0) continue;
+            sent[i] = 1;
+            MSFM_CUDA(ctx, cudaMemcpyAsync(static_cast<float2 *>(ctx->kp_xy.ptr) + ctx->images[i].off, g.image_xy[i],
+                                           (size_t)ctx->images[i].rows * sizeof(float2), cudaMemcpyHostToDevice, ctx->stream));
+        }
+    return MSFM_OK;
+}
+
+// msfm_match_pairs, and msfm_match_pairs_guided when `guided` is set: the same batches, with the forward and twin passes
+// of the matching kernel under the epipolar gate and every mutual pair routed to the twin pass.
 msfm_status match_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pairs, const msfm_params *params, const OutSpec *out,
-                             bool resident, int64_t *n_matches_total) {
+                             bool resident, int64_t *n_matches_total, const GuidedArgs *guided = nullptr) {
     if (!ctx) return MSFM_ERR_INVALID_ARG;
     std::lock_guard<std::mutex> lock(ctx->mu);
     if (n_pairs < 0 || (n_pairs > 0 && !pairs) || !params) return fail(ctx, MSFM_ERR_INVALID_ARG, "null pair list / params or negative n_pairs");
@@ -703,9 +794,15 @@ msfm_status match_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pa
     if (!(params->ratio > 0.0f)) return fail(ctx, MSFM_ERR_INVALID_ARG, "ratio must be > 0");
     msfm_status st;
     if ((st = check_pairs(ctx, pairs, n_pairs)) != MSFM_OK) return st;
+    std::vector<float> fq;  // guided: F of every pair in fp32
+    if (guided && (st = check_guided(ctx, pairs, n_pairs, params, *guided, fq)) != MSFM_OK) return st;
     ctx->timing = msfm_timing{};
     DrainListCopy drain_list_copy{ctx};
     MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_begin, ctx->stream));
+    if (guided) {
+        if ((st = upload_keypoints(ctx, pairs, n_pairs, *guided)) != MSFM_OK) return st;
+        ctx->guided_t2 = guided->th * guided->th;
+    }
     const bool mutual = params->mutual != 0;
     const bool want_good = params->ratio_good > 0.0f && (resident || out->has_good);
     const int64_t max_rows = mutual ? kBatchMaxQueryRowsMutual : kBatchMaxQueryRows;
@@ -744,6 +841,7 @@ msfm_status match_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pa
                 const uint64_t need = std::max(r.ready_seq, q.ready_seq);
                 if (!c.plan.pairs.empty() && need > c.plan.need_seq && !uploads_landed(ctx, need)) break;
                 plan_add_pair(ctx, c.plan, next, pairs[next].ref, pairs[next].query);
+                if (guided) c.plan.fmat.insert(c.plan.fmat.end(), fq.begin() + 9 * next, fq.begin() + 9 * (next + 1));
             }
             ++next;
         }
@@ -821,7 +919,7 @@ msfm_status match_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pa
             sp.counts = static_cast<int32_t *>(ctx->cand_counts.ptr);
             sp.float_mutual = (mutual && float_rescoring) ? 1 : 0;
             sp.mutual = mutual ? 1 : 0;
-            sp.force_twin = ctx->force_twin ? 1 : 0;
+            sp.force_twin = (ctx->force_twin || guided) ? 1 : 0;  // the forward-result check is not proven under a gate
             sp.colbest = static_cast<unsigned long long *>(ctx->colbest.ptr);
             sp.smem_table_rows = msfm::kSmemTableRows;
             sp.danger = static_cast<int2 *>(ctx->matches.ptr);  // the match scratch is written by the emission afterwards
@@ -1157,6 +1255,10 @@ msfm_status msfm_create(const msfm_config *cfg, msfm_ctx **out) {
                              cudaFuncAttributeMaxDynamicSharedMemorySize, KCfg::kSmemAlloc) != cudaSuccess ||
         cudaFuncSetAttribute(msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, false, 1>,
                              cudaFuncAttributeMaxDynamicSharedMemorySize, KCfg::kSmemAlloc) != cudaSuccess ||
+        cudaFuncSetAttribute(msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, false, 2>,
+                             cudaFuncAttributeMaxDynamicSharedMemorySize, KCfg::kSmemAlloc) != cudaSuccess ||
+        cudaFuncSetAttribute(msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, true, 2>,
+                             cudaFuncAttributeMaxDynamicSharedMemorySize, KCfg::kSmemAlloc) != cudaSuccess ||
         cudaFuncSetAttribute(msfm::select_candidates_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msfm::kSelectSmemBytes) != cudaSuccess)
         return bail(MSFM_ERR_CUDA);
     if (ctx->debug_flags & 8u) {
@@ -1201,7 +1303,7 @@ msfm_status msfm_destroy(msfm_ctx *ctx) {
     if (ctx->resid) cudaFree(ctx->resid);
     if (ctx->img_rmax) cudaFree(ctx->img_rmax);
     DeviceBuf *bufs[] = {&ctx->knn_ids, &ctx->knn_dists, &ctx->knn_ids_b, &ctx->knn_dists_b, &ctx->band_q, &ctx->band_counts, &ctx->band_thr, &ctx->band_state, &ctx->band_events, &ctx->band_event_keys, &ctx->band_event_count, &ctx->cand_q, &ctx->cand_j, &ctx->cand_d0, &ctx->cand_good, &ctx->cand_counts, &ctx->cand_desc, &ctx->cand_ckeys, &ctx->colbest, &ctx->twin_counts, &ctx->tilemin,
-                         &ctx->staging, &ctx->knn, &ctx->matches, &ctx->good, &ctx->counts, &ctx->offsets,
+                         &ctx->kp_xy, &ctx->staging, &ctx->knn, &ctx->matches, &ctx->good, &ctx->counts, &ctx->offsets,
                          &ctx->pairdesc, &ctx->items, &ctx->tight_matches, &ctx->tight_good, &ctx->tight_matches_b, &ctx->tight_good_b};
     for (DeviceBuf *b : bufs)
         if (b->ptr) cudaFree(b->ptr);
@@ -1659,6 +1761,23 @@ msfm_status msfm_match_pairs(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pa
     spec.sink = caller_sink;
     spec.user = &cb;
     return match_pairs_impl(ctx, pairs, n_pairs, params, &spec, false, nullptr);
+}
+
+msfm_status msfm_match_pairs_guided(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pairs, const msfm_params *params,
+                                    const double (*F)[9], float th_epipolar, const float *const *image_xy,
+                                    const int32_t *image_npts, int32_t n_images, msfm_result *out) {
+    if (!ctx) return MSFM_ERR_INVALID_ARG;
+    if (cudaSetDevice(ctx->device) != cudaSuccess) return MSFM_ERR_CUDA;
+    const GuidedArgs g{F, th_epipolar, image_xy, image_npts, n_images};
+    if (!out || (!out->matches && out->match_capacity > 0)) return match_pairs_impl(ctx, pairs, n_pairs, params, nullptr, false, nullptr, &g);
+    CallerBuffers cb{out->matches, out->good, out->match_capacity};
+    OutSpec spec;
+    spec.offsets = out->offsets;
+    spec.ok = out->ok;
+    spec.has_good = out->good != nullptr;
+    spec.sink = caller_sink;
+    spec.user = &cb;
+    return match_pairs_impl(ctx, pairs, n_pairs, params, &spec, false, nullptr, &g);
 }
 
 msfm_status msfm_internal_match_pairs_sink(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pairs, const msfm_params *params, int64_t *offsets,

@@ -318,6 +318,18 @@ bool MatchGraphB200::ReleaseImage(int idx) {
 
 bool MatchGraphB200::MatchPairs(const std::vector<std::vector<int>> &match_graph_init, std::vector<std::vector<PairMatches>> &out,
                                 float th_good, float th_all, bool mutual, int th_reject) {
+    return Match(match_graph_init, nullptr, out, th_good, th_all, mutual, th_reject);
+}
+
+bool MatchGraphB200::MatchPairsGuided(const std::vector<std::vector<int>> &match_graph_init, const std::vector<std::array<double, 9>> &F,
+                                      const std::vector<std::vector<cv::KeyPoint>> &keypoints, float th_epipolar,
+                                      std::vector<std::vector<PairMatches>> &out, float th_good, float th_all, bool mutual, int th_reject) {
+    const Guide g = {&F, &keypoints, th_epipolar};
+    return Match(match_graph_init, &g, out, th_good, th_all, mutual, th_reject);
+}
+
+bool MatchGraphB200::Match(const std::vector<std::vector<int>> &match_graph_init, const Guide *guide, std::vector<std::vector<PairMatches>> &out,
+                           float th_good, float th_all, bool mutual, int th_reject) {
     if (!ctx_) return false;
     std::vector<msfm_pair> pairs;
     long long capacity = 0;
@@ -350,7 +362,31 @@ bool MatchGraphB200::MatchPairs(const std::vector<std::vector<int>> &match_graph
     res.matches = reinterpret_cast<int32_t(*)[2]>(buf.data());
     res.good = good.data();
     res.match_capacity = capacity;
-    msfm_status st = msfm_match_pairs(ctx_, pairs.data(), (int64_t)pairs.size(), &prm, &res);
+    msfm_status st;
+    if (guide) {
+        if (guide->F->size() != pairs.size()) {
+            err_ = "MatchPairsGuided needs one F per pair";
+            return false;
+        }
+        // keypoints as the library takes them: (x, y) per descriptor row, one array per image
+        const size_t n_images = rows_.size();
+        std::vector<std::vector<float>> xy(n_images);
+        std::vector<const float *> xy_ptr(n_images, nullptr);
+        std::vector<int32_t> npts(n_images, 0);
+        for (size_t i = 0; i < n_images && i < guide->keypoints->size(); ++i) {
+            const std::vector<cv::KeyPoint> &kp = (*guide->keypoints)[i];
+            for (const cv::KeyPoint &k : kp) {
+                xy[i].push_back(k.pt.x);
+                xy[i].push_back(k.pt.y);
+            }
+            xy_ptr[i] = xy[i].data();
+            npts[i] = (int32_t)kp.size();
+        }
+        st = msfm_match_pairs_guided(ctx_, pairs.data(), (int64_t)pairs.size(), &prm, reinterpret_cast<const double(*)[9]>(guide->F->data()),
+                                     guide->th, xy_ptr.data(), npts.data(), (int32_t)n_images, &res);
+    } else {
+        st = msfm_match_pairs(ctx_, pairs.data(), (int64_t)pairs.size(), &prm, &res);
+    }
     if (st != MSFM_OK) {
         err_ = msfm_last_error(ctx_);
         return false;

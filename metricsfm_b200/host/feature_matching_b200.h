@@ -16,6 +16,7 @@
 //
 // Everything here is a thin marshalling layer: all arithmetic runs in the CUDA library behind msfm_match.h.
 #pragma once
+#include <array>
 #include <string>
 #include <utility>
 #include <vector>
@@ -172,8 +173,24 @@ public:
     // match_graph_init[idx1] = partner list, as produced by InitialMatchingGraph (initial_matching_graph.h:64).
     bool MatchPairs(const std::vector<std::vector<int>> &match_graph_init, std::vector<std::vector<PairMatches>> &out,
                     float th_good = 0.6f, float th_all = 0.85f, bool mutual = false, int th_reject = 20);
+    // Guided re-matching of verified pairs (msfm_match_pairs_guided, GUIDED-SPEC in msfm_match.h): MatchPairs with every
+    // row's two nearest neighbours searched only among the keypoints within th_epipolar pixels of the pair's epipolar
+    // geometry.  F[k] belongs to the k-th pair of match_graph_init in order (row-major, p2^T F p1 = 0 for a keypoint p1 of
+    // idx1 and p2 of idx2: what msfm_geo_verify returns); keypoints[idx] holds one keypoint per descriptor row of image
+    // idx, in the centred coordinates of the feature files.
+    bool MatchPairsGuided(const std::vector<std::vector<int>> &match_graph_init, const std::vector<std::array<double, 9>> &F,
+                          const std::vector<std::vector<cv::KeyPoint>> &keypoints, float th_epipolar,
+                          std::vector<std::vector<PairMatches>> &out, float th_good = 0.6f, float th_all = 0.85f,
+                          bool mutual = false, int th_reject = 20);
 
 private:
+    struct Guide {  // the epipolar gate of MatchPairsGuided
+        const std::vector<std::array<double, 9>> *F;
+        const std::vector<std::vector<cv::KeyPoint>> *keypoints;
+        float th;
+    };
+    bool Match(const std::vector<std::vector<int>> &match_graph_init, const Guide *guide, std::vector<std::vector<PairMatches>> &out,
+               float th_good, float th_all, bool mutual, int th_reject);
     msfm_ctx *ctx_ = nullptr;
     float scale_;
     std::vector<int> rows_;

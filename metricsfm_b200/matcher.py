@@ -289,6 +289,15 @@ class Matcher:
         band of a threshold are decided on exact fp32 distances."""
         pa = self._pairs(pairs)
         n = pa.shape[0]
+        out, res = self._result_buffers(pa, ratio_good, capacity, out)
+        prm = self._params(ratio, ratio_good, max_dist_sq, mutual, min_keypoints, orientation, rescore_band, flags)
+        self._check(self._L.msfm_match_pairs(self._h, pa.ctypes.data, n, C.byref(prm), C.byref(res)))
+        total = int(out.offsets[n])
+        return MatchResult(out.offsets, out.ok, out.matches[:total], out.good[:total] if out.good is not None else None)
+
+    def _result_buffers(self, pa: np.ndarray, ratio_good: float, capacity: int | None, out: MatchResult | None):
+        """(MatchResult, msfm_result) over the caller's `out` or new buffers with room for one match per query row."""
+        n = pa.shape[0]
         if out is None:
             if capacity is None:
                 capacity = 0
@@ -307,8 +316,39 @@ class Matcher:
         res.matches = _host_ptr(out.matches)[0]
         res.good = out.good.ctypes.data_as(_lib._u8p) if out.good is not None else None
         res.match_capacity = out.matches.shape[0]
-        prm = self._params(ratio, ratio_good, max_dist_sq, mutual, min_keypoints, orientation, rescore_band, flags)
-        self._check(self._L.msfm_match_pairs(self._h, pa.ctypes.data, n, C.byref(prm), C.byref(res)))
+        return out, res
+
+    @staticmethod
+    def _keypoint_table(image_xy: dict, n_images: int):
+        """(pointer array, point counts, keepalive) of {image id: [n, 2] float32 keypoints} for ids < n_images."""
+        xy_keep, ptrs, npts = [], (C.c_void_p * max(n_images, 1))(), np.zeros((max(n_images, 1),), np.int32)
+        for i, xy in image_xy.items():
+            if i < n_images:
+                a = np.ascontiguousarray(xy, np.float32).reshape(-1, 2)
+                xy_keep.append(a)
+                ptrs[i] = a.ctypes.data
+                npts[i] = a.shape[0]
+        return ptrs, npts, xy_keep
+
+    def match_pairs_guided(self, pairs, F, image_xy: dict, *, th_epipolar: float = 3.0, ratio: float = 0.6,
+                           ratio_good: float = 0.0, max_dist_sq: float = 0.0, mutual: bool = False, min_keypoints: int = 20,
+                           orientation: int = 0, flags: int = 0, capacity: int | None = None) -> MatchResult:
+        """msfm_match_pairs_guided (GUIDED-SPEC in include/msfm_match.h): match_pairs with every query row's 2-NN searched
+        only among the reference keypoints within th_epipolar pixels of the pair's epipolar geometry.  F: [n, 3, 3]
+        float64 as geo_verify returns it (p_query^T F p_ref = 0); image_xy: {image id: [rows, 2] float32 centred
+        keypoints}, one per descriptor row of every image the pairs touch."""
+        pa = self._pairs(pairs)
+        n = pa.shape[0]
+        Fa = np.ascontiguousarray(F, np.float64).reshape(-1, 9)
+        if Fa.shape[0] != n:
+            raise ValueError(f"F must hold one 3x3 matrix per pair: {Fa.shape[0]} for {n} pairs")
+        n_images = int(pa.max()) + 1 if n else 0
+        ptrs, npts, xy_keep = self._keypoint_table(image_xy, n_images)
+        out, res = self._result_buffers(pa, ratio_good, capacity, None)
+        prm = self._params(ratio, ratio_good, max_dist_sq, mutual, min_keypoints, orientation, 0.0, flags)
+        self._check(self._L.msfm_match_pairs_guided(self._h, pa.ctypes.data, n, C.byref(prm), Fa.ctypes.data, th_epipolar,
+                                                    C.cast(ptrs, C.c_void_p), npts.ctypes.data, n_images, C.byref(res)))
+        del xy_keep
         total = int(out.offsets[n])
         return MatchResult(out.offsets, out.ok, out.matches[:total], out.good[:total] if out.good is not None else None)
 
@@ -333,13 +373,7 @@ class Matcher:
         pa = self._pairs(pairs)
         n = pa.shape[0]
         n_images = int(pa.max()) + 1 if n else 0
-        xy_keep, ptrs, npts = [], (C.c_void_p * max(n_images, 1))(), np.zeros((max(n_images, 1),), np.int32)
-        for i, xy in image_xy.items():
-            if i < n_images:
-                a = np.ascontiguousarray(xy, np.float32).reshape(-1, 2)
-                xy_keep.append(a)
-                ptrs[i] = a.ctypes.data
-                npts[i] = a.shape[0]
+        ptrs, npts, xy_keep = self._keypoint_table(image_xy, n_images)
         gp = _lib.GeoParams(th_epipolar, min_points, min_inliers, iters, seed, pair_index_base)
         total = int(result.offsets[n])
         ok = np.zeros((max(n, 1),), np.int32)
