@@ -50,6 +50,15 @@
  *   fewer than two allowed rows gets id -1 / +inf and is rejected.  Ratio, ratio_good, max_dist_sq, MSFM_RATIO_REJECT_GT,
  *   orientation and the min_keypoints gate (on the images' rows) are those of MATCH-SPEC; the mutual check keeps
  *   (q, nn0) iff q is the closest allowed query row of nn0 (lowest index on ties).
+ *   Float regime under the gate (rescore_band > 0 on a keep_float context, pairs whose images both keep float rows at
+ *   one scale; every other pair follows the integer rule above): a query row is a band row when both of its gated
+ *   quantised neighbours exist and fl(d0/d1) lies within ratio*(1 +- band) or ratio_good*(1 +- band) (the rule of
+ *   msfm_params.rescore_band applied to the guided 2-NN).  A band row is decided on its exact fp32 top-2 (b0, b1) among
+ *   the allowed reference rows, with the arithmetic of the float regime: squared L2 accumulated in index order with
+ *   separate multiply and add, lowest index on ties; the ratio tests on fl(b0/b1), max_dist_sq on fl(b0*fl(s*s)), the
+ *   match on the fp32 nearest allowed row.  Every other row keeps the integer guided decision; the allowed set is the
+ *   same in both arithmetics, so a row with fewer than two allowed rows is never a band row and stays rejected.  With
+ *   mutual = 1 the check is the float regime's heuristic filter of the one-way list, under the gate (not exact in fp32).
  */
 #ifndef MSFM_MATCH_H_
 #define MSFM_MATCH_H_
@@ -302,7 +311,9 @@ msfm_status msfm_geo_ransac(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pai
  * Errors (before any launch): the statuses of msfm_match_pairs, and INVALID_ARG (the message names the pair or image)
  * for a null F, image_xy or image_npts; a pair naming an image >= n_images; a touched image without keypoints, with
  * image_npts different from its uploaded rows, or with a non-finite coordinate; an F with a non-finite entry or that
- * is zero after rounding to fp32; th_epipolar not finite or not > 0; rescore_band != 0 (no float regime under a gate). */
+ * is zero after rounding to fp32; th_epipolar not finite or not > 0; rescore_band negative or not finite, or > 0 on a
+ * context without retained float rows (keep_float = 0).  rescore_band > 0 on a keep_float context: the float regime
+ * under the gate (GUIDED-SPEC). */
 msfm_status msfm_match_pairs_guided(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pairs, const msfm_params *params,
                                     const double (*F)[9], float th_epipolar,
                                     const float *const *image_xy, const int32_t *image_npts, int32_t n_images,
@@ -311,10 +322,12 @@ msfm_status msfm_match_pairs_guided(msfm_ctx *ctx, const msfm_pair *pairs, int64
 /* ---- GPU-side cross-check kernel (CUDA cores, dp4a); used by the tests to localise faults, never by the fast path */
 msfm_status msfm_knn2_crosscheck(msfm_ctx *ctx, int32_t ref_id, int32_t query_id, int32_t *ids, float *dists);
 /* Test hook: capacity of the float regime's event list (-1 = default sizing; 0 forces the brute-force fallback).
- * Applies to msfm_match_pairs' rescore_band and to msfm_knn2_pairs' MSFM_KNN_EXACT_F32 alike. */
+ * Applies to the rescore_band of msfm_match_pairs and msfm_match_pairs_guided and to msfm_knn2_pairs'
+ * MSFM_KNN_EXACT_F32 alike. */
 msfm_status msfm_test_set_band_event_cap(msfm_ctx *ctx, int64_t cap);
-/* Test hook: for the last MSFM_KNN_EXACT_F32 call of msfm_knn2_pairs or the last msfm_match_pairs call with
- * rescore_band > 0 on a keep_float context, whichever came later, the events the collect path scored and the batches
+/* Test hook: for the last MSFM_KNN_EXACT_F32 call of msfm_knn2_pairs or the last msfm_match_pairs /
+ * msfm_match_pairs_guided call with rescore_band > 0 on a keep_float context, whichever came later, the events the
+ * collect path scored (in a guided call: only elements the gate allows) and the batches
  * whose event list overflowed, i.e. that the brute force decided.  Either pointer may be NULL. */
 msfm_status msfm_test_last_knn_stats(msfm_ctx *ctx, int64_t *events, int32_t *brute_force_batches);
 /* Test hook: 1 routes every pair's mutual check through the tensor twin pass (the fallback of the bound-based check). */

@@ -23,7 +23,7 @@
 //   over the B ring (immediate addresses) and they sleep between polls (see the comment at the role dispatch).
 // MODE 1 ("collect", float regime) replaces the top-2 merge by "append every element under the row's fixed threshold
 // to an event list"; MODE 2 ("guided") bars the elements that fail an epipolar gate from the top-2 in the exact phase;
-// everything else is shared.
+// MODE 3 is MODE 1 under MODE 2's gate (band rows of a guided call); everything else is shared.
 // Work distribution: CTA b takes items b, b + grid, ...; every role walks that list on its own.
 // Pipelines (all mbarrier based):
 //   A ring (2 deep)     : query strips of a work item, STRIPS x [128 rows x 128 B]
@@ -87,11 +87,27 @@ struct MatchKernelParams {
     const PairDesc *pairs;
     const WorkItem *items;
     int32_t n_items;
-    uint32_t debug_flags;         // timing experiments only (results are wrong): 1 = skip the exact phase,
+    // MODE 3 ("collect under the gate", float regime of msfm_match_pairs_guided): MODE 1's event append restricted to the
+    // elements that pass the epipolar gate, which runs in the exact phase as in MODE 2.  Item of band twin d (cand_idx =
+    // p): row = band row q of forward pair p (scratch row qry_off + q), at the keypoint of its query row
+    // band_q[qry_off + q]; columns = p's reference rows; F = row p of the F table.  MODE 3 needs the event fields and
+    // the gate at once, and the block cannot grow: past 128 bytes nvcc addresses the parameter block through a pointer
+    // and the code of every mode changes.  So its three gate fields share the slots of fields that only the debug build
+    // (debug_flags, stats) or the kNN output (knn) reads, neither of which MODE 3 has.
+    union {
+        uint32_t debug_flags;     // timing experiments only (results are wrong): 1 = skip the exact phase,
                                   // 2 = no epilogue work at all, 4 = TMEM loads + hand-back only
-    unsigned long long *stats;    // optional debug counter (slow-path group visits); null in production
-    int4 *knn;                    // [sum qry_rows] {id0, id1, d0, d1} per query row; id = -1 / d = INT_MAX when absent;
+        uint32_t gate_f_desc;     // MODE 3: the F table ([forward pairs][9] fp32) starts after this many PairDescs of `pairs`
+    };
+    union {
+        unsigned long long *stats;  // optional debug counter (slow-path group visits); null in production
+        const float2 *gate_xy;      // MODE 3: keypoints (x, y), indexed like the column-key arena
+    };
+    union {
+        int4 *knn;                // [sum qry_rows] {id0, id1, d0, d1} per query row; id = -1 / d = INT_MAX when absent;
                                   // consumers read it with load_knn()
+        const int32_t *band_q;    // MODE 3: [forward kNN rows] query row of every band row (mark_band_kernel)
+    };
     // MODE 1 ("collect", float regime): instead of a top-2 the kernel lists every (query row, reference row) whose
     // squared distance is <= cand_d0[row], as {scratch row, reference row, cand_idx, 0}.
     // MODE 2 ("guided", msfm_match_pairs_guided): only elements that pass the epipolar gate (epi_allowed) can enter a
@@ -115,7 +131,7 @@ struct MatchKernelParams {
     uint32_t prune_q8;            // "dead row" rule of the forward pass (see the epilogue): a row whose two nearest neighbours
                                   // so far satisfy d0 > (prune_q8 / 256) * d1 only follows its NEAREST neighbour exactly.
                                   // kNoPrune = off (exact 2-NN of every row: msfm_knn2, twin and collect passes)
-    float t2;                     // MODE 2: th_epipolar^2, rounded to fp32
+    float t2;                     // MODE 2 and 3: th_epipolar^2, rounded to fp32
 };
 constexpr uint32_t kNoPrune = 4096;  // ((d1 >> 8) + 1) * 4096 >= 16 * d1 > d0 for every row, and fits in 32 bits (d < 2^25)
 
@@ -439,7 +455,7 @@ match_pairs_kernel(const MatchKernelParams p) {
             // which is what the mutual check's dangerous-row bound needs (select_candidates_kernel).
             // Under the epipolar gate (MODE 2) the rule stays on: it only reasons about elements that can enter the row's
             // top-2, and the gate only removes elements (barred ones never reach the running state).
-            const int rho8 = (MODE != 1 && pd.cand_idx < 0) ? (int)p.prune_q8 : (int)kNoPrune;
+            const int rho8 = (MODE != 1 && MODE != 3 && pd.cand_idx < 0) ? (int)p.prune_q8 : (int)kNoPrune;
             // Guided items: the row's half of the gate, once per item.  Forward row (query q): g = (a0, a1, a2, |a|^2);
             // twin row (candidate of reference row j): g = (xj, yj, b0, b1), gn = |b|^2.
             float g0 = 0.f, g1 = 0.f, g2 = 0.f, g3 = 0.f, gn = 0.f;
@@ -459,6 +475,17 @@ match_pairs_kernel(const MatchKernelParams p) {
                     g2 = epi_lin(fm[0], k.x, fm[1], k.y, fm[2]);
                     g3 = epi_lin(fm[3], k.x, fm[4], k.y, fm[5]);
                     gn = epi_sq(g2, g3);
+                }
+            } else if (MODE == 3) {
+                // band row: the same four values as its query row's forward item (bit for bit, so the allowed set of the
+                // row is the one its gated quantised 2-NN, and hence its threshold T(q), came from)
+                fm = reinterpret_cast<const float *>(p.pairs + p.gate_f_desc) + 9 * pd.cand_idx;
+                if (valid) {
+                    const float2 k = p.gate_xy[p.pairs[pd.cand_idx].qry_off + p.band_q[pd.qry_off + q]];
+                    g0 = epi_lin(fm[0], k.x, fm[3], k.y, fm[6]);
+                    g1 = epi_lin(fm[1], k.x, fm[4], k.y, fm[7]);
+                    g2 = epi_lin(fm[2], k.x, fm[5], k.y, fm[8]);
+                    g3 = epi_sq(g0, g1);
                 }
             }
             const int ntiles = (pd.ref_rows + TILE_N - 1) / TILE_N;
@@ -525,11 +552,12 @@ match_pairs_kernel(const MatchKernelParams p) {
                                               16 * (int)v[3] + c0.w, 16 * (int)v[4] + c1.x, 16 * (int)v[5] + c1.y,
                                               16 * (int)v[6] + c1.z, 16 * (int)v[7] + c1.w};
                                 const int jb8 = jtile + gq * 8;
-                                if (MODE == 2) {
+                                if (MODE == 2 || MODE == 3) {
                                     // the group's 8 column keypoints (64 bytes, L2-resident); a barred element gets the
                                     // smallest key, whose score lies below kAbsent: it can only fill an empty slot as
-                                    // "no neighbour" and loses against every allowed element
-                                    const float4 *kp = reinterpret_cast<const float4 *>(p.xy + pd.ref_off + jb8);
+                                    // "no neighbour" and loses against every allowed element (MODE 3: it lies below
+                                    // every row's collect threshold and is never listed)
+                                    const float4 *kp = reinterpret_cast<const float4 *>((MODE == 3 ? p.gate_xy : p.xy) + pd.ref_off + jb8);
 #pragma unroll
                                     for (int h = 0; h < 4; ++h) {
                                         const float4 c = __ldg(kp + h);
@@ -537,7 +565,7 @@ match_pairs_kernel(const MatchKernelParams p) {
 #pragma unroll
                                         for (int e = 0; e < 2; ++e) {
                                             bool ok;
-                                            if (pd.cand_idx < 0) {  // column = reference row j
+                                            if (MODE == 3 || pd.cand_idx < 0) {  // column = reference row j
                                                 const float b0 = epi_lin(__ldg(fm + 0), cx[e], __ldg(fm + 1), cy[e], __ldg(fm + 2));
                                                 const float b1 = epi_lin(__ldg(fm + 3), cx[e], __ldg(fm + 4), cy[e], __ldg(fm + 5));
                                                 ok = epi_allowed(epi_lin(g0, cx[e], g1, cy[e], g2), g3, epi_sq(b0, b1), p.t2);
@@ -551,7 +579,7 @@ match_pairs_kernel(const MatchKernelParams p) {
                                         }
                                     }
                                 }
-                                if (MODE == 1) {
+                                if (MODE == 1 || MODE == 3) {
 #pragma unroll
                                     for (int i = 0; i < 8; ++i)
                                         if ((key[i] >> 3) > S1) {
@@ -592,7 +620,7 @@ match_pairs_kernel(const MatchKernelParams p) {
                 atomicAdd(p.stats + 8 + 2 * quarter, (unsigned long long)acc_wait);  // per SM sub-partition
                 atomicAdd(p.stats + 9 + 2 * quarter, (unsigned long long)(acc_load + acc_p1 + acc_p2));
             }
-            if (valid && MODE != 1) {
+            if (valid && MODE != 1 && MODE != 3) {
                 if (prune_score(S0, S1, na, rho8, kAbsent) != S1) S1 = S0;  // ended dead: d1 := d0 (lower bound)
                 int4 out;
                 out.x = (S0 > kAbsent && J0 >= 0) ? (J0 ^ 7) : -1;  // low three bits hold 7 - (column mod 8), as in the packed keys;

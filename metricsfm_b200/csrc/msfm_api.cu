@@ -347,7 +347,7 @@ struct BatchPlan {
 //   forward  2-NN of the forward pairs' query rows, with the dead-row rule `value` (prune_q8)
 //   twin     2-NN of the mutual twins' candidate rows, skipped on the device unless select_candidates_kernel routed a pair
 //   collect  the items are band twins: every reference row within band_thr of a band row is appended to the event list,
-//            which holds `value` events
+//            which holds `value` events; in a guided call only the rows the epipolar gate allows
 enum class Pass { forward, twin, collect };
 
 msfm_status launch_match_kernel(msfm_ctx *ctx, Pass pass, size_t first_item, size_t n_items, uint32_t value = 0) {
@@ -361,27 +361,35 @@ msfm_status launch_match_kernel(msfm_ctx *ctx, Pass pass, size_t first_item, siz
     kp.counts = static_cast<const int32_t *>(collect ? ctx->band_counts.ptr : ctx->twin_counts.ptr);
     // mutual twin pass: the launch returns at once unless select_candidates_kernel routed some pair to it
     kp.gate = twin ? reinterpret_cast<const unsigned int *>(static_cast<const int32_t *>(ctx->twin_counts.ptr) + ctx->twin_gate_index) : nullptr;
-    const bool guided = ctx->guided_f != nullptr && !collect;
-    if (guided) {
+    // a guided call's collect pass lists only the elements its gate allows (MODE 3)
+    const bool guided = ctx->guided_f != nullptr;
+    if (guided && !collect) {
         kp.xy = static_cast<const float2 *>(ctx->kp_xy.ptr);
         kp.fmat = ctx->guided_f;
         kp.cand_j = static_cast<const int32_t *>(ctx->cand_j.ptr);
-        kp.t2 = ctx->guided_t2;
     } else {
         kp.events = static_cast<int4 *>(ctx->band_events.ptr);
         kp.event_count = static_cast<unsigned int *>(ctx->band_event_count.ptr);
         kp.event_cap = collect ? value : 0;
-        kp.t2 = 0.0f;
     }
+    kp.t2 = guided ? ctx->guided_t2 : 0.0f;
     kp.pairs = static_cast<const PairDesc *>(ctx->pairdesc.ptr);
     kp.items = static_cast<const WorkItem *>(ctx->items.ptr) + first_item;
     kp.n_items = (int32_t)n_items;
-    kp.stats = static_cast<unsigned long long *>(ctx->dbg_stats.ptr);  // null unless MSFM_DEBUG_FLAGS & 8
-    kp.debug_flags = ctx->debug_flags;
-    kp.knn = static_cast<int4 *>(ctx->knn.ptr);
+    if (guided && collect) {  // MODE 3: the gate's fields in the slots of the debug and kNN fields (match_kernel.cuh)
+        kp.gate_f_desc = (uint32_t)((ctx->guided_f - static_cast<const float *>(ctx->pairdesc.ptr)) * sizeof(float) / sizeof(PairDesc));
+        kp.gate_xy = static_cast<const float2 *>(ctx->kp_xy.ptr);
+        kp.band_q = static_cast<const int32_t *>(ctx->band_q.ptr);
+    } else {
+        kp.stats = static_cast<unsigned long long *>(ctx->dbg_stats.ptr);  // null unless MSFM_DEBUG_FLAGS & 8
+        kp.debug_flags = ctx->debug_flags;
+        kp.knn = static_cast<int4 *>(ctx->knn.ptr);
+    }
     kp.prune_q8 = (pass == Pass::forward && !ctx->no_prune) ? value : msfm::kNoPrune;
     const int grid = std::max(1, std::min<int>(ctx->num_sms, kp.n_items));
-    if (collect)
+    if (collect && guided)
+        msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, false, 3><<<grid, KCfg::kThreads, KCfg::kSmemAlloc, ctx->stream>>>(kp);
+    else if (collect)
         msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, false, 1><<<grid, KCfg::kThreads, KCfg::kSmemAlloc, ctx->stream>>>(kp);
     else if (guided && ctx->debug_flags)
         msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, true, 2><<<grid, KCfg::kThreads, KCfg::kSmemAlloc, ctx->stream>>>(kp);
@@ -667,7 +675,12 @@ msfm_status run_collect_pass(msfm_ctx *ctx, const BatchPlan &plan, const msfm::B
     msfm::finish_band_kernel<<<nb, 256, 0, ctx->stream>>>(bp);
     const int gx = std::min(nb, 4 * ctx->num_sms);
     const int gy = std::max(1, std::min(32, (4 * ctx->num_sms + gx - 1) / gx));
-    msfm::rescore_band_kernel<<<dim3(gx, gy), 256, 0, ctx->stream>>>(bp, nb);
+    // a guided batch: the brute force applies the gate as the collect pass does (launch_match_kernel)
+    if (ctx->guided_f)
+        msfm::rescore_band_kernel<true><<<dim3(gx, gy), 256, 0, ctx->stream>>>(
+            bp, nb, msfm::BandGate{static_cast<const float2 *>(ctx->kp_xy.ptr), ctx->guided_f, ctx->guided_t2});
+    else
+        msfm::rescore_band_kernel<false><<<dim3(gx, gy), 256, 0, ctx->stream>>>(bp, nb, msfm::BandGate{nullptr, nullptr, 0.0f});
     MSFM_CUDA(ctx, cudaGetLastError());
     ctx->timing.total_launches += 4;
     return MSFM_OK;
@@ -728,7 +741,10 @@ struct GuidedArgs {
 // rounded to fp32.  The image ids have been checked.
 msfm_status check_guided(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pairs, const msfm_params *params, const GuidedArgs &g,
                          std::vector<float> &fq) {
-    if (params->rescore_band != 0.0f) return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_match_pairs_guided: rescore_band must be 0");
+    if (!std::isfinite(params->rescore_band) || params->rescore_band < 0.0f)
+        return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_match_pairs_guided: rescore_band %g must be finite and >= 0", (double)params->rescore_band);
+    if (params->rescore_band > 0.0f && !ctx->fdesc)
+        return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_match_pairs_guided: rescore_band > 0 needs a keep_float context (retained float rows)");
     if (!std::isfinite(g.th) || !(g.th > 0.0f))
         return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_match_pairs_guided: th_epipolar %g must be finite and > 0", (double)g.th);
     if (n_pairs == 0) return MSFM_OK;
@@ -1258,6 +1274,8 @@ msfm_status msfm_create(const msfm_config *cfg, msfm_ctx **out) {
         cudaFuncSetAttribute(msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, false, 2>,
                              cudaFuncAttributeMaxDynamicSharedMemorySize, KCfg::kSmemAlloc) != cudaSuccess ||
         cudaFuncSetAttribute(msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, true, 2>,
+                             cudaFuncAttributeMaxDynamicSharedMemorySize, KCfg::kSmemAlloc) != cudaSuccess ||
+        cudaFuncSetAttribute(msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, false, 3>,
                              cudaFuncAttributeMaxDynamicSharedMemorySize, KCfg::kSmemAlloc) != cudaSuccess ||
         cudaFuncSetAttribute(msfm::select_candidates_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msfm::kSelectSmemBytes) != cudaSuccess)
         return bail(MSFM_ERR_CUDA);

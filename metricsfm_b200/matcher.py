@@ -247,7 +247,7 @@ class Matcher:
 
     def _test_last_knn_stats(self):
         """(events scored by the collect path, batches decided by the brute force) of the last exact knn2_pairs call or
-        re-scoring match_pairs call (rescore_band > 0 on a keep_float context)."""
+        re-scoring match_pairs / match_pairs_guided call (rescore_band > 0 on a keep_float context)."""
         ev, bf = C.c_int64(), C.c_int32()
         self._check(self._L.msfm_test_last_knn_stats(self._h, C.byref(ev), C.byref(bf)))
         return ev.value, bf.value
@@ -332,11 +332,14 @@ class Matcher:
 
     def match_pairs_guided(self, pairs, F, image_xy: dict, *, th_epipolar: float = 3.0, ratio: float = 0.6,
                            ratio_good: float = 0.0, max_dist_sq: float = 0.0, mutual: bool = False, min_keypoints: int = 20,
-                           orientation: int = 0, flags: int = 0, capacity: int | None = None) -> MatchResult:
+                           orientation: int = 0, flags: int = 0, rescore_band: float = 0.0,
+                           capacity: int | None = None) -> MatchResult:
         """msfm_match_pairs_guided (GUIDED-SPEC in include/msfm_match.h): match_pairs with every query row's 2-NN searched
         only among the reference keypoints within th_epipolar pixels of the pair's epipolar geometry.  F: [n, 3, 3]
         float64 as geo_verify returns it (p_query^T F p_ref = 0); image_xy: {image id: [rows, 2] float32 centred
-        keypoints}, one per descriptor row of every image the pairs touch."""
+        keypoints}, one per descriptor row of every image the pairs touch.  rescore_band > 0 (float uploads on a
+        keep_float context): rows whose gated quantised ratio lies within that relative band of a ratio threshold are
+        decided on their exact fp32 top-2 among the allowed reference rows, as match_pairs does without a gate."""
         pa = self._pairs(pairs)
         n = pa.shape[0]
         Fa = np.ascontiguousarray(F, np.float64).reshape(-1, 9)
@@ -345,7 +348,7 @@ class Matcher:
         n_images = int(pa.max()) + 1 if n else 0
         ptrs, npts, xy_keep = self._keypoint_table(image_xy, n_images)
         out, res = self._result_buffers(pa, ratio_good, capacity, None)
-        prm = self._params(ratio, ratio_good, max_dist_sq, mutual, min_keypoints, orientation, 0.0, flags)
+        prm = self._params(ratio, ratio_good, max_dist_sq, mutual, min_keypoints, orientation, rescore_band, flags)
         self._check(self._L.msfm_match_pairs_guided(self._h, pa.ctypes.data, n, C.byref(prm), Fa.ctypes.data, th_epipolar,
                                                     C.cast(ptrs, C.c_void_p), npts.ctypes.data, n_images, C.byref(res)))
         del xy_keep
