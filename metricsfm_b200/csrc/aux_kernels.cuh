@@ -1,6 +1,6 @@
 // aux_kernels.cuh — the small HBM-bound kernels around the matching kernel:
 //   * descriptor packer (north_star subsystem 1): f32/u8 rows -> 128-byte u8 rows + uint32 squared norms
-//   * finalize: ratio test (+ max-dist gate, + mutual check) and ordered per-pair compaction
+//   * finalize: ratio test (+ max-dist test, + mutual check) and ordered per-pair compaction
 //   * offsets scan + tight gather of the per-pair match lists
 //   * a CUDA-core dp4a brute-force kNN used only by tests as a GPU-side cross-check
 #pragma once
@@ -206,15 +206,6 @@ struct BandParams {
     float *out_dists = nullptr;
 };
 
-// The epipolar gate of a guided batch, for the brute force (rescore_band_kernel<true>); the other stages of the collect
-// path see gated rows only.  A separate argument: a longer BandParams would move the parameters after it in every kernel
-// that takes one.
-struct BandGate {
-    const float2 *xy;   // keypoints (x, y), indexed like the packed arena
-    const float *fmat;  // [forward pairs of the batch][9] F rounded to fp32, row-major
-    float t2;           // th_epipolar^2, rounded to fp32
-};
-
 // A quantised-distance threshold T(q) that provably holds every fp32 top-2 neighbour of query row x (the band rows of
 // msfm_match_pairs and every row of the exact kNN mode).
 // With s the scale, q_y the packed row of y and r_y = ||s*y - q_y|| its quantisation residual (clamping included), the
@@ -386,16 +377,18 @@ __global__ void __launch_bounds__(256) finish_band_kernel(const BandParams bp) {
     }
 }
 
-// GUIDED: a reference row enters a band row's top-2 only if the epipolar gate allows the element, evaluated with the
-// operations of the matching kernel's MODE 2 (bit for bit: the allowed set is the one the row's threshold came from).
+// GUIDED: a reference row enters a band row's top-2 only if the epipolar gate allows the element, evaluated like the
+// matching kernel does (bit for bit: the allowed set is the one the row's threshold came from).  The gate is a separate
+// argument because a longer BandParams would move the parameters after it in every kernel that takes one; the other
+// stages of the collect path see gated rows only.
 template <bool GUIDED>
-__global__ void __launch_bounds__(256) rescore_band_kernel(const BandParams bp, int n_pairs, const BandGate gate) {
+__global__ void __launch_bounds__(256) rescore_band_kernel(const BandParams bp, int n_pairs, const EpiGate gate) {
     __shared__ float sq[kRescoreRows][kDim];                  // band rows, float
     __shared__ __align__(16) uint32_t sq8[kRescoreRows][kDim / 4];  // the same rows, packed u8
     __shared__ int s_na[kRescoreRows], s_thr[kRescoreRows];
     __shared__ float red_d[8][kRescoreRows][2];
     __shared__ int red_i[8][kRescoreRows][2];
-    __shared__ float s_gate[GUIDED ? kRescoreRows : 1][4];   // GUIDED: the band rows' query lines (a0, a1, a2, |a|^2)
+    __shared__ EpiLine s_line[GUIDED ? kRescoreRows : 1];    // GUIDED: the band rows' query lines
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     if (bp.event_count && *bp.event_count <= bp.event_cap) return;  // the collect path has every event: nothing to do
     for (int p = blockIdx.x; p < n_pairs; p += gridDim.x) {
@@ -424,15 +417,7 @@ __global__ void __launch_bounds__(256) rescore_band_kernel(const BandParams bp, 
                     na = ckey_to_norm(bp.ckeys[pd.qry_off + q]);
                     // Prefilter on the quantised distance: the threshold the collect pass used (exact_threshold)
                     thr = bp.band_thr[pd.knn_off + c0 + qi];
-                    if (GUIDED) {
-                        const float *fm = gate.fmat + 9 * p;
-                        const float2 k = gate.xy[pd.qry_off + q];
-                        const float a0 = epi_lin(fm[0], k.x, fm[3], k.y, fm[6]), a1 = epi_lin(fm[1], k.x, fm[4], k.y, fm[7]);
-                        s_gate[qi][0] = a0;
-                        s_gate[qi][1] = a1;
-                        s_gate[qi][2] = epi_lin(fm[2], k.x, fm[5], k.y, fm[8]);
-                        s_gate[qi][3] = epi_sq(a0, a1);
-                    }
+                    if (GUIDED) s_line[qi] = epi_query_line(gate.fmat + 9 * p, gate.xy[pd.qry_off + q]);
                 }
                 s_na[qi] = na;
                 s_thr[qi] = thr;
@@ -460,19 +445,17 @@ __global__ void __launch_bounds__(256) rescore_band_kernel(const BandParams bp, 
                     }
                 }
                 const int nb = ckey_to_norm(refk[j]);
-                float xj = 0.f, yj = 0.f, nbj = 0.f;  // GUIDED: reference row j's keypoint and |b|^2
+                float2 kj{};      // GUIDED: reference row j's keypoint ...
+                float nbj = 0.f;  // ... and |b|^2
                 if (GUIDED) {
-                    const float *fm = gate.fmat + 9 * p;
-                    const float2 k = gate.xy[pd.ref_off + j];
-                    xj = k.x;
-                    yj = k.y;
-                    nbj = epi_sq(epi_lin(fm[0], xj, fm[1], yj, fm[2]), epi_lin(fm[3], xj, fm[4], yj, fm[5]));
+                    kj = gate.xy[pd.ref_off + j];
+                    nbj = epi_ref_line(gate.fmat + 9 * p, kj).n;
                 }
 #pragma unroll
                 for (int qi = 0; qi < kRescoreRows; ++qi) {
                     const int dint = s_na[qi] + nb - 2 * (int)ab[qi];
                     if (dint <= s_thr[qi] &&
-                        (!GUIDED || epi_allowed(epi_lin(s_gate[qi][0], xj, s_gate[qi][1], yj, s_gate[qi][2]), s_gate[qi][3], nbj, gate.t2))) {
+                        (!GUIDED || epi_allowed(s_line[qi], kj, nbj, gate.t2))) {
                         // rare: exact fp32 distance, accumulated in index order without contraction
                         float acc = 0.0f;
                         const float *rf = ref + (int64_t)j * kDim;
@@ -562,7 +545,7 @@ struct SelectParams {
     int32_t smem_table_rows;
     int2 *danger;              // [forward kNN rows] per-pair list of (row, d1) of the dangerous rows
     int32_t *twin_counts;      // [n_pairs] candidates routed to the tensor twin pass (0: decided here)
-    unsigned int *twin_gate;   // number of pairs routed to the twin pass (the twin launch returns at once when 0)
+    unsigned int *routed;      // number of pairs routed to the twin pass (the twin launch returns at once when 0)
     const uint8_t *desc_arena;
     const int32_t *ckeys;
     uint8_t *cand_desc;        // [forward kNN rows][128]
@@ -859,7 +842,7 @@ __global__ void __launch_bounds__(1024) select_candidates_kernel(const SelectPar
     }
     if (threadIdx.x == 0) {
         sp.twin_counts[blockIdx.x] = overflow ? running : 0;
-        if (overflow && running > 0) atomicAdd(sp.twin_gate, 1u);
+        if (overflow && running > 0) atomicAdd(sp.routed, 1u);
     }
     if (!overflow) return;
     // ---- tensor twin pass for this pair: gather the candidates' reference rows (+ column keys) into the scratch image

@@ -21,9 +21,9 @@
 //   (padding warps) idle; the auxiliary warpgroups hand their registers to the epilogue warps (setmaxnreg)
 //   The service warps share issue slots with the epilogue warps of their sub-partition: their tile loops are unrolled
 //   over the B ring (immediate addresses) and they sleep between polls (see the comment at the role dispatch).
-// MODE 1 ("collect", float regime) replaces the top-2 merge by "append every element under the row's fixed threshold
-// to an event list"; MODE 2 ("guided") bars the elements that fail an epipolar gate from the top-2 in the exact phase;
-// MODE 3 is MODE 1 under MODE 2's gate (band rows of a guided call); everything else is shared.
+// Two template flags vary the epilogue's exact phase, everything else is shared: COLLECT (float regime) replaces the
+// top-2 merge by "append every element under the row's fixed threshold to an event list"; GATED (guided matching) bars
+// the elements that fail the epipolar gate (epi_allowed) from the row's top-2 or event list.
 // Work distribution: CTA b takes items b, b + grid, ...; every role walks that list on its own.
 // Pipelines (all mbarrier based):
 //   A ring (2 deep)     : query strips of a work item, STRIPS x [128 rows x 128 B]
@@ -34,6 +34,7 @@
 //   TMEM                : TBUFS x STRIPS accumulator blocks of TILE_N int32 columns, each with its own full/empty
 //                         barrier pair, so the MMA of tile t+1 runs under the epilogue of tile t
 #pragma once
+#include <cstddef>
 #include <cstdint>
 #include <climits>
 #include <cuda.h>
@@ -87,52 +88,47 @@ struct MatchKernelParams {
     const PairDesc *pairs;
     const WorkItem *items;
     int32_t n_items;
-    // MODE 3 ("collect under the gate", float regime of msfm_match_pairs_guided): MODE 1's event append restricted to the
-    // elements that pass the epipolar gate, which runs in the exact phase as in MODE 2.  Item of band twin d (cand_idx =
-    // p): row = band row q of forward pair p (scratch row qry_off + q), at the keypoint of its query row
-    // band_q[qry_off + q]; columns = p's reference rows; F = row p of the F table.  MODE 3 needs the event fields and
-    // the gate at once, and the block cannot grow: past 128 bytes nvcc addresses the parameter block through a pointer
-    // and the code of every mode changes.  So its three gate fields share the slots of fields that only the debug build
-    // (debug_flags, stats) or the kNN output (knn) reads, neither of which MODE 3 has.
+    // A pass writes either top-2 records (and, in the debug build, counters) or events (COLLECT), never both, so those
+    // outputs share slots.  COLLECT lists every (row, reference row) whose squared distance is <= cand_d0[row], as
+    // {scratch row, reference row, cand_idx, 0}.
     union {
         uint32_t debug_flags;     // timing experiments only (results are wrong): 1 = skip the exact phase,
                                   // 2 = no epilogue work at all, 4 = TMEM loads + hand-back only
-        uint32_t gate_f_desc;     // MODE 3: the F table ([forward pairs][9] fp32) starts after this many PairDescs of `pairs`
+        uint32_t event_cap;       // COLLECT
     };
     union {
         unsigned long long *stats;  // optional debug counter (slow-path group visits); null in production
-        const float2 *gate_xy;      // MODE 3: keypoints (x, y), indexed like the column-key arena
+        unsigned int *event_count;  // COLLECT: total events seen (may exceed event_cap: the consumer then falls back)
     };
     union {
         int4 *knn;                // [sum qry_rows] {id0, id1, d0, d1} per query row; id = -1 / d = INT_MAX when absent;
                                   // consumers read it with load_knn()
-        const int32_t *band_q;    // MODE 3: [forward kNN rows] query row of every band row (mark_band_kernel)
+        int4 *events;             // COLLECT: [event_cap]
     };
-    // MODE 1 ("collect", float regime): instead of a top-2 the kernel lists every (query row, reference row) whose
-    // squared distance is <= cand_d0[row], as {scratch row, reference row, cand_idx, 0}.
-    // MODE 2 ("guided", msfm_match_pairs_guided): only elements that pass the epipolar gate (epi_allowed) can enter a
-    // row's top-2.  Forward item of pair p: row = query row, columns = reference rows, F = fmat[p]; twin item of pair p
-    // (cand_idx = p): row = candidate i, whose reference row is cand_j[qry_off + i], columns = query rows, same F.
-    // The two modes share these fields, which keeps the parameter block (and the code of modes 0 and 1) as it was.
-    union {
-        int4 *events;
-        const float2 *xy;         // MODE 2: keypoints (x, y), indexed like the column-key arena
-    };
-    union {
-        unsigned int *event_count;  // total events seen (may exceed event_cap: the consumer then falls back)
-        const float *fmat;          // MODE 2: [forward pairs of the batch][9] F rounded to fp32, row-major
-    };
-    union {
-        uint32_t event_cap;
-        const int32_t *cand_j;      // MODE 2: reference row of every gathered candidate (twin items)
-    };
-    const unsigned int *gate;     // optional: the whole launch returns at once when *gate == 0 (mutual twin pass with no
-                                  // pair left for the tensor path, see select_candidates_kernel)
+    // GATED (msfm_match_pairs_guided): only elements that pass the epipolar gate (epi_allowed) can enter a row's top-2 or
+    // event list.  F is row p of fmat for a forward item of pair p and for every item with cand_idx = p.  A forward row
+    // and a band row (a collect item's row) are query keypoints, so the gate takes their query line; a twin row is a
+    // reference keypoint, and the gate takes the query line of each column instead.
+    const float2 *xy;             // keypoints (x, y), indexed like the column-key arena
+    const float *fmat;            // [forward pairs of the batch][9] F rounded to fp32, row-major
+    const int32_t *src_row;       // [candidate scratch rows] the image row a scratch row came from: a reference row of pair
+                                  // cand_idx for a twin row (cand_j), a query row of it for a band row (band_q)
+    const unsigned int *routed;   // optional: the whole launch returns at once when *routed == 0 (mutual twin pass with no
+                                  // pair routed to the tensor path, see select_candidates_kernel)
     uint32_t prune_q8;            // "dead row" rule of the forward pass (see the epilogue): a row whose two nearest neighbours
                                   // so far satisfy d0 > (prune_q8 / 256) * d1 only follows its NEAREST neighbour exactly.
                                   // kNoPrune = off (exact 2-NN of every row: msfm_knn2, twin and collect passes)
-    float t2;                     // MODE 2 and 3: th_epipolar^2, rounded to fp32
+    float t2;                     // GATED: th_epipolar^2, rounded to fp32
 };
+// The kernel takes the block by value.  Past 128 bytes nvcc addresses it through a pointer and the code of every
+// instantiation changes; the top-2 passes, the headline path, read their fields at these offsets.
+static_assert(sizeof(MatchKernelParams) == 128, "MatchKernelParams must stay 128 bytes");
+static_assert(offsetof(MatchKernelParams, n_items) == 64 && offsetof(MatchKernelParams, debug_flags) == 68 &&
+              offsetof(MatchKernelParams, stats) == 72 && offsetof(MatchKernelParams, knn) == 80 &&
+              offsetof(MatchKernelParams, xy) == 88 && offsetof(MatchKernelParams, fmat) == 96 &&
+              offsetof(MatchKernelParams, src_row) == 104 && offsetof(MatchKernelParams, routed) == 112 &&
+              offsetof(MatchKernelParams, prune_q8) == 120 && offsetof(MatchKernelParams, t2) == 124,
+              "top-2 passes read the parameter block at fixed offsets");
 constexpr uint32_t kNoPrune = 4096;  // ((d1 >> 8) + 1) * 4096 >= 16 * d1 > d0 for every row, and fits in 32 bits (d < 2^25)
 
 template <int STRIPS, int TILE_N, int STAGES, int TBUFS>
@@ -210,17 +206,54 @@ __device__ __forceinline__ int prune_score(int S0, int S1, int na, int rho8, int
 
 // Epipolar gate of GUIDED-SPEC (include/msfm_match.h).  Query line a = F^T (xq, yq, 1), reference line b = F (xj, yj, 1),
 // s = a . (xj, yj, 1): element (q, j) is allowed iff s^2 <= t2 * min(|a|^2, |b|^2) over the first two components.  Every
-// operation is one fp32 rounding (no contraction), so the forward item (row q) and the twin item (row j) decide an element
-// identically, and a numpy float32 restatement reproduces it bit for bit.
+// operation is one fp32 rounding (no contraction), and every stage that evaluates the gate (the matching kernel's rows
+// and columns in both roles, the brute force rescore_band_kernel) goes through epi_query_line, epi_ref_line and
+// epi_allowed below: an element is decided identically everywhere, and a numpy float32 restatement reproduces it bit for bit.
 __device__ __forceinline__ float epi_lin(float u, float x, float v, float y, float w) {  // ((u*x) + (v*y)) + w
     return __fadd_rn(__fadd_rn(__fmul_rn(u, x), __fmul_rn(v, y)), w);
 }
 __device__ __forceinline__ float epi_sq(float u, float v) { return __fadd_rn(__fmul_rn(u, u), __fmul_rn(v, v)); }
-__device__ __forceinline__ bool epi_allowed(float s, float na, float nb, float t2) {
-    return __fmul_rn(s, s) <= __fmul_rn(t2, nb < na ? nb : na);
+
+struct EpiLine {
+    float u, v, w;  // the line u x + v y + w = 0
+    float n;        // u^2 + v^2
+};
+// F is row-major; LDG reads it through the read-only cache (the per-element tests of the matching kernel).
+template <bool LDG>
+__device__ __forceinline__ float epi_f(const float *F, int i) { return LDG ? __ldg(F + i) : F[i]; }
+template <bool LDG = false>
+__device__ __forceinline__ EpiLine epi_query_line(const float *F, float2 k) {  // a = F^T (x, y, 1)
+    EpiLine a;
+    a.u = epi_lin(epi_f<LDG>(F, 0), k.x, epi_f<LDG>(F, 3), k.y, epi_f<LDG>(F, 6));
+    a.v = epi_lin(epi_f<LDG>(F, 1), k.x, epi_f<LDG>(F, 4), k.y, epi_f<LDG>(F, 7));
+    a.w = epi_lin(epi_f<LDG>(F, 2), k.x, epi_f<LDG>(F, 5), k.y, epi_f<LDG>(F, 8));
+    a.n = epi_sq(a.u, a.v);
+    return a;
+}
+template <bool LDG = false>
+__device__ __forceinline__ EpiLine epi_ref_line(const float *F, float2 k) {  // b = F (x, y, 1)
+    EpiLine b;
+    b.u = epi_lin(epi_f<LDG>(F, 0), k.x, epi_f<LDG>(F, 1), k.y, epi_f<LDG>(F, 2));
+    b.v = epi_lin(epi_f<LDG>(F, 3), k.x, epi_f<LDG>(F, 4), k.y, epi_f<LDG>(F, 5));
+    b.w = epi_lin(epi_f<LDG>(F, 6), k.x, epi_f<LDG>(F, 7), k.y, epi_f<LDG>(F, 8));
+    b.n = epi_sq(b.u, b.v);
+    return b;
+}
+// Element (q, j) from q's query line a, j's keypoint kj and |b|^2 of j's reference line.
+__device__ __forceinline__ bool epi_allowed(const EpiLine &a, float2 kj, float nb, float t2) {
+    const float s = epi_lin(a.u, kj.x, a.v, kj.y, a.w);
+    return __fmul_rn(s, s) <= __fmul_rn(t2, nb < a.n ? nb : a.n);
 }
 
-template <int STRIPS, int TILE_N, int STAGES, int TBUFS, bool DEBUG, int MODE = 0>
+// The epipolar gate of a guided batch as the host passes it: keypoints (x, y) indexed like the column-key arena, the
+// batch's F table ([forward pairs][9] rounded to fp32, row-major) and th_epipolar^2 rounded to fp32.
+struct EpiGate {
+    const float2 *xy;
+    const float *fmat;
+    float t2;
+};
+
+template <int STRIPS, int TILE_N, int STAGES, int TBUFS, bool DEBUG, bool COLLECT = false, bool GATED = false>
 __global__ void __launch_bounds__(MatchKernelCfg<STRIPS, TILE_N, STAGES, TBUFS>::kThreads, 1)
 match_pairs_kernel(const MatchKernelParams p) {
     using Cfg = MatchKernelCfg<STRIPS, TILE_N, STAGES, TBUFS>;
@@ -244,7 +277,7 @@ match_pairs_kernel(const MatchKernelParams p) {
     const int warp = __shfl_sync(0xFFFFFFFFu, (int)(threadIdx.x >> 5), 0);  // warp-uniform by construction: lets the compiler keep
                                                                             // everything derived from it in uniform registers
     const int lane = threadIdx.x & 31;
-    if (p.gate != nullptr && *p.gate == 0u) return;  // uniform over the grid: nothing was routed to this pass
+    if (p.routed != nullptr && *p.routed == 0u) return;  // uniform over the grid: nothing was routed to this pass
     if (threadIdx.x == 0 && (ptx::smem_u32(smem) & 1023u) != 0) __trap();
 
     if (warp == Cfg::kEpiWarps && lane == 0) {
@@ -453,39 +486,24 @@ match_pairs_kernel(const MatchKernelParams p) {
             // the running-top-2 records of such rows (most rows of an image pair) never reach the exact phase.  A row that
             // ends dead reports d1 := d0: "rejected", and still a valid lower bound of its distance to every row but nn0,
             // which is what the mutual check's dangerous-row bound needs (select_candidates_kernel).
-            // Under the epipolar gate (MODE 2) the rule stays on: it only reasons about elements that can enter the row's
-            // top-2, and the gate only removes elements (barred ones never reach the running state).
-            const int rho8 = (MODE != 1 && MODE != 3 && pd.cand_idx < 0) ? (int)p.prune_q8 : (int)kNoPrune;
-            // Guided items: the row's half of the gate, once per item.  Forward row (query q): g = (a0, a1, a2, |a|^2);
-            // twin row (candidate of reference row j): g = (xj, yj, b0, b1), gn = |b|^2.
-            float g0 = 0.f, g1 = 0.f, g2 = 0.f, g3 = 0.f, gn = 0.f;
+            // Under the epipolar gate the rule stays on: it only reasons about elements that can enter the row's top-2,
+            // and the gate only removes elements (barred ones never reach the running state).
+            const int rho8 = (!COLLECT && pd.cand_idx < 0) ? (int)p.prune_q8 : (int)kNoPrune;
+            // Gated items: the row's half of the gate, once per item.  A forward or band row is a query keypoint: its
+            // query line.  A band row takes its query row's keypoint and F, so it gets that row's line bit for bit, and
+            // its allowed set is the one its gated quantised 2-NN, and hence its threshold T(q), came from.  A twin row is
+            // a reference keypoint kr: its reference line, of which the test needs |b|^2 only.
+            const bool query_row = COLLECT || pd.cand_idx < 0;
+            EpiLine line{};
+            float2 kr{};
             const float *fm = nullptr;
-            if (MODE == 2) {
+            if (GATED) {
                 fm = p.fmat + 9 * (pd.cand_idx >= 0 ? pd.cand_idx : wi.pair);
-                if (valid && pd.cand_idx < 0) {
-                    const float2 k = p.xy[pd.qry_off + q];
-                    g0 = epi_lin(fm[0], k.x, fm[3], k.y, fm[6]);
-                    g1 = epi_lin(fm[1], k.x, fm[4], k.y, fm[7]);
-                    g2 = epi_lin(fm[2], k.x, fm[5], k.y, fm[8]);
-                    g3 = epi_sq(g0, g1);
+                if (valid && query_row) {
+                    line = epi_query_line(fm, p.xy[pd.cand_idx < 0 ? pd.qry_off + q : p.pairs[pd.cand_idx].qry_off + p.src_row[pd.qry_off + q]]);
                 } else if (valid) {
-                    const float2 k = p.xy[p.pairs[pd.cand_idx].ref_off + p.cand_j[pd.qry_off + q]];
-                    g0 = k.x;
-                    g1 = k.y;
-                    g2 = epi_lin(fm[0], k.x, fm[1], k.y, fm[2]);
-                    g3 = epi_lin(fm[3], k.x, fm[4], k.y, fm[5]);
-                    gn = epi_sq(g2, g3);
-                }
-            } else if (MODE == 3) {
-                // band row: the same four values as its query row's forward item (bit for bit, so the allowed set of the
-                // row is the one its gated quantised 2-NN, and hence its threshold T(q), came from)
-                fm = reinterpret_cast<const float *>(p.pairs + p.gate_f_desc) + 9 * pd.cand_idx;
-                if (valid) {
-                    const float2 k = p.gate_xy[p.pairs[pd.cand_idx].qry_off + p.band_q[pd.qry_off + q]];
-                    g0 = epi_lin(fm[0], k.x, fm[3], k.y, fm[6]);
-                    g1 = epi_lin(fm[1], k.x, fm[4], k.y, fm[7]);
-                    g2 = epi_lin(fm[2], k.x, fm[5], k.y, fm[8]);
-                    g3 = epi_sq(g0, g1);
+                    kr = p.xy[p.pairs[pd.cand_idx].ref_off + p.src_row[pd.qry_off + q]];
+                    line = epi_ref_line(fm, kr);
                 }
             }
             const int ntiles = (pd.ref_rows + TILE_N - 1) / TILE_N;
@@ -552,34 +570,26 @@ match_pairs_kernel(const MatchKernelParams p) {
                                               16 * (int)v[3] + c0.w, 16 * (int)v[4] + c1.x, 16 * (int)v[5] + c1.y,
                                               16 * (int)v[6] + c1.z, 16 * (int)v[7] + c1.w};
                                 const int jb8 = jtile + gq * 8;
-                                if (MODE == 2 || MODE == 3) {
+                                if (GATED) {
                                     // the group's 8 column keypoints (64 bytes, L2-resident); a barred element gets the
                                     // smallest key, whose score lies below kAbsent: it can only fill an empty slot as
-                                    // "no neighbour" and loses against every allowed element (MODE 3: it lies below
+                                    // "no neighbour" and loses against every allowed element (COLLECT: it lies below
                                     // every row's collect threshold and is never listed)
-                                    const float4 *kp = reinterpret_cast<const float4 *>((MODE == 3 ? p.gate_xy : p.xy) + pd.ref_off + jb8);
+                                    const float4 *kp = reinterpret_cast<const float4 *>(p.xy + pd.ref_off + jb8);
 #pragma unroll
                                     for (int h = 0; h < 4; ++h) {
                                         const float4 c = __ldg(kp + h);
-                                        const float cx[2] = {c.x, c.z}, cy[2] = {c.y, c.w};
+                                        const float2 kc[2] = {make_float2(c.x, c.y), make_float2(c.z, c.w)};
 #pragma unroll
                                         for (int e = 0; e < 2; ++e) {
-                                            bool ok;
-                                            if (MODE == 3 || pd.cand_idx < 0) {  // column = reference row j
-                                                const float b0 = epi_lin(__ldg(fm + 0), cx[e], __ldg(fm + 1), cy[e], __ldg(fm + 2));
-                                                const float b1 = epi_lin(__ldg(fm + 3), cx[e], __ldg(fm + 4), cy[e], __ldg(fm + 5));
-                                                ok = epi_allowed(epi_lin(g0, cx[e], g1, cy[e], g2), g3, epi_sq(b0, b1), p.t2);
-                                            } else {                // column = query row q
-                                                const float a0 = epi_lin(__ldg(fm + 0), cx[e], __ldg(fm + 3), cy[e], __ldg(fm + 6));
-                                                const float a1 = epi_lin(__ldg(fm + 1), cx[e], __ldg(fm + 4), cy[e], __ldg(fm + 7));
-                                                const float a2 = epi_lin(__ldg(fm + 2), cx[e], __ldg(fm + 5), cy[e], __ldg(fm + 8));
-                                                ok = epi_allowed(epi_lin(a0, g0, a1, g1, a2), epi_sq(a0, a1), gn, p.t2);
-                                            }
+                                            const bool ok = query_row  // column = reference row j, or query row q
+                                                ? epi_allowed(line, kc[e], epi_ref_line<true>(fm, kc[e]).n, p.t2)
+                                                : epi_allowed(epi_query_line<true>(fm, kc[e]), kr, line.n, p.t2);
                                             if (!ok) key[2 * h + e] = INT_MIN;
                                         }
                                     }
                                 }
-                                if (MODE == 1 || MODE == 3) {
+                                if (COLLECT) {
 #pragma unroll
                                     for (int i = 0; i < 8; ++i)
                                         if ((key[i] >> 3) > S1) {
@@ -620,7 +630,7 @@ match_pairs_kernel(const MatchKernelParams p) {
                 atomicAdd(p.stats + 8 + 2 * quarter, (unsigned long long)acc_wait);  // per SM sub-partition
                 atomicAdd(p.stats + 9 + 2 * quarter, (unsigned long long)(acc_load + acc_p1 + acc_p2));
             }
-            if (valid && MODE != 1 && MODE != 3) {
+            if (valid && !COLLECT) {
                 if (prune_score(S0, S1, na, rho8, kAbsent) != S1) S1 = S0;  // ended dead: d1 := d0 (lower bound)
                 int4 out;
                 out.x = (S0 > kAbsent && J0 >= 0) ? (J0 ^ 7) : -1;  // low three bits hold 7 - (column mod 8), as in the packed keys;

@@ -39,6 +39,18 @@ constexpr int kTbufs = 2;    // TMEM accumulator buffers per strip
 using KCfg = msfm::MatchKernelCfg<kStrips, kTileN, kStages, kTbufs>;
 constexpr int kItemRows = kStrips * msfm::kStripRows;
 
+// The instantiations of the matching kernel, (DEBUG, COLLECT, GATED): every combination but a debug build of the
+// collect pass, for which `debug` is ignored.
+using MatchKernelFn = void (*)(msfm::MatchKernelParams);
+template <bool DEBUG, bool COLLECT>
+MatchKernelFn match_kernel(bool gated) {
+    return gated ? msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, DEBUG, COLLECT, true>
+                 : msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, DEBUG, COLLECT, false>;
+}
+MatchKernelFn match_kernel(bool debug, bool collect, bool gated) {
+    return collect ? match_kernel<false, true>(gated) : debug ? match_kernel<true, false>(gated) : match_kernel<false, false>(gated);
+}
+
 // Per-batch scratch bounds (rows).  16 Mi query rows -> 256 MiB kNN scratch + 128 MiB match scratch.
 constexpr int64_t kBatchMaxQueryRows = 16ll << 20;
 constexpr int64_t kBatchMaxQueryRowsMutual = 16ll << 20;  // mutual: + 128 B of gathered candidate row per query row
@@ -114,7 +126,7 @@ struct msfm_ctx {
     DeviceBuf dbg_stats;  // debug flag 8: per-phase cycle counters of the matching kernel, dumped at destroy
     DeviceBuf cand_q, cand_j, cand_d0, cand_good, cand_counts, cand_desc, cand_ckeys;  // one-way candidates + gathered rows
     DeviceBuf tilemin;       // per reference tile: smallest squared norm (tile_min_kernel, refreshed per batch)
-    DeviceBuf colbest, twin_counts;  // mutual check: per-pair column table (nearest claimant per reference row); [n_pairs] + gate word
+    DeviceBuf colbest, twin_counts;  // mutual check: per-pair column table (nearest claimant per reference row); [n_pairs] + routed word
     DeviceBuf band_q, band_counts;  // float regime: query rows near a ratio threshold, per pair
     DeviceBuf band_thr, band_state, band_events, band_event_keys, band_event_count;  // ... and the collect pass over them
     int64_t band_event_cap_override = -1;  // msfm_test_set_band_event_cap (tests: 0 forces the brute-force fallback)
@@ -124,9 +136,6 @@ struct msfm_ctx {
     bool force_twin = false;               // msfm_test_force_twin_pass
     bool no_prune = false;                 // msfm_test_disable_pruning: the forward pass keeps exact 2-NN rows for every query row
     DeviceBuf kp_xy;                       // msfm_match_pairs_guided: keypoints (x, y) per arena row (allocated on the first call)
-    const float *guided_f = nullptr;       // F matrices (fp32) of the current batch of a guided call, null otherwise: set per batch
-                                           // by run_match_stage (they travel in the pair-descriptor upload)
-    float guided_t2 = 0.0f;                // ... and th_epipolar^2
     DeviceBuf staging, knn, matches, good, counts, offsets, pairdesc, items, tight_matches, tight_good;
     DeviceBuf tight_matches_b, tight_good_b;  // second set: a batch's lists are copied out while the next batch is gathered
     void *h_pinned = nullptr;
@@ -134,7 +143,7 @@ struct msfm_ctx {
     cudaEvent_t ev_begin = nullptr, ev_end = nullptr, ev_k0 = nullptr, ev_k1 = nullptr, ev_k2 = nullptr, ev_k3 = nullptr,
                 ev_f1 = nullptr;
 
-    int64_t twin_gate_index = 0;  // the gate word sits after the per-pair twin counts
+    int64_t routed_index = 0;  // the routed word (pairs routed to the twin pass) sits after the per-pair twin counts
     msfm_timing timing{};
     uint32_t debug_flags = 0;  // MSFM_DEBUG_FLAGS environment variable (timing experiments)
     std::string err;
@@ -321,7 +330,7 @@ msfm_status reserve_locked(msfm_ctx *ctx, int32_t image_id, int32_t rows, int64_
 }
 
 struct BatchPlan {
-    std::vector<PairDesc> pairs;     // forward pair descriptors (only pairs passing the gate)
+    std::vector<PairDesc> pairs;     // forward pair descriptors (only pairs with min_keypoints rows on both sides)
     std::vector<PairDesc> twins;     // mutual cross-check: candidate rows of pair p searched against its query image
     std::vector<int64_t> src_index;  // index into the caller's pair list
     std::vector<WorkItem> items;     // forward work items
@@ -340,6 +349,9 @@ struct BatchPlan {
     bool has_empty = false;          // some pair has no work items: its kNN rows must read "absent"
     bool any_float = false;          // some pair has retained float rows on both sides (rescoring possible)
     std::vector<float> fmat;         // guided call: F of every forward pair, 9 floats each (uploaded after the descriptors)
+    msfm::EpiGate gate{};            // guided call: keypoints and t2 from the carve, the F table's device address from
+                                     // run_match_stage
+    const msfm::EpiGate *epi_gate() const { return gate.fmat ? &gate : nullptr; }  // null: ungated
     int64_t knn_rows() const { return mutual ? 2 * query_rows : query_rows; }
 };
 
@@ -347,10 +359,12 @@ struct BatchPlan {
 //   forward  2-NN of the forward pairs' query rows, with the dead-row rule `value` (prune_q8)
 //   twin     2-NN of the mutual twins' candidate rows, skipped on the device unless select_candidates_kernel routed a pair
 //   collect  the items are band twins: every reference row within band_thr of a band row is appended to the event list,
-//            which holds `value` events; in a guided call only the rows the epipolar gate allows
+//            which holds `value` events
+// `gate` (null: none) bars the elements that fail the epipolar gate in every pass.
 enum class Pass { forward, twin, collect };
 
-msfm_status launch_match_kernel(msfm_ctx *ctx, Pass pass, size_t first_item, size_t n_items, uint32_t value = 0) {
+msfm_status launch_match_kernel(msfm_ctx *ctx, Pass pass, size_t first_item, size_t n_items, uint32_t value,
+                                const msfm::EpiGate *gate) {
     const bool collect = pass == Pass::collect, twin = pass == Pass::twin;
     msfm::MatchKernelParams kp;
     kp.maps = ctx->d_maps;
@@ -359,46 +373,27 @@ msfm_status launch_match_kernel(msfm_ctx *ctx, Pass pass, size_t first_item, siz
     kp.cand_ckeys = static_cast<const int32_t *>(ctx->cand_ckeys.ptr);
     kp.cand_d0 = static_cast<const int32_t *>(collect ? ctx->band_thr.ptr : ctx->cand_d0.ptr);
     kp.counts = static_cast<const int32_t *>(collect ? ctx->band_counts.ptr : ctx->twin_counts.ptr);
-    // mutual twin pass: the launch returns at once unless select_candidates_kernel routed some pair to it
-    kp.gate = twin ? reinterpret_cast<const unsigned int *>(static_cast<const int32_t *>(ctx->twin_counts.ptr) + ctx->twin_gate_index) : nullptr;
-    // a guided call's collect pass lists only the elements its gate allows (MODE 3)
-    const bool guided = ctx->guided_f != nullptr;
-    if (guided && !collect) {
-        kp.xy = static_cast<const float2 *>(ctx->kp_xy.ptr);
-        kp.fmat = ctx->guided_f;
-        kp.cand_j = static_cast<const int32_t *>(ctx->cand_j.ptr);
-    } else {
-        kp.events = static_cast<int4 *>(ctx->band_events.ptr);
-        kp.event_count = static_cast<unsigned int *>(ctx->band_event_count.ptr);
-        kp.event_cap = collect ? value : 0;
-    }
-    kp.t2 = guided ? ctx->guided_t2 : 0.0f;
     kp.pairs = static_cast<const PairDesc *>(ctx->pairdesc.ptr);
     kp.items = static_cast<const WorkItem *>(ctx->items.ptr) + first_item;
     kp.n_items = (int32_t)n_items;
-    if (guided && collect) {  // MODE 3: the gate's fields in the slots of the debug and kNN fields (match_kernel.cuh)
-        kp.gate_f_desc = (uint32_t)((ctx->guided_f - static_cast<const float *>(ctx->pairdesc.ptr)) * sizeof(float) / sizeof(PairDesc));
-        kp.gate_xy = static_cast<const float2 *>(ctx->kp_xy.ptr);
-        kp.band_q = static_cast<const int32_t *>(ctx->band_q.ptr);
+    if (collect) {
+        kp.event_cap = value;
+        kp.event_count = static_cast<unsigned int *>(ctx->band_event_count.ptr);
+        kp.events = static_cast<int4 *>(ctx->band_events.ptr);
     } else {
-        kp.stats = static_cast<unsigned long long *>(ctx->dbg_stats.ptr);  // null unless MSFM_DEBUG_FLAGS & 8
         kp.debug_flags = ctx->debug_flags;
+        kp.stats = static_cast<unsigned long long *>(ctx->dbg_stats.ptr);  // null unless MSFM_DEBUG_FLAGS & 8
         kp.knn = static_cast<int4 *>(ctx->knn.ptr);
     }
+    kp.xy = gate ? gate->xy : nullptr;
+    kp.fmat = gate ? gate->fmat : nullptr;
+    kp.src_row = static_cast<const int32_t *>(collect ? ctx->band_q.ptr : ctx->cand_j.ptr);
+    // mutual twin pass: the launch returns at once unless select_candidates_kernel routed some pair to it
+    kp.routed = twin ? reinterpret_cast<const unsigned int *>(static_cast<const int32_t *>(ctx->twin_counts.ptr) + ctx->routed_index) : nullptr;
     kp.prune_q8 = (pass == Pass::forward && !ctx->no_prune) ? value : msfm::kNoPrune;
+    kp.t2 = gate ? gate->t2 : 0.0f;
     const int grid = std::max(1, std::min<int>(ctx->num_sms, kp.n_items));
-    if (collect && guided)
-        msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, false, 3><<<grid, KCfg::kThreads, KCfg::kSmemAlloc, ctx->stream>>>(kp);
-    else if (collect)
-        msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, false, 1><<<grid, KCfg::kThreads, KCfg::kSmemAlloc, ctx->stream>>>(kp);
-    else if (guided && ctx->debug_flags)
-        msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, true, 2><<<grid, KCfg::kThreads, KCfg::kSmemAlloc, ctx->stream>>>(kp);
-    else if (guided)
-        msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, false, 2><<<grid, KCfg::kThreads, KCfg::kSmemAlloc, ctx->stream>>>(kp);
-    else if (ctx->debug_flags)
-        msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, true><<<grid, KCfg::kThreads, KCfg::kSmemAlloc, ctx->stream>>>(kp);
-    else
-        msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, false><<<grid, KCfg::kThreads, KCfg::kSmemAlloc, ctx->stream>>>(kp);
+    match_kernel(ctx->debug_flags != 0, collect, gate != nullptr)<<<grid, KCfg::kThreads, KCfg::kSmemAlloc, ctx->stream>>>(kp);
     MSFM_CUDA(ctx, cudaGetLastError());
     ctx->timing.match_launches += 1;
     ctx->timing.total_launches += 1;
@@ -479,8 +474,9 @@ void finish_plan(msfm_ctx *ctx, BatchPlan &plan) {
     }
 }
 
-// Upload the plan and run the forward matching launch (timed); leaves the kNN rows in scratch.
-msfm_status run_match_stage(msfm_ctx *ctx, const BatchPlan &plan) {
+// Upload the plan and run the forward matching launch (timed); leaves the kNN rows in scratch.  A guided plan's F table
+// travels behind the pair descriptors, and its address completes plan.gate.
+msfm_status run_match_stage(msfm_ctx *ctx, BatchPlan &plan) {
     msfm_status st;
     const size_t fw_bytes = plan.pairs.size() * sizeof(PairDesc);
     const size_t tw_bytes = plan.twins.size() * sizeof(PairDesc), bt_bytes = plan.band_twins.size() * sizeof(PairDesc);
@@ -502,7 +498,7 @@ msfm_status run_match_stage(msfm_ctx *ctx, const BatchPlan &plan) {
     if (tw_bytes) memcpy(hp + fw_bytes, plan.twins.data(), tw_bytes);
     if (bt_bytes) memcpy(hp + fw_bytes + tw_bytes, plan.band_twins.data(), bt_bytes);
     if (f_bytes) memcpy(hp + fw_bytes + tw_bytes + bt_bytes, plan.fmat.data(), f_bytes);
-    ctx->guided_f = f_bytes ? reinterpret_cast<const float *>(static_cast<const char *>(ctx->pairdesc.ptr) + fw_bytes + tw_bytes + bt_bytes) : nullptr;
+    plan.gate.fmat = f_bytes ? reinterpret_cast<const float *>(static_cast<const char *>(ctx->pairdesc.ptr) + fw_bytes + tw_bytes + bt_bytes) : nullptr;
     memcpy(hp + pd_pad, plan.items.data(), it_fw);
     if (!plan.twin_items.empty()) memcpy(hp + pd_pad + it_fw, plan.twin_items.data(), plan.twin_items.size() * sizeof(WorkItem));
     if (!plan.band_items.empty())
@@ -524,7 +520,7 @@ msfm_status run_match_stage(msfm_ctx *ctx, const BatchPlan &plan) {
         ctx->timing.total_launches += 1;
     }
     MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_k0, ctx->stream));
-    if (!plan.items.empty() && (st = launch_match_kernel(ctx, Pass::forward, 0, plan.items.size(), plan.prune_q8)) != MSFM_OK) return st;
+    if (!plan.items.empty() && (st = launch_match_kernel(ctx, Pass::forward, 0, plan.items.size(), plan.prune_q8, plan.epi_gate())) != MSFM_OK) return st;
     MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_k1, ctx->stream));
     ctx->timing.int8_ops += plan.ops;
     return MSFM_OK;
@@ -667,7 +663,8 @@ msfm::BandParams collect_params(const msfm_ctx *ctx, size_t event_cap) {
 msfm_status run_collect_pass(msfm_ctx *ctx, const BatchPlan &plan, const msfm::BandParams &bp) {
     msfm_status st;
     if (!plan.band_items.empty() &&
-        (st = launch_match_kernel(ctx, Pass::collect, plan.items.size() + plan.twin_items.size(), plan.band_items.size(), bp.event_cap)) != MSFM_OK)
+        (st = launch_match_kernel(ctx, Pass::collect, plan.items.size() + plan.twin_items.size(), plan.band_items.size(), bp.event_cap,
+                                  plan.epi_gate())) != MSFM_OK)
         return st;
     const int nb = (int)plan.pairs.size();
     msfm::score_events_kernel<<<4 * ctx->num_sms, 256, 0, ctx->stream>>>(bp);
@@ -675,12 +672,11 @@ msfm_status run_collect_pass(msfm_ctx *ctx, const BatchPlan &plan, const msfm::B
     msfm::finish_band_kernel<<<nb, 256, 0, ctx->stream>>>(bp);
     const int gx = std::min(nb, 4 * ctx->num_sms);
     const int gy = std::max(1, std::min(32, (4 * ctx->num_sms + gx - 1) / gx));
-    // a guided batch: the brute force applies the gate as the collect pass does (launch_match_kernel)
-    if (ctx->guided_f)
-        msfm::rescore_band_kernel<true><<<dim3(gx, gy), 256, 0, ctx->stream>>>(
-            bp, nb, msfm::BandGate{static_cast<const float2 *>(ctx->kp_xy.ptr), ctx->guided_f, ctx->guided_t2});
+    // a guided batch: the brute force applies the gate as the collect pass does
+    if (const msfm::EpiGate *gate = plan.epi_gate())
+        msfm::rescore_band_kernel<true><<<dim3(gx, gy), 256, 0, ctx->stream>>>(bp, nb, *gate);
     else
-        msfm::rescore_band_kernel<false><<<dim3(gx, gy), 256, 0, ctx->stream>>>(bp, nb, msfm::BandGate{nullptr, nullptr, 0.0f});
+        msfm::rescore_band_kernel<false><<<dim3(gx, gy), 256, 0, ctx->stream>>>(bp, nb, msfm::EpiGate{nullptr, nullptr, 0.0f});
     MSFM_CUDA(ctx, cudaGetLastError());
     ctx->timing.total_launches += 4;
     return MSFM_OK;
@@ -693,7 +689,7 @@ void note_collect_events(msfm_ctx *ctx, unsigned int events, size_t event_cap) {
     else ctx->knn_events += events;
 }
 
-// kNN of a single pair into scratch (no gate).  Caller holds the lock.
+// kNN of a single pair into scratch (no min_keypoints test).  Caller holds the lock.
 msfm_status knn_single(msfm_ctx *ctx, int32_t ref_id, int32_t query_id, BatchPlan &plan) {
     msfm_status st;
     if ((st = check_image_id(ctx, ref_id, true)) != MSFM_OK) return st;
@@ -815,10 +811,7 @@ msfm_status match_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pa
     ctx->timing = msfm_timing{};
     DrainListCopy drain_list_copy{ctx};
     MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_begin, ctx->stream));
-    if (guided) {
-        if ((st = upload_keypoints(ctx, pairs, n_pairs, *guided)) != MSFM_OK) return st;
-        ctx->guided_t2 = guided->th * guided->th;
-    }
+    if (guided && (st = upload_keypoints(ctx, pairs, n_pairs, *guided)) != MSFM_OK) return st;
     const bool mutual = params->mutual != 0;
     const bool want_good = params->ratio_good > 0.0f && (resident || out->has_good);
     const int64_t max_rows = mutual ? kBatchMaxQueryRowsMutual : kBatchMaxQueryRows;
@@ -845,11 +838,12 @@ msfm_status match_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pa
         c.plan.mutual = mutual;
         c.plan.rescoring = params->rescore_band > 0.0f && ctx->fdesc != nullptr;
         c.plan.prune_q8 = prune_q8;
+        if (guided) c.plan.gate = msfm::EpiGate{static_cast<const float2 *>(ctx->kp_xy.ptr), nullptr, guided->th * guided->th};
         c.first = next;
         while (next < n_pairs && (int64_t)c.plan.pairs.size() < kBatchMaxPairs) {
             const ImageSlot &r = ctx->images[pairs[next].ref], &q = ctx->images[pairs[next].query];
-            const bool gated = r.rows < params->min_keypoints || q.rows < params->min_keypoints;
-            if (!gated) {
+            const bool too_few = r.rows < params->min_keypoints || q.rows < params->min_keypoints;
+            if (!too_few) {
                 if (!c.plan.pairs.empty() && (c.plan.query_rows + q.rows > max_rows || (mutual && c.plan.ref_rows + r.rows > kBatchMaxRefRows))) break;
                 // A pair whose images are still being uploaded does not hold back the pairs before it: the batch is cut
                 // there, runs on what has landed, and the transfer goes on underneath (the caller orders the list by the
@@ -917,7 +911,7 @@ msfm_status match_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pa
             if (mutual) {
                 if ((st = ensure(ctx, ctx->colbest, plan.big_ref ? (size_t)std::max<int64_t>(plan.ref_rows, 1) * 8 : 256)) != MSFM_OK) return st;
                 if ((st = ensure(ctx, ctx->twin_counts, (size_t)(nb + 1) * 4)) != MSFM_OK) return st;
-                ctx->twin_gate_index = nb;
+                ctx->routed_index = nb;
                 if (plan.big_ref) MSFM_CUDA(ctx, cudaMemsetAsync(ctx->colbest.ptr, 0xFF, (size_t)plan.ref_rows * 8, ctx->stream));
                 MSFM_CUDA(ctx, cudaMemsetAsync(static_cast<int32_t *>(ctx->twin_counts.ptr) + nb, 0, 4, ctx->stream));
             }
@@ -940,7 +934,7 @@ msfm_status match_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pa
             sp.smem_table_rows = msfm::kSmemTableRows;
             sp.danger = static_cast<int2 *>(ctx->matches.ptr);  // the match scratch is written by the emission afterwards
             sp.twin_counts = static_cast<int32_t *>(ctx->twin_counts.ptr);
-            sp.twin_gate = reinterpret_cast<unsigned int *>(static_cast<int32_t *>(ctx->twin_counts.ptr) + nb);
+            sp.routed = reinterpret_cast<unsigned int *>(static_cast<int32_t *>(ctx->twin_counts.ptr) + nb);
             sp.desc_arena = ctx->desc;
             sp.ckeys = ctx->norms;
             sp.cand_desc = static_cast<uint8_t *>(ctx->cand_desc.ptr);
@@ -951,7 +945,7 @@ msfm_status match_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pa
             // ---- tensor twin pass (nearest query row of every candidate's reference row) for the routed pairs only
             MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_k2, ctx->stream));
             if (mutual && !plan.twin_items.empty() &&
-                (st = launch_match_kernel(ctx, Pass::twin, plan.items.size(), plan.twin_items.size())) != MSFM_OK)
+                (st = launch_match_kernel(ctx, Pass::twin, plan.items.size(), plan.twin_items.size(), 0, plan.epi_gate())) != MSFM_OK)
                 return st;
             MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_k3, ctx->stream));
             // ---- emission, offsets, tight gather
@@ -1153,6 +1147,22 @@ msfm_status knn2_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pai
     return MSFM_OK;
 }
 
+// msfm_match_pairs and msfm_match_pairs_guided: the caller's msfm_result receives the match lists.
+msfm_status match_pairs_to_result(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pairs, const msfm_params *params, msfm_result *out,
+                                  const GuidedArgs *guided) {
+    if (!ctx) return MSFM_ERR_INVALID_ARG;
+    if (cudaSetDevice(ctx->device) != cudaSuccess) return MSFM_ERR_CUDA;
+    if (!out || (!out->matches && out->match_capacity > 0)) return match_pairs_impl(ctx, pairs, n_pairs, params, nullptr, false, nullptr, guided);
+    CallerBuffers cb{out->matches, out->good, out->match_capacity};
+    OutSpec spec;
+    spec.offsets = out->offsets;
+    spec.ok = out->ok;
+    spec.has_good = out->good != nullptr;
+    spec.sink = caller_sink;
+    spec.user = &cb;
+    return match_pairs_impl(ctx, pairs, n_pairs, params, &spec, false, nullptr, guided);
+}
+
 }  // namespace
 
 // =====================================================================================================================
@@ -1265,19 +1275,12 @@ msfm_status msfm_create(const msfm_config *cfg, msfm_ctx **out) {
     // one tensor map per image + one for the candidate scratch
     if (cudaMalloc(&ctx->d_maps, (size_t)(ctx->max_images + 1) * sizeof(CUtensorMap)) != cudaSuccess) return bail(MSFM_ERR_OUT_OF_MEMORY);
     if (cudaMallocHost(&ctx->h_maps, (size_t)(ctx->max_images + 1) * sizeof(CUtensorMap)) != cudaSuccess) return bail(MSFM_ERR_OUT_OF_MEMORY);
-    if (cudaFuncSetAttribute(msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, false>,
-                             cudaFuncAttributeMaxDynamicSharedMemorySize, KCfg::kSmemAlloc) != cudaSuccess ||
-        cudaFuncSetAttribute(msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, true>,
-                             cudaFuncAttributeMaxDynamicSharedMemorySize, KCfg::kSmemAlloc) != cudaSuccess ||
-        cudaFuncSetAttribute(msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, false, 1>,
-                             cudaFuncAttributeMaxDynamicSharedMemorySize, KCfg::kSmemAlloc) != cudaSuccess ||
-        cudaFuncSetAttribute(msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, false, 2>,
-                             cudaFuncAttributeMaxDynamicSharedMemorySize, KCfg::kSmemAlloc) != cudaSuccess ||
-        cudaFuncSetAttribute(msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, true, 2>,
-                             cudaFuncAttributeMaxDynamicSharedMemorySize, KCfg::kSmemAlloc) != cudaSuccess ||
-        cudaFuncSetAttribute(msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, false, 3>,
-                             cudaFuncAttributeMaxDynamicSharedMemorySize, KCfg::kSmemAlloc) != cudaSuccess ||
-        cudaFuncSetAttribute(msfm::select_candidates_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msfm::kSelectSmemBytes) != cudaSuccess)
+    for (const bool debug : {false, true})
+        for (const bool collect : {false, true})
+            for (const bool gated : {false, true})
+                if (cudaFuncSetAttribute(match_kernel(debug, collect, gated), cudaFuncAttributeMaxDynamicSharedMemorySize, KCfg::kSmemAlloc) != cudaSuccess)
+                    return bail(MSFM_ERR_CUDA);
+    if (cudaFuncSetAttribute(msfm::select_candidates_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msfm::kSelectSmemBytes) != cudaSuccess)
         return bail(MSFM_ERR_CUDA);
     if (ctx->debug_flags & 8u) {
         if (cudaMalloc(&ctx->dbg_stats.ptr, 512) != cudaSuccess) return bail(MSFM_ERR_OUT_OF_MEMORY);
@@ -1768,34 +1771,14 @@ msfm_status msfm_colbest(msfm_ctx *ctx, int32_t ref_id, int32_t query_id, int32_
 }
 
 msfm_status msfm_match_pairs(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pairs, const msfm_params *params, msfm_result *out) {
-    if (!ctx) return MSFM_ERR_INVALID_ARG;
-    if (cudaSetDevice(ctx->device) != cudaSuccess) return MSFM_ERR_CUDA;
-    if (!out || (!out->matches && out->match_capacity > 0)) return match_pairs_impl(ctx, pairs, n_pairs, params, nullptr, false, nullptr);
-    CallerBuffers cb{out->matches, out->good, out->match_capacity};
-    OutSpec spec;
-    spec.offsets = out->offsets;
-    spec.ok = out->ok;
-    spec.has_good = out->good != nullptr;
-    spec.sink = caller_sink;
-    spec.user = &cb;
-    return match_pairs_impl(ctx, pairs, n_pairs, params, &spec, false, nullptr);
+    return match_pairs_to_result(ctx, pairs, n_pairs, params, out, nullptr);
 }
 
 msfm_status msfm_match_pairs_guided(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pairs, const msfm_params *params,
                                     const double (*F)[9], float th_epipolar, const float *const *image_xy,
                                     const int32_t *image_npts, int32_t n_images, msfm_result *out) {
-    if (!ctx) return MSFM_ERR_INVALID_ARG;
-    if (cudaSetDevice(ctx->device) != cudaSuccess) return MSFM_ERR_CUDA;
     const GuidedArgs g{F, th_epipolar, image_xy, image_npts, n_images};
-    if (!out || (!out->matches && out->match_capacity > 0)) return match_pairs_impl(ctx, pairs, n_pairs, params, nullptr, false, nullptr, &g);
-    CallerBuffers cb{out->matches, out->good, out->match_capacity};
-    OutSpec spec;
-    spec.offsets = out->offsets;
-    spec.ok = out->ok;
-    spec.has_good = out->good != nullptr;
-    spec.sink = caller_sink;
-    spec.user = &cb;
-    return match_pairs_impl(ctx, pairs, n_pairs, params, &spec, false, nullptr, &g);
+    return match_pairs_to_result(ctx, pairs, n_pairs, params, out, &g);
 }
 
 msfm_status msfm_internal_match_pairs_sink(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pairs, const msfm_params *params, int64_t *offsets,
