@@ -18,15 +18,15 @@ namespace msfm {
 // Quantisation rule (mirrored by oracle_quantize_f32): q = min(255, max(0, rint(x * scale))), NaN -> 0.
 // resid (keep_float contexts, else null): per row the quantisation residual r = ||scale*x - q||_2, rounded up, and
 // *rmax the largest residual of the image (the exact kNN mode's candidate bound, see exact_threshold).
-__global__ void pack_f32_kernel(const float *__restrict__ src, int64_t src_stride_floats, int rows, int rows_padded,
-                                float scale, uint8_t *__restrict__ dst, int32_t *__restrict__ ckeys,
+__global__ void pack_f32_kernel(const float *__restrict__ src, int rows, int rows_padded, float scale,
+                                uint8_t *__restrict__ dst, int32_t *__restrict__ ckeys,
                                 float *__restrict__ resid = nullptr, float *__restrict__ rmax = nullptr) {
     const int warps_per_block = blockDim.x >> 5;
     const int lane = threadIdx.x & 31;
     for (int r = blockIdx.x * warps_per_block + (threadIdx.x >> 5); r < rows_padded; r += gridDim.x * warps_per_block) {
         uint32_t packed = 0, nrm = kNormPad;
         if (r < rows) {
-            const float *s = src + (int64_t)r * src_stride_floats + lane * 4;
+            const float *s = src + (int64_t)r * kDim + lane * 4;
             const float f[4] = {s[0], s[1], s[2], s[3]};
             uint32_t acc = 0;
             double e2 = 0.0;  // x*scale is exact in double (24 x 24 bit significands), so is its distance to q
@@ -61,21 +61,22 @@ __global__ void pack_f32_kernel(const float *__restrict__ src, int64_t src_strid
     }
 }
 
-__global__ void pack_u8_kernel(const uint8_t *__restrict__ src, int64_t src_stride_bytes, int rows, int rows_padded,
-                               uint8_t *__restrict__ dst, int32_t *__restrict__ ckeys) {
+// u8 rows already copied to their place in the arena: keys for every row, zero bytes for the pad rows.
+__global__ void pack_u8_kernel(int rows, int rows_padded, uint8_t *__restrict__ rows_inout, int32_t *__restrict__ ckeys) {
     const int warps_per_block = blockDim.x >> 5;
     const int lane = threadIdx.x & 31;
     for (int r = blockIdx.x * warps_per_block + (threadIdx.x >> 5); r < rows_padded; r += gridDim.x * warps_per_block) {
-        uint32_t packed = 0, nrm = kNormPad;
+        uint32_t *row = reinterpret_cast<uint32_t *>(rows_inout + (int64_t)r * kDim);
+        uint32_t nrm = kNormPad;
         if (r < rows) {
-            const uint8_t *s8 = src + (int64_t)r * src_stride_bytes + lane * 4;
-            packed = (uint32_t)s8[0] | ((uint32_t)s8[1] << 8) | ((uint32_t)s8[2] << 16) | ((uint32_t)s8[3] << 24);
+            const uint32_t packed = row[lane];
             uint32_t acc = __dp4a(packed, packed, 0u);
 #pragma unroll
             for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xFFFFFFFFu, acc, o);
             nrm = acc;
+        } else {
+            row[lane] = 0u;
         }
-        reinterpret_cast<uint32_t *>(dst + (int64_t)r * kDim)[lane] = packed;
         if (lane == 0) ckeys[r] = make_ckey(nrm, r);
     }
 }

@@ -13,6 +13,7 @@
 #include <mutex>
 #include <new>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include <cuda.h>
@@ -97,14 +98,14 @@ struct msfm_ctx {
     int num_sms = 0;
     cudaStream_t stream = nullptr;         // matching: plans, kernels, result copies
     cudaStream_t upload_stream = nullptr;  // table changes: packer launches, tensor maps, pad rows (overlaps matching)
-    cudaStream_t copy_stream = nullptr;    // host->device copies of the asynchronous batch uploads: they never queue behind a
-                                           // packer launch that is waiting for an SM (the matching kernel is persistent)
+    cudaStream_t copy_stream = nullptr;    // host->device copies of every table upload: they never queue behind a packer
+                                           // launch that is waiting for an SM (the matching kernel is persistent)
     cudaEvent_t ev_copy = nullptr;
     cudaStream_t d2h_stream = nullptr;     // match lists of batch k go back to the host under batch k+1's kernels
     cudaEvent_t ev_d2h0 = nullptr, ev_d2h1 = nullptr;  // brackets of the list copy in flight (timed)
     bool d2h_in_flight = false;
-    struct StageBuf { void *ptr; size_t bytes; cudaEvent_t done; bool used; };
-    std::vector<StageBuf> stage_pool;      // float staging of msfm_upload_f32_batch_async calls still in flight
+    struct StageBuf { void *ptr; size_t bytes; cudaEvent_t done; };
+    std::vector<StageBuf> stage_pool;      // float rows of plain-context msfm_upload_f32* calls, until their packers have run
     std::vector<UploadMark> marks;         // asynchronous uploads still to be ordered before matching launches
     std::vector<cudaEvent_t> event_pool;
     uint64_t upload_seq = 0, waited_seq = 0;
@@ -136,7 +137,7 @@ struct msfm_ctx {
     bool force_twin = false;               // msfm_test_force_twin_pass
     bool no_prune = false;                 // msfm_test_disable_pruning: the forward pass keeps exact 2-NN rows for every query row
     DeviceBuf kp_xy;                       // msfm_match_pairs_guided: keypoints (x, y) per arena row (allocated on the first call)
-    DeviceBuf staging, knn, matches, good, counts, offsets, pairdesc, items, tight_matches, tight_good;
+    DeviceBuf knn, matches, good, counts, offsets, pairdesc, items, tight_matches, tight_good;
     DeviceBuf tight_matches_b, tight_good_b;  // second set: a batch's lists are copied out while the next batch is gathered
     void *h_pinned = nullptr;
     size_t h_pinned_bytes = 0;
@@ -170,10 +171,9 @@ msfm_status fail(msfm_ctx *ctx, msfm_status st, const char *fmt, ...) {
                         "%s failed: %s (%s:%d)", #call, cudaGetErrorString(e__), __FILE__, __LINE__);          \
     } while (0)
 
-msfm_status ensure(msfm_ctx *ctx, DeviceBuf &b, size_t bytes, cudaStream_t also = nullptr) {
+msfm_status ensure(msfm_ctx *ctx, DeviceBuf &b, size_t bytes) {
     if (b.bytes >= bytes && b.ptr) return MSFM_OK;
     if (b.ptr) {
-        if (also) MSFM_CUDA(ctx, cudaStreamSynchronize(also));
         MSFM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
         MSFM_CUDA(ctx, cudaFree(b.ptr));
         b.ptr = nullptr;
@@ -1324,7 +1324,7 @@ msfm_status msfm_destroy(msfm_ctx *ctx) {
     if (ctx->resid) cudaFree(ctx->resid);
     if (ctx->img_rmax) cudaFree(ctx->img_rmax);
     DeviceBuf *bufs[] = {&ctx->knn_ids, &ctx->knn_dists, &ctx->knn_ids_b, &ctx->knn_dists_b, &ctx->band_q, &ctx->band_counts, &ctx->band_thr, &ctx->band_state, &ctx->band_events, &ctx->band_event_keys, &ctx->band_event_count, &ctx->cand_q, &ctx->cand_j, &ctx->cand_d0, &ctx->cand_good, &ctx->cand_counts, &ctx->cand_desc, &ctx->cand_ckeys, &ctx->colbest, &ctx->twin_counts, &ctx->tilemin,
-                         &ctx->kp_xy, &ctx->staging, &ctx->knn, &ctx->matches, &ctx->good, &ctx->counts, &ctx->offsets,
+                         &ctx->kp_xy, &ctx->knn, &ctx->matches, &ctx->good, &ctx->counts, &ctx->offsets,
                          &ctx->pairdesc, &ctx->items, &ctx->tight_matches, &ctx->tight_good, &ctx->tight_matches_b, &ctx->tight_good_b};
     for (DeviceBuf *b : bufs)
         if (b->ptr) cudaFree(b->ptr);
@@ -1349,11 +1349,12 @@ msfm_status msfm_destroy(msfm_ctx *ctx) {
 }
 
 // ---------------------------------------------------------------------------------------------------- table uploads
-// Everything that changes the packed table (host->device copies, packer launches, tensor-map writes, pad rows) runs on
-// the context's UPLOAD stream, so that staging overlaps matching on the main stream.  The synchronous entry points wait
-// for the upload stream before they return (the images are then simply "ready"); the *_async ones return at once and
-// leave an upload mark — an event on the upload stream plus a sequence number stored in the images it covers.  A matching
-// launch makes the main stream wait for the newest mark among the images it touches (marks complete in order).
+// Everything that changes the packed table (packer launches, tensor-map writes, pad rows) runs on the context's UPLOAD
+// stream, so that staging overlaps matching on the main stream; the host->device copies run on the copy stream, and the
+// upload stream waits for them before the packers.  The synchronous entry points wait for the upload stream before they
+// return (the images are then simply "ready"); the *_async ones return at once and leave an upload mark — an event on
+// the upload stream plus a sequence number stored in the images it covers.  A matching launch makes the main stream wait
+// for the newest mark among the images it touches (marks complete in order).
 static msfm_status finish_upload_sync(msfm_ctx *ctx) {
     MSFM_CUDA(ctx, cudaStreamSynchronize(ctx->upload_stream));
     return MSFM_OK;
@@ -1385,17 +1386,15 @@ static void unreserve_locked(msfm_ctx *ctx, const std::vector<int32_t> &ids) {
     }
 }
 
-// CUDA call inside an upload: on failure the images reserved so far by this call are rolled back.
-#define MSFM_CUDA_UPLOAD(ctx, reserved, call)                                                                   \
-    do {                                                                                                       \
-        cudaError_t e__ = (call);                                                                              \
-        if (e__ != cudaSuccess) {                                                                              \
-            cudaStreamSynchronize((ctx)->upload_stream);                                                       \
-            unreserve_locked(ctx, reserved);                                                                   \
-            return fail(ctx, e__ == cudaErrorMemoryAllocation ? MSFM_ERR_OUT_OF_MEMORY : MSFM_ERR_CUDA,         \
-                        "%s failed: %s (%s:%d)", #call, cudaGetErrorString(e__), __FILE__, __LINE__);          \
-        }                                                                                                      \
-    } while (0)
+// A CUDA failure after the images in `reserved` were reserved: once no copy or packer launch can still write into their
+// rows, they are rolled back, and `reserved` is left empty.
+static msfm_status fail_reserved(msfm_ctx *ctx, std::vector<int32_t> &reserved, cudaError_t e) {
+    cudaStreamSynchronize(ctx->copy_stream);
+    cudaStreamSynchronize(ctx->upload_stream);
+    unreserve_locked(ctx, reserved);
+    reserved.clear();
+    return fail(ctx, e == cudaErrorMemoryAllocation ? MSFM_ERR_OUT_OF_MEMORY : MSFM_ERR_CUDA, "table upload failed: %s", cudaGetErrorString(e));
+}
 
 msfm_status msfm_reserve(msfm_ctx *ctx, int32_t image_id, int32_t rows, int64_t *row_offset) {
     return msfm_reserve_batch(ctx, 1, &image_id, &rows, row_offset);
@@ -1411,8 +1410,11 @@ static msfm_status reserve_batch_locked(msfm_ctx *ctx, int32_t n, const int32_t 
         const ImageSlot &s = ctx->images[image_ids[i]];
         if (s.rows_padded > s.rows) {
             msfm::init_pad_kernel<<<8, 256, 0, ctx->upload_stream>>>(s.rows, s.rows_padded, ctx->desc + off * kDim, ctx->norms + off);
-            const std::vector<int32_t> one{image_ids[i]};
-            MSFM_CUDA_UPLOAD(ctx, one, cudaGetLastError());
+            const cudaError_t e = cudaGetLastError();
+            if (e != cudaSuccess) {
+                std::vector<int32_t> one{image_ids[i]};
+                return fail_reserved(ctx, one, e);
+            }
         }
         if (row_offsets) row_offsets[i] = off;
     }
@@ -1428,110 +1430,142 @@ msfm_status msfm_reserve_batch(msfm_ctx *ctx, int32_t n, const int32_t *image_id
     return st != MSFM_OK ? st : fin;
 }
 
-// One image, enqueued on the upload stream without a host sync.  Contiguous rows go straight into the arena and are
-// keyed in place; strided rows pass through the staging buffer (which must not be reused before the stream got there).
-static msfm_status upload_u8_enqueue(msfm_ctx *ctx, int32_t image_id, const uint8_t *desc, int32_t rows, int64_t row_stride_bytes,
-                                     bool *used_staging) {
-    if ((rows > 0 && !desc) || row_stride_bytes < kDim) return fail(ctx, MSFM_ERR_INVALID_ARG, "null descriptors or stride < 128 bytes");
-    int64_t off = 0;
-    msfm_status st = reserve_locked(ctx, image_id, rows, &off);
-    if (st != MSFM_OK) return st;
-    const std::vector<int32_t> mine{image_id};
-    const ImageSlot &s = ctx->images[image_id];
-    const int blocks = std::max(1, std::min(4 * ctx->num_sms, (s.rows_padded + 7) / 8));
-    const uint8_t *src = ctx->desc + off * kDim;
-    int64_t src_stride = kDim;
-    if (row_stride_bytes == kDim) {
-        if (rows > 0) MSFM_CUDA_UPLOAD(ctx, mine, cudaMemcpyAsync(ctx->desc + off * kDim, desc, (size_t)rows * kDim, cudaMemcpyHostToDevice, ctx->upload_stream));
-    } else {
-        const size_t bytes = rows > 0 ? (size_t)(rows - 1) * row_stride_bytes + kDim : 0;
-        if ((st = ensure(ctx, ctx->staging, bytes, ctx->upload_stream)) != MSFM_OK) { unreserve_locked(ctx, mine); return st; }
-        if (bytes) MSFM_CUDA_UPLOAD(ctx, mine, cudaMemcpyAsync(ctx->staging.ptr, desc, bytes, cudaMemcpyHostToDevice, ctx->upload_stream));
-        src = static_cast<const uint8_t *>(ctx->staging.ptr);
-        src_stride = row_stride_bytes;
-        *used_staging = true;
+// A float staging buffer of at least `bytes` that no queued packer launch still reads: a pool buffer whose last user's
+// packers have run (an event never recorded counts as complete), else a new one of at least 64 MiB.
+static cudaError_t take_stage(msfm_ctx *ctx, size_t bytes, msfm_ctx::StageBuf **out) {
+    for (msfm_ctx::StageBuf &b : ctx->stage_pool)
+        if (b.bytes >= bytes && cudaEventQuery(b.done) == cudaSuccess) {
+            *out = &b;
+            return cudaSuccess;
+        }
+    msfm_ctx::StageBuf nb{nullptr, std::max<size_t>(bytes, (size_t)64 << 20), nullptr};
+    cudaError_t e = cudaMalloc(&nb.ptr, nb.bytes);
+    if (e != cudaSuccess) return e;
+    if ((e = cudaEventCreateWithFlags(&nb.done, cudaEventDisableTiming)) != cudaSuccess) {
+        cudaFree(nb.ptr);
+        return e;
     }
-    msfm::pack_u8_kernel<<<blocks, 256, 0, ctx->upload_stream>>>(src, src_stride, rows, s.rows_padded, ctx->desc + off * kDim, ctx->norms + off);
-    MSFM_CUDA_UPLOAD(ctx, mine, cudaGetLastError());
-    return MSFM_OK;
+    ctx->stage_pool.push_back(nb);
+    *out = &ctx->stage_pool.back();
+    return cudaSuccess;
 }
+
+// The one path of the five upload entry points: images [0, n) of a call, u8 or float rows `strides[i]` elements apart
+// (strides null: dense rows).  `dense_only` names an entry point that refuses strided rows.
+//  1. Each image is checked and reserved in turn; the first failing one ends the loop, the images before it are uploaded.
+//  2. Every destination is dense: u8 rows go to the arena, float rows to the retained float rows of a keep_float context,
+//     else to one staging buffer of this call.
+//  3. The host->device copies are queued back to back on the copy stream, so they never wait behind a packer launch that
+//     waits for an SM (the matching kernel is persistent).  Images adjacent both in host memory and in the destination
+//     are one copy; strided rows are one 2-D copy each.
+//  4. The packers follow on the upload stream: u8 rows are keyed in place, one launch per copy (images start on
+//     multiples of kAlignRows, so row % 8 and with it the column keys do not depend on where a copy starts; only its
+//     last image can have pad rows); float rows are quantised per image (each image has its own largest residual).
+// A CUDA failure rolls back every image of the call.  `uploaded` receives the images queued.
+extern "C++" {  // a template cannot have C linkage
+template <typename T>
+static msfm_status upload_locked(msfm_ctx *ctx, int32_t n, const int32_t *image_ids, const T *const *descs, const int32_t *rows,
+                                 const int64_t *strides, float scale, const char *dense_only, std::vector<int32_t> &uploaded) {
+    constexpr bool kFloat = std::is_same<T, float>::value;
+    MSFM_CUDA(ctx, cudaSetDevice(ctx->device));
+    struct Job { int32_t id; const T *src; int64_t stride; T *dst; };
+    std::vector<Job> jobs;
+    msfm_status st = MSFM_OK;
+    for (int32_t i = 0; i < n; ++i) {
+        const int64_t stride = strides ? strides[i] : kDim;
+        if (stride != kDim && dense_only) { st = fail(ctx, MSFM_ERR_INVALID_ARG, "%s takes contiguous 128-byte rows only", dense_only); break; }
+        if (rows[i] > 0 && !descs[i] && stride == kDim) { st = fail(ctx, MSFM_ERR_INVALID_ARG, "null descriptors"); break; }
+        if ((rows[i] > 0 && !descs[i]) || stride < kDim) {
+            st = fail(ctx, MSFM_ERR_INVALID_ARG, "null descriptors or stride < 128 %s", kFloat ? "floats" : "bytes");
+            break;
+        }
+        if ((st = reserve_locked(ctx, image_ids[i], rows[i], nullptr)) != MSFM_OK) break;
+        uploaded.push_back(image_ids[i]);
+        jobs.push_back({image_ids[i], descs[i], stride, nullptr});
+    }
+    cudaError_t e = cudaSuccess;
+    msfm_ctx::StageBuf *stage = nullptr;
+    if (kFloat && !ctx->fdesc) {
+        size_t bytes = 0;
+        for (const Job &j : jobs) bytes += (size_t)ctx->images[j.id].rows * kDim * sizeof(float);
+        if (bytes > 0 && (e = take_stage(ctx, bytes, &stage)) != cudaSuccess) return fail_reserved(ctx, uploaded, e);
+    }
+    struct Run { const T *src; int64_t stride; T *dst; int64_t off, rows, rows_padded; };
+    std::vector<Run> runs;
+    size_t stage_pos = 0;
+    for (Job &j : jobs) {
+        ImageSlot &s = ctx->images[j.id];
+        if constexpr (kFloat) {
+            if (ctx->fdesc) {
+                j.dst = ctx->fdesc + s.off * kDim;
+                if (s.rows > 0) {
+                    s.has_float = true;
+                    s.scale = scale;
+                }
+            } else {
+                j.dst = static_cast<float *>(stage ? stage->ptr : nullptr) + stage_pos;
+                stage_pos += (size_t)s.rows * kDim;
+            }
+        } else {
+            j.dst = ctx->desc + s.off * kDim;
+        }
+        Run *last = runs.empty() ? nullptr : &runs.back();
+        if (last && j.stride == kDim && last->stride == kDim && j.src == last->src + last->rows * kDim &&
+            j.dst == last->dst + last->rows * kDim && last->rows + s.rows_padded < (int64_t)INT32_MAX) {
+            last->rows += s.rows;
+            last->rows_padded += s.rows_padded;
+        } else {
+            runs.push_back({j.src, j.stride, j.dst, s.off, s.rows, s.rows_padded});
+        }
+    }
+    for (const Run &r : runs) {
+        if (r.rows == 0) continue;
+        e = r.stride == kDim ? cudaMemcpyAsync(r.dst, r.src, (size_t)r.rows * kDim * sizeof(T), cudaMemcpyHostToDevice, ctx->copy_stream)
+                             : cudaMemcpy2DAsync(r.dst, kDim * sizeof(T), r.src, (size_t)r.stride * sizeof(T), kDim * sizeof(T), (size_t)r.rows,
+                                                 cudaMemcpyHostToDevice, ctx->copy_stream);
+        if (e != cudaSuccess) return fail_reserved(ctx, uploaded, e);
+    }
+    if (!jobs.empty()) {
+        if ((e = cudaEventRecord(ctx->ev_copy, ctx->copy_stream)) != cudaSuccess) return fail_reserved(ctx, uploaded, e);
+        if ((e = cudaStreamWaitEvent(ctx->upload_stream, ctx->ev_copy, 0)) != cudaSuccess) return fail_reserved(ctx, uploaded, e);
+    }
+    if constexpr (kFloat) {
+        for (const Job &j : jobs) {
+            const ImageSlot &s = ctx->images[j.id];
+            const int blocks = std::max(1, std::min(4 * ctx->num_sms, (s.rows_padded + 7) / 8));
+            msfm::pack_f32_kernel<<<blocks, 256, 0, ctx->upload_stream>>>(j.dst, s.rows, s.rows_padded, scale, ctx->desc + s.off * kDim, ctx->norms + s.off,
+                                                                          ctx->resid ? ctx->resid + s.off : nullptr, ctx->img_rmax ? ctx->img_rmax + j.id : nullptr);
+            if ((e = cudaGetLastError()) != cudaSuccess) return fail_reserved(ctx, uploaded, e);
+        }
+        if (stage && (e = cudaEventRecord(stage->done, ctx->upload_stream)) != cudaSuccess) return fail_reserved(ctx, uploaded, e);
+    } else {
+        for (const Run &r : runs) {
+            const int blocks = (int)std::max<int64_t>(1, std::min<int64_t>(8 * ctx->num_sms, (r.rows_padded + 7) / 8));
+            msfm::pack_u8_kernel<<<blocks, 256, 0, ctx->upload_stream>>>((int)r.rows, (int)r.rows_padded, r.dst, ctx->norms + r.off);
+            if ((e = cudaGetLastError()) != cudaSuccess) return fail_reserved(ctx, uploaded, e);
+        }
+    }
+    return st;
+}
+}  // extern "C++"
 
 msfm_status msfm_upload_u8(msfm_ctx *ctx, int32_t image_id, const uint8_t *desc, int32_t rows, int64_t row_stride_bytes) {
     if (!ctx) return MSFM_ERR_INVALID_ARG;
     std::lock_guard<std::mutex> lock(ctx->mu);
-    MSFM_CUDA(ctx, cudaSetDevice(ctx->device));
-    bool staged = false;
-    msfm_status st = upload_u8_enqueue(ctx, image_id, desc, rows, row_stride_bytes, &staged);
+    if ((rows > 0 && !desc) || row_stride_bytes < kDim) return fail(ctx, MSFM_ERR_INVALID_ARG, "null descriptors or stride < 128 bytes");
+    std::vector<int32_t> uploaded;
+    const msfm_status st = upload_locked(ctx, 1, &image_id, &desc, &rows, &row_stride_bytes, 0.0f, nullptr, uploaded);
     if (st != MSFM_OK) return st;
     return finish_upload_sync(ctx);  // the caller may free `desc` on return
-}
-
-// Batch upload.  Contiguous-row images are reserved first, their host->device copies are queued back to back (runs
-// that are adjacent both in host memory and in the arena become one copy) and the packer launches follow, so the copy
-// engine is not held up by the keying kernels in between; strided images take the per-image staging path.
-// `uploaded` receives the ids this call staged (for the upload mark of the asynchronous variant).
-static msfm_status upload_u8_batch_locked(msfm_ctx *ctx, int32_t n, const int32_t *image_ids, const uint8_t *const *descs, const int32_t *rows,
-                                          const int64_t *row_stride_bytes, bool allow_strided, std::vector<int32_t> &uploaded) {
-    if (n < 0 || (n > 0 && (!image_ids || !descs || !rows))) return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_upload_u8_batch: null argument");
-    MSFM_CUDA(ctx, cudaSetDevice(ctx->device));
-    msfm_status st = MSFM_OK;
-    // A run = images adjacent both in host memory and in the arena: one copy, one packer launch (images start on
-    // multiples of kAlignRows, so row % 8 and with it the column keys do not depend on where the run starts; only the
-    // last image of a run can have pad rows).
-    struct Run { const uint8_t *src; int64_t off; int64_t rows, rows_padded; };
-    std::vector<Run> runs;
-    std::vector<int32_t> in_runs;  // reserved here, copies not queued yet
-    for (int32_t i = 0; i < n && st == MSFM_OK; ++i) {
-        const int64_t stride = row_stride_bytes ? row_stride_bytes[i] : kDim;
-        if (stride != kDim) {
-            if (!allow_strided) { st = fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_upload_u8_batch_async takes contiguous 128-byte rows only"); break; }
-            bool staged = false;
-            st = upload_u8_enqueue(ctx, image_ids[i], descs[i], rows[i], stride, &staged);
-            if (st == MSFM_OK) {
-                uploaded.push_back(image_ids[i]);
-                if (staged) MSFM_CUDA_UPLOAD(ctx, in_runs, cudaStreamSynchronize(ctx->upload_stream));  // the staging buffer is reused by the next image
-            }
-            continue;
-        }
-        if (rows[i] > 0 && !descs[i]) { st = fail(ctx, MSFM_ERR_INVALID_ARG, "null descriptors"); break; }
-        int64_t off = 0;
-        if ((st = reserve_locked(ctx, image_ids[i], rows[i], &off)) != MSFM_OK) break;
-        in_runs.push_back(image_ids[i]);
-        const ImageSlot &sl = ctx->images[image_ids[i]];
-        if (!runs.empty() && runs.back().rows == runs.back().rows_padded && off == runs.back().off + runs.back().rows &&
-            descs[i] == runs.back().src + runs.back().rows * kDim && runs.back().rows + sl.rows_padded < (int64_t)INT32_MAX) {
-            runs.back().rows += sl.rows;
-            runs.back().rows_padded += sl.rows_padded;
-        } else {
-            runs.push_back({descs[i], off, sl.rows, sl.rows_padded});
-        }
-    }
-    // On an argument error the images before the failing one stay uploaded (documented); a CUDA failure below rolls back
-    // every image whose rows this call has not provably written.
-    // copies back to back on the copy stream (never held up by a keying kernel that waits for an SM), keys afterwards
-    for (const Run &r : runs)
-        if (r.rows > 0) MSFM_CUDA_UPLOAD(ctx, in_runs, cudaMemcpyAsync(ctx->desc + r.off * kDim, r.src, (size_t)r.rows * kDim, cudaMemcpyHostToDevice, ctx->copy_stream));
-    if (!runs.empty()) {
-        MSFM_CUDA_UPLOAD(ctx, in_runs, cudaEventRecord(ctx->ev_copy, ctx->copy_stream));
-        MSFM_CUDA_UPLOAD(ctx, in_runs, cudaStreamWaitEvent(ctx->upload_stream, ctx->ev_copy, 0));
-    }
-    for (const Run &r : runs) {    // keys + pad rows, in place
-        if (r.rows_padded == 0) continue;
-        const int blocks = (int)std::max<int64_t>(1, std::min<int64_t>(8 * ctx->num_sms, (r.rows_padded + 7) / 8));
-        uint8_t *d = ctx->desc + r.off * kDim;
-        msfm::pack_u8_kernel<<<blocks, 256, 0, ctx->upload_stream>>>(d, kDim, (int)r.rows, (int)r.rows_padded, d, ctx->norms + r.off);
-        MSFM_CUDA_UPLOAD(ctx, in_runs, cudaGetLastError());
-    }
-    uploaded.insert(uploaded.end(), in_runs.begin(), in_runs.end());
-    return st;
 }
 
 msfm_status msfm_upload_u8_batch(msfm_ctx *ctx, int32_t n, const int32_t *image_ids, const uint8_t *const *descs, const int32_t *rows,
                                  const int64_t *row_stride_bytes) {
     if (!ctx) return MSFM_ERR_INVALID_ARG;
     std::lock_guard<std::mutex> lock(ctx->mu);
+    if (n < 0 || (n > 0 && (!image_ids || !descs || !rows))) return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_upload_u8_batch: null argument");
     std::vector<int32_t> uploaded;
-    const msfm_status st = upload_u8_batch_locked(ctx, n, image_ids, descs, rows, row_stride_bytes, true, uploaded);
+    const msfm_status st = upload_locked(ctx, n, image_ids, descs, rows, row_stride_bytes, 0.0f, nullptr, uploaded);
     const msfm_status fin = finish_upload_sync(ctx);  // one sync for the batch: the caller may free every `descs[i]` on return
     return st != MSFM_OK ? st : fin;
 }
@@ -1540,8 +1574,9 @@ msfm_status msfm_upload_u8_batch_async(msfm_ctx *ctx, int32_t n, const int32_t *
                                        const int64_t *row_stride_bytes) {
     if (!ctx) return MSFM_ERR_INVALID_ARG;
     std::lock_guard<std::mutex> lock(ctx->mu);
+    if (n < 0 || (n > 0 && (!image_ids || !descs || !rows))) return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_upload_u8_batch: null argument");
     std::vector<int32_t> uploaded;
-    const msfm_status st = upload_u8_batch_locked(ctx, n, image_ids, descs, rows, row_stride_bytes, false, uploaded);
+    const msfm_status st = upload_locked(ctx, n, image_ids, descs, rows, row_stride_bytes, 0.0f, "msfm_upload_u8_batch_async", uploaded);
     const msfm_status mk = leave_upload_mark(ctx, uploaded);
     return st != MSFM_OK ? st : mk;
 }
@@ -1556,114 +1591,27 @@ msfm_status msfm_sync(msfm_ctx *ctx) {
     return MSFM_OK;
 }
 
-// float rows of one image: staged at `stage` (device), quantised + keyed into the arena; with keep_float the rows are
-// copied to the float arena first and packed from there (no staging).
-static msfm_status upload_f32_enqueue(msfm_ctx *ctx, int32_t image_id, const float *desc, int32_t rows, int64_t row_stride_floats, float scale,
-                                      float *stage) {
-    const ImageSlot &s = ctx->images[image_id];
-    const std::vector<int32_t> mine{image_id};
-    const int64_t off = s.off;
-    const float *src = stage;
-    int64_t src_stride = row_stride_floats;
-    if (ctx->fdesc && rows > 0) {
-        // straight into the retained float rows (dense 128-float rows), then packed from there
-        MSFM_CUDA_UPLOAD(ctx, mine, cudaMemcpy2DAsync(ctx->fdesc + off * kDim, kDim * sizeof(float), desc, (size_t)row_stride_floats * sizeof(float),
-                                                      kDim * sizeof(float), (size_t)rows, cudaMemcpyHostToDevice, ctx->upload_stream));
-        src = ctx->fdesc + off * kDim;
-        src_stride = kDim;
-        ctx->images[image_id].has_float = true;
-        ctx->images[image_id].scale = scale;
-    } else if (rows > 0) {
-        const size_t bytes = ((size_t)(rows - 1) * row_stride_floats + kDim) * sizeof(float);
-        MSFM_CUDA_UPLOAD(ctx, mine, cudaMemcpyAsync(stage, desc, bytes, cudaMemcpyHostToDevice, ctx->upload_stream));
-    }
-    const int blocks = std::max(1, std::min(4 * ctx->num_sms, (s.rows_padded + 7) / 8));
-    msfm::pack_f32_kernel<<<blocks, 256, 0, ctx->upload_stream>>>(src, src_stride, rows, s.rows_padded, scale, ctx->desc + off * kDim, ctx->norms + off,
-                                                                  ctx->resid ? ctx->resid + off : nullptr, ctx->img_rmax ? ctx->img_rmax + image_id : nullptr);
-    MSFM_CUDA_UPLOAD(ctx, mine, cudaGetLastError());
-    return MSFM_OK;
-}
-
 msfm_status msfm_upload_f32(msfm_ctx *ctx, int32_t image_id, const float *desc, int32_t rows, int64_t row_stride_floats, float scale) {
     if (!ctx) return MSFM_ERR_INVALID_ARG;
     std::lock_guard<std::mutex> lock(ctx->mu);
     if ((rows > 0 && !desc) || row_stride_floats < kDim || !(scale > 0.0f))
         return fail(ctx, MSFM_ERR_INVALID_ARG, "null descriptors, stride < 128 floats or scale <= 0");
-    MSFM_CUDA(ctx, cudaSetDevice(ctx->device));
-    int64_t off = 0;
-    msfm_status st = reserve_locked(ctx, image_id, rows, &off);
+    std::vector<int32_t> uploaded;
+    const msfm_status st = upload_locked(ctx, 1, &image_id, &desc, &rows, &row_stride_floats, scale, nullptr, uploaded);
     if (st != MSFM_OK) return st;
-    const size_t bytes = (rows > 0 && !ctx->fdesc) ? ((size_t)(rows - 1) * row_stride_floats + kDim) * sizeof(float) : 0;
-    if ((st = ensure(ctx, ctx->staging, bytes, ctx->upload_stream)) != MSFM_OK) {
-        unreserve_locked(ctx, std::vector<int32_t>{image_id});
-        return st;
-    }
-    if ((st = upload_f32_enqueue(ctx, image_id, desc, rows, row_stride_floats, scale, static_cast<float *>(ctx->staging.ptr))) != MSFM_OK) return st;
     return finish_upload_sync(ctx);
 }
 
 // Several float images (dense 128-float rows) without a host wait: the rows must sit in page-locked memory and stay
-// valid until msfm_sync() or a later call that returns results.  All host->device copies of the call are queued back to
-// back on the copy stream — into a staging buffer that belongs to this call until its packer launches have run, or
-// straight into the retained float rows — and the packer launches follow on the upload stream.
+// valid until msfm_sync() or a later call that returns results.
 msfm_status msfm_upload_f32_batch_async(msfm_ctx *ctx, int32_t n, const int32_t *image_ids, const float *const *descs, const int32_t *rows,
                                         float scale) {
     if (!ctx) return MSFM_ERR_INVALID_ARG;
     std::lock_guard<std::mutex> lock(ctx->mu);
     if (n < 0 || (n > 0 && (!image_ids || !descs || !rows)) || !(scale > 0.0f))
         return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_upload_f32_batch_async: null argument or scale <= 0");
-    MSFM_CUDA(ctx, cudaSetDevice(ctx->device));
-    size_t total = 0;
-    for (int32_t i = 0; i < n; ++i)
-        if (rows[i] > 0) total += (size_t)rows[i] * kDim * sizeof(float);
-    msfm_status st = MSFM_OK;
-    msfm_ctx::StageBuf *stage = nullptr;
-    if (!ctx->fdesc && total > 0) {
-        for (msfm_ctx::StageBuf &b : ctx->stage_pool)
-            if (b.bytes >= total && (!b.used || cudaEventQuery(b.done) == cudaSuccess)) { stage = &b; break; }
-        if (!stage) {
-            msfm_ctx::StageBuf nb{nullptr, std::max<size_t>(total, (size_t)64 << 20), nullptr, false};
-            MSFM_CUDA(ctx, cudaMalloc(&nb.ptr, nb.bytes));
-            if (cudaEventCreateWithFlags(&nb.done, cudaEventDisableTiming) != cudaSuccess) {
-                cudaFree(nb.ptr);
-                return fail(ctx, MSFM_ERR_CUDA, "cudaEventCreate failed");
-            }
-            ctx->stage_pool.push_back(nb);
-            stage = &ctx->stage_pool.back();
-        }
-        stage->used = true;
-    }
-    struct Job { int32_t id; int32_t rows; const float *src; };
-    std::vector<Job> jobs;
     std::vector<int32_t> uploaded;
-    size_t pos = 0;
-    for (int32_t i = 0; i < n && st == MSFM_OK; ++i) {  // reserve + copies
-        if (rows[i] > 0 && !descs[i]) { st = fail(ctx, MSFM_ERR_INVALID_ARG, "null descriptors"); break; }
-        int64_t off = 0;
-        if ((st = reserve_locked(ctx, image_ids[i], rows[i], &off)) != MSFM_OK) break;
-        uploaded.push_back(image_ids[i]);
-        const size_t bytes = (size_t)std::max(rows[i], 0) * kDim * sizeof(float);
-        float *dst = ctx->fdesc ? ctx->fdesc + off * kDim : reinterpret_cast<float *>(static_cast<char *>(stage ? stage->ptr : nullptr) + pos);
-        if (bytes) MSFM_CUDA_UPLOAD(ctx, uploaded, cudaMemcpyAsync(dst, descs[i], bytes, cudaMemcpyHostToDevice, ctx->copy_stream));
-        if (ctx->fdesc && rows[i] > 0) {
-            ctx->images[image_ids[i]].has_float = true;
-            ctx->images[image_ids[i]].scale = scale;
-        }
-        jobs.push_back({image_ids[i], rows[i], dst});
-        if (!ctx->fdesc) pos += bytes;
-    }
-    if (!jobs.empty()) {
-        MSFM_CUDA_UPLOAD(ctx, uploaded, cudaEventRecord(ctx->ev_copy, ctx->copy_stream));
-        MSFM_CUDA_UPLOAD(ctx, uploaded, cudaStreamWaitEvent(ctx->upload_stream, ctx->ev_copy, 0));
-    }
-    for (const Job &j : jobs) {  // quantise + key
-        const ImageSlot &sl = ctx->images[j.id];
-        const int blocks = std::max(1, std::min(4 * ctx->num_sms, (sl.rows_padded + 7) / 8));
-        msfm::pack_f32_kernel<<<blocks, 256, 0, ctx->upload_stream>>>(j.src, kDim, j.rows, sl.rows_padded, scale, ctx->desc + sl.off * kDim, ctx->norms + sl.off,
-                                                                      ctx->resid ? ctx->resid + sl.off : nullptr, ctx->img_rmax ? ctx->img_rmax + j.id : nullptr);
-        MSFM_CUDA_UPLOAD(ctx, uploaded, cudaGetLastError());
-    }
-    if (stage) MSFM_CUDA_UPLOAD(ctx, uploaded, cudaEventRecord(stage->done, ctx->upload_stream));
+    const msfm_status st = upload_locked(ctx, n, image_ids, descs, rows, nullptr, scale, nullptr, uploaded);
     const msfm_status mk = leave_upload_mark(ctx, uploaded);
     return st != MSFM_OK ? st : mk;
 }
@@ -1804,10 +1752,6 @@ msfm_status msfm_reserve_batch_async(msfm_ctx *ctx, int32_t n, const int32_t *im
         if (image_ids[i] >= 0 && image_ids[i] < ctx->max_images && ctx->images[image_ids[i]].present) ids.push_back(image_ids[i]);
     const msfm_status mk = (st == MSFM_OK) ? leave_upload_mark(ctx, ids) : MSFM_OK;
     return st != MSFM_OK ? st : mk;
-}
-
-msfm_status msfm_internal_reserve_batch_nosync(msfm_ctx *ctx, int32_t n, const int32_t *image_ids, const int32_t *rows) {
-    return msfm_reserve_batch_async(ctx, n, image_ids, rows, nullptr);
 }
 
 msfm_status msfm_internal_mark_on_stream(msfm_ctx *ctx, int32_t n, const int32_t *image_ids, cudaStream_t stream) {

@@ -18,8 +18,6 @@ typedef int (*msfm_sink_fn)(void *user, int64_t first_match, int64_t n_matches, 
 // are plain host arrays).
 MSFM_HIDDEN msfm_status msfm_internal_match_pairs_sink(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pairs, const msfm_params *params,
                                                        int64_t *offsets, int32_t *ok, int want_good, msfm_sink_fn sink, void *user);
-// msfm_reserve_batch without the host wait: pad rows and tensor maps are queued on the upload stream.
-MSFM_HIDDEN msfm_status msfm_internal_reserve_batch_nosync(msfm_ctx *ctx, int32_t n, const int32_t *image_ids, const int32_t *rows);
 // The images become usable once the work queued on `stream` so far has completed (a collective wrote their rows there):
 // leaves an upload mark recorded on that stream.
 MSFM_HIDDEN msfm_status msfm_internal_mark_on_stream(msfm_ctx *ctx, int32_t n, const int32_t *image_ids, cudaStream_t stream);

@@ -197,7 +197,7 @@ msfm_status stage_group(msfm_multi *mm, int32_t n, const int32_t *ids, const int
         DeviceSlot &ds = mm->dev[d];
         for (const Run &r : runs) {
             if (r.owner == d) MM_CTX(mm, ds, upload(ds, r.a, r.b));
-            else MM_CTX(mm, ds, msfm_internal_reserve_batch_nosync(ds.ctx, r.b - r.a, ids + r.a, rows + r.a));
+            else MM_CTX(mm, ds, msfm_reserve_batch_async(ds.ctx, r.b - r.a, ids + r.a, rows + r.a, nullptr));
         }
         if (W > 1) {
             MM_CUDA(mm, cudaSetDevice(ds.device));

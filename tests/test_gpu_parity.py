@@ -55,6 +55,10 @@ def test_packer_roundtrip_and_norms(matcher, golden):
     big[::2] = g["qry"]
     matcher.upload(2, big[::2])
     np.testing.assert_array_equal(matcher.download_packed(2)[0], g["qry"])
+    bigf = np.zeros((2 * g["qry"].shape[0], 128), np.float32)
+    bigf[::2] = g["qry"]
+    matcher.upload(3, bigf[::2], scale=1.0)
+    np.testing.assert_array_equal(matcher.download_packed(3)[0], g["qry"])
 
 
 @pytest.mark.parametrize("case", GOLDEN_CASES)
@@ -618,13 +622,16 @@ def test_build_match_graph_with_gpu_geo_verification(oracle_mod, native_lib, tmp
 
 def test_upload_batch_equals_single_uploads(oracle_mod, matcher):
     """msfm_upload_u8_batch (one host wait per batch; contiguous rows go straight into the arena and are keyed in place)
-    leaves the same table as per-image uploads, including a strided member and an empty image."""
+    leaves the same table as per-image uploads, including two strided members (one with a stride that is not a multiple
+    of 128 bytes) and an empty image."""
     col = synth.Collection(700, seed=13)
-    imgs = [col.image_u8(0, 700), col.image_u8(1, 513), np.empty((0, 128), np.uint8), col.image_u8(3, 64)]
+    imgs = [col.image_u8(0, 700), col.image_u8(1, 513), np.empty((0, 128), np.uint8), col.image_u8(3, 64), col.image_u8(4, 300)]
     big = np.zeros((2 * 513, 128), np.uint8)
     big[::2] = imgs[1]
+    wide = np.zeros((300, 200), np.uint8)                     # a 128-byte ROI at byte 64 of 200-byte rows
+    wide[:, 64:192] = imgs[4]
     matcher.release_all()
-    matcher.upload_batch([0, 1, 2, 3], [imgs[0], big[::2], imgs[2], imgs[3]])
+    matcher.upload_batch([0, 1, 2, 3, 4], [imgs[0], big[::2], imgs[2], imgs[3], wide[:, 64:192]])
     for i, d in enumerate(imgs):
         got, norms = matcher.download_packed(i)
         np.testing.assert_array_equal(got, d)
@@ -667,6 +674,48 @@ def test_upload_batch_async_overlaps_and_matches(oracle_mod, matcher):
     strided = np.zeros((200, 256), np.uint8)[:, :128]
     with pytest.raises(MsfmError):
         matcher.upload_batch([0], [strided], wait=False)
+
+
+def test_upload_f32_three_ways_equal():
+    """The same float images uploaded with contiguous rows, with strided rows and with msfm_upload_f32_batch_async from
+    adjacent page-locked views (adjacent images coalesced into one copy) leave identical tables, and on a keep_float
+    context identical retained float rows, residuals and largest residuals: msfm_knn2_pairs in exact fp32 mode gives
+    identical arrays."""
+    import torch
+    from metricsfm_b200.matcher import Matcher
+    col = synth.Collection(768, seed=15)
+    rows = [768, 512, 300, 0, 256]                       # 768 and 512 rows are adjacent in the arena too
+    imgs = [col.image_unit(i, r) for i, r in enumerate(rows)]
+    host = torch.from_numpy(np.concatenate(imgs)).pin_memory()
+    bounds = np.cumsum([0] + rows)
+    views = [host[a:b] for a, b in zip(bounds[:-1], bounds[1:])]
+    pairs = [(0, 1), (1, 2), (2, 4), (4, 0), (1, 0)]
+
+    def strided(x):
+        big = np.zeros((2 * x.shape[0], 128), np.float32)
+        big[::2] = x
+        return big[::2]
+
+    for keep_float in (True, False):
+        out = []
+        for how in ("contiguous", "strided", "batch_async"):
+            with Matcher(device=0, max_images=8, arena_rows=1 << 15, keep_float=keep_float) as m:
+                if how == "batch_async":
+                    m.upload_f32_batch_async(list(range(len(rows))), views, scale=512.0)
+                    m.sync()
+                else:
+                    for i, x in enumerate(imgs):
+                        m.upload(i, x if how == "contiguous" else strided(x), scale=512.0)
+                tables = [m.download_packed(i) for i in range(len(rows))]
+                knn = m.knn2_pairs(pairs, exact_f32=keep_float)
+            out.append((how, tables, knn))
+        _, tables0, knn0 = out[0]
+        for how, tables, knn in out[1:]:
+            for (d0, n0), (d, n) in zip(tables0, tables):
+                np.testing.assert_array_equal(d, d0, err_msg=f"{how} keep_float {keep_float}")
+                np.testing.assert_array_equal(n, n0, err_msg=f"{how} keep_float {keep_float}")
+            for a0, a in zip(knn0, knn):
+                np.testing.assert_array_equal(a, a0, err_msg=f"{how} keep_float {keep_float}")
 
 
 def test_reserve_batch_equals_single_reserves(matcher):
