@@ -59,6 +59,25 @@
  *   match on the fp32 nearest allowed row.  Every other row keeps the integer guided decision; the allowed set is the
  *   same in both arithmetics, so a row with fewer than two allowed rows is never a band row and stays rejected.  With
  *   mutual = 1 the check is the float regime's heuristic filter of the one-way list, under the gate (not exact in fp32).
+ *
+ * HOMOG-SPEC (msfm_match_pairs_guided_homography): MATCH-SPEC with the candidate set of every query row restricted to the
+ *   reference rows whose keypoint the pair's homography carries to within th of the query keypoint.  H is given as
+ *   msfm_geo_homography writes it (double[9], row-major, p_q ~ H p_r with p_r a keypoint of the reference image and p_q
+ *   one of the query image, centred feature-file coordinates) and rounded once to float h[9]; t2 = th*th in fp32
+ *   (th = th_transfer).  Every operation below is one IEEE fp32 rounding, with no fused multiply-add:
+ *     reference row j at (xj, yj):  U = ((h0*xj) + (h1*yj)) + h2,  V = ((h3*xj) + (h4*yj)) + h5,  W = ((h6*xj) + (h7*yj)) + h8
+ *     query row q at (xq, yq):      du = U - (xq*W),  dv = V - (yq*W)
+ *     element (q, j) is allowed iff (du*du) + (dv*dv) <= t2 * (W*W)
+ *   i.e. the squared transfer distance |p_q - pi(H p_j)|^2 <= th^2 without the division; it does not depend on the sign
+ *   of H, and W = 0 bars the element unless U = V = 0 too (only possible for a singular H).  Everything else is
+ *   GUIDED-SPEC's integer rule unchanged: nn0 / nn1 are the two closest allowed reference rows (lowest index on ties), a
+ *   row with fewer than two allowed rows gets id -1 / +inf and is rejected, ratio, ratio_good, max_dist_sq,
+ *   MSFM_RATIO_REJECT_GT, orientation and min_keypoints as in MATCH-SPEC, and the mutual check keeps (q, nn0) iff q is
+ *   the closest allowed query row of nn0.  There is no float regime under this gate (rescore_band must be 0).
+ *   Caution: at th of a few pixels the disc around pi(H p_j) seldom holds two reference keypoints at ordinary keypoint
+ *   densities, and a row with fewer than two allowed rows is rejected.  The gate then keeps only rows that have a second
+ *   keypoint inside the disc (e.g. a second orientation at the same location), and can keep far fewer true matches than
+ *   msfm_match_pairs or the epipolar gate (DESIGN.md §8c).
  */
 #ifndef MSFM_MATCH_H_
 #define MSFM_MATCH_H_
@@ -303,6 +322,33 @@ msfm_status msfm_geo_ransac(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pai
                             const int32_t *image_npts, int32_t n_images, const msfm_geo_params *gp, int32_t *pair_ok,
                             int32_t *pair_inliers, uint8_t *inlier_mask, double *F);
 
+/* msfm_geo_ransac with a homography model, p_q ~ H p_r (matches in orientation 0: reference keypoint -> query keypoint;
+ * cv::findHomography(RANSAC, th) without its refinement).  gp->th_epipolar is the transfer threshold in pixels.  Shared
+ * with msfm_geo_ransac: the used matches (a strided subsample above 2048, in list order), the isotropic scale
+ * s = 1 / max(1, max |coordinate| of those points) in fp32, the counter-based draws from (seed, pair_index_base + p, h),
+ * the winner (most inliers, then lowest hypothesis id h), and the decision: inliers of the returned H among all used
+ * matches in double, pair_ok iff >= max(min_points, 4) used matches, a model exists and inliers >= min_inliers.
+ * The search, step by step (hypotheses h = 0 .. iters-1, iters 0 = 1024):
+ *   sample   4 distinct indices of the scaled points, drawn like msfm_geo_ransac's 7 (each slot repeats the draw until new)
+ *   subset   an orientation test derived from cv::findHomography's checkSubset: for each triple {0,1,2}, {1,2,3},
+ *            {0,2,3}, {0,1,3}, the product det[p_a p_b p_c] (reference, homogeneous, double) * det[...] (query) must not
+ *            be negative, otherwise the sample gives no model.  Stricter than OpenCV, which also accepts a sample whose
+ *            four triples all flip (a mirror); OpenCV's collinearity test (haveCollinearPoints) is not applied
+ *   solver   normalised DLT: the 8 x 9 system with rows (x, y, 1, 0, 0, 0, -u x, -u y, -u) and (0, 0, 0, x, y, 1, -v x,
+ *            -v y, -v) per correspondence (x, y) -> (u, v), in double, Gauss-Jordan elimination with full pivoting (as the
+ *            7-point solver of msfm_geo_ransac; a pivot below 1e-12 means no model), h = the null vector with the free
+ *            component 1, divided by its norm, rounded to fp32
+ *   score    cv::findHomography's one-sided reprojection error |p_q - pi(H p_r)|^2 in fp32 on the scaled points,
+ *            inlier iff <= (th*s)^2; a zero or non-finite w = (H p_r)_2 makes the match an outlier
+ *   result   H in pixel coordinates (T^-1 H' T, T = diag(s, s, 1)), scaled so that H22 = 1 unless
+ *            |H22| <= 1e-12 |H| (then to unit norm); no Levenberg-Marquardt refinement
+ * inlier_mask[k] = 1 iff match k is used and its double-precision error against the returned H is <= th^2.  H[n_pairs][9]
+ * row-major (zero for rejected pairs) or NULL.  Errors as msfm_geo_ransac. */
+msfm_status msfm_geo_homography(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pairs, const int64_t *offsets,
+                                const int32_t (*matches)[2], const uint8_t *use, const float *const *image_xy,
+                                const int32_t *image_npts, int32_t n_images, const msfm_geo_params *gp,
+                                int32_t *pair_ok, int32_t *pair_inliers, uint8_t *inlier_mask, double *H);
+
 /* ---- guided re-matching of verified pairs (GUIDED-SPEC above) ------------------------------------------------- */
 /* msfm_match_pairs with each query row's 2-NN searched only among the reference rows consistent with F[p] (typically
  * msfm_geo_verify's F of the pairs with pair_ok).  image_xy / image_npts / n_images as in msfm_geo_verify; image_npts[i]
@@ -318,6 +364,14 @@ msfm_status msfm_match_pairs_guided(msfm_ctx *ctx, const msfm_pair *pairs, int64
                                     const double (*F)[9], float th_epipolar,
                                     const float *const *image_xy, const int32_t *image_npts, int32_t n_images,
                                     msfm_result *out);
+/* msfm_match_pairs with each query row's 2-NN searched only among the reference rows that H[p] carries to within
+ * th_transfer pixels of the row's keypoint (HOMOG-SPEC above; typically msfm_geo_homography's H of the pairs with
+ * pair_ok).  Arguments, results, timing and errors as msfm_match_pairs_guided with H in place of F and th_transfer in
+ * place of th_epipolar, and every rescore_band > 0 is refused with INVALID_ARG. */
+msfm_status msfm_match_pairs_guided_homography(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pairs,
+                                               const msfm_params *params, const double (*H)[9], float th_transfer,
+                                               const float *const *image_xy, const int32_t *image_npts, int32_t n_images,
+                                               msfm_result *out);
 
 /* ---- GPU-side cross-check kernel (CUDA cores, dp4a); used by the tests to localise faults, never by the fast path */
 msfm_status msfm_knn2_crosscheck(msfm_ctx *ctx, int32_t ref_id, int32_t query_id, int32_t *ids, float *dists);

@@ -26,7 +26,8 @@ EXPORTED_SYMBOLS = [
     "msfm_download_packed", "msfm_knn2", "msfm_colbest", "msfm_match_pairs", "msfm_match_pairs_resident",
     "msfm_last_timing", "msfm_get_stream", "msfm_knn2_crosscheck", "msfm_geo_verify", "msfm_geo_ransac",
     "msfm_upload_f32_batch_async", "msfm_get_upload_stream", "msfm_wait_event", "msfm_test_set_band_event_cap", "msfm_test_force_twin_pass", "msfm_test_disable_pruning", "msfm_reserve_batch_async", "msfm_host_alloc", "msfm_host_free", "msfm_device_memory",
-    "msfm_knn2_pairs", "msfm_test_last_knn_stats", "msfm_match_pairs_guided",
+    "msfm_knn2_pairs", "msfm_test_last_knn_stats", "msfm_match_pairs_guided", "msfm_geo_homography",
+    "msfm_match_pairs_guided_homography",
 ]
 
 
@@ -124,6 +125,7 @@ def load() -> C.CDLL:
     L.msfm_match_pairs.argtypes = [vp, vp, C.c_int64, C.POINTER(Params), C.POINTER(Result)]
     L.msfm_match_pairs_guided.argtypes = [vp, vp, C.c_int64, C.POINTER(Params), vp, C.c_float, vp, vp, C.c_int32,
                                           C.POINTER(Result)]
+    L.msfm_match_pairs_guided_homography.argtypes = L.msfm_match_pairs_guided.argtypes
     L.msfm_match_pairs_resident.argtypes = [vp, vp, C.c_int64, C.POINTER(Params), _i64p]
     L.msfm_last_timing.argtypes = [vp, C.POINTER(Timing)]
     L.msfm_get_stream.argtypes = [vp, C.POINTER(vp)]
@@ -139,6 +141,7 @@ def load() -> C.CDLL:
     L.msfm_knn2_crosscheck.argtypes = [vp, C.c_int32, C.c_int32, vp, vp]
     L.msfm_geo_verify.argtypes = [vp, vp, C.c_int64, vp, vp, vp, vp, vp, C.c_int32, C.POINTER(GeoParams), vp, vp, vp, vp]
     L.msfm_geo_ransac.argtypes = L.msfm_geo_verify.argtypes
+    L.msfm_geo_homography.argtypes = L.msfm_geo_verify.argtypes
     for name in EXPORTED_SYMBOLS:
         fn = getattr(L, name)
         if name not in ("msfm_abi_version", "msfm_status_string", "msfm_last_error"):

@@ -67,12 +67,13 @@ def build_native(force: bool = False, verbose: bool = False) -> str:
 
 SHIM_BIN = os.path.join(HOST_DIR, "shim_selftest")
 GUIDED_BIN = os.path.join(HOST_DIR, "guided_selftest")  # MatchGraphB200::MatchPairsGuided driver
+HOMOGRAPHY_BIN = os.path.join(HOST_DIR, "homography_selftest")  # MatchGraphB200::MatchPairsGuidedHomography driver
 
 
 def build_host_shim(force: bool = False) -> str:
     """Compile the C++ mirror of the reference's matcher interface + its self-test drivers against the C ABI library.
-    Returns the path of the main self-test (the guided-matching driver is GUIDED_BIN)."""
-    for exe in (SHIM_BIN, GUIDED_BIN):
+    Returns the path of the main self-test (the guided-matching drivers are GUIDED_BIN and HOMOGRAPHY_BIN)."""
+    for exe in (SHIM_BIN, GUIDED_BIN, HOMOGRAPHY_BIN):
         srcs = [exe + ".cc", os.path.join(HOST_DIR, "feature_matching_b200.cc")]
         deps = srcs + [os.path.join(HOST_DIR, f) for f in ("feature_matching_b200.h", "cv_standin.h")] + [LIB_PATH]
         if not force and os.path.exists(exe) and all(os.path.getmtime(d) <= os.path.getmtime(exe) for d in deps):

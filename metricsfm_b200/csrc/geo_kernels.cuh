@@ -8,6 +8,8 @@
 // One CTA per image pair; pairs are independent, so the batch is data parallel like the matching itself.  The RANSAC
 // draws are counter-based (seed, pair, hypothesis), i.e. reproducible, but they are not OpenCV's RNG stream: parity with
 // the reference is statistical for stage A (inlier sets / accept decisions) and exact for stage B given F.
+// The same search with a homography model (4-point DLT, one-sided transfer error) is msfm_geo_homography
+// (cv::findHomography with RANSAC, without its Levenberg-Marquardt refinement).
 #pragma once
 #include <cstdint>
 #include <cuda_runtime.h>
@@ -32,7 +34,7 @@ struct GeoParams {
     int32_t *pair_ok;          // [n_pairs]
     int32_t *pair_inliers;     // [n_pairs] stage-A inliers among the good matches
     uint8_t *keep;             // [total matches] stage-B mask
-    double *F;                 // [n_pairs][9] row-major, pixel coordinates
+    double *F;                 // [n_pairs][9] row-major, pixel coordinates (F, or H of geo_homography_kernel)
 };
 
 __device__ __forceinline__ unsigned long long geo_mix(unsigned long long z) {  // splitmix64
@@ -153,7 +155,106 @@ __device__ __forceinline__ T sym_epi_err(const T *F, T ax, T ay, T bx, T by) {
     return d1 > d2 ? d1 : d2;
 }
 
-__global__ void __launch_bounds__(kGeoThreads) geo_verify_kernel(const GeoParams gp, int n_pairs) {
+// Normalised DLT through four correspondences (x1, y1) -> (x2, y2), p2 ~ H p1 (row-major H, scaled coordinates): the
+// 8 x 9 system [x y 1 0 0 0 -u x -u y -u; 0 0 0 x y 1 -v x -v y -v] reduced by Gauss-Jordan elimination with full
+// pivoting as in seven_point; h = its null vector (free column 8), unit-normalised.  False: degenerate sample.
+static __device__ bool four_point_h(const float (&x1)[4], const float (&y1)[4], const float (&x2)[4], const float (&y2)[4], double (&H)[9]) {
+    double A[8][9];
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        const double x = x1[i], y = y1[i], u = x2[i], v = y2[i];
+        A[2 * i][0] = x;   A[2 * i][1] = y;   A[2 * i][2] = 1.0; A[2 * i][3] = 0.0; A[2 * i][4] = 0.0; A[2 * i][5] = 0.0;
+        A[2 * i][6] = -u * x; A[2 * i][7] = -u * y; A[2 * i][8] = -u;
+        A[2 * i + 1][0] = 0.0; A[2 * i + 1][1] = 0.0; A[2 * i + 1][2] = 0.0; A[2 * i + 1][3] = x; A[2 * i + 1][4] = y; A[2 * i + 1][5] = 1.0;
+        A[2 * i + 1][6] = -v * x; A[2 * i + 1][7] = -v * y; A[2 * i + 1][8] = -v;
+    }
+    int perm[9];
+    for (int j = 0; j < 9; ++j) perm[j] = j;
+    for (int k = 0; k < 8; ++k) {
+        int pr = k, pc = k;
+        double best = 0.0;
+        for (int i = k; i < 8; ++i)
+            for (int j = k; j < 9; ++j)
+                if (fabs(A[i][j]) > best) { best = fabs(A[i][j]); pr = i; pc = j; }
+        if (best < 1e-12) return false;
+        for (int j = 0; j < 9; ++j) { const double t = A[k][j]; A[k][j] = A[pr][j]; A[pr][j] = t; }
+        for (int i = 0; i < 8; ++i) { const double t = A[i][k]; A[i][k] = A[i][pc]; A[i][pc] = t; }
+        { const int t = perm[k]; perm[k] = perm[pc]; perm[pc] = t; }
+        const double inv = 1.0 / A[k][k];
+        for (int j = k; j < 9; ++j) A[k][j] *= inv;
+        for (int i = 0; i < 8; ++i) {
+            if (i == k) continue;
+            const double f = A[i][k];
+            if (f != 0.0)
+                for (int j = k; j < 9; ++j) A[i][j] -= f * A[k][j];
+        }
+    }
+    double nrm = 1.0;
+    for (int k = 0; k < 8; ++k) { H[perm[k]] = -A[k][8]; nrm += A[k][8] * A[k][8]; }
+    H[perm[8]] = 1.0;
+    if (!isfinite(nrm)) return false;
+    const double inv = rsqrt(nrm);
+    for (int j = 0; j < 9; ++j) H[j] *= inv;
+    return true;
+}
+
+// Orientation check derived from cv::findHomography's subset check (HomographyEstimatorCallback::checkSubset): every
+// triple of the sample must keep its orientation, det[p_a p_b p_c] of image 1 times that of image 2 not negative
+// (double, homogeneous points).  Stricter than OpenCV, which also accepts a sample whose four triples all flip (a
+// mirror, which no camera motion produces), and without OpenCV's collinearity test (haveCollinearPoints): a sample
+// with a collinear triple passes here (det 0) and gives a degenerate model, or none when a DLT pivot falls below 1e-12.
+__device__ __forceinline__ bool h_subset_ok(const float (&x1)[4], const float (&y1)[4], const float (&x2)[4], const float (&y2)[4]) {
+    const int tt[4][3] = {{0, 1, 2}, {1, 2, 3}, {0, 2, 3}, {0, 1, 3}};
+    bool ok = true;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        const int a = tt[i][0], b = tt[i][1], c = tt[i][2];
+        const double A[9] = {x1[a], y1[a], 1.0, x1[b], y1[b], 1.0, x1[c], y1[c], 1.0};
+        const double B[9] = {x2[a], y2[a], 1.0, x2[b], y2[b], 1.0, x2[c], y2[c], 1.0};
+        ok = ok && !(det3(A) * det3(B) < 0.0);
+    }
+    return ok;
+}
+
+// cv::findHomography's RANSAC error (calib3d fundam.cpp HomographyEstimatorCallback::computeError): the squared
+// distance of p2 to H p1 in image 2.  A zero or non-finite w makes the point an outlier (+inf).
+template <typename T>
+__device__ __forceinline__ T h_transfer_err(const T *H, T ax, T ay, T bx, T by) {
+    const T w = H[6] * ax + H[7] * ay + H[8];
+    if (w == T(0) || !isfinite(w)) return T(INFINITY);
+    const T dx = (H[0] * ax + H[1] * ay + H[2]) / w - bx, dy = (H[3] * ax + H[4] * ay + H[5]) / w - by;
+    return dx * dx + dy * dy;
+}
+
+enum class GeoModel { fundamental, homography };
+
+// The sample of hypothesis h of the pair with global index `pair`: K distinct indices of the n_pts scaled points, drawn
+// from the counter-based state mix(seed ^ mix((pair << 32) | h)) (each slot repeats st = mix(st), idx = (st >> 11) %
+// n_pts until the index is new), and their coordinates.  Both models draw through here.
+template <int K>
+__device__ __forceinline__ void geo_draw(unsigned long long seed, long long pair, int h, int n_pts, const float *sx1,
+                                         const float *sy1, const float *sx2, const float *sy2, float (&a)[K], float (&b)[K],
+                                         float (&cc)[K], float (&d)[K]) {
+    unsigned long long st = geo_mix(seed ^ geo_mix(((unsigned long long)pair << 32) | (unsigned)h));
+    int idx[K];
+    for (int k = 0; k < K; ++k) {
+        bool dup;
+        do {
+            st = geo_mix(st);
+            idx[k] = (int)((st >> 11) % (unsigned long long)n_pts);
+            dup = false;
+            for (int l = 0; l < k; ++l) dup |= idx[l] == idx[k];
+        } while (dup);
+    }
+    for (int k = 0; k < K; ++k) { a[k] = sx1[idx[k]]; b[k] = sy1[idx[k]]; cc[k] = sx2[idx[k]]; d[k] = sy2[idx[k]]; }
+}
+
+// One CTA per pair (msfm_geo_verify / msfm_geo_ransac with the fundamental model, msfm_geo_homography with the
+// homography model): used matches into shared memory, hypothesis search, winner, final count over all used matches.
+template <GeoModel MODEL>
+__device__ __forceinline__ void geo_pairs(const GeoParams gp, int n_pairs) {
+    constexpr bool HOMOG = MODEL == GeoModel::homography;
+    constexpr int kSample = HOMOG ? 4 : 7;
     __shared__ float sx1[kGeoPointCap], sy1[kGeoPointCap], sx2[kGeoPointCap], sy2[kGeoPointCap];
     __shared__ int s_cnt[kGeoThreads / 32];
     __shared__ int s_red_cnt[kGeoThreads];
@@ -181,7 +282,7 @@ __global__ void __launch_bounds__(kGeoThreads) geo_verify_kernel(const GeoParams
         }
         __syncthreads();
         const int n_good = s_ngood;
-        bool ok = n_good >= gp.min_points && n_good >= 7;
+        bool ok = n_good >= gp.min_points && n_good >= kSample;
         int n_pts = 0;
         float scale = 1.0f;
         if (ok) {
@@ -223,25 +324,33 @@ __global__ void __launch_bounds__(kGeoThreads) geo_verify_kernel(const GeoParams
             __syncthreads();
         }
         // ---- RANSAC: every thread draws hypotheses, solves the 7-point system and scores its candidates on all points
+        //      (homography: a 4-point sample that passes the subset check gives one model, id h)
         int best_cnt = -1, best_id = 0x7fffffff;
         float bestF[9];
         for (int j = 0; j < 9; ++j) bestF[j] = 0.0f;
-        if (ok && n_pts >= 7) {
+        if constexpr (HOMOG) if (ok && n_pts >= 4) {
             const float th2 = gp.th * scale * gp.th * scale;
             for (int h = threadIdx.x; h < gp.iters; h += kGeoThreads) {
-                unsigned long long st = geo_mix(gp.seed ^ geo_mix(((unsigned long long)(gp.pair_base + p) << 32) | (unsigned)h));
-                int idx[7];
-                for (int k = 0; k < 7; ++k) {
-                    bool dup;
-                    do {
-                        st = geo_mix(st);
-                        idx[k] = (int)((st >> 11) % (unsigned long long)n_pts);
-                        dup = false;
-                        for (int l = 0; l < k; ++l) dup |= idx[l] == idx[k];
-                    } while (dup);
+                float a[4], b[4], cc[4], d[4];
+                geo_draw(gp.seed, gp.pair_base + p, h, n_pts, sx1, sy1, sx2, sy2, a, b, cc, d);
+                double Hc[9];
+                if (!h_subset_ok(a, b, cc, d) || !four_point_h(a, b, cc, d, Hc)) continue;
+                float Hf[9];
+                for (int j = 0; j < 9; ++j) Hf[j] = (float)Hc[j];
+                int cnt = 0;
+                for (int i = 0; i < n_pts; ++i) cnt += h_transfer_err<float>(Hf, sx1[i], sy1[i], sx2[i], sy2[i]) <= th2 ? 1 : 0;
+                if (cnt > best_cnt || (cnt == best_cnt && h < best_id)) {
+                    best_cnt = cnt;
+                    best_id = h;
+                    for (int j = 0; j < 9; ++j) bestF[j] = Hf[j];
                 }
+            }
+        }
+        if constexpr (!HOMOG) if (ok && n_pts >= 7) {
+            const float th2 = gp.th * scale * gp.th * scale;
+            for (int h = threadIdx.x; h < gp.iters; h += kGeoThreads) {
                 float a[7], b[7], cc[7], d[7];
-                for (int k = 0; k < 7; ++k) { a[k] = sx1[idx[k]]; b[k] = sy1[idx[k]]; cc[k] = sx2[idx[k]]; d[k] = sy2[idx[k]]; }
+                geo_draw(gp.seed, gp.pair_base + p, h, n_pts, sx1, sy1, sx2, sy2, a, b, cc, d);
                 double Fc[3][9];
                 const int nf = seven_point(a, b, cc, d, Fc);
                 for (int f = 0; f < nf; ++f) {
@@ -270,12 +379,14 @@ __global__ void __launch_bounds__(kGeoThreads) geo_verify_kernel(const GeoParams
         __syncthreads();
         if (s_best_thread < 0) ok = false;
         if (ok && threadIdx.x == s_best_thread) {
-            // back to pixel coordinates: F = T^T F' T with T = diag(s, s, 1)
+            // back to pixel coordinates: F = T^T F' T with T = diag(s, s, 1); H = T^-1 H' T
             const double s = scale;
-            const double T[9] = {s * s, s * s, s, s * s, s * s, s, s, s, 1.0};
+            double T[9] = {s * s, s * s, s, s * s, s * s, s, s, s, 1.0};
+            if constexpr (HOMOG) { T[0] = T[1] = T[3] = T[4] = 1.0; T[2] = T[5] = 1.0 / s; }
             double nrm = 0.0;
             for (int j = 0; j < 9; ++j) { s_F[j] = (double)bestF[j] * T[j]; nrm += s_F[j] * s_F[j]; }
-            // cv::findFundamentalMat scales the result so that F(2,2) = 1 when it is not ~0 (fundam.cpp run7Point)
+            // cv::findFundamentalMat scales the result so that F(2,2) = 1 when it is not ~0 (fundam.cpp run7Point);
+            // cv::findHomography returns H with H(2,2) = 1
             const double f22 = s_F[8];
             const double k = fabs(f22) > 1e-12 * sqrt(nrm) ? 1.0 / f22 : 1.0 / sqrt(nrm);
             for (int j = 0; j < 9; ++j) s_F[j] *= k;
@@ -288,7 +399,10 @@ __global__ void __launch_bounds__(kGeoThreads) geo_verify_kernel(const GeoParams
             for (int i = threadIdx.x; i < n_all; i += kGeoThreads) {
                 if (!gd[i]) continue;
                 const int2 m = mt[i];
-                inl += sym_epi_err<double>(s_F, xy1[2 * m.x], xy1[2 * m.x + 1], xy2[2 * m.y], xy2[2 * m.y + 1]) <= th2 ? 1 : 0;
+                if constexpr (HOMOG)
+                    inl += h_transfer_err<double>(s_F, xy1[2 * m.x], xy1[2 * m.x + 1], xy2[2 * m.y], xy2[2 * m.y + 1]) <= th2 ? 1 : 0;
+                else
+                    inl += sym_epi_err<double>(s_F, xy1[2 * m.x], xy1[2 * m.x + 1], xy2[2 * m.y], xy2[2 * m.y + 1]) <= th2 ? 1 : 0;
             }
         }
         for (int o = 16; o > 0; o >>= 1) inl += __shfl_xor_sync(0xFFFFFFFFu, inl, o);
@@ -298,7 +412,21 @@ __global__ void __launch_bounds__(kGeoThreads) geo_verify_kernel(const GeoParams
         int inliers = 0;
         for (int w = 0; w < kGeoThreads / 32; ++w) inliers += s_cnt[w];
         ok = ok && inliers >= gp.min_inliers;
-        // ---- stage B: one-sided distance of p2 to the epipolar line F p1 on every "all" match (geo_verification.cc:60-79)
+        // ---- the per-match mask.  Homography: the consensus set, transfer error of the used matches against H <= th^2.
+        //      Fundamental, stage B: one-sided distance of p2 to the epipolar line F p1 on every "all" match
+        //      (geo_verification.cc:60-79); msfm_geo_ransac: the consensus set of the good matches
+        if constexpr (HOMOG) {
+            for (int i = threadIdx.x; i < n_all; i += kGeoThreads) {
+                uint8_t k = 0;
+                if (ok) {
+                    const int2 m = mt[i];
+                    k = gd[i] && h_transfer_err<double>(s_F, xy1[2 * m.x], xy1[2 * m.x + 1], xy2[2 * m.y], xy2[2 * m.y + 1]) <=
+                                     (double)gp.th * (double)gp.th
+                            ? 1 : 0;
+                }
+                gp.keep[m0 + i] = k;
+            }
+        } else
         for (int i = threadIdx.x; i < n_all; i += kGeoThreads) {
             uint8_t k = 0;
             if (ok && !gp.stage_b) {
@@ -324,6 +452,14 @@ __global__ void __launch_bounds__(kGeoThreads) geo_verify_kernel(const GeoParams
                 for (int j = 0; j < 9; ++j) gp.F[9 * (int64_t)p + j] = ok ? s_F[j] : 0.0;
         }
     }
+}
+
+__global__ void __launch_bounds__(kGeoThreads) geo_verify_kernel(const GeoParams gp, int n_pairs) {
+    geo_pairs<GeoModel::fundamental>(gp, n_pairs);
+}
+
+__global__ void __launch_bounds__(kGeoThreads) geo_homography_kernel(const GeoParams gp, int n_pairs) {
+    geo_pairs<GeoModel::homography>(gp, n_pairs);
 }
 
 }  // namespace msfm

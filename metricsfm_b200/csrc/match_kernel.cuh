@@ -21,9 +21,10 @@
 //   (padding warps) idle; the auxiliary warpgroups hand their registers to the epilogue warps (setmaxnreg)
 //   The service warps share issue slots with the epilogue warps of their sub-partition: their tile loops are unrolled
 //   over the B ring (immediate addresses) and they sleep between polls (see the comment at the role dispatch).
-// Two template flags vary the epilogue's exact phase, everything else is shared: COLLECT (float regime) replaces the
-// top-2 merge by "append every element under the row's fixed threshold to an event list"; GATED (guided matching) bars
-// the elements that fail the epipolar gate (epi_allowed) from the row's top-2 or event list.
+// Two template parameters vary the epilogue's exact phase, everything else is shared: COLLECT (float regime) replaces the
+// top-2 merge by "append every element under the row's fixed threshold to an event list"; GATE (guided matching) bars
+// the elements that fail the epipolar gate (epi_allowed) or the homography gate (hom_allowed) from the row's top-2 or
+// event list.
 // Work distribution: CTA b takes items b, b + grid, ...; every role walks that list on its own.
 // Pipelines (all mbarrier based):
 //   A ring (2 deep)     : query strips of a work item, STRIPS x [128 rows x 128 B]
@@ -105,12 +106,14 @@ struct MatchKernelParams {
                                   // consumers read it with load_knn()
         int4 *events;             // COLLECT: [event_cap]
     };
-    // GATED (msfm_match_pairs_guided): only elements that pass the epipolar gate (epi_allowed) can enter a row's top-2 or
-    // event list.  F is row p of fmat for a forward item of pair p and for every item with cand_idx = p.  A forward row
-    // and a band row (a collect item's row) are query keypoints, so the gate takes their query line; a twin row is a
-    // reference keypoint, and the gate takes the query line of each column instead.
+    // GATE (msfm_match_pairs_guided / _guided_homography): only elements that pass the gate can enter a row's top-2 or
+    // event list.  F (or H) is row p of fmat for a forward item of pair p and for every item with cand_idx = p.  A forward
+    // row and a band row (a collect item's row) are query keypoints, so the epipolar gate takes their query line; a twin
+    // row is a reference keypoint, and the gate takes the query line of each column instead.  The homography gate
+    // transfers the reference keypoint of each element: per column on a forward row, once per row on a twin row.
     const float2 *xy;             // keypoints (x, y), indexed like the column-key arena
-    const float *fmat;            // [forward pairs of the batch][9] F rounded to fp32, row-major
+    const float *fmat;            // [forward pairs of the batch][9] F (epipolar gate) or H (homography gate) rounded to
+                                  // fp32, row-major
     const int32_t *src_row;       // [candidate scratch rows] the image row a scratch row came from: a reference row of pair
                                   // cand_idx for a twin row (cand_j), a query row of it for a band row (band_q)
     const unsigned int *routed;   // optional: the whole launch returns at once when *routed == 0 (mutual twin pass with no
@@ -118,7 +121,7 @@ struct MatchKernelParams {
     uint32_t prune_q8;            // "dead row" rule of the forward pass (see the epilogue): a row whose two nearest neighbours
                                   // so far satisfy d0 > (prune_q8 / 256) * d1 only follows its NEAREST neighbour exactly.
                                   // kNoPrune = off (exact 2-NN of every row: msfm_knn2, twin and collect passes)
-    float t2;                     // GATED: th_epipolar^2, rounded to fp32
+    float t2;                     // GATE: th_epipolar^2 or th_transfer^2, rounded to fp32
 };
 // The kernel takes the block by value.  Past 128 bytes nvcc addresses it through a pointer and the code of every
 // instantiation changes; the top-2 passes, the headline path, read their fields at these offsets.
@@ -245,18 +248,44 @@ __device__ __forceinline__ bool epi_allowed(const EpiLine &a, float2 kj, float n
     return __fmul_rn(s, s) <= __fmul_rn(t2, nb < a.n ? nb : a.n);
 }
 
-// The epipolar gate of a guided batch as the host passes it: keypoints (x, y) indexed like the column-key arena, the
-// batch's F table ([forward pairs][9] rounded to fp32, row-major) and th_epipolar^2 rounded to fp32.
+// Homography gate of HOMOG-SPEC (include/msfm_match.h).  The reference keypoint kj is transferred once,
+// (U, V, W) = H (xj, yj, 1); element (q, j) is allowed iff |(U, V) - (xq, yq) W|^2 <= t2 W^2, the squared transfer
+// distance |p_q - pi(H p_j)|^2 <= th^2 without the division (independent of the sign of H; W = 0 bars the element unless
+// U = V = 0).  One fp32 rounding per operation, no contraction; every site of the matching kernel goes through
+// hom_transfer and hom_allowed.
+struct HomPoint {
+    float U, V, W;
+};
+template <bool LDG = false>
+__device__ __forceinline__ HomPoint hom_transfer(const float *H, float2 k) {
+    HomPoint t;
+    t.U = epi_lin(epi_f<LDG>(H, 0), k.x, epi_f<LDG>(H, 1), k.y, epi_f<LDG>(H, 2));
+    t.V = epi_lin(epi_f<LDG>(H, 3), k.x, epi_f<LDG>(H, 4), k.y, epi_f<LDG>(H, 5));
+    t.W = epi_lin(epi_f<LDG>(H, 6), k.x, epi_f<LDG>(H, 7), k.y, epi_f<LDG>(H, 8));
+    return t;
+}
+__device__ __forceinline__ bool hom_allowed(const HomPoint &t, float2 kq, float t2) {
+    const float du = __fsub_rn(t.U, __fmul_rn(kq.x, t.W)), dv = __fsub_rn(t.V, __fmul_rn(kq.y, t.W));
+    return epi_sq(du, dv) <= __fmul_rn(t2, __fmul_rn(t.W, t.W));
+}
+
+// Which gate a guided launch applies (the matching kernel's GATE parameter).
+enum class GateKind : int { none = 0, epipolar = 1, homography = 2 };
+
+// The gate of a guided batch as the host passes it: keypoints (x, y) indexed like the column-key arena, the
+// batch's F (or H) table ([forward pairs][9] rounded to fp32, row-major) and th^2 rounded to fp32.
 struct EpiGate {
     const float2 *xy;
     const float *fmat;
     float t2;
 };
 
-template <int STRIPS, int TILE_N, int STAGES, int TBUFS, bool DEBUG, bool COLLECT = false, bool GATED = false>
+template <int STRIPS, int TILE_N, int STAGES, int TBUFS, bool DEBUG, bool COLLECT = false, GateKind GATE = GateKind::none>
 __global__ void __launch_bounds__(MatchKernelCfg<STRIPS, TILE_N, STAGES, TBUFS>::kThreads, 1)
 match_pairs_kernel(const MatchKernelParams p) {
     using Cfg = MatchKernelCfg<STRIPS, TILE_N, STAGES, TBUFS>;
+    constexpr bool GATED = GATE != GateKind::none, HOMOG = GATE == GateKind::homography;
+    static_assert(!(COLLECT && HOMOG), "the float regime has no homography gate");
     // No static shared memory is declared, so the dynamic window starts at shared offset 0 (1024-byte aligned, as
     // the 128B-swizzled operand tiles require); checked once below.
     extern __shared__ __align__(1024) uint8_t smem[];
@@ -493,11 +522,17 @@ match_pairs_kernel(const MatchKernelParams p) {
             // query line.  A band row takes its query row's keypoint and F, so it gets that row's line bit for bit, and
             // its allowed set is the one its gated quantised 2-NN, and hence its threshold T(q), came from.  A twin row is
             // a reference keypoint kr: its reference line, of which the test needs |b|^2 only.
+            // Homography gate: a forward row keeps its query keypoint kr, a twin row its transferred keypoint ht.
             const bool query_row = COLLECT || pd.cand_idx < 0;
             EpiLine line{};
             float2 kr{};
+            HomPoint ht{};
             const float *fm = nullptr;
-            if (GATED) {
+            if (HOMOG) {
+                fm = p.fmat + 9 * (pd.cand_idx >= 0 ? pd.cand_idx : wi.pair);
+                if (valid && query_row) kr = p.xy[pd.qry_off + q];
+                else if (valid) ht = hom_transfer(fm, p.xy[p.pairs[pd.cand_idx].ref_off + p.src_row[pd.qry_off + q]]);
+            } else if (GATED) {
                 fm = p.fmat + 9 * (pd.cand_idx >= 0 ? pd.cand_idx : wi.pair);
                 if (valid && query_row) {
                     line = epi_query_line(fm, p.xy[pd.cand_idx < 0 ? pd.qry_off + q : p.pairs[pd.cand_idx].qry_off + p.src_row[pd.qry_off + q]]);
@@ -582,9 +617,14 @@ match_pairs_kernel(const MatchKernelParams p) {
                                         const float2 kc[2] = {make_float2(c.x, c.y), make_float2(c.z, c.w)};
 #pragma unroll
                                         for (int e = 0; e < 2; ++e) {
-                                            const bool ok = query_row  // column = reference row j, or query row q
-                                                ? epi_allowed(line, kc[e], epi_ref_line<true>(fm, kc[e]).n, p.t2)
-                                                : epi_allowed(epi_query_line<true>(fm, kc[e]), kr, line.n, p.t2);
+                                            bool ok;  // column = reference row j, or query row q
+                                            if (HOMOG)
+                                                ok = query_row ? hom_allowed(hom_transfer<true>(fm, kc[e]), kr, p.t2)
+                                                               : hom_allowed(ht, kc[e], p.t2);
+                                            else
+                                                ok = query_row
+                                                    ? epi_allowed(line, kc[e], epi_ref_line<true>(fm, kc[e]).n, p.t2)
+                                                    : epi_allowed(epi_query_line<true>(fm, kc[e]), kr, line.n, p.t2);
                                             if (!ok) key[2 * h + e] = INT_MIN;
                                         }
                                     }

@@ -40,16 +40,20 @@ constexpr int kTbufs = 2;    // TMEM accumulator buffers per strip
 using KCfg = msfm::MatchKernelCfg<kStrips, kTileN, kStages, kTbufs>;
 constexpr int kItemRows = kStrips * msfm::kStripRows;
 
-// The instantiations of the matching kernel, (DEBUG, COLLECT, GATED): every combination but a debug build of the
-// collect pass, for which `debug` is ignored.
+// The instantiations of the matching kernel, (DEBUG, COLLECT, GATE): every combination but a debug build of the
+// collect pass, for which `debug` is ignored, and a collect pass under the homography gate (the float regime has none:
+// null).
 using MatchKernelFn = void (*)(msfm::MatchKernelParams);
+using msfm::GateKind;
 template <bool DEBUG, bool COLLECT>
-MatchKernelFn match_kernel(bool gated) {
-    return gated ? msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, DEBUG, COLLECT, true>
-                 : msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, DEBUG, COLLECT, false>;
+MatchKernelFn match_kernel(GateKind gate) {
+    if (gate == GateKind::none) return msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, DEBUG, COLLECT, GateKind::none>;
+    if (gate == GateKind::epipolar) return msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, DEBUG, COLLECT, GateKind::epipolar>;
+    if constexpr (!COLLECT) return msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, DEBUG, COLLECT, GateKind::homography>;
+    return nullptr;
 }
-MatchKernelFn match_kernel(bool debug, bool collect, bool gated) {
-    return collect ? match_kernel<false, true>(gated) : debug ? match_kernel<true, false>(gated) : match_kernel<false, false>(gated);
+MatchKernelFn match_kernel(bool debug, bool collect, GateKind gate) {
+    return collect ? match_kernel<false, true>(gate) : debug ? match_kernel<true, false>(gate) : match_kernel<false, false>(gate);
 }
 
 // Per-batch scratch bounds (rows).  16 Mi query rows -> 256 MiB kNN scratch + 128 MiB match scratch.
@@ -348,9 +352,11 @@ struct BatchPlan {
     uint32_t prune_q8 = msfm::kNoPrune;  // forward pass: dead-row rule of the matching kernel (match_kernel.cuh); off = exact 2-NN rows
     bool has_empty = false;          // some pair has no work items: its kNN rows must read "absent"
     bool any_float = false;          // some pair has retained float rows on both sides (rescoring possible)
-    std::vector<float> fmat;         // guided call: F of every forward pair, 9 floats each (uploaded after the descriptors)
+    std::vector<float> fmat;         // guided call: F (or H) of every forward pair, 9 floats each (uploaded after the
+                                     // descriptors)
     msfm::EpiGate gate{};            // guided call: keypoints and t2 from the carve, the F table's device address from
                                      // run_match_stage
+    GateKind gate_kind = GateKind::none;  // what the table in gate.fmat holds and which test the matching kernel applies
     const msfm::EpiGate *epi_gate() const { return gate.fmat ? &gate : nullptr; }  // null: ungated
     int64_t knn_rows() const { return mutual ? 2 * query_rows : query_rows; }
 };
@@ -360,12 +366,13 @@ struct BatchPlan {
 //   twin     2-NN of the mutual twins' candidate rows, skipped on the device unless select_candidates_kernel routed a pair
 //   collect  the items are band twins: every reference row within band_thr of a band row is appended to the event list,
 //            which holds `value` events
-// `gate` (null: none) bars the elements that fail the epipolar gate in every pass.
+// A guided plan's gate bars the elements that fail it in every pass.
 enum class Pass { forward, twin, collect };
 
 msfm_status launch_match_kernel(msfm_ctx *ctx, Pass pass, size_t first_item, size_t n_items, uint32_t value,
-                                const msfm::EpiGate *gate) {
+                                const BatchPlan &plan) {
     const bool collect = pass == Pass::collect, twin = pass == Pass::twin;
+    const msfm::EpiGate *gate = plan.epi_gate();
     msfm::MatchKernelParams kp;
     kp.maps = ctx->d_maps;
     kp.ckeys = ctx->norms;
@@ -393,7 +400,7 @@ msfm_status launch_match_kernel(msfm_ctx *ctx, Pass pass, size_t first_item, siz
     kp.prune_q8 = (pass == Pass::forward && !ctx->no_prune) ? value : msfm::kNoPrune;
     kp.t2 = gate ? gate->t2 : 0.0f;
     const int grid = std::max(1, std::min<int>(ctx->num_sms, kp.n_items));
-    match_kernel(ctx->debug_flags != 0, collect, gate != nullptr)<<<grid, KCfg::kThreads, KCfg::kSmemAlloc, ctx->stream>>>(kp);
+    match_kernel(ctx->debug_flags != 0, collect, gate ? plan.gate_kind : GateKind::none)<<<grid, KCfg::kThreads, KCfg::kSmemAlloc, ctx->stream>>>(kp);
     MSFM_CUDA(ctx, cudaGetLastError());
     ctx->timing.match_launches += 1;
     ctx->timing.total_launches += 1;
@@ -520,7 +527,7 @@ msfm_status run_match_stage(msfm_ctx *ctx, BatchPlan &plan) {
         ctx->timing.total_launches += 1;
     }
     MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_k0, ctx->stream));
-    if (!plan.items.empty() && (st = launch_match_kernel(ctx, Pass::forward, 0, plan.items.size(), plan.prune_q8, plan.epi_gate())) != MSFM_OK) return st;
+    if (!plan.items.empty() && (st = launch_match_kernel(ctx, Pass::forward, 0, plan.items.size(), plan.prune_q8, plan)) != MSFM_OK) return st;
     MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_k1, ctx->stream));
     ctx->timing.int8_ops += plan.ops;
     return MSFM_OK;
@@ -664,7 +671,7 @@ msfm_status run_collect_pass(msfm_ctx *ctx, const BatchPlan &plan, const msfm::B
     msfm_status st;
     if (!plan.band_items.empty() &&
         (st = launch_match_kernel(ctx, Pass::collect, plan.items.size() + plan.twin_items.size(), plan.band_items.size(), bp.event_cap,
-                                  plan.epi_gate())) != MSFM_OK)
+                                  plan)) != MSFM_OK)
         return st;
     const int nb = (int)plan.pairs.size();
     msfm::score_events_kernel<<<4 * ctx->num_sms, 256, 0, ctx->stream>>>(bp);
@@ -724,55 +731,62 @@ int caller_sink(void *user, int64_t first, int64_t n, int32_t (**m)[2], uint8_t 
     return 0;
 }
 
-// The epipolar gate of msfm_match_pairs_guided, as the caller passed it.
+// The gate of msfm_match_pairs_guided (epipolar: M = F) or msfm_match_pairs_guided_homography (homography: M = H), as
+// the caller passed it.
 struct GuidedArgs {
-    const double (*F)[9];
+    GateKind kind;
+    const double (*M)[9];
     float th;
     const float *const *image_xy;
     const int32_t *image_npts;
     int32_t n_images;
 };
 
-// Everything msfm_match_pairs_guided rejects is rejected here, before any launch.  On success `fq` holds every pair's F
-// rounded to fp32.  The image ids have been checked.
+// Everything the guided entry points reject is rejected here, before any launch.  On success `fq` holds every pair's
+// matrix rounded to fp32.  The image ids have been checked.
 msfm_status check_guided(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pairs, const msfm_params *params, const GuidedArgs &g,
                          std::vector<float> &fq) {
+    const bool homog = g.kind == GateKind::homography;
+    const char *fn = homog ? "msfm_match_pairs_guided_homography" : "msfm_match_pairs_guided";
+    const char *mat = homog ? "H" : "F";
     if (!std::isfinite(params->rescore_band) || params->rescore_band < 0.0f)
-        return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_match_pairs_guided: rescore_band %g must be finite and >= 0", (double)params->rescore_band);
+        return fail(ctx, MSFM_ERR_INVALID_ARG, "%s: rescore_band %g must be finite and >= 0", fn, (double)params->rescore_band);
+    if (homog && params->rescore_band > 0.0f)
+        return fail(ctx, MSFM_ERR_INVALID_ARG, "%s: rescore_band > 0 is not supported under the homography gate", fn);
     if (params->rescore_band > 0.0f && !ctx->fdesc)
-        return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_match_pairs_guided: rescore_band > 0 needs a keep_float context (retained float rows)");
+        return fail(ctx, MSFM_ERR_INVALID_ARG, "%s: rescore_band > 0 needs a keep_float context (retained float rows)", fn);
     if (!std::isfinite(g.th) || !(g.th > 0.0f))
-        return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_match_pairs_guided: th_epipolar %g must be finite and > 0", (double)g.th);
+        return fail(ctx, MSFM_ERR_INVALID_ARG, "%s: %s %g must be finite and > 0", fn, homog ? "th_transfer" : "th_epipolar", (double)g.th);
     if (n_pairs == 0) return MSFM_OK;
-    if (!g.F) return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_match_pairs_guided: null F");
-    if (!g.image_xy || !g.image_npts) return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_match_pairs_guided: null image_xy / image_npts");
+    if (!g.M) return fail(ctx, MSFM_ERR_INVALID_ARG, "%s: null %s", fn, mat);
+    if (!g.image_xy || !g.image_npts) return fail(ctx, MSFM_ERR_INVALID_ARG, "%s: null image_xy / image_npts", fn);
     std::vector<char> checked((size_t)std::max(g.n_images, 0), 0);
     fq.resize((size_t)n_pairs * 9);
     for (int64_t p = 0; p < n_pairs; ++p) {
         for (const int32_t i : {pairs[p].ref, pairs[p].query}) {
             if (i >= g.n_images)
-                return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_match_pairs_guided: pair %lld names image %d, outside [0, n_images = %d)",
+                return fail(ctx, MSFM_ERR_INVALID_ARG, "%s: pair %lld names image %d, outside [0, n_images = %d)", fn,
                             (long long)p, i, g.n_images);
             if (checked[i]) continue;
             checked[i] = 1;
             const int32_t rows = ctx->images[i].rows;
             if (g.image_npts[i] != rows)
-                return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_match_pairs_guided: image %d has %d keypoints and %d uploaded rows", i,
+                return fail(ctx, MSFM_ERR_INVALID_ARG, "%s: image %d has %d keypoints and %d uploaded rows", fn, i,
                             g.image_npts[i], rows);
-            if (rows > 0 && !g.image_xy[i]) return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_match_pairs_guided: image %d has no keypoints", i);
+            if (rows > 0 && !g.image_xy[i]) return fail(ctx, MSFM_ERR_INVALID_ARG, "%s: image %d has no keypoints", fn, i);
             for (int64_t k = 0; k < 2ll * rows; ++k)
                 if (!std::isfinite(g.image_xy[i][k]))
-                    return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_match_pairs_guided: keypoint %lld of image %d is not finite", (long long)(k / 2), i);
+                    return fail(ctx, MSFM_ERR_INVALID_ARG, "%s: keypoint %lld of image %d is not finite", fn, (long long)(k / 2), i);
         }
         bool nonzero = false;
         for (int k = 0; k < 9; ++k) {
-            const float f = (float)g.F[p][k];  // one rounding to nearest
+            const float f = (float)g.M[p][k];  // one rounding to nearest
             if (!std::isfinite(f))
-                return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_match_pairs_guided: F of pair %lld has a non-finite entry (in fp32)", (long long)p);
+                return fail(ctx, MSFM_ERR_INVALID_ARG, "%s: %s of pair %lld has a non-finite entry (in fp32)", fn, mat, (long long)p);
             nonzero = nonzero || f != 0.0f;
             fq[(size_t)p * 9 + k] = f;
         }
-        if (!nonzero) return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_match_pairs_guided: F of pair %lld is zero", (long long)p);
+        if (!nonzero) return fail(ctx, MSFM_ERR_INVALID_ARG, "%s: %s of pair %lld is zero", fn, mat, (long long)p);
     }
     return MSFM_OK;
 }
@@ -794,8 +808,8 @@ msfm_status upload_keypoints(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pa
     return MSFM_OK;
 }
 
-// msfm_match_pairs, and msfm_match_pairs_guided when `guided` is set: the same batches, with the forward and twin passes
-// of the matching kernel under the epipolar gate and every mutual pair routed to the twin pass.
+// msfm_match_pairs, and the guided entry points when `guided` is set: the same batches, with the forward and twin passes
+// of the matching kernel under the epipolar or homography gate and every mutual pair routed to the twin pass.
 msfm_status match_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pairs, const msfm_params *params, const OutSpec *out,
                              bool resident, int64_t *n_matches_total, const GuidedArgs *guided = nullptr) {
     if (!ctx) return MSFM_ERR_INVALID_ARG;
@@ -806,7 +820,7 @@ msfm_status match_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pa
     if (!(params->ratio > 0.0f)) return fail(ctx, MSFM_ERR_INVALID_ARG, "ratio must be > 0");
     msfm_status st;
     if ((st = check_pairs(ctx, pairs, n_pairs)) != MSFM_OK) return st;
-    std::vector<float> fq;  // guided: F of every pair in fp32
+    std::vector<float> fq;  // guided: F (or H) of every pair in fp32
     if (guided && (st = check_guided(ctx, pairs, n_pairs, params, *guided, fq)) != MSFM_OK) return st;
     ctx->timing = msfm_timing{};
     DrainListCopy drain_list_copy{ctx};
@@ -838,7 +852,10 @@ msfm_status match_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pa
         c.plan.mutual = mutual;
         c.plan.rescoring = params->rescore_band > 0.0f && ctx->fdesc != nullptr;
         c.plan.prune_q8 = prune_q8;
-        if (guided) c.plan.gate = msfm::EpiGate{static_cast<const float2 *>(ctx->kp_xy.ptr), nullptr, guided->th * guided->th};
+        if (guided) {
+            c.plan.gate = msfm::EpiGate{static_cast<const float2 *>(ctx->kp_xy.ptr), nullptr, guided->th * guided->th};
+            c.plan.gate_kind = guided->kind;
+        }
         c.first = next;
         while (next < n_pairs && (int64_t)c.plan.pairs.size() < kBatchMaxPairs) {
             const ImageSlot &r = ctx->images[pairs[next].ref], &q = ctx->images[pairs[next].query];
@@ -945,7 +962,7 @@ msfm_status match_pairs_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pa
             // ---- tensor twin pass (nearest query row of every candidate's reference row) for the routed pairs only
             MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_k2, ctx->stream));
             if (mutual && !plan.twin_items.empty() &&
-                (st = launch_match_kernel(ctx, Pass::twin, plan.items.size(), plan.twin_items.size(), 0, plan.epi_gate())) != MSFM_OK)
+                (st = launch_match_kernel(ctx, Pass::twin, plan.items.size(), plan.twin_items.size(), 0, plan)) != MSFM_OK)
                 return st;
             MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_k3, ctx->stream));
             // ---- emission, offsets, tight gather
@@ -1277,8 +1294,9 @@ msfm_status msfm_create(const msfm_config *cfg, msfm_ctx **out) {
     if (cudaMallocHost(&ctx->h_maps, (size_t)(ctx->max_images + 1) * sizeof(CUtensorMap)) != cudaSuccess) return bail(MSFM_ERR_OUT_OF_MEMORY);
     for (const bool debug : {false, true})
         for (const bool collect : {false, true})
-            for (const bool gated : {false, true})
-                if (cudaFuncSetAttribute(match_kernel(debug, collect, gated), cudaFuncAttributeMaxDynamicSharedMemorySize, KCfg::kSmemAlloc) != cudaSuccess)
+            for (const GateKind gate : {GateKind::none, GateKind::epipolar, GateKind::homography})
+                if (!(collect && gate == GateKind::homography) &&
+                    cudaFuncSetAttribute(match_kernel(debug, collect, gate), cudaFuncAttributeMaxDynamicSharedMemorySize, KCfg::kSmemAlloc) != cudaSuccess)
                     return bail(MSFM_ERR_CUDA);
     if (cudaFuncSetAttribute(msfm::select_candidates_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msfm::kSelectSmemBytes) != cudaSuccess)
         return bail(MSFM_ERR_CUDA);
@@ -1725,7 +1743,14 @@ msfm_status msfm_match_pairs(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pa
 msfm_status msfm_match_pairs_guided(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pairs, const msfm_params *params,
                                     const double (*F)[9], float th_epipolar, const float *const *image_xy,
                                     const int32_t *image_npts, int32_t n_images, msfm_result *out) {
-    const GuidedArgs g{F, th_epipolar, image_xy, image_npts, n_images};
+    const GuidedArgs g{GateKind::epipolar, F, th_epipolar, image_xy, image_npts, n_images};
+    return match_pairs_to_result(ctx, pairs, n_pairs, params, out, &g);
+}
+
+msfm_status msfm_match_pairs_guided_homography(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pairs, const msfm_params *params,
+                                               const double (*H)[9], float th_transfer, const float *const *image_xy,
+                                               const int32_t *image_npts, int32_t n_images, msfm_result *out) {
+    const GuidedArgs g{GateKind::homography, H, th_transfer, image_xy, image_npts, n_images};
     return match_pairs_to_result(ctx, pairs, n_pairs, params, out, &g);
 }
 
@@ -1830,52 +1855,64 @@ msfm_status msfm_test_last_knn_stats(msfm_ctx *ctx, int64_t *events, int32_t *br
     return MSFM_OK;
 }
 
+// The three geometric-verification entry points share validation, staging and timing; `call` picks the model and the
+// meaning of `keep`.
+enum class GeoCall { verify, ransac, homography };
 static msfm_status geo_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pairs, const int64_t *offsets, const int32_t (*matches)[2],
                             const uint8_t *good, const float *const *image_xy, const int32_t *image_npts, int32_t n_images,
-                            const msfm_geo_params *gp, int32_t *pair_ok, int32_t *pair_inliers, uint8_t *keep, double *F, bool stage_b);
+                            const msfm_geo_params *gp, int32_t *pair_ok, int32_t *pair_inliers, uint8_t *keep, double *F, GeoCall call);
 
 msfm_status msfm_geo_verify(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pairs, const int64_t *offsets,
                             const int32_t (*matches)[2], const uint8_t *good, const float *const *image_xy,
                             const int32_t *image_npts, int32_t n_images, const msfm_geo_params *gp, int32_t *pair_ok,
                             int32_t *pair_inliers, uint8_t *keep, double *F) {
-    return geo_impl(ctx, pairs, n_pairs, offsets, matches, good, image_xy, image_npts, n_images, gp, pair_ok, pair_inliers, keep, F, true);
+    return geo_impl(ctx, pairs, n_pairs, offsets, matches, good, image_xy, image_npts, n_images, gp, pair_ok, pair_inliers, keep, F, GeoCall::verify);
 }
 
 msfm_status msfm_geo_ransac(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pairs, const int64_t *offsets,
                             const int32_t (*matches)[2], const uint8_t *use, const float *const *image_xy,
                             const int32_t *image_npts, int32_t n_images, const msfm_geo_params *gp, int32_t *pair_ok,
                             int32_t *pair_inliers, uint8_t *inlier_mask, double *F) {
-    return geo_impl(ctx, pairs, n_pairs, offsets, matches, use, image_xy, image_npts, n_images, gp, pair_ok, pair_inliers, inlier_mask, F, false);
+    return geo_impl(ctx, pairs, n_pairs, offsets, matches, use, image_xy, image_npts, n_images, gp, pair_ok, pair_inliers, inlier_mask, F, GeoCall::ransac);
+}
+
+msfm_status msfm_geo_homography(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pairs, const int64_t *offsets,
+                                const int32_t (*matches)[2], const uint8_t *use, const float *const *image_xy,
+                                const int32_t *image_npts, int32_t n_images, const msfm_geo_params *gp, int32_t *pair_ok,
+                                int32_t *pair_inliers, uint8_t *inlier_mask, double *H) {
+    return geo_impl(ctx, pairs, n_pairs, offsets, matches, use, image_xy, image_npts, n_images, gp, pair_ok, pair_inliers, inlier_mask, H,
+                    GeoCall::homography);
 }
 
 static msfm_status geo_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pairs, const int64_t *offsets, const int32_t (*matches)[2],
                             const uint8_t *good, const float *const *image_xy, const int32_t *image_npts, int32_t n_images,
-                            const msfm_geo_params *gp, int32_t *pair_ok, int32_t *pair_inliers, uint8_t *keep, double *F, bool stage_b) {
+                            const msfm_geo_params *gp, int32_t *pair_ok, int32_t *pair_inliers, uint8_t *keep, double *F, GeoCall call) {
     if (!ctx) return MSFM_ERR_INVALID_ARG;
+    const char *fn = call == GeoCall::homography ? "msfm_geo_homography" : call == GeoCall::ransac ? "msfm_geo_ransac" : "msfm_geo_verify";
     std::lock_guard<std::mutex> lock(ctx->mu);
     if (n_pairs < 0 || !gp || (n_pairs > 0 && (!pairs || !offsets || !pair_ok || !pair_inliers || !image_xy || !image_npts)))
-        return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_geo_verify: null argument");
+        return fail(ctx, MSFM_ERR_INVALID_ARG, "%s: null argument", fn);
     if (n_pairs == 0) return MSFM_OK;
     const int64_t total = offsets[n_pairs];
-    if (total < 0 || (total > 0 && (!matches || !good || !keep))) return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_geo_verify: null match buffers");
+    if (total < 0 || (total > 0 && (!matches || !good || !keep))) return fail(ctx, MSFM_ERR_INVALID_ARG, "%s: null match buffers", fn);
     MSFM_CUDA(ctx, cudaSetDevice(ctx->device));
     // keypoints of the images the pairs touch, concatenated
     std::vector<int64_t> xy_off((size_t)n_images + 1, 0);
     std::vector<char> used((size_t)n_images, 0);
     for (int64_t p = 0; p < n_pairs; ++p) {
         if (pairs[p].ref < 0 || pairs[p].ref >= n_images || pairs[p].query < 0 || pairs[p].query >= n_images)
-            return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_geo_verify: pair %lld names an image outside [0, %d)", (long long)p, n_images);
+            return fail(ctx, MSFM_ERR_INVALID_ARG, "%s: pair %lld names an image outside [0, %d)", fn, (long long)p, n_images);
         used[pairs[p].ref] = used[pairs[p].query] = 1;
     }
     for (int32_t i = 0; i < n_images; ++i) {
         if (used[i] && (image_npts[i] < 0 || (image_npts[i] > 0 && !image_xy[i])))
-            return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_geo_verify: image %d has no keypoints", i);
+            return fail(ctx, MSFM_ERR_INVALID_ARG, "%s: image %d has no keypoints", fn, i);
         xy_off[i + 1] = xy_off[i] + (used[i] ? image_npts[i] : 0);
     }
     for (int64_t p = 0; p < n_pairs; ++p)
         for (int64_t k = offsets[p]; k < offsets[p + 1]; ++k)
             if (matches[k][0] < 0 || matches[k][0] >= image_npts[pairs[p].ref] || matches[k][1] < 0 || matches[k][1] >= image_npts[pairs[p].query])
-                return fail(ctx, MSFM_ERR_INVALID_ARG, "msfm_geo_verify: match %lld of pair %lld indexes past the keypoints", (long long)k, (long long)p);
+                return fail(ctx, MSFM_ERR_INVALID_ARG, "%s: match %lld of pair %lld indexes past the keypoints", fn, (long long)k, (long long)p);
     const int64_t n_xy = xy_off[n_images];
     std::vector<float> xy((size_t)std::max<int64_t>(n_xy, 1) * 2);
     for (int32_t i = 0; i < n_images; ++i)
@@ -1922,13 +1959,17 @@ static msfm_status geo_impl(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pai
     kp.iters = gp->iters > 0 ? gp->iters : 1024;
     kp.seed = gp->seed;
     kp.pair_base = gp->pair_index_base;
-    kp.stage_b = stage_b ? 1 : 0;
+    kp.stage_b = call == GeoCall::verify ? 1 : 0;
     kp.pair_ok = static_cast<int32_t *>(d.ok.ptr);
     kp.pair_inliers = static_cast<int32_t *>(d.inl.ptr);
     kp.keep = static_cast<uint8_t *>(d.keep.ptr);
     kp.F = static_cast<double *>(d.F.ptr);
     MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_k0, ctx->stream));
-    msfm::geo_verify_kernel<<<(int)std::min<int64_t>(n_pairs, 8 * ctx->num_sms), msfm::kGeoThreads, 0, ctx->stream>>>(kp, (int)n_pairs);
+    const int geo_grid = (int)std::min<int64_t>(n_pairs, 8 * ctx->num_sms);
+    if (call == GeoCall::homography)
+        msfm::geo_homography_kernel<<<geo_grid, msfm::kGeoThreads, 0, ctx->stream>>>(kp, (int)n_pairs);
+    else
+        msfm::geo_verify_kernel<<<geo_grid, msfm::kGeoThreads, 0, ctx->stream>>>(kp, (int)n_pairs);
     MSFM_CUDA(ctx, cudaGetLastError());
     MSFM_CUDA(ctx, cudaEventRecord(ctx->ev_k1, ctx->stream));
     MSFM_CUDA(ctx, cudaMemcpyAsync(pair_ok, d.ok.ptr, (size_t)n_pairs * 4, cudaMemcpyDeviceToHost, ctx->stream));

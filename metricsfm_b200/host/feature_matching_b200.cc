@@ -324,7 +324,16 @@ bool MatchGraphB200::MatchPairs(const std::vector<std::vector<int>> &match_graph
 bool MatchGraphB200::MatchPairsGuided(const std::vector<std::vector<int>> &match_graph_init, const std::vector<std::array<double, 9>> &F,
                                       const std::vector<std::vector<cv::KeyPoint>> &keypoints, float th_epipolar,
                                       std::vector<std::vector<PairMatches>> &out, float th_good, float th_all, bool mutual, int th_reject) {
-    const Guide g = {&F, &keypoints, th_epipolar};
+    const Guide g = {Guide::epipolar, &F, &keypoints, th_epipolar};
+    return Match(match_graph_init, &g, out, th_good, th_all, mutual, th_reject);
+}
+
+bool MatchGraphB200::MatchPairsGuidedHomography(const std::vector<std::vector<int>> &match_graph_init,
+                                                const std::vector<std::array<double, 9>> &H,
+                                                const std::vector<std::vector<cv::KeyPoint>> &keypoints, float th_transfer,
+                                                std::vector<std::vector<PairMatches>> &out, float th_good, float th_all, bool mutual,
+                                                int th_reject) {
+    const Guide g = {Guide::homography, &H, &keypoints, th_transfer};
     return Match(match_graph_init, &g, out, th_good, th_all, mutual, th_reject);
 }
 
@@ -364,8 +373,8 @@ bool MatchGraphB200::Match(const std::vector<std::vector<int>> &match_graph_init
     res.match_capacity = capacity;
     msfm_status st;
     if (guide) {
-        if (guide->F->size() != pairs.size()) {
-            err_ = "MatchPairsGuided needs one F per pair";
+        if (guide->M->size() != pairs.size()) {
+            err_ = guide->kind == Guide::homography ? "MatchPairsGuidedHomography needs one H per pair" : "MatchPairsGuided needs one F per pair";
             return false;
         }
         // keypoints as the library takes them: (x, y) per descriptor row, one array per image
@@ -382,8 +391,12 @@ bool MatchGraphB200::Match(const std::vector<std::vector<int>> &match_graph_init
             xy_ptr[i] = xy[i].data();
             npts[i] = (int32_t)kp.size();
         }
-        st = msfm_match_pairs_guided(ctx_, pairs.data(), (int64_t)pairs.size(), &prm, reinterpret_cast<const double(*)[9]>(guide->F->data()),
-                                     guide->th, xy_ptr.data(), npts.data(), (int32_t)n_images, &res);
+        const double(*M)[9] = reinterpret_cast<const double(*)[9]>(guide->M->data());
+        st = guide->kind == Guide::homography
+                 ? msfm_match_pairs_guided_homography(ctx_, pairs.data(), (int64_t)pairs.size(), &prm, M, guide->th, xy_ptr.data(),
+                                                      npts.data(), (int32_t)n_images, &res)
+                 : msfm_match_pairs_guided(ctx_, pairs.data(), (int64_t)pairs.size(), &prm, M, guide->th, xy_ptr.data(), npts.data(),
+                                           (int32_t)n_images, &res);
     } else {
         st = msfm_match_pairs(ctx_, pairs.data(), (int64_t)pairs.size(), &prm, &res);
     }

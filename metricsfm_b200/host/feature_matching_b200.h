@@ -182,10 +182,19 @@ public:
                           const std::vector<std::vector<cv::KeyPoint>> &keypoints, float th_epipolar,
                           std::vector<std::vector<PairMatches>> &out, float th_good = 0.6f, float th_all = 0.85f,
                           bool mutual = false, int th_reject = 20);
+    // Homography-guided re-matching (msfm_match_pairs_guided_homography, HOMOG-SPEC in msfm_match.h): MatchPairs with every
+    // row's two nearest neighbours searched only among the keypoints of idx1 that H carries to within th_transfer pixels
+    // of the row's keypoint.  H[k] belongs to the k-th pair of match_graph_init in order (row-major, p2 ~ H p1 for a
+    // keypoint p1 of idx1 and p2 of idx2: what msfm_geo_homography returns); keypoints as in MatchPairsGuided.
+    bool MatchPairsGuidedHomography(const std::vector<std::vector<int>> &match_graph_init, const std::vector<std::array<double, 9>> &H,
+                                    const std::vector<std::vector<cv::KeyPoint>> &keypoints, float th_transfer,
+                                    std::vector<std::vector<PairMatches>> &out, float th_good = 0.6f, float th_all = 0.85f,
+                                    bool mutual = false, int th_reject = 20);
 
 private:
-    struct Guide {  // the epipolar gate of MatchPairsGuided
-        const std::vector<std::array<double, 9>> *F;
+    struct Guide {  // the gate of MatchPairsGuided (epipolar, M = F) or MatchPairsGuidedHomography (homography, M = H)
+        enum Kind { epipolar, homography } kind;
+        const std::vector<std::array<double, 9>> *M;
         const std::vector<std::vector<cv::KeyPoint>> *keypoints;
         float th;
     };

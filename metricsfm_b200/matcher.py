@@ -340,20 +340,35 @@ class Matcher:
         keypoints}, one per descriptor row of every image the pairs touch.  rescore_band > 0 (float uploads on a
         keep_float context): rows whose gated quantised ratio lies within that relative band of a ratio threshold are
         decided on their exact fp32 top-2 among the allowed reference rows, as match_pairs does without a gate."""
+        prm = self._params(ratio, ratio_good, max_dist_sq, mutual, min_keypoints, orientation, rescore_band, flags)
+        return self._match_guided(self._L.msfm_match_pairs_guided, pairs, F, image_xy, th_epipolar, prm, ratio_good, capacity)
+
+    def _match_guided(self, fn, pairs, M, image_xy, th, prm, ratio_good, capacity) -> MatchResult:
         pa = self._pairs(pairs)
         n = pa.shape[0]
-        Fa = np.ascontiguousarray(F, np.float64).reshape(-1, 9)
+        Fa = np.ascontiguousarray(M, np.float64).reshape(-1, 9)
         if Fa.shape[0] != n:
-            raise ValueError(f"F must hold one 3x3 matrix per pair: {Fa.shape[0]} for {n} pairs")
+            raise ValueError(f"one 3x3 matrix per pair is needed: {Fa.shape[0]} for {n} pairs")
         n_images = int(pa.max()) + 1 if n else 0
         ptrs, npts, xy_keep = self._keypoint_table(image_xy, n_images)
         out, res = self._result_buffers(pa, ratio_good, capacity, None)
-        prm = self._params(ratio, ratio_good, max_dist_sq, mutual, min_keypoints, orientation, rescore_band, flags)
-        self._check(self._L.msfm_match_pairs_guided(self._h, pa.ctypes.data, n, C.byref(prm), Fa.ctypes.data, th_epipolar,
-                                                    C.cast(ptrs, C.c_void_p), npts.ctypes.data, n_images, C.byref(res)))
+        self._check(fn(self._h, pa.ctypes.data, n, C.byref(prm), Fa.ctypes.data, th, C.cast(ptrs, C.c_void_p), npts.ctypes.data,
+                       n_images, C.byref(res)))
         del xy_keep
         total = int(out.offsets[n])
         return MatchResult(out.offsets, out.ok, out.matches[:total], out.good[:total] if out.good is not None else None)
+
+    def match_pairs_guided_homography(self, pairs, H, image_xy: dict, *, th_transfer: float = 3.0, ratio: float = 0.6,
+                                      ratio_good: float = 0.0, max_dist_sq: float = 0.0, mutual: bool = False,
+                                      min_keypoints: int = 20, orientation: int = 0, flags: int = 0,
+                                      capacity: int | None = None) -> MatchResult:
+        """msfm_match_pairs_guided_homography (HOMOG-SPEC in include/msfm_match.h): match_pairs with every query row's 2-NN
+        searched only among the reference keypoints that H carries to within th_transfer pixels of the row's keypoint.
+        H: [n, 3, 3] float64 as geo_homography returns it (p_query ~ H p_ref); image_xy as in match_pairs_guided.  There
+        is no float regime under this gate."""
+        prm = self._params(ratio, ratio_good, max_dist_sq, mutual, min_keypoints, orientation, 0.0, flags)
+        return self._match_guided(self._L.msfm_match_pairs_guided_homography, pairs, H, image_xy, th_transfer, prm, ratio_good,
+                                  capacity)
 
     def match_pairs_resident(self, pairs, ratio: float = 0.6, *, ratio_good: float = 0.0, max_dist_sq: float = 0.0,
                              mutual: bool = False, min_keypoints: int = 20, orientation: int = 0) -> int:
@@ -373,11 +388,24 @@ class Matcher:
         `result.good` selects the participating matches and `keep` is the RANSAC consensus mask instead of the F-filter.
         pair_index_base: global index of the first pair in the RANSAC counter, so that a pair list verified in slices
         draws the same hypotheses as in one call."""
+        fn = self._L.msfm_geo_ransac if ransac_only else self._L.msfm_geo_verify
+        return self._geo_call(fn, pairs, result, image_xy, th_epipolar, min_points, min_inliers, iters, seed, pair_index_base)
+
+    def geo_homography(self, pairs, result: "MatchResult", image_xy: dict, *, th: float = 3.0, min_points: int = 30,
+                       min_inliers: int = 30, iters: int = 1024, seed: int = 0, pair_index_base: int = 0):
+        """msfm_geo_homography: batched RANSAC homography (p_query ~ H p_ref, cv::findHomography(RANSAC, th) without the
+        refinement) of the pairs of a match_pairs result (orientation 0); `result.good` selects the participating matches,
+        as geo_verify(ransac_only=True) does.  Returns (pair_ok [n] int32, pair_inliers [n] int32, inlier_mask [total]
+        uint8, H [n, 3, 3] float64, H22 = 1)."""
+        return self._geo_call(self._L.msfm_geo_homography, pairs, result, image_xy, th, min_points, min_inliers, iters, seed,
+                              pair_index_base)
+
+    def _geo_call(self, fn, pairs, result, image_xy, th, min_points, min_inliers, iters, seed, pair_index_base):
         pa = self._pairs(pairs)
         n = pa.shape[0]
         n_images = int(pa.max()) + 1 if n else 0
         ptrs, npts, xy_keep = self._keypoint_table(image_xy, n_images)
-        gp = _lib.GeoParams(th_epipolar, min_points, min_inliers, iters, seed, pair_index_base)
+        gp = _lib.GeoParams(th, min_points, min_inliers, iters, seed, pair_index_base)
         total = int(result.offsets[n])
         ok = np.zeros((max(n, 1),), np.int32)
         inl = np.zeros((max(n, 1),), np.int32)
@@ -386,7 +414,6 @@ class Matcher:
         offs = np.ascontiguousarray(result.offsets, np.int64)
         m = np.ascontiguousarray(result.matches, np.int32)
         g = np.ascontiguousarray(result.good if result.good is not None else np.ones((total,), np.uint8), np.uint8)
-        fn = self._L.msfm_geo_ransac if ransac_only else self._L.msfm_geo_verify
         self._check(fn(self._h, pa.ctypes.data, n, offs.ctypes.data, m.ctypes.data if total else None,
                                             g.ctypes.data if total else None, C.cast(ptrs, C.c_void_p), npts.ctypes.data, n_images,
                                             C.byref(gp), ok.ctypes.data, inl.ctypes.data, keep.ctypes.data, F.ctypes.data)
