@@ -480,17 +480,22 @@ match_pairs_kernel(const MatchKernelParams p) {
         const int strip = warp >> 2;
         const int quarter = warp & 3;
         const int row_local = strip * kStripRows + quarter * 32 + lane;
-        const uint32_t warp_taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + strip * TILE_N;
+        const uint32_t warp_taddr = ptx::opaque(tmem_base + ((uint32_t)(quarter * 32) << 16) + strip * TILE_N);
         constexpr int kAbsent = -0x08000000;  // scores below this are pad columns / "no neighbour"
         // everything the tile loop touches in shared memory, as 32-bit shared addresses
-        const uint32_t key_base = ptx::smem_u32(sKey);
-        const uint32_t tmin_base = ptx::smem_u32(sTmin);
-        const uint32_t t_full_base = ptx::smem_u32(t_full + strip);
-        const uint32_t t_empty_base = ptx::smem_u32(t_empty + strip);
-        // ring positions are carried incrementally (no divisions in the tile loop)
-        // ring positions all derive from ONE running tile counter g (TBUFS and kKeySlots are powers of two)
+        // (made opaque: otherwise they are re-derived from the shared-window base and the warp index in every tile)
+        const uint32_t key_base = ptx::opaque(ptx::smem_u32(sKey));
+        const uint32_t tmin_base = ptx::opaque(ptx::smem_u32(sTmin));
+        const uint32_t t_full_base = ptx::opaque(ptx::smem_u32(t_full + strip));
+        const uint32_t t_empty_base = ptx::opaque(ptx::smem_u32(t_empty + strip));
+        const uint32_t lane_pinned = ptx::opaque((uint32_t)lane);  // (not re-read from %tid per tile)
+        // Ring positions of the CTA's running tile sequence, carried from tile to tile: the accumulator buffer, its
+        // barrier phase and the key slot, as byte offsets (a few ALU operations per tile instead of re-deriving every
+        // address from a tile counter and the shared-memory window base).
         static_assert((TBUFS & (TBUFS - 1)) == 0 && (Cfg::kKeySlots & (Cfg::kKeySlots - 1)) == 0, "ring sizes must be powers of two");
-        uint32_t g = 0;
+        uint32_t buf = 0, t_phase = 0;  // accumulator buffer of the next tile and the parity of its full barrier
+        uint32_t koff = 0;              // key slot of the next tile, in bytes of the key ring (TILE_N * 4 per slot)
+        constexpr uint32_t kKeyRingBytes = Cfg::kKeySlots * TILE_N * 4, kKeyToTmin = TILE_N * 4 / 16;
         for (int item = blockIdx.x; item < p.n_items; item += gridDim.x) {
             const WorkItem wi = p.items[item];
             const PairDesc pd = p.pairs[wi.pair];
@@ -550,8 +555,6 @@ match_pairs_kernel(const MatchKernelParams p) {
                 long long c0 = 0, c1 = 0, c2 = 0, c3 = 0;
                 const bool prof = DEBUG && (p.debug_flags & 8u) && p.stats != nullptr;
                 if (prof) c0 = clock64();
-                const uint32_t buf = g % TBUFS, t_phase = (g / TBUFS) & 1;
-                const uint32_t ks = g % Cfg::kKeySlots;
                 ptx::mbar_wait_a(t_full_base + buf * (STRIPS * 8), t_phase);
                 ptx::tc_fence_after();
                 if (prof) c1 = clock64();
@@ -561,13 +564,13 @@ match_pairs_kernel(const MatchKernelParams p) {
                 for (int c = 0; c < TILE_N / 16; ++c) ptx::tmem_ld_32x32b_x16(tile_taddr + c * 16, acc[c]);
                 // ---- while the loads fly: column keys of the tile, smallest reference norm, pruning threshold
                 // (the tile's keys and minimum norm landed before its MMAs were issued: they share the B stage's barrier)
-                const uint32_t ck = key_base + ks * (TILE_N * 4);
-                const int nbmin = ptx::lds_s32(tmin_base + ks * 16);  // smallest reference norm of the tile (tile_min_kernel)
+                const uint32_t ck = key_base + koff;
+                const int nbmin = ptx::lds_s32(tmin_base + koff / kKeyToTmin);  // smallest reference norm of the tile (tile_min_kernel)
                 const int T = (theta + nbmin) >> 1;  // dead rows are pruned against their best score, the others against their second best
                 ptx::tmem_ld_wait();
                 ptx::tc_fence_before();
                 __syncwarp();
-                if (lane == 0) ptx::mbar_arrive_a(t_empty_base + buf * (STRIPS * 8));
+                if (lane_pinned == 0) ptx::mbar_arrive_a(t_empty_base + buf * (STRIPS * 8));
                 if (prof) c2 = clock64();
                 if (DEBUG && (p.debug_flags & 6u)) {  // experiments: 2/4 = TMEM loads + hand-back only
                     if (acc[0][0] == 0x7fffffffu) S1 = 0;
@@ -656,7 +659,9 @@ match_pairs_kernel(const MatchKernelParams p) {
                     acc_p1 += c3 - c2;    // phase 1
                     acc_p2 += c4 - c3;    // phase 2
                 }
-                ++g;
+                koff = (koff + TILE_N * 4) & (kKeyRingBytes - 1);
+                buf = (buf + 1) & (TBUFS - 1);
+                t_phase ^= (buf == 0);
             }
             if (DEBUG && (p.debug_flags & 8u) && p.stats != nullptr && lane == 0) {
                 atomicAdd(p.stats + 0, (unsigned long long)acc_hot);

@@ -9,6 +9,13 @@ namespace ptx {
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
+// The value, as something the compiler cannot re-derive: a loop-invariant address computed once before a loop stays in
+// a register instead of being rematerialised (shared-window base, warp-index arithmetic) in every iteration.
+__device__ __forceinline__ uint32_t opaque(uint32_t x) {
+    asm volatile("mov.b32 %0, %0;" : "+r"(x));
+    return x;
+}
+
 __device__ __forceinline__ uint32_t lane_id() {
     uint32_t l;
     asm volatile("mov.u32 %0, %%laneid;" : "=r"(l));
