@@ -73,7 +73,16 @@
  *   GUIDED-SPEC's integer rule unchanged: nn0 / nn1 are the two closest allowed reference rows (lowest index on ties), a
  *   row with fewer than two allowed rows gets id -1 / +inf and is rejected, ratio, ratio_good, max_dist_sq,
  *   MSFM_RATIO_REJECT_GT, orientation and min_keypoints as in MATCH-SPEC, and the mutual check keeps (q, nn0) iff q is
- *   the closest allowed query row of nn0.  There is no float regime under this gate (rescore_band must be 0).
+ *   the closest allowed query row of nn0.
+ *   Float regime under the gate (rescore_band > 0 on a keep_float context, pairs whose images both keep float rows at
+ *   one scale; every other pair follows the integer rule above): GUIDED-SPEC's float regime with this test in place of
+ *   the epipolar one.  A query row is a band row when both of its gated quantised neighbours exist and fl(d0/d1) lies
+ *   within ratio*(1 +- band) or ratio_good*(1 +- band).  A band row is decided on its exact fp32 top-2 (b0, b1) among
+ *   the reference rows H allows, with the arithmetic of the float regime: squared L2 accumulated in index order with
+ *   separate multiply and add, lowest index on ties; the ratio tests on fl(b0/b1), max_dist_sq on fl(b0*fl(s*s)), the
+ *   match on the fp32 nearest allowed row.  Every other row keeps the integer H-guided decision; the allowed set is the
+ *   same in both arithmetics, so a row with fewer than two allowed rows is never a band row and stays rejected.  With
+ *   mutual = 1 the check is the float regime's heuristic filter of the one-way list, under the gate (not exact in fp32).
  *   Caution: at th of a few pixels the disc around pi(H p_j) seldom holds two reference keypoints at ordinary keypoint
  *   densities, and a row with fewer than two allowed rows is rejected.  The gate then keeps only rows that have a second
  *   keypoint inside the disc (e.g. a second orientation at the same location), and can keep far fewer true matches than
@@ -367,7 +376,7 @@ msfm_status msfm_match_pairs_guided(msfm_ctx *ctx, const msfm_pair *pairs, int64
 /* msfm_match_pairs with each query row's 2-NN searched only among the reference rows that H[p] carries to within
  * th_transfer pixels of the row's keypoint (HOMOG-SPEC above; typically msfm_geo_homography's H of the pairs with
  * pair_ok).  Arguments, results, timing and errors as msfm_match_pairs_guided with H in place of F and th_transfer in
- * place of th_epipolar, and every rescore_band > 0 is refused with INVALID_ARG. */
+ * place of th_epipolar.  rescore_band > 0 on a keep_float context: the float regime under the gate (HOMOG-SPEC). */
 msfm_status msfm_match_pairs_guided_homography(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pairs,
                                                const msfm_params *params, const double (*H)[9], float th_transfer,
                                                const float *const *image_xy, const int32_t *image_npts, int32_t n_images,
@@ -376,11 +385,12 @@ msfm_status msfm_match_pairs_guided_homography(msfm_ctx *ctx, const msfm_pair *p
 /* ---- GPU-side cross-check kernel (CUDA cores, dp4a); used by the tests to localise faults, never by the fast path */
 msfm_status msfm_knn2_crosscheck(msfm_ctx *ctx, int32_t ref_id, int32_t query_id, int32_t *ids, float *dists);
 /* Test hook: capacity of the float regime's event list (-1 = default sizing; 0 forces the brute-force fallback).
- * Applies to the rescore_band of msfm_match_pairs and msfm_match_pairs_guided and to msfm_knn2_pairs'
- * MSFM_KNN_EXACT_F32 alike. */
+ * Applies to the rescore_band of msfm_match_pairs, msfm_match_pairs_guided and msfm_match_pairs_guided_homography and
+ * to msfm_knn2_pairs' MSFM_KNN_EXACT_F32 alike. */
 msfm_status msfm_test_set_band_event_cap(msfm_ctx *ctx, int64_t cap);
 /* Test hook: for the last MSFM_KNN_EXACT_F32 call of msfm_knn2_pairs or the last msfm_match_pairs /
- * msfm_match_pairs_guided call with rescore_band > 0 on a keep_float context, whichever came later, the events the
+ * msfm_match_pairs_guided / msfm_match_pairs_guided_homography call with rescore_band > 0 on a keep_float context,
+ * whichever came later, the events the
  * collect path scored (in a guided call: only elements the gate allows) and the batches
  * whose event list overflowed, i.e. that the brute force decided.  Either pointer may be NULL. */
 msfm_status msfm_test_last_knn_stats(msfm_ctx *ctx, int64_t *events, int32_t *brute_force_batches);

@@ -378,18 +378,21 @@ __global__ void __launch_bounds__(256) finish_band_kernel(const BandParams bp) {
     }
 }
 
-// GUIDED: a reference row enters a band row's top-2 only if the epipolar gate allows the element, evaluated like the
-// matching kernel does (bit for bit: the allowed set is the one the row's threshold came from).  The gate is a separate
-// argument because a longer BandParams would move the parameters after it in every kernel that takes one; the other
-// stages of the collect path see gated rows only.
-template <bool GUIDED>
+// GATE: a reference row enters a band row's top-2 only if the epipolar or homography gate allows the element, evaluated
+// like the matching kernel does (bit for bit: the allowed set is the one the row's threshold came from).  Under the
+// homography gate a band row keeps its query keypoint and each reference column is transferred (hom_transfer,
+// hom_allowed).  The gate is a separate argument because a longer BandParams would move the parameters after it in
+// every kernel that takes one; the other stages of the collect path see gated rows only.
+template <GateKind GATE>
 __global__ void __launch_bounds__(256) rescore_band_kernel(const BandParams bp, int n_pairs, const EpiGate gate) {
+    constexpr bool GUIDED = GATE != GateKind::none, HOMOG = GATE == GateKind::homography;
     __shared__ float sq[kRescoreRows][kDim];                  // band rows, float
     __shared__ __align__(16) uint32_t sq8[kRescoreRows][kDim / 4];  // the same rows, packed u8
     __shared__ int s_na[kRescoreRows], s_thr[kRescoreRows];
     __shared__ float red_d[8][kRescoreRows][2];
     __shared__ int red_i[8][kRescoreRows][2];
-    __shared__ EpiLine s_line[GUIDED ? kRescoreRows : 1];    // GUIDED: the band rows' query lines
+    __shared__ EpiLine s_line[GUIDED && !HOMOG ? kRescoreRows : 1];  // epipolar gate: the band rows' query lines
+    __shared__ float2 s_kq[HOMOG ? kRescoreRows : 1];                 // homography gate: the band rows' keypoints
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     if (bp.event_count && *bp.event_count <= bp.event_cap) return;  // the collect path has every event: nothing to do
     for (int p = blockIdx.x; p < n_pairs; p += gridDim.x) {
@@ -418,7 +421,8 @@ __global__ void __launch_bounds__(256) rescore_band_kernel(const BandParams bp, 
                     na = ckey_to_norm(bp.ckeys[pd.qry_off + q]);
                     // Prefilter on the quantised distance: the threshold the collect pass used (exact_threshold)
                     thr = bp.band_thr[pd.knn_off + c0 + qi];
-                    if (GUIDED) s_line[qi] = epi_query_line(gate.fmat + 9 * p, gate.xy[pd.qry_off + q]);
+                    if (HOMOG) s_kq[qi] = gate.xy[pd.qry_off + q];
+                    else if (GUIDED) s_line[qi] = epi_query_line(gate.fmat + 9 * p, gate.xy[pd.qry_off + q]);
                 }
                 s_na[qi] = na;
                 s_thr[qi] = thr;
@@ -446,9 +450,12 @@ __global__ void __launch_bounds__(256) rescore_band_kernel(const BandParams bp, 
                     }
                 }
                 const int nb = ckey_to_norm(refk[j]);
-                float2 kj{};      // GUIDED: reference row j's keypoint ...
+                float2 kj{};      // epipolar gate: reference row j's keypoint ...
                 float nbj = 0.f;  // ... and |b|^2
-                if (GUIDED) {
+                HomPoint hj{};    // homography gate: its transferred keypoint
+                if (HOMOG) {
+                    hj = hom_transfer(gate.fmat + 9 * p, gate.xy[pd.ref_off + j]);
+                } else if (GUIDED) {
                     kj = gate.xy[pd.ref_off + j];
                     nbj = epi_ref_line(gate.fmat + 9 * p, kj).n;
                 }
@@ -456,7 +463,7 @@ __global__ void __launch_bounds__(256) rescore_band_kernel(const BandParams bp, 
                 for (int qi = 0; qi < kRescoreRows; ++qi) {
                     const int dint = s_na[qi] + nb - 2 * (int)ab[qi];
                     if (dint <= s_thr[qi] &&
-                        (!GUIDED || epi_allowed(s_line[qi], kj, nbj, gate.t2))) {
+                        (!GUIDED || (HOMOG ? hom_allowed(hj, s_kq[qi], gate.t2) : epi_allowed(s_line[qi], kj, nbj, gate.t2)))) {
                         // rare: exact fp32 distance, accumulated in index order without contraction
                         float acc = 0.0f;
                         const float *rf = ref + (int64_t)j * kDim;

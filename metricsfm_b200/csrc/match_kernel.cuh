@@ -110,7 +110,7 @@ struct MatchKernelParams {
     // event list.  F (or H) is row p of fmat for a forward item of pair p and for every item with cand_idx = p.  A forward
     // row and a band row (a collect item's row) are query keypoints, so the epipolar gate takes their query line; a twin
     // row is a reference keypoint, and the gate takes the query line of each column instead.  The homography gate
-    // transfers the reference keypoint of each element: per column on a forward row, once per row on a twin row.
+    // transfers the reference keypoint of each element: per column on a forward or band row, once per row on a twin row.
     const float2 *xy;             // keypoints (x, y), indexed like the column-key arena
     const float *fmat;            // [forward pairs of the batch][9] F (epipolar gate) or H (homography gate) rounded to
                                   // fp32, row-major
@@ -251,8 +251,8 @@ __device__ __forceinline__ bool epi_allowed(const EpiLine &a, float2 kj, float n
 // Homography gate of HOMOG-SPEC (include/msfm_match.h).  The reference keypoint kj is transferred once,
 // (U, V, W) = H (xj, yj, 1); element (q, j) is allowed iff |(U, V) - (xq, yq) W|^2 <= t2 W^2, the squared transfer
 // distance |p_q - pi(H p_j)|^2 <= th^2 without the division (independent of the sign of H; W = 0 bars the element unless
-// U = V = 0).  One fp32 rounding per operation, no contraction; every site of the matching kernel goes through
-// hom_transfer and hom_allowed.
+// U = V = 0).  One fp32 rounding per operation, no contraction; every site (the matching kernel's rows and columns in
+// every pass, the brute force rescore_band_kernel) goes through hom_transfer and hom_allowed.
 struct HomPoint {
     float U, V, W;
 };
@@ -285,7 +285,6 @@ __global__ void __launch_bounds__(MatchKernelCfg<STRIPS, TILE_N, STAGES, TBUFS>:
 match_pairs_kernel(const MatchKernelParams p) {
     using Cfg = MatchKernelCfg<STRIPS, TILE_N, STAGES, TBUFS>;
     constexpr bool GATED = GATE != GateKind::none, HOMOG = GATE == GateKind::homography;
-    static_assert(!(COLLECT && HOMOG), "the float regime has no homography gate");
     // No static shared memory is declared, so the dynamic window starts at shared offset 0 (1024-byte aligned, as
     // the 128B-swizzled operand tiles require); checked once below.
     extern __shared__ __align__(1024) uint8_t smem[];
@@ -527,7 +526,8 @@ match_pairs_kernel(const MatchKernelParams p) {
             // query line.  A band row takes its query row's keypoint and F, so it gets that row's line bit for bit, and
             // its allowed set is the one its gated quantised 2-NN, and hence its threshold T(q), came from.  A twin row is
             // a reference keypoint kr: its reference line, of which the test needs |b|^2 only.
-            // Homography gate: a forward row keeps its query keypoint kr, a twin row its transferred keypoint ht.
+            // Homography gate: a forward row keeps its query keypoint kr, a band row its query row's keypoint (and with
+            // that row's H, that row's allowed set bit for bit), a twin row its transferred keypoint ht.
             const bool query_row = COLLECT || pd.cand_idx < 0;
             EpiLine line{};
             float2 kr{};
@@ -535,7 +535,8 @@ match_pairs_kernel(const MatchKernelParams p) {
             const float *fm = nullptr;
             if (HOMOG) {
                 fm = p.fmat + 9 * (pd.cand_idx >= 0 ? pd.cand_idx : wi.pair);
-                if (valid && query_row) kr = p.xy[pd.qry_off + q];
+                if (valid && query_row)
+                    kr = p.xy[(!COLLECT || pd.cand_idx < 0) ? pd.qry_off + q : p.pairs[pd.cand_idx].qry_off + p.src_row[pd.qry_off + q]];
                 else if (valid) ht = hom_transfer(fm, p.xy[p.pairs[pd.cand_idx].ref_off + p.src_row[pd.qry_off + q]]);
             } else if (GATED) {
                 fm = p.fmat + 9 * (pd.cand_idx >= 0 ? pd.cand_idx : wi.pair);

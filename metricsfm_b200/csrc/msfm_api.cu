@@ -41,16 +41,14 @@ using KCfg = msfm::MatchKernelCfg<kStrips, kTileN, kStages, kTbufs>;
 constexpr int kItemRows = kStrips * msfm::kStripRows;
 
 // The instantiations of the matching kernel, (DEBUG, COLLECT, GATE): every combination but a debug build of the
-// collect pass, for which `debug` is ignored, and a collect pass under the homography gate (the float regime has none:
-// null).
+// collect pass, for which `debug` is ignored.
 using MatchKernelFn = void (*)(msfm::MatchKernelParams);
 using msfm::GateKind;
 template <bool DEBUG, bool COLLECT>
 MatchKernelFn match_kernel(GateKind gate) {
     if (gate == GateKind::none) return msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, DEBUG, COLLECT, GateKind::none>;
     if (gate == GateKind::epipolar) return msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, DEBUG, COLLECT, GateKind::epipolar>;
-    if constexpr (!COLLECT) return msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, DEBUG, COLLECT, GateKind::homography>;
-    return nullptr;
+    return msfm::match_pairs_kernel<kStrips, kTileN, kStages, kTbufs, DEBUG, COLLECT, GateKind::homography>;
 }
 MatchKernelFn match_kernel(bool debug, bool collect, GateKind gate) {
     return collect ? match_kernel<false, true>(gate) : debug ? match_kernel<true, false>(gate) : match_kernel<false, false>(gate);
@@ -679,11 +677,16 @@ msfm_status run_collect_pass(msfm_ctx *ctx, const BatchPlan &plan, const msfm::B
     msfm::finish_band_kernel<<<nb, 256, 0, ctx->stream>>>(bp);
     const int gx = std::min(nb, 4 * ctx->num_sms);
     const int gy = std::max(1, std::min(32, (4 * ctx->num_sms + gx - 1) / gx));
-    // a guided batch: the brute force applies the gate as the collect pass does
-    if (const msfm::EpiGate *gate = plan.epi_gate())
-        msfm::rescore_band_kernel<true><<<dim3(gx, gy), 256, 0, ctx->stream>>>(bp, nb, *gate);
+    // a guided batch: the brute force applies the plan's gate as the collect pass does
+    const msfm::EpiGate *gate = plan.epi_gate();
+    const GateKind kind = gate ? plan.gate_kind : GateKind::none;
+    const msfm::EpiGate g = gate ? *gate : msfm::EpiGate{nullptr, nullptr, 0.0f};
+    if (kind == GateKind::homography)
+        msfm::rescore_band_kernel<GateKind::homography><<<dim3(gx, gy), 256, 0, ctx->stream>>>(bp, nb, g);
+    else if (kind == GateKind::epipolar)
+        msfm::rescore_band_kernel<GateKind::epipolar><<<dim3(gx, gy), 256, 0, ctx->stream>>>(bp, nb, g);
     else
-        msfm::rescore_band_kernel<false><<<dim3(gx, gy), 256, 0, ctx->stream>>>(bp, nb, msfm::EpiGate{nullptr, nullptr, 0.0f});
+        msfm::rescore_band_kernel<GateKind::none><<<dim3(gx, gy), 256, 0, ctx->stream>>>(bp, nb, g);
     MSFM_CUDA(ctx, cudaGetLastError());
     ctx->timing.total_launches += 4;
     return MSFM_OK;
@@ -751,8 +754,6 @@ msfm_status check_guided(msfm_ctx *ctx, const msfm_pair *pairs, int64_t n_pairs,
     const char *mat = homog ? "H" : "F";
     if (!std::isfinite(params->rescore_band) || params->rescore_band < 0.0f)
         return fail(ctx, MSFM_ERR_INVALID_ARG, "%s: rescore_band %g must be finite and >= 0", fn, (double)params->rescore_band);
-    if (homog && params->rescore_band > 0.0f)
-        return fail(ctx, MSFM_ERR_INVALID_ARG, "%s: rescore_band > 0 is not supported under the homography gate", fn);
     if (params->rescore_band > 0.0f && !ctx->fdesc)
         return fail(ctx, MSFM_ERR_INVALID_ARG, "%s: rescore_band > 0 needs a keep_float context (retained float rows)", fn);
     if (!std::isfinite(g.th) || !(g.th > 0.0f))
@@ -1295,8 +1296,7 @@ msfm_status msfm_create(const msfm_config *cfg, msfm_ctx **out) {
     for (const bool debug : {false, true})
         for (const bool collect : {false, true})
             for (const GateKind gate : {GateKind::none, GateKind::epipolar, GateKind::homography})
-                if (!(collect && gate == GateKind::homography) &&
-                    cudaFuncSetAttribute(match_kernel(debug, collect, gate), cudaFuncAttributeMaxDynamicSharedMemorySize, KCfg::kSmemAlloc) != cudaSuccess)
+                if (cudaFuncSetAttribute(match_kernel(debug, collect, gate), cudaFuncAttributeMaxDynamicSharedMemorySize, KCfg::kSmemAlloc) != cudaSuccess)
                     return bail(MSFM_ERR_CUDA);
     if (cudaFuncSetAttribute(msfm::select_candidates_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msfm::kSelectSmemBytes) != cudaSuccess)
         return bail(MSFM_ERR_CUDA);

@@ -247,7 +247,8 @@ class Matcher:
 
     def _test_last_knn_stats(self):
         """(events scored by the collect path, batches decided by the brute force) of the last exact knn2_pairs call or
-        re-scoring match_pairs / match_pairs_guided call (rescore_band > 0 on a keep_float context)."""
+        re-scoring match_pairs / match_pairs_guided / match_pairs_guided_homography call (rescore_band > 0 on a
+        keep_float context)."""
         ev, bf = C.c_int64(), C.c_int32()
         self._check(self._L.msfm_test_last_knn_stats(self._h, C.byref(ev), C.byref(bf)))
         return ev.value, bf.value
@@ -361,12 +362,14 @@ class Matcher:
     def match_pairs_guided_homography(self, pairs, H, image_xy: dict, *, th_transfer: float = 3.0, ratio: float = 0.6,
                                       ratio_good: float = 0.0, max_dist_sq: float = 0.0, mutual: bool = False,
                                       min_keypoints: int = 20, orientation: int = 0, flags: int = 0,
-                                      capacity: int | None = None) -> MatchResult:
+                                      rescore_band: float = 0.0, capacity: int | None = None) -> MatchResult:
         """msfm_match_pairs_guided_homography (HOMOG-SPEC in include/msfm_match.h): match_pairs with every query row's 2-NN
         searched only among the reference keypoints that H carries to within th_transfer pixels of the row's keypoint.
-        H: [n, 3, 3] float64 as geo_homography returns it (p_query ~ H p_ref); image_xy as in match_pairs_guided.  There
-        is no float regime under this gate."""
-        prm = self._params(ratio, ratio_good, max_dist_sq, mutual, min_keypoints, orientation, 0.0, flags)
+        H: [n, 3, 3] float64 as geo_homography returns it (p_query ~ H p_ref); image_xy as in match_pairs_guided.
+        rescore_band > 0 (float uploads on a keep_float context): rows whose gated quantised ratio lies within that
+        relative band of a ratio threshold are decided on their exact fp32 top-2 among the reference rows H allows, as
+        match_pairs_guided does under F."""
+        prm = self._params(ratio, ratio_good, max_dist_sq, mutual, min_keypoints, orientation, rescore_band, flags)
         return self._match_guided(self._L.msfm_match_pairs_guided_homography, pairs, H, image_xy, th_transfer, prm, ratio_good,
                                   capacity)
 

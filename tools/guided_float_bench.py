@@ -58,14 +58,16 @@ def card_info():
                 max_sm_clock=parts[2] if len(parts) > 2 else None)
 
 
-def fp32_guided_rows(s):
-    """Per query row of an fp32 guided matcher: (kept, reference row, good).  The fp32 top-2 among the allowed rows is
-    found exactly in index order among the allowed rows whose float64 distance is within a relative 2^-14 of the
-    float64 second distance (the fp32 sum is within 130 * 2^-24 of it), so only a few rows per query are summed in fp32."""
+def fp32_guided_rows(s, allowed=None):
+    """Per query row of an fp32 guided matcher: (kept, reference row, good); `allowed` defaults to the epipolar gate.
+    The fp32 top-2 among the allowed rows is found exactly in index order among the allowed rows whose float64 distance
+    is within a relative 2^-14 of the float64 second distance (the fp32 sum is within 130 * 2^-24 of it), so only a few
+    rows per query are summed in fp32."""
     from oracle import guided_float_oracle as gfo
     from oracle import guided_oracle as gdo
     ref, qry = s["ref"].astype(np.float64), s["qry"].astype(np.float64)
-    allowed = gdo.gate_f32(s["F"], s["xy_ref"], s["xy_qry"], TH)
+    if allowed is None:
+        allowed = gdo.gate_f32(s["F"], s["xy_ref"], s["xy_qry"], TH)
     D = (qry * qry).sum(1)[:, None] + (ref * ref).sum(1)[None, :] - 2.0 * (qry @ ref.T)
     D[~allowed] = np.inf
     n = len(qry)
